@@ -263,6 +263,11 @@ int vag_last_total_alias(vag_context* ctx);
  * rounding).  mode 0 (default): chosen per request by cost; 1: never; 2: whenever the request has <= 8 frequencies. */
 int vag_set_series_mode(vag_context* ctx, int mode);
 
+/* Lanes that cooperate on one model's grid (K0): 0 (default) chooses by batch size -- the widest group whose launch
+ * still fits into one wave on the device; 4, 8, 16 or 32 forces that width for every batch.  The grid
+ * is the same bit for bit at every width; forcing one is for tests and A/B timing. */
+int vag_set_grid_lanes(vag_context* ctx, int lanes);
+
 /* per-stage device time of the most recent batched call on this context, milliseconds:
  * [0]=grid (K0) [1]=dynamics (K1) [2]=radiation (K2) [3]=EATS flux (K3) [4]=likelihood (K4)
  * Only filled when vag_set_profiling(ctx, 1) was called (adds event records + one sync). */

@@ -55,6 +55,7 @@ def load():
     lib.vag_debug_set_ode_limits.argtypes = [vp, C.c_int, C.c_int]
     lib.vag_last_total_alias.argtypes = [vp]
     lib.vag_set_series_mode.argtypes = [vp, C.c_int]
+    lib.vag_set_grid_lanes.argtypes = [vp, C.c_int]
     lib.vag_last_work.argtypes = [vp, C.POINTER(C.c_double)]
     lib.vag_details.argtypes = [vp, vp, C.c_double, C.c_double, vp, dp, dp, ip, dp, dp, dp, ip]
     lib.vag_details_photons.argtypes = [vp, vp, C.c_double, C.c_double, dp, dp]
@@ -68,6 +69,7 @@ EXPORTS = [
     "vag_flux_density_grid", "vag_flux_density_series", "vag_flux_band", "vag_chi2_series", "vag_flux_density_grid_dev",
     "vag_flux_density_series_dev", "vag_chi2_series_dev", "vag_synchronize", "vag_set_capacity", "vag_details", "vag_details_photons",
     "vag_set_profiling", "vag_set_output_mode", "vag_last_stage_ms", "vag_last_launch_count", "vag_measure_fp64_peak", "vag_selftest_libm", "vag_chi2", "vag_params_validate_batch", "vag_debug_set_ode_limits", "vag_last_total_alias", "vag_last_work", "vag_set_series_mode", "vag_details_ic",
+    "vag_set_grid_lanes",
 ]
 
 

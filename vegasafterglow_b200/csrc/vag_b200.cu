@@ -2,7 +2,7 @@
 // VegasAfterglow model-evaluation path.  Kernel bodies live in vag_pipeline.cuh / vag_observer.cuh.
 //
 // Launch geometry (B200: 148 SMs, FP64 path, no tensor cores -- nothing here is a contraction):
-//   k_grid<G>        : G = 8 / 16 / 32 lanes per model (32 / G models share a warp's scalar instruction stream)
+//   k_grid<G>        : G = 4 / 8 / 16 / 32 lanes per model (32 / G models share a warp's scalar instruction stream)
 //   k_dynamics<PAIR> : one thread per unique ODE row, 8 rows per warp for small batches; forward-only rows on a
 //                      register-resident dopri5, pair rows with the stage vectors in shared memory
 //   k_radiation      : one 64-thread CTA per unique row: finishes the shock tables from the raw node states,
@@ -614,6 +614,7 @@ struct vag_context {
     long long* h_cells = nullptr;   // pinned
     int* h_bands = nullptr;         // pinned: distinct frequencies of the series request in flight
     int series_mode = 0;            // vag_set_series_mode: 0 auto, 1 per-point spectra always, 2 banded whenever possible
+    int grid_lanes = 0;             // vag_set_grid_lanes: 0 by batch size, else k_grid<grid_lanes> for every batch
     int cap_theta = 384, cap_phi = 128;            // capacities of the batch in flight (host calls derive them per batch)
     int dbg_max_ode_steps = 0, dbg_max_ode_fails = 0;
     int user_cap_theta = 384, user_cap_phi = 128;  // vag_set_capacity: what the *_dev entry points run with
@@ -763,18 +764,36 @@ void mark(vag_context* ctx, int i, cudaStream_t s) {
     if (ctx->profiling) cudaEventRecord(ctx->ev[i], s);
 }
 
+template <int G>
+void launch_grid(const BatchWs& w, size_t n, const double* d_t, size_t n_t, cudaStream_t s) {
+    k_grid<G><<<(unsigned)((n * G + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
+}
+
+// Lanes per model of k_grid: the widest group whose launch fits into one wave of resident CTAs (GRID_MIN_BLOCKS CTAs of
+// 128 threads per SM).  Narrower groups only pay once a wider launch would need a second wave: the models of one warp
+// still diverge outside the quadrature rounds (GroupPar::lockstep), and with fewer than 6 lanes the six stage
+// evaluations of an attempt take two passes.  k_grid stage per batch on the bench draw (B200, 1000 W;
+// G = 4 / 8 / 16 / 32, ms): 16384 models 0.74 / 0.82 / 1.21 / 1.95, 4096: 0.50 / 0.36 / 0.36 / 0.52,
+// 1024: 0.45 / 0.31 / 0.28 / 0.26 (G = 2 was never the fastest: 1.23 ms at 16384 before the lockstep rounds).
+int grid_lanes_for(size_t n, int sm_count) {
+    const size_t resident_lanes = (size_t)sm_count * GRID_MIN_BLOCKS * 128;
+    int g = 32;
+    while (g > 4 && n * g > resident_lanes) g >>= 1;
+    return g;
+}
+
 // grid + dynamics + radiation for a batch; fills w and the totals
 int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, const double* d_t, size_t n_t,
               cudaStream_t s, int* totals_out, long long* cells_out) {
     int rc = setup_models(ctx, w, d_params, n);
     if (rc) return rc;
     mark(ctx, 0, s);
-    if (n >= 8192)
-        k_grid<8><<<(unsigned)((n * 8 + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
-    else if (n >= 1024)
-        k_grid<16><<<(unsigned)((n * 16 + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
-    else
-        k_grid<32><<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
+    switch (ctx->grid_lanes ? ctx->grid_lanes : grid_lanes_for(n, ctx->sm_count)) {
+        case 4: launch_grid<4>(w, n, d_t, n_t, s); break;
+        case 8: launch_grid<8>(w, n, d_t, n_t, s); break;
+        case 16: launch_grid<16>(w, n, d_t, n_t, s); break;
+        default: launch_grid<32>(w, n, d_t, n_t, s); break;
+    }
     k_scan<<<1, 1024, 0, s>>>(w);
     ctx->launches += 2;
     CK(cudaMemcpyAsync(ctx->h_totals, w.totals, sizeof(int) * TOT_N, cudaMemcpyDeviceToHost, s));
@@ -1150,6 +1169,7 @@ int vag_create(int device, vag_context** out) {
     }
     // k_grid spills its scratch to local memory: prefer L1.  k_dynamics keeps its dopri5 stage vectors
     // in shared memory (23 KB per 32-row CTA): give it the full carve-out so several CTAs share an SM.
+    cudaFuncSetCacheConfig(k_grid<4>, cudaFuncCachePreferL1);
     cudaFuncSetCacheConfig(k_grid<8>, cudaFuncCachePreferL1);
     cudaFuncSetCacheConfig(k_grid<16>, cudaFuncCachePreferL1);
     cudaFuncSetCacheConfig(k_grid<32>, cudaFuncCachePreferL1);
@@ -1222,6 +1242,12 @@ int vag_last_total_alias(vag_context* ctx) { return ctx ? ctx->total_alias : -1;
 int vag_set_series_mode(vag_context* ctx, int mode) {
     if (mode < 0 || mode > 2) return fail(VAG_ERR_INVALID, "unknown series mode");
     ctx->series_mode = mode;
+    return VAG_OK;
+}
+int vag_set_grid_lanes(vag_context* ctx, int lanes) {
+    if (lanes != 0 && lanes != 4 && lanes != 8 && lanes != 16 && lanes != 32)
+        return fail(VAG_ERR_INVALID, "grid lanes must be 0, 4, 8, 16 or 32");
+    ctx->grid_lanes = lanes;
     return VAG_OK;
 }
 int vag_set_capacity(vag_context* ctx, int cap_theta, int cap_phi) {

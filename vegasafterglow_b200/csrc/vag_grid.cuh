@@ -62,6 +62,11 @@ struct SeqPar {
             if (pred(j)) return j;
         return end;
     }
+    // while (active) active = round();  -- see GroupPar::lockstep
+    template <class R>
+    VAG_HD void lockstep(bool active, R round) const {
+        while (active) active = round();
+    }
 };
 #if defined(__CUDACC__)
 // one warp: index space strided over the lanes, warp barrier (with memory ordering) afterwards
@@ -83,8 +88,12 @@ struct WarpPar {
         }
         return end;
     }
+    template <class R>
+    __device__ __forceinline__ void lockstep(bool active, R round) const {
+        while (active) active = round();
+    }
 };
-// G lanes of a warp (G = 8): the same contract for a sub-warp group, so that 32 / G models share one warp.
+// G lanes of a warp (G = 2 ... 32): the same contract for a sub-warp group, so that 32 / G models share one warp.
 // The grid builder is mostly uniform (scalar) code that every cooperating lane executes redundantly;
 // with narrower groups the same instruction stream serves 32 / G models at once, while the strided
 // regions keep all lanes busy.  Groups synchronise with their own lane mask (they diverge freely).
@@ -107,6 +116,16 @@ struct GroupPar {
             if (hits) return j0 + __ffs(hits) - 1;
         }
         return end;
+    }
+    // `while (active) active = round();` for a loop whose trip count differs between models.  The groups that enter
+    // together run their rounds together until the last of them is done (a finished group idles): a group that needs
+    // another round does not leave the others to run theirs alone later, so the warp issues each round's stage
+    // evaluations and uniform code once for all of its groups instead of once per group.
+    template <class R>
+    __device__ __forceinline__ void lockstep(bool active, R round) const {
+        const unsigned peers = __activemask();
+        while (__any_sync(peers, active))
+            if (active) active = round();
     }
 };
 #endif
@@ -407,25 +426,20 @@ VAG_HD int inverse_cdf_sampling(const Par& par, const Pdf& pdf, double lo, doubl
     }
     CdfQuad<VARIANT> st;
     st.initialize(lo, gl::mul(gl::sub(hi, lo), 1.0 / 1e3));
-    int k = 1, attempts = 0;
-    for (int steps = 0; st.t <= hi;) {
+    int k = 1, attempts = 0, steps = 0, fails = 0;
+    // one attempt per round: while st.t <= hi, up to 500 attempts per step, at most max_ode_steps accepted steps
+    par.lockstep(st.t <= hi, [&]() {
         if (!st.deriv_ready) {
             st.k1 = pdf(st.t);
             st.deriv_ready = true;
         }
-        bool ok = false;
-        for (int fails = 0; fails < 500; ++fails) {
-            const double t0 = st.t, dt = st.dt;
-            // the six stage evaluations of an attempt are independent (a pure quadrature): one lane each
-            par.for_each(6, [&](int s) { kk[s] = pdf(CdfQuad<VARIANT>::stage_time(t0, dt, s)); });
-            ++attempts;
-            if (st.try_step(kk, rtol)) {
-                ok = true;
-                break;
-            }
-        }
-        if (!ok) break;
-        if (++steps > dflt::max_ode_steps) break;
+        const double t0 = st.t, dt = st.dt;
+        // the six stage evaluations of an attempt are independent (a pure quadrature): one lane each
+        par.for_each(6, [&](int s) { kk[s] = pdf(CdfQuad<VARIANT>::stage_time(t0, dt, s)); });
+        ++attempts;
+        if (!st.try_step(kk, rtol)) return ++fails < 500;
+        fails = 0;
+        if (++steps > dflt::max_ode_steps) return false;
         // dense output for every sample abscissa the accepted step passed
         // m = number of sample abscissae the step passed: first q >= k with !(st.t > x_i[q]), searched G at a time
         const double t_now = st.t;
@@ -435,7 +449,8 @@ VAG_HD int inverse_cdf_sampling(const Par& par, const Pdf& pdf, double lo, doubl
             par.for_each(m, [&](int i) { cdf_i[k0 + i] = st.calc_state(x_i[k0 + i]); });
             k += m;
         }
-    }
+        return st.t <= hi;
+    });
     const double c0 = cdf_i[0], c1 = cdf_i[n_samp - 1];
     // first j with target <= cdf_i[j].  A lane visits its queries in ascending q, hence (c1 >= c0) ascending target, and
     // every sample below the previous hit has already failed the test for a smaller target: the scan resumes there

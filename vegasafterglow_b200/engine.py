@@ -177,6 +177,11 @@ class Engine:
         1 per-point spectra always, 2 banded whenever possible."""
         _lib.check(self._lib.vag_set_series_mode(self._h, int(mode)))
 
+    def set_grid_lanes(self, lanes: int):
+        """Lanes per model of the grid builder (vag.h vag_set_grid_lanes): 0 by batch size (default), or 4 / 8 / 16 / 32 for
+        every batch.  The grid is the same bit for bit at every width."""
+        _lib.check(self._lib.vag_set_grid_lanes(self._h, int(lanes)))
+
     def last_total_alias(self):
         """Index into ``abi.COMPONENTS`` of the plane that holds `total` after the last host call, or -1."""
         return int(self._lib.vag_last_total_alias(self._h))
