@@ -1,5 +1,5 @@
 // TEST INFRASTRUCTURE ONLY: sequential host execution of the *same* kernel bodies that
-// vegasafterglow_b200/csrc/vag_kernels.cu launches on the GPU (every body is an HD function of the
+// vegasafterglow_b200/csrc/vag_b200.cu launches on the GPU (every body is an HD function of the
 // thread index; barriers become loop boundaries).  Lets the CPU-only test tier compare the
 // device algorithm against the reference stage by stage.  It is never built into, linked with or
 // called by the product library (libvag_b200.so).
@@ -29,8 +29,6 @@ struct HostBatch {
     }
 };
 
-void caps_for(const vag_params* p, size_t n, int& cap_theta, int& cap_phi);
-
 const double* softplus_table() {
     static std::vector<double> lut;
     if (lut.empty()) {
@@ -44,7 +42,9 @@ void run_front(HostBatch& hb, const vag_params* params, size_t n, double t_min, 
     BatchWs& w = hb.w;
     w.n_models = (int)n;
     w.sp_lut = softplus_table();
-    caps_for(params, n, w.cap_theta, w.cap_phi);
+    const Caps caps = caps_for(params, n);  // vag_b200.cu plans its host-buffer batches the same way
+    w.cap_theta = caps.theta;
+    w.cap_phi = caps.phi;
     w.work_per_model = grid_work_doubles(w.cap_theta, w.cap_phi);
     w.params = params;
     w.cfg = hb.alloc<ModelCfg>(n);
@@ -87,8 +87,7 @@ void run_front(HostBatch& hb, const vag_params* params, size_t n, double t_min, 
     w.coef_rvs = hb.alloc<double>((size_t)cells * PH_NCOEF);
     w.max_n_t = std::max(w.totals[TOT_MAX_NT], 1);
     w.max_erows = std::max(w.totals[TOT_MAX_EROWS], 1);
-    w.any_ssc = 0;
-    for (size_t i = 0; i < n; ++i) w.any_ssc |= (params[i].fwd.ssc || (params[i].has_rvs && params[i].rvs.ssc)) ? 1 : 0;
+    w.any_ssc = w.totals[TOT_ANY_SSC];
     for (size_t i = 0; i < n; ++i) k0c_rowmap_body(w, (int)i);
     for (int r = 0; r < rows; ++r) k1_lattice_body(w, r, 0, 1);
     for (int r = 0; r < rows; ++r) {
@@ -159,23 +158,7 @@ void run_ic_tables(HostBatch& hb, const double* nu_range) {
     }
 }
 
-// mirrors the host-side capacity planning of vag_api.cu (kept in sync by tests)
-void caps_for(const vag_params* p, size_t n, int& cap_theta, int& cap_phi) {
-    cap_theta = 64;
-    cap_phi = 8;
-    for (size_t i = 0; i < n; ++i) {
-        const bool r = p[i].has_rvs != 0;
-        const double th_res = p[i].theta_resol > 0 ? p[i].theta_resol : (r ? 0.2 : 0.15);
-        const double ph_res = p[i].phi_resol > 0 ? p[i].phi_resol : 0.06;
-        const double lg = std::log10(std::max(1.0, std::max(p[i].Gamma0, p[i].Gamma0_w) * 1.5708));
-        const int ct = 36 + (int)(90 * th_res) + (int)(std::max(0.0, lg - 1) * th_res * 55) + (int)(lg * th_res * 25) + 64;
-        const int cp = std::max((int)(360 * ph_res), 1) * 5 + 8;
-        cap_theta = std::max(cap_theta, ct);
-        cap_phi = std::max(cap_phi, cp);
-    }
-}
-
-// sequential emulation of the K3 CTA (vag_kernels.cu: k_eats) for one (model, shock)
+// sequential emulation of the K3 CTA (vag_b200.cu: k_eats) for one (model, shock)
 void eats_emulate(const BatchWs& w, int mi, int which, const EatsRequest& rq0, double* out /*[n_nu][n_t] or [n]*/) {
     const int NTHR = 128;
     EatsModel M = make_eats_model(w, mi, which);
@@ -280,9 +263,7 @@ int run_flux(const vag_params* params, size_t n, const double* t, size_t n_t, co
             }
             band_of[i] = q;
         }
-        int max_n_t = 1;
-        for (size_t mi = 0; mi < n; ++mi) max_n_t = std::max(max_n_t, hb.w.hdr[mi].n_t);
-        if (ok && !b_lg2.empty() && (g_series_mode == 2 || b_lg2.size() * (size_t)max_n_t <= 3 * n_t)) {
+        if (series_banded(ok ? (int)b_lg2.size() : 0, hb.w.max_n_t, n_t, g_series_mode)) {
             rq.n_bands = (int)b_lg2.size();
             rq.band_of = band_of.data();
             rq.lg2_nu_obs = b_lg2.data();

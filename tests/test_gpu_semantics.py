@@ -34,7 +34,7 @@ def test_chi2_with_band_terms_equals_manual_formula(engine):
         manual = manual + _manual_chi2(b["lnF_obs"], engine.flux_band(P, b["t"], b["nu_min"], b["nu_max"], b["num_nu"])[:, 0],
                                        b["sigma_ln"], b["w"])
     np.testing.assert_allclose(chi2, manual, rtol=1e-12)
-    np.testing.assert_allclose(engine.chi2(P, pts, ()), engine.chi2_series(P, *pts), rtol=1e-13)
+    np.testing.assert_array_equal(engine.chi2(P, pts, ()), engine.chi2_series(P, *pts))
     only_bands = engine.chi2(P, None, bands)
     np.testing.assert_allclose(only_bands, chi2 - engine.chi2_series(P, *pts), rtol=1e-9)
     # the sampler-side object routes band data the same way

@@ -584,9 +584,16 @@ int fail(int code, const std::string& msg) {
             return fail(VAG_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));                \
     } while (0)
 
+// device buffer grown on demand; freed with the context that owns it (vag_destroy makes its device current)
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -597,11 +604,6 @@ struct DevBuf {
         if (e == cudaSuccess) cap = want;
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
 };
 
 }  // namespace
@@ -609,22 +611,21 @@ struct DevBuf {
 struct vag_context {
     int device = 0;
     cudaStream_t stream = nullptr;
-    DevBuf model_buf, row_buf, cell_buf, obs_buf, io_params, io_t, io_nu, io_out, io_status, io_aux, ic_buf, lut_buf, sp_buf, geom_buf, io_w, io_obs, io_chi2, split_buf;
+    DevBuf model_buf, row_buf, cell_buf, obs_buf, ic_buf, lut_buf, sp_buf, geom_buf, split_buf, work_buf;
+    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs;  // staging of the host-buffer entry points
     int* h_totals = nullptr;        // pinned
     long long* h_cells = nullptr;   // pinned
     int* h_bands = nullptr;         // pinned: distinct frequencies of the series request in flight
     int series_mode = 0;            // vag_set_series_mode: 0 auto, 1 per-point spectra always, 2 banded whenever possible
     int grid_lanes = 0;             // vag_set_grid_lanes: 0 by batch size, else k_grid<grid_lanes> for every batch
-    int cap_theta = 384, cap_phi = 128;            // capacities of the batch in flight (host calls derive them per batch)
+    int cap_theta = 384, cap_phi = 128;  // vag_set_capacity: what the *_dev entry points run with (host calls size each batch)
     int dbg_max_ode_steps = 0, dbg_max_ode_fails = 0;
-    int user_cap_theta = 384, user_cap_phi = 128;  // vag_set_capacity: what the *_dev entry points run with
     bool profiling = false;
     int out_mode = VAG_OUT_DENSE;
     int total_alias = -1;  // VAG_OUT_PRESENT_ALIAS_TOTAL: component plane the last host call's `total` equals, or -1
     cudaEvent_t ev[8] = {};
     float stage_ms[8] = {};
     double work[8] = {};   // k_work counters of the last profiled pass
-    DevBuf work_buf;
     int launches = 0;
     int sm_count = 148;
     // warps of k_ic_spectrum per SM (one warp per cell in flight, 30 KB of scratch each): as many as are resident.  Measured
@@ -645,23 +646,6 @@ size_t carve_sz(size_t n) {
     return ((n * sizeof(T) + 255) / 256) * 256;
 }
 
-// capacity planning from host-side parameters (upper bounds of auto_grid's node counts,
-// src/core/grid-refinement.h:246-262,655,664-677)
-void caps_for(const vag_params* p, size_t n, int& cap_theta, int& cap_phi) {
-    cap_theta = 64;
-    cap_phi = 8;
-    for (size_t i = 0; i < n; ++i) {
-        const bool r = p[i].has_rvs != 0;
-        const double th_res = p[i].theta_resol > 0 ? p[i].theta_resol : (r ? 0.2 : 0.15);
-        const double ph_res = p[i].phi_resol > 0 ? p[i].phi_resol : 0.06;
-        const double lg = std::log10(std::max(1.0, std::max(p[i].Gamma0, p[i].Gamma0_w) * 1.5708));
-        const int ct = 36 + (int)(90 * th_res) + (int)(std::max(0.0, lg - 1) * th_res * 55) + (int)(lg * th_res * 25) + 64;
-        const int cp = std::max((int)(360 * ph_res), 1) * 5 + 8;
-        cap_theta = std::max(cap_theta, ct);
-        cap_phi = std::max(cap_phi, cp);
-    }
-}
-
 constexpr size_t EATS_SMEM_BUDGET = 200 * 1024;  // dynamic shared memory k_eats may ask for
 // models per pipeline pass: k_rowgeom / k_rowcos / k_dop_extrema index the model with gridDim.y (<= 65535), and the
 // per-model workspaces of a pass stay below a few GB; larger batches are processed in consecutive passes
@@ -673,15 +657,16 @@ struct Request {
     const double* d_nu;
     size_t n_t, n_nu;
     bool nu_code_units = false;
+    const double *d_lnF = nullptr, *d_sig = nullptr, *d_w = nullptr;  // [n_t] observations of a chi-squared series
 };
 
-int setup_models(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n) {
+int setup_models(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps) {
     w = BatchWs{};
     w.n_models = (int)n;
     w.dbg_max_ode_steps = ctx->dbg_max_ode_steps;
     w.dbg_max_ode_fails = ctx->dbg_max_ode_fails;
-    w.cap_theta = ctx->cap_theta;
-    w.cap_phi = ctx->cap_phi;
+    w.cap_theta = caps.theta;
+    w.cap_phi = caps.phi;
     w.work_per_model = grid_work_doubles(w.cap_theta, w.cap_phi);
     w.params = d_params;
     w.sp_lut = static_cast<const double*>(ctx->sp_buf.p);
@@ -764,10 +749,15 @@ void mark(vag_context* ctx, int i, cudaStream_t s) {
     if (ctx->profiling) cudaEventRecord(ctx->ev[i], s);
 }
 
-template <int G>
-void launch_grid(const BatchWs& w, size_t n, const double* d_t, size_t n_t, cudaStream_t s) {
-    k_grid<G><<<(unsigned)((n * G + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
-}
+// The kernel variants: the launch sites and vag_create's function attributes take them from here
+using GridKernel = void (*)(BatchWs, const double*, int);
+using EatsKernel = void (*)(BatchWs, EatsRequest, double*, int, int, int, int, size_t);
+constexpr int GRID_LANES[] = {4, 8, 16, 32};
+constexpr int EATS_MODES = 3, EATS_KINDS = 3;
+
+// (defined after run_front: the cubin lists the kernel templates in the order the source first names them)
+GridKernel grid_kernel(int lanes);
+EatsKernel eats_kernel(int mode, int kind);
 
 // Lanes per model of k_grid: the widest group whose launch fits into one wave of resident CTAs (GRID_MIN_BLOCKS CTAs of
 // 128 threads per SM).  Narrower groups only pay once a wider launch would need a second wave: the models of one warp
@@ -783,17 +773,13 @@ int grid_lanes_for(size_t n, int sm_count) {
 }
 
 // grid + dynamics + radiation for a batch; fills w and the totals
-int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, const double* d_t, size_t n_t,
-              cudaStream_t s, int* totals_out, long long* cells_out) {
-    int rc = setup_models(ctx, w, d_params, n);
+int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps, const double* d_t,
+              size_t n_t, cudaStream_t s, int* totals_out, long long* cells_out) {
+    int rc = setup_models(ctx, w, d_params, n, caps);
     if (rc) return rc;
     mark(ctx, 0, s);
-    switch (ctx->grid_lanes ? ctx->grid_lanes : grid_lanes_for(n, ctx->sm_count)) {
-        case 4: launch_grid<4>(w, n, d_t, n_t, s); break;
-        case 8: launch_grid<8>(w, n, d_t, n_t, s); break;
-        case 16: launch_grid<16>(w, n, d_t, n_t, s); break;
-        default: launch_grid<32>(w, n, d_t, n_t, s); break;
-    }
+    const int lanes = ctx->grid_lanes ? ctx->grid_lanes : grid_lanes_for(n, ctx->sm_count);
+    grid_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
     k_scan<<<1, 1024, 0, s>>>(w);
     ctx->launches += 2;
     CK(cudaMemcpyAsync(ctx->h_totals, w.totals, sizeof(int) * TOT_N, cudaMemcpyDeviceToHost, s));
@@ -856,20 +842,26 @@ int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n
     return VAG_OK;
 }
 
-template <int MODE>
-void launch_eats(int kind, dim3 eg, size_t sb, cudaStream_t s, const BatchWs& w, const EatsRequest& rq, double* out,
-                 int n_split, int row_chunk, int max_n_t, int nu_tile, size_t elems) {
-    if (kind == EATS_GRID)
-        k_eats<MODE, EATS_GRID><<<eg, 128, sb, s>>>(w, rq, out, n_split, row_chunk, max_n_t, nu_tile, elems);
-    else if (kind == EATS_POINT)
-        k_eats<MODE, EATS_POINT><<<eg, 128, sb, s>>>(w, rq, out, n_split, row_chunk, max_n_t, nu_tile, elems);
-    else
-        k_eats<MODE, EATS_BANDED><<<eg, 128, sb, s>>>(w, rq, out, n_split, row_chunk, max_n_t, nu_tile, elems);
+GridKernel grid_kernel(int lanes) {
+    switch (lanes) {
+        case 4: return k_grid<4>;
+        case 8: return k_grid<8>;
+        case 16: return k_grid<16>;
+        default: return k_grid<32>;
+    }
 }
 
-int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const Request& rq_in, double* d_out,
-                  int32_t* d_status, const double* d_lnF, const double* d_sig, const double* d_w, double* d_chi2,
-                  cudaStream_t s) {
+EatsKernel eats_kernel(int mode, int kind) {
+    static const EatsKernel k[EATS_MODES][EATS_KINDS] = {
+        {k_eats<0, EATS_GRID>, k_eats<0, EATS_POINT>, k_eats<0, EATS_BANDED>},
+        {k_eats<1, EATS_GRID>, k_eats<1, EATS_POINT>, k_eats<1, EATS_BANDED>},
+        {k_eats<2, EATS_GRID>, k_eats<2, EATS_POINT>, k_eats<2, EATS_BANDED>}};
+    return k[mode][kind];
+}
+
+// flux of a batch into d_out [n][VAG_NCOMP][comp]; with d_chi2, also the chi-squared of the series against rq_in's data
+int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, const Request& rq_in, double* d_out,
+                  int32_t* d_status, double* d_chi2, cudaStream_t s) {
     const size_t n_t = rq_in.n_t, n_nu = rq_in.n_nu;
     // observation arrays
     CK(ctx->obs_buf.ensure(sizeof(double) * (2 * n_t + 3 * n_nu + 8 + 3 * EATS_NU_TILE) + sizeof(int) * (n_t + 2)));
@@ -900,7 +892,7 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const 
     BatchWs w;
     int totals[TOT_N];
     long long cells = 0;
-    int rc = run_front(ctx, w, d_params, n, rq_in.d_t, n_t, s, totals, &cells);
+    int rc = run_front(ctx, w, d_params, n, caps, rq_in.d_t, n_t, s, totals, &cells);
     if (rc) return rc;
 
     if (w.any_ssc && totals[TOT_ROWS] > 0) {
@@ -921,13 +913,8 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const 
         // shared-memory budget -> rows staged per pass
         const size_t budget = EATS_SMEM_BUDGET;
         int row_chunk = EATS_ROW_CHUNK;
-        // Banded series: the boundary luminosities of every (node, band) are staged once per row instead of two spectra
-        // per (point, row): n_bands * n_t tile evaluations against 2 * n_points per-point ones.  Measured on the
-        // config-5 batch (5 bands, ~100-node lattices, scripts/series_ab.py): 3.18 ms banded, flat in the number of
-        // points, against 1.97 ms per 100 points -- the break-even is n_bands * n_t ~ 3 n_points.
         const int n_bands_req = rq_in.series ? *ctx->h_bands : 0;
-        const bool banded = n_bands_req >= 1 && n_bands_req <= EATS_NU_TILE &&
-                            (ctx->series_mode == 2 || (size_t)n_bands_req * max_n_t <= 3 * n_t);
+        const bool banded = series_banded(n_bands_req, max_n_t, n_t, ctx->series_mode);
         const int nu_tile = rq_in.series ? (banded ? n_bands_req : 1) : (int)std::min<size_t>(EATS_NU_TILE, n_nu);
         const int acc_cols = rq_in.series ? 1 : nu_tile;
         auto smem_bytes = [&](int rc_) {
@@ -975,13 +962,10 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const 
             CK(cudaMemsetAsync(eats_out, 0, sizeof(double) * elems * n_split, s));
         }
         const int kind = !rq_in.series ? EATS_GRID : banded ? EATS_BANDED : EATS_POINT;
-        launch_eats<0>(kind, eg, sb, s, w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
-        ctx->launches++;
-        if (w.any_ssc) {
-            launch_eats<1>(kind, eg, sb, s, w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
-            launch_eats<2>(kind, eg, sb, s, w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
-            ctx->launches += 2;
-        }
+        const int n_modes = w.any_ssc ? EATS_MODES : 1;
+        for (int mode = 0; mode < n_modes; ++mode)
+            eats_kernel(mode, kind)<<<eg, 128, sb, s>>>(w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
+        ctx->launches += n_modes;
         if (n_split > 1) {
             k_sum_splits<<<(unsigned)((elems + 255) / 256), 256, 0, s>>>(d_out, eats_out, n_split, elems);
             ctx->launches++;
@@ -1000,7 +984,8 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const 
         }
     }
     if (d_chi2) {
-        k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, d_lnF, d_sig, d_w, d_chi2, w.status, 0);
+        k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
+                                                                 d_chi2, w.status, 0);
         ctx->launches++;
     }
     mark(ctx, 5, s);
@@ -1017,23 +1002,17 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, const 
     return VAG_OK;
 }
 
-int run_flux(vag_context* ctx, const vag_params* d_params, size_t n, const Request& rq, double* d_out, int32_t* d_status,
-             const double* d_lnF, const double* d_sig, const double* d_w, double* d_chi2, cudaStream_t s) {
+int run_flux(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, const Request& rq, double* d_out,
+             int32_t* d_status, double* d_chi2, cudaStream_t s) {
     ctx->launches = 0;
     const size_t comp_sz = rq.series ? rq.n_t : rq.n_nu * rq.n_t;
     for (size_t lo = 0; lo < n; lo += MAX_MODELS_PER_PASS) {
         const size_t m = std::min(MAX_MODELS_PER_PASS, n - lo);
-        if (int rc = run_flux_pass(ctx, d_params + lo, m, rq, d_out + lo * VAG_NCOMP * comp_sz, d_status ? d_status + lo : nullptr,
-                                   d_lnF, d_sig, d_w, d_chi2 ? d_chi2 + lo : nullptr, s))
+        if (int rc = run_flux_pass(ctx, d_params + lo, m, caps, rq, d_out + lo * VAG_NCOMP * comp_sz,
+                                   d_status ? d_status + lo : nullptr, d_chi2 ? d_chi2 + lo : nullptr, s))
             return rc;
     }
     return VAG_OK;
-}
-
-int check_ascending(const double* t, size_t n) {  // is_ascending, pybind/pybind.h:28
-    for (size_t i = 1; i < n; ++i)
-        if (!(t[i - 1] <= t[i])) return 0;
-    return 1;
 }
 
 bool finite_pos(double x) { return std::isfinite(x) && x > 0; }
@@ -1169,25 +1148,13 @@ int vag_create(int device, vag_context** out) {
     }
     // k_grid spills its scratch to local memory: prefer L1.  k_dynamics keeps its dopri5 stage vectors
     // in shared memory (23 KB per 32-row CTA): give it the full carve-out so several CTAs share an SM.
-    cudaFuncSetCacheConfig(k_grid<4>, cudaFuncCachePreferL1);
-    cudaFuncSetCacheConfig(k_grid<8>, cudaFuncCachePreferL1);
-    cudaFuncSetCacheConfig(k_grid<16>, cudaFuncCachePreferL1);
-    cudaFuncSetCacheConfig(k_grid<32>, cudaFuncCachePreferL1);
+    for (int lanes : GRID_LANES) cudaFuncSetCacheConfig(grid_kernel(lanes), cudaFuncCachePreferL1);
     cudaFuncSetAttribute(k_dynamics<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     // per-function process state: set once, to the largest request run_flux can make (not per call, where two contexts
     // with different request shapes would race on it)
-#define VAG_EATS_ATTR(M_, K_) \
-    CK(cudaFuncSetAttribute(k_eats<M_, K_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET))
-    VAG_EATS_ATTR(0, EATS_GRID);
-    VAG_EATS_ATTR(0, EATS_POINT);
-    VAG_EATS_ATTR(0, EATS_BANDED);
-    VAG_EATS_ATTR(1, EATS_GRID);
-    VAG_EATS_ATTR(1, EATS_POINT);
-    VAG_EATS_ATTR(1, EATS_BANDED);
-    VAG_EATS_ATTR(2, EATS_GRID);
-    VAG_EATS_ATTR(2, EATS_POINT);
-    VAG_EATS_ATTR(2, EATS_BANDED);
-#undef VAG_EATS_ATTR
+    for (int mode = 0; mode < EATS_MODES; ++mode)
+        for (int kind = 0; kind < EATS_KINDS; ++kind)
+            CK(cudaFuncSetAttribute(eats_kernel(mode, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET));
     {
         int blocks = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum, 128, 0) == cudaSuccess && blocks > 0)
@@ -1201,17 +1168,13 @@ void vag_destroy(vag_context* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
-    for (DevBuf* b : {&c->model_buf, &c->row_buf, &c->cell_buf, &c->obs_buf, &c->io_params, &c->io_t, &c->io_nu,
-                      &c->io_out, &c->io_status, &c->io_aux, &c->ic_buf, &c->lut_buf, &c->sp_buf, &c->geom_buf, &c->io_w, &c->io_obs,
-                      &c->io_chi2, &c->split_buf, &c->work_buf})
-        b->release();
     if (c->h_totals) cudaFreeHost(c->h_totals);
     if (c->h_cells) cudaFreeHost(c->h_cells);
     if (c->h_bands) cudaFreeHost(c->h_bands);
     for (auto& ev : c->ev)
         if (ev) cudaEventDestroy(ev);
     cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;  // frees the DevBufs
 }
 
 int vag_set_profiling(vag_context* ctx, int enable) {
@@ -1252,8 +1215,8 @@ int vag_set_grid_lanes(vag_context* ctx, int lanes) {
 }
 int vag_set_capacity(vag_context* ctx, int cap_theta, int cap_phi) {
     if (cap_theta < 40 || cap_phi < 2) return fail(VAG_ERR_INVALID, "capacity too small");
-    ctx->cap_theta = ctx->user_cap_theta = cap_theta;
-    ctx->cap_phi = ctx->user_cap_phi = cap_phi;
+    ctx->cap_theta = cap_theta;
+    ctx->cap_phi = cap_phi;
     return VAG_OK;
 }
 
@@ -1266,7 +1229,7 @@ int vag_debug_set_ode_limits(vag_context* ctx, int max_steps, int max_fails) {
 
 int vag_measure_fp64_peak(vag_context* ctx, double* tflops) {
     CK(cudaSetDevice(ctx->device));
-    CK(ctx->io_aux.ensure(64));
+    CK(ctx->io_out.ensure(64));
     const int iters = 1 << 16, blocks = ctx->sm_count * 8, threads = 256;
     cudaEvent_t a, b;
     CK(cudaEventCreate(&a));
@@ -1274,7 +1237,7 @@ int vag_measure_fp64_peak(vag_context* ctx, double* tflops) {
     double best = 0;
     for (int rep = 0; rep < 4; ++rep) {
         CK(cudaEventRecord(a, ctx->stream));
-        k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(static_cast<double*>(ctx->io_aux.p), iters);
+        k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(static_cast<double*>(ctx->io_out.p), iters);
         CK(cudaEventRecord(b, ctx->stream));
         CK(cudaEventSynchronize(b));
         float ms = 0;
@@ -1293,8 +1256,8 @@ int vag_selftest_libm(vag_context* ctx, int fn, const double* x, const double* y
     if ((fn == 5) != (y != nullptr)) return fail(VAG_ERR_INVALID, "vag_selftest_libm: y is required for pow only");
     if (n == 0) return VAG_OK;
     CK(cudaSetDevice(ctx->device));
-    CK(ctx->io_aux.ensure(3 * n * sizeof(double)));
-    double* d_x = static_cast<double*>(ctx->io_aux.p);
+    CK(ctx->io_out.ensure(3 * n * sizeof(double)));
+    double* d_x = static_cast<double*>(ctx->io_out.p);
     double* d_y = d_x + n;
     double* d_o = d_y + n;
     CK(cudaMemcpyAsync(d_x, x, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
@@ -1306,83 +1269,86 @@ int vag_selftest_libm(vag_context* ctx, int fn, const double* x, const double* y
     return VAG_OK;
 }
 
+// ---- preparation of the host-buffer entry points ------------------------------------------------------
+// validates the parameter sets and uploads them; *caps: the capacities their grids need
+static int prepare_params(vag_context* ctx, const vag_params* params, size_t n_models, Caps* caps) {
+    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
+    if (!params && n_models) return fail(VAG_ERR_INVALID, "params is NULL");
+    for (size_t i = 0; i < n_models; ++i)
+        if (int rc = vag_params_validate(&params[i])) return rc;
+    CK(cudaSetDevice(ctx->device));
+    *caps = caps_for(params, n_models);
+    CK(ctx->io_params.ensure(sizeof(vag_params) * std::max<size_t>(n_models, 1)));
+    CK(ctx->io_status.ensure(sizeof(int32_t) * std::max<size_t>(n_models, 1)));
+    CK(cudaMemcpyAsync(ctx->io_params.p, params, sizeof(vag_params) * n_models, cudaMemcpyHostToDevice, ctx->stream));
+    return VAG_OK;
+}
+
+// log10(t_end / t_start) sizes the time lattice: a zero, negative or non-finite epoch has no meaning
+static int check_times(const double* t, size_t n_t) {
+    if (n_t == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
+    for (size_t i = 1; i < n_t; ++i)  // is_ascending, pybind/pybind.h:28
+        if (!(t[i - 1] <= t[i])) return fail(VAG_ERR_INVALID, "time array must be in ascending order");
+    for (size_t i = 0; i < n_t; ++i)
+        if (!finite_pos(t[i])) return fail(VAG_ERR_INVALID, "observation times must be finite and > 0");
+    return VAG_OK;
+}
+
+// times -> io_t, frequencies -> io_nu, checked by the caller
+static int upload_request(vag_context* ctx, const double* t, size_t n_t, const double* nu, size_t n_nu) {
+    CK(ctx->io_t.ensure(sizeof(double) * n_t));
+    CK(ctx->io_nu.ensure(sizeof(double) * n_nu));
+    CK(cudaMemcpyAsync(ctx->io_t.p, t, sizeof(double) * n_t, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->io_nu.p, nu, sizeof(double) * n_nu, cudaMemcpyHostToDevice, ctx->stream));
+    return VAG_OK;
+}
+
+static int prepare_request(vag_context* ctx, const double* t, size_t n_t, const double* nu, size_t n_nu) {
+    if (int rc = check_times(t, n_t)) return rc;
+    if (n_nu == 0 || !nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
+    for (size_t i = 0; i < n_nu; ++i)
+        if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, "observation frequencies must be finite and > 0");
+    return upload_request(ctx, t, n_t, nu, n_nu);
+}
+
 // ---- device-buffer entry points ----------------------------------------------------------------
+// the caller's buffers and stream, the capacities of vag_set_capacity; with d_chi2 the series flux is scratch
+static int flux_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const Request& rq, double* d_out,
+                    int32_t* d_status, double* d_chi2, void* stream) {
+    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
+    if (rq.n_t == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
+    if (rq.n_nu == 0) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    if (d_chi2) {
+        CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * rq.n_t));
+        d_out = static_cast<double*>(ctx->io_out.p);
+    }
+    return run_flux(ctx, d_params, n_models, Caps{ctx->cap_theta, ctx->cap_phi}, rq, d_out, d_status, d_chi2, s);
+}
+
 int vag_flux_density_grid_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t,
                               size_t n_t, const double* d_nu, size_t n_nu, double* d_out, int32_t* d_status,
                               void* stream) {
-    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
-    if (n_t == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
-    if (n_nu == 0) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
-    ctx->cap_theta = ctx->user_cap_theta;  // host-buffer calls in between may have run with tighter per-batch capacities
-    ctx->cap_phi = ctx->user_cap_phi;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Request rq{false, d_t, d_nu, n_t, n_nu};
-    return run_flux(ctx, d_params, n_models, rq, d_out, d_status, nullptr, nullptr, nullptr, nullptr, s);
+    return flux_dev(ctx, d_params, n_models, Request{false, d_t, d_nu, n_t, n_nu}, d_out, d_status, nullptr, stream);
 }
 
 int vag_flux_density_series_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t,
                                 const double* d_nu, size_t n, double* d_out, int32_t* d_status, void* stream) {
-    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
-    if (n == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
-    ctx->cap_theta = ctx->user_cap_theta;  // host-buffer calls in between may have run with tighter per-batch capacities
-    ctx->cap_phi = ctx->user_cap_phi;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    Request rq{true, d_t, d_nu, n, n};
-    return run_flux(ctx, d_params, n_models, rq, d_out, d_status, nullptr, nullptr, nullptr, nullptr, s);
+    return flux_dev(ctx, d_params, n_models, Request{true, d_t, d_nu, n, n}, d_out, d_status, nullptr, stream);
 }
 
 int vag_chi2_series_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t,
                         const double* d_nu, const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w,
                         size_t n, double* d_chi2, int32_t* d_status, void* stream) {
-    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
-    if (n == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
-    ctx->cap_theta = ctx->user_cap_theta;  // host-buffer calls in between may have run with tighter per-batch capacities
-    ctx->cap_phi = ctx->user_cap_phi;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * n));
     Request rq{true, d_t, d_nu, n, n};
-    return run_flux(ctx, d_params, n_models, rq, static_cast<double*>(ctx->io_out.p), d_status, d_lnF_obs, d_sigma_ln,
-                    d_w, d_chi2, s);
+    rq.d_lnF = d_lnF_obs;
+    rq.d_sig = d_sigma_ln;
+    rq.d_w = d_w;
+    return flux_dev(ctx, d_params, n_models, rq, nullptr, d_status, d_chi2, stream);
 }
 
 // ---- host-buffer entry points --------------------------------------------------------------------
-static int host_prepare(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, size_t n_t,
-                        const double* nu, size_t n_nu, bool series) {
-    if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
-    if (!params && n_models) return fail(VAG_ERR_INVALID, "params is NULL");
-    if (n_t == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
-    if (n_nu == 0 || !nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
-    if (series && n_t != n_nu)
-        return fail(VAG_ERR_INVALID,
-                    "time and frequency arrays must have the same size\nIf you intend to get grid-like output, use "
-                    "the generic `flux_density_grid` instead");
-    if (!check_ascending(t, n_t)) return fail(VAG_ERR_INVALID, "time array must be in ascending order");
-    // log10(t_end / t_start) sizes the time lattice: a zero, negative or non-finite epoch / frequency has no meaning
-    for (size_t i = 0; i < n_t; ++i)
-        if (!finite_pos(t[i])) return fail(VAG_ERR_INVALID, "observation times must be finite and > 0");
-    for (size_t i = 0; i < n_nu; ++i)
-        if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, "observation frequencies must be finite and > 0");
-    for (size_t i = 0; i < n_models; ++i)
-        if (int rc = vag_params_validate(&params[i])) return rc;
-    CK(cudaSetDevice(ctx->device));
-    int ct, cp;
-    caps_for(params, n_models, ct, cp);
-    ctx->cap_theta = ct;
-    ctx->cap_phi = cp;
-    CK(ctx->io_params.ensure(sizeof(vag_params) * std::max<size_t>(n_models, 1)));
-    CK(ctx->io_t.ensure(sizeof(double) * n_t));
-    CK(ctx->io_nu.ensure(sizeof(double) * n_nu));
-    CK(ctx->io_status.ensure(sizeof(int32_t) * std::max<size_t>(n_models, 1)));
-    cudaStream_t s = ctx->stream;
-    CK(cudaMemcpyAsync(ctx->io_params.p, params, sizeof(vag_params) * n_models, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_t.p, t, sizeof(double) * n_t, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_nu.p, nu, sizeof(double) * n_nu, cudaMemcpyHostToDevice, s));
-    return VAG_OK;
-}
-
 // device -> host transfer of out[n_models][VAG_NCOMP][comp_sz] under the context's output mode
 static int copy_out(vag_context* ctx, const vag_params* params, size_t n_models, size_t comp_sz, double* out,
                     cudaStream_t s) {
@@ -1429,49 +1395,48 @@ static int copy_out(vag_context* ctx, const vag_params* params, size_t n_models,
     return VAG_OK;
 }
 
-int vag_flux_density_grid(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, size_t n_t,
-                          const double* nu, size_t n_nu, double* out, int32_t* status) {
-    if (int rc = host_prepare(ctx, params, n_models, t, n_t, nu, n_nu, false)) return rc;
+static int flux_host(vag_context* ctx, const vag_params* params, size_t n_models, bool series, const double* t,
+                     size_t n_t, const double* nu, size_t n_nu, double* out, int32_t* status) {
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (int rc = prepare_request(ctx, t, n_t, nu, n_nu)) return rc;
     if (n_models == 0) return VAG_OK;
-    const size_t out_bytes = sizeof(double) * n_models * VAG_NCOMP * n_nu * n_t;
-    CK(ctx->io_out.ensure(out_bytes));
+    const size_t comp_sz = series ? n_t : n_nu * n_t;
+    CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * comp_sz));
     cudaStream_t s = ctx->stream;
-    Request rq{false, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_t, n_nu};
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, rq,
-                          static_cast<double*>(ctx->io_out.p), static_cast<int32_t*>(ctx->io_status.p), nullptr, nullptr,
-                          nullptr, nullptr, s))
+    const Request rq{series, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_t, n_nu};
+    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq,
+                          static_cast<double*>(ctx->io_out.p), static_cast<int32_t*>(ctx->io_status.p), nullptr, s))
         return rc;
-    if (int rc = copy_out(ctx, params, n_models, out_bytes / (sizeof(double) * n_models * VAG_NCOMP), out, s)) return rc;
+    if (int rc = copy_out(ctx, params, n_models, comp_sz, out, s)) return rc;
     if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
 }
 
+int vag_flux_density_grid(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, size_t n_t,
+                          const double* nu, size_t n_nu, double* out, int32_t* status) {
+    return flux_host(ctx, params, n_models, false, t, n_t, nu, n_nu, out, status);
+}
+
 int vag_flux_density_series(vag_context* ctx, const vag_params* params, size_t n_models, const double* t,
                             const double* nu, size_t n, double* out, int32_t* status) {
-    if (int rc = host_prepare(ctx, params, n_models, t, n, nu, n, true)) return rc;
-    if (n_models == 0) return VAG_OK;
-    const size_t out_bytes = sizeof(double) * n_models * VAG_NCOMP * n;
-    CK(ctx->io_out.ensure(out_bytes));
-    cudaStream_t s = ctx->stream;
-    Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n, n};
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, rq,
-                          static_cast<double*>(ctx->io_out.p), static_cast<int32_t*>(ctx->io_status.p), nullptr, nullptr,
-                          nullptr, nullptr, s))
-        return rc;
-    if (int rc = copy_out(ctx, params, n_models, out_bytes / (sizeof(double) * n_models * VAG_NCOMP), out, s)) return rc;
-    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return VAG_OK;
+    return flux_host(ctx, params, n_models, true, t, n, nu, n, out, status);
 }
 
 // Frequency grid (code units) and quadrature weights of PyModel::flux (pybind/pymodel.cpp:391-410): xt::logspace of the
 // unit-scaled bounds, Boole's rule in ln(nu) with 3/8 / Simpson / trapezoid remainders (src/core/quadrature.h:138-191),
 // times the Jacobian nu and the code-unit -> Hz factor, so that sum_i F_nu[cgs](nu_i) w_i is erg cm^-2 s^-1.
-static int band_grid(double nu_min, double nu_max, size_t num_nu, std::vector<double>& nu, std::vector<double>& wgt) {
+struct BandGrid {
+    std::vector<double> nu, wgt;
+};
+
+static int band_grid(double nu_min, double nu_max, size_t num_nu, BandGrid& g) {
     if (!(nu_min > 0) || !std::isfinite(nu_min)) return fail(VAG_ERR_INVALID, "nu_min must be positive");
     if (!(nu_max > nu_min) || !std::isfinite(nu_max)) return fail(VAG_ERR_INVALID, "nu_max must be greater than nu_min");
     if (num_nu < 2) return fail(VAG_ERR_INVALID, "num_nu must be at least 2");
+    std::vector<double>& nu = g.nu;
+    std::vector<double>& wgt = g.wgt;
     nu.assign(num_nu, 0.0);
     wgt.assign(num_nu, 0.0);
     const double a = std::log10(nu_min * unit::Hz), b = std::log10(nu_max * unit::Hz);
@@ -1507,30 +1472,21 @@ static int band_grid(double nu_min, double nu_max, size_t num_nu, std::vector<do
     return VAG_OK;
 }
 
-// Band-integrated flux of a batch whose parameters are already on the device: grid evaluation on the band's
-// frequency nodes, then the weighted sum over frequency.  *d_band -> [n_models][VAG_NCOMP][n_t] inside io_out.
-static int run_band(vag_context* ctx, size_t n_models, const double* t, size_t n_t, double nu_min, double nu_max,
-                    size_t num_nu, double** d_band, cudaStream_t s) {
-    std::vector<double> nu, wgt;
-    if (int rc = band_grid(nu_min, nu_max, num_nu, nu, wgt)) return rc;
-    if (!check_ascending(t, n_t)) return fail(VAG_ERR_INVALID, "time array must be in ascending order");
-    for (size_t i = 0; i < n_t; ++i)
-        if (!finite_pos(t[i])) return fail(VAG_ERR_INVALID, "observation times must be finite and > 0");
-    CK(ctx->io_t.ensure(sizeof(double) * n_t));
-    CK(ctx->io_nu.ensure(sizeof(double) * num_nu));
+// Band-integrated flux of a batch whose parameters, times (io_t) and band nodes g.nu (io_nu) are on the device: grid
+// evaluation on the band's frequency nodes, then the weighted sum over frequency.  *d_band -> [n_models][VAG_NCOMP][n_t]
+// inside io_out.
+static int run_band(vag_context* ctx, size_t n_models, Caps caps, size_t n_t, const BandGrid& g, double** d_band,
+                    cudaStream_t s) {
+    const size_t num_nu = g.nu.size();
     CK(ctx->io_w.ensure(sizeof(double) * num_nu));
     const size_t grid_elems = n_models * VAG_NCOMP * num_nu * n_t;
     CK(ctx->io_out.ensure(sizeof(double) * (grid_elems + n_models * VAG_NCOMP * n_t)));
-    // (the previous pass over these staging buffers has completed on this stream; pageable copies are staged by the runtime)
-    CK(cudaMemcpyAsync(ctx->io_t.p, t, sizeof(double) * n_t, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_nu.p, nu.data(), sizeof(double) * num_nu, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_w.p, wgt.data(), sizeof(double) * num_nu, cudaMemcpyHostToDevice, s));
-    CK(cudaStreamSynchronize(s));  // nu / wgt are locals
+    CK(cudaMemcpyAsync(ctx->io_w.p, g.wgt.data(), sizeof(double) * num_nu, cudaMemcpyHostToDevice, s));
     double* d_grid = static_cast<double*>(ctx->io_out.p);
     *d_band = d_grid + grid_elems;
     Request rq{false, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_t, num_nu, true};
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, rq, d_grid,
-                          static_cast<int32_t*>(ctx->io_status.p), nullptr, nullptr, nullptr, nullptr, s))
+    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq, d_grid,
+                          static_cast<int32_t*>(ctx->io_status.p), nullptr, s))
         return rc;
     const size_t n_mc = n_models * VAG_NCOMP;
     k_band_reduce<<<(unsigned)((n_mc * n_t + 255) / 256), 256, 0, s>>>(d_grid, static_cast<double*>(ctx->io_w.p), *d_band,
@@ -1543,13 +1499,15 @@ static int run_band(vag_context* ctx, size_t n_models, const double* t, size_t n
 // Replaces PyModel::flux (pybind/pymodel.cpp:391-410): band-integrated flux over [nu_min, nu_max]
 int vag_flux_band(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, size_t n_t,
                   double nu_min, double nu_max, size_t num_nu, double* out, int32_t* status) {
-    std::vector<double> nu, wgt;
-    if (int rc = band_grid(nu_min, nu_max, num_nu, nu, wgt)) return rc;
-    if (int rc = host_prepare(ctx, params, n_models, t, n_t, nu.data(), num_nu, false)) return rc;
+    BandGrid g;
+    if (int rc = band_grid(nu_min, nu_max, num_nu, g)) return rc;
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (int rc = prepare_request(ctx, t, n_t, g.nu.data(), num_nu)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
     double* d_band = nullptr;
-    if (int rc = run_band(ctx, n_models, t, n_t, nu_min, nu_max, num_nu, &d_band, s)) return rc;
+    if (int rc = run_band(ctx, n_models, caps, n_t, g, &d_band, s)) return rc;
     CK(cudaMemcpyAsync(out, d_band, sizeof(double) * n_models * VAG_NCOMP * n_t, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -1565,64 +1523,74 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
     if (n_points && (!t || !nu || !lnF_obs || !sigma_ln || !w)) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL");
     if (n_bands && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
     if (n_points == 0 && n_bands == 0) return fail(VAG_ERR_INVALID, "no data: n_points and n_bands are both 0");
+    // every band is checked before any work is enqueued
+    std::vector<BandGrid> grids(n_bands);
+    size_t max_obs = n_points;
     for (size_t b = 0; b < n_bands; ++b) {
         const vag_band_obs& B = bands[b];
         if (B.n == 0 || !B.t || !B.lnF_obs || !B.sigma_ln || !B.w) return fail(VAG_ERR_INVALID, "band data arrays must be non-empty");
-        std::vector<double> gnu, gw;
-        if (int rc = band_grid(B.nu_min, B.nu_max, B.num_nu, gnu, gw)) return rc;
+        if (int rc = band_grid(B.nu_min, B.nu_max, B.num_nu, grids[b])) return rc;
+        if (int rc = check_times(B.t, B.n)) return rc;
+        max_obs = std::max(max_obs, B.n);
     }
-    // validation + upload of the parameters (and of the point request when there is one)
-    const double one = 1.0;
-    if (int rc = n_points ? host_prepare(ctx, params, n_models, t, n_points, nu, n_points, true)
-                          : host_prepare(ctx, params, n_models, bands[0].t, bands[0].n, &one, 1, false))
-        return rc;
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_points)
+        if (int rc = prepare_request(ctx, t, n_points, nu, n_points)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
-    size_t max_obs = n_points;
-    for (size_t b = 0; b < n_bands; ++b) max_obs = std::max(max_obs, bands[b].n);
-    CK(ctx->io_obs.ensure(sizeof(double) * 3 * max_obs));
-    CK(ctx->io_chi2.ensure(sizeof(double) * n_models + sizeof(int32_t) * n_models));
-    double* d_lnF = static_cast<double*>(ctx->io_obs.p);
+    // observation staging: chi2 [n_models], lnF / sigma_ln / w [max_obs] of the term in flight, status OR [n_models]
+    CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * max_obs) + sizeof(int32_t) * n_models));
+    double* d_chi2 = static_cast<double*>(ctx->io_obs.p);
+    double* d_lnF = d_chi2 + n_models;
     double* d_sig = d_lnF + max_obs;
     double* d_w = d_sig + max_obs;
-    double* d_chi2 = static_cast<double*>(ctx->io_chi2.p);
-    int32_t* d_stat_or = reinterpret_cast<int32_t*>(d_chi2 + n_models);
-    CK(cudaMemsetAsync(d_chi2, 0, sizeof(double) * n_models, s));
-    CK(cudaMemsetAsync(d_stat_or, 0, sizeof(int32_t) * n_models, s));
-    int launches = 0;
+    int32_t* d_stat_or = reinterpret_cast<int32_t*>(d_w + max_obs);
+    int32_t* d_status = static_cast<int32_t*>(ctx->io_status.p);
     auto upload = [&](const double* a, const double* b_, const double* c, size_t n) -> int {
         CK(cudaMemcpyAsync(d_lnF, a, sizeof(double) * n, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(d_sig, b_, sizeof(double) * n, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(d_w, c, sizeof(double) * n, cudaMemcpyHostToDevice, s));
         return VAG_OK;
     };
-    const unsigned cg = (unsigned)((n_models * 32 + 127) / 128);
-    if (n_points) {
+    // with band terms, the status is the OR over every term's status; a lone point term's status is the status
+    const bool or_status = n_bands > 0;
+    const unsigned og = (unsigned)((n_models + 255) / 256), cg = (unsigned)((n_models * 32 + 127) / 128);
+    if (or_status) CK(cudaMemsetAsync(d_stat_or, 0, sizeof(int32_t) * n_models, s));
+    int launches = 0;
+    if (n_points) {  // the first term: run_flux writes chi2
         if (int rc = upload(lnF_obs, sigma_ln, w, n_points)) return rc;
         CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * n_points));
         Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points, n_points};
-        if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, rq, static_cast<double*>(ctx->io_out.p),
-                              static_cast<int32_t*>(ctx->io_status.p), nullptr, nullptr, nullptr, nullptr, s))
+        rq.d_lnF = d_lnF;
+        rq.d_sig = d_sig;
+        rq.d_w = d_w;
+        if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq,
+                              static_cast<double*>(ctx->io_out.p), d_status, d_chi2, s))
             return rc;
-        k_chi2<<<cg, 128, 0, s>>>(static_cast<double*>(ctx->io_out.p), n_models, (int)n_points, d_lnF, d_sig, d_w, d_chi2,
-                                  static_cast<int32_t*>(ctx->io_status.p), 1);
-        k_or_status<<<(unsigned)((n_models + 255) / 256), 256, 0, s>>>(d_stat_or, static_cast<int32_t*>(ctx->io_status.p), n_models);
-        launches += ctx->launches + 2;
+        launches += ctx->launches;
+        if (or_status) {
+            k_or_status<<<og, 256, 0, s>>>(d_stat_or, d_status, n_models);
+            launches++;
+        }
+    } else {
+        CK(cudaMemsetAsync(d_chi2, 0, sizeof(double) * n_models, s));
     }
     for (size_t b = 0; b < n_bands; ++b) {
         const vag_band_obs& B = bands[b];
+        if (int rc = upload_request(ctx, B.t, B.n, grids[b].nu.data(), grids[b].nu.size())) return rc;
         double* d_band = nullptr;
-        if (int rc = run_band(ctx, n_models, B.t, B.n, B.nu_min, B.nu_max, B.num_nu, &d_band, s)) return rc;
+        if (int rc = run_band(ctx, n_models, caps, B.n, grids[b], &d_band, s)) return rc;
         if (int rc = upload(B.lnF_obs, B.sigma_ln, B.w, B.n)) return rc;
-        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, d_lnF, d_sig, d_w, d_chi2, static_cast<int32_t*>(ctx->io_status.p), 1);
-        k_or_status<<<(unsigned)((n_models + 255) / 256), 256, 0, s>>>(d_stat_or, static_cast<int32_t*>(ctx->io_status.p), n_models);
+        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, d_lnF, d_sig, d_w, d_chi2, d_status, 1);
+        k_or_status<<<og, 256, 0, s>>>(d_stat_or, d_status, n_models);
         launches += ctx->launches + 2;
-        CK(cudaStreamSynchronize(s));  // the observation staging buffers are reused by the next band
     }
     ctx->launches = launches;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
-    if (status) CK(cudaMemcpyAsync(status, d_stat_or, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    if (status)
+        CK(cudaMemcpyAsync(status, or_status ? d_stat_or : d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
 }
@@ -1639,52 +1607,32 @@ int vag_chi2_series(vag_context* ctx, const vag_params* params, size_t n_models,
                     const double* lnF_obs, const double* sigma_ln, const double* w, size_t n, double* chi2,
                     int32_t* status) {
     if (!lnF_obs || !sigma_ln || !w || !chi2) return fail(VAG_ERR_INVALID, "data arrays must not be NULL");
-    if (int rc = host_prepare(ctx, params, n_models, t, n, nu, n, true)) return rc;
-    if (n_models == 0) return VAG_OK;
-    cudaStream_t s = ctx->stream;
-    CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * n));
-    CK(ctx->io_aux.ensure(sizeof(double) * (3 * n + n_models)));
-    double* d_lnF = static_cast<double*>(ctx->io_aux.p);
-    double* d_sig = d_lnF + n;
-    double* d_w = d_sig + n;
-    double* d_chi2 = d_w + n;
-    CK(cudaMemcpyAsync(d_lnF, lnF_obs, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_sig, sigma_ln, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_w, w, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-    Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n, n};
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, rq,
-                          static_cast<double*>(ctx->io_out.p), static_cast<int32_t*>(ctx->io_status.p), d_lnF, d_sig,
-                          d_w, d_chi2, s))
-        return rc;
-    CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
-    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return VAG_OK;
+    if (n == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
+    if (!nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
+    return vag_chi2(ctx, params, n_models, t, nu, lnF_obs, sigma_ln, w, n, nullptr, 0, chi2, status);
 }
 
 // ---- introspection ---------------------------------------------------------------------------------
+// one parameter set through grid, dynamics and radiation over [t_min, t_max]
+static int details_front(vag_context* ctx, const vag_params* p, double t_min, double t_max, BatchWs& w, long long* cells) {
+    Caps caps;
+    if (int rc = prepare_params(ctx, p, 1, &caps)) return rc;
+    const double tt[2] = {t_min, t_max};
+    CK(ctx->io_t.ensure(sizeof(tt)));
+    CK(cudaMemcpyAsync(ctx->io_t.p, tt, sizeof(tt), cudaMemcpyHostToDevice, ctx->stream));
+    int totals[TOT_N];
+    ctx->launches = 0;
+    return run_front(ctx, w, static_cast<vag_params*>(ctx->io_params.p), 1, caps, static_cast<double*>(ctx->io_t.p), 2,
+                     ctx->stream, totals, cells);
+}
+
 int vag_details(vag_context* ctx, const vag_params* p, double t_min, double t_max, vag_grid_info* info, double* theta,
                 double* phi, int32_t* reps, double* t_rows, double* fwd_shock, double* rvs_shock, int32_t* inj_idx) {
     if (!ctx || !p) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (int rc = vag_params_validate(p)) return rc;
-    CK(cudaSetDevice(ctx->device));
-    int ct, cp;
-    caps_for(p, 1, ct, cp);
-    ctx->cap_theta = ct;
-    ctx->cap_phi = cp;
-    cudaStream_t s = ctx->stream;
-    CK(ctx->io_params.ensure(sizeof(vag_params)));
-    CK(ctx->io_t.ensure(sizeof(double) * 2));
-    const double tt[2] = {t_min, t_max};
-    CK(cudaMemcpyAsync(ctx->io_params.p, p, sizeof(vag_params), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_t.p, tt, sizeof(tt), cudaMemcpyHostToDevice, s));
     BatchWs w;
-    int totals[TOT_N];
     long long cells = 0;
-    ctx->launches = 0;
-    if (int rc = run_front(ctx, w, static_cast<vag_params*>(ctx->io_params.p), 1, static_cast<double*>(ctx->io_t.p), 2,
-                           s, totals, &cells))
-        return rc;
+    if (int rc = details_front(ctx, p, t_min, t_max, w, &cells)) return rc;
+    cudaStream_t s = ctx->stream;
     GridHeader h;
     int st = 0;
     CK(cudaMemcpyAsync(&h, w.hdr, sizeof(h), cudaMemcpyDeviceToHost, s));
@@ -1701,20 +1649,15 @@ int vag_details(vag_context* ctx, const vag_params* p, double t_min, double t_ma
         info->status = st;
     }
     const size_t nc = (size_t)h.n_reps * h.n_t;
-    if (theta) CK(cudaMemcpyAsync(theta, w.theta, sizeof(double) * h.n_theta, cudaMemcpyDeviceToHost, s));
+    // theta and the theta index of every ODE row (the representatives of the symmetry groups, or r % n_theta for a
+    // rows3d model) serve the output arrays and the theta plane of the shock tables
+    std::vector<double> th(h.n_theta);
+    std::vector<int32_t> rep(h.n_reps);
+    CK(cudaMemcpyAsync(th.data(), w.theta, sizeof(double) * h.n_theta, cudaMemcpyDeviceToHost, s));
+    if (!h.rows3d) CK(cudaMemcpyAsync(rep.data(), w.reps, sizeof(int) * h.n_reps, cudaMemcpyDeviceToHost, s));
     if (phi) CK(cudaMemcpyAsync(phi, w.phi, sizeof(double) * h.n_phi, cudaMemcpyDeviceToHost, s));
-    // theta index of every ODE row: the representatives of the symmetry groups, or r % n_theta for a rows3d model
-    if (reps && !h.rows3d) CK(cudaMemcpyAsync(reps, w.reps, sizeof(int) * h.n_reps, cudaMemcpyDeviceToHost, s));
-    if (reps && h.rows3d)
-        for (int r = 0; r < h.n_reps; ++r) reps[r] = r % h.n_theta;
     if (t_rows) CK(cudaMemcpyAsync(t_rows, w.t_rows, sizeof(double) * nc, cudaMemcpyDeviceToHost, s));
     if (inj_idx) CK(cudaMemcpyAsync(inj_idx, w.inj_idx, sizeof(int) * h.n_reps, cudaMemcpyDeviceToHost, s));
-    std::vector<double> th_host(h.n_theta);
-    std::vector<int> reps_host(h.n_reps);
-    CK(cudaMemcpyAsync(th_host.data(), w.theta, sizeof(double) * h.n_theta, cudaMemcpyDeviceToHost, s));
-    if (!h.rows3d) CK(cudaMemcpyAsync(reps_host.data(), w.reps, sizeof(int) * h.n_reps, cudaMemcpyDeviceToHost, s));
-    if (h.rows3d)
-        for (int r = 0; r < h.n_reps; ++r) reps_host[r] = r % h.n_theta;
     auto dump = [&](double* const* pl, double* o) -> int {
         const int map[7] = {0, 1, -1, 2, 3, 4, 5};
         for (int a = 0; a < 7; ++a)
@@ -1726,9 +1669,13 @@ int vag_details(vag_context* ctx, const vag_params* p, double t_min, double t_ma
     if (rvs_shock && p->has_rvs)
         if (int rc = dump(w.rvs, rvs_shock)) return rc;
     CK(cudaStreamSynchronize(s));
+    if (h.rows3d)
+        for (int r = 0; r < h.n_reps; ++r) rep[r] = r % h.n_theta;
+    if (theta) std::copy(th.begin(), th.end(), theta);
+    if (reps) std::copy(rep.begin(), rep.end(), reps);
     auto fill_theta = [&](double* o) {
         for (int r = 0; r < h.n_reps; ++r)
-            for (int k = 0; k < h.n_t; ++k) o[(2 * (size_t)h.n_reps + r) * h.n_t + k] = th_host[reps_host[r]];
+            for (int k = 0; k < h.n_t; ++k) o[(2 * (size_t)h.n_reps + r) * h.n_t + k] = th[rep[r]];
     };
     if (fwd_shock) fill_theta(fwd_shock);
     if (fwd_shock && w.sh_theta) {  // spreading model: Shock::theta varies along k
@@ -1741,25 +1688,10 @@ int vag_details(vag_context* ctx, const vag_params* p, double t_min, double t_ma
 
 int vag_details_photons(vag_context* ctx, const vag_params* p, double t_min, double t_max, double* fwd, double* rvs) {
     if (!ctx || !p || !fwd) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (int rc = vag_params_validate(p)) return rc;
-    CK(cudaSetDevice(ctx->device));
-    int ct, cp;
-    caps_for(p, 1, ct, cp);
-    ctx->cap_theta = ct;
-    ctx->cap_phi = cp;
-    cudaStream_t s = ctx->stream;
-    CK(ctx->io_params.ensure(sizeof(vag_params)));
-    CK(ctx->io_t.ensure(sizeof(double) * 2));
-    const double tt[2] = {t_min, t_max};
-    CK(cudaMemcpyAsync(ctx->io_params.p, p, sizeof(vag_params), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_t.p, tt, sizeof(tt), cudaMemcpyHostToDevice, s));
     BatchWs w;
-    int totals[TOT_N];
     long long cells = 0;
-    ctx->launches = 0;
-    if (int rc = run_front(ctx, w, static_cast<vag_params*>(ctx->io_params.p), 1, static_cast<double*>(ctx->io_t.p), 2,
-                           s, totals, &cells))
-        return rc;
+    if (int rc = details_front(ctx, p, t_min, t_max, w, &cells)) return rc;
+    cudaStream_t s = ctx->stream;
     const int planes[6] = {PH_LOG2_NU_M, PH_LOG2_NU_C, PH_LOG2_NU_A, PH_LOG2_NU_M_MAX, PH_LOG2_I_MAX, PH_INV_NU_M_MAX};
     const size_t nc = (size_t)cells;
     for (int a = 0; a < 6; ++a) {
@@ -1774,25 +1706,10 @@ int vag_details_photons(vag_context* ctx, const vag_params* p, double t_min, dou
 // Electron / inverse-Compton bookkeeping of the shocks with ssc=True (after KN_cooling / Thomson_cooling), per unique cell
 int vag_details_ic(vag_context* ctx, const vag_params* p, double t_min, double t_max, double* fwd, double* rvs) {
     if (!ctx || !p || !fwd) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (int rc = vag_params_validate(p)) return rc;
-    CK(cudaSetDevice(ctx->device));
-    int ct, cp;
-    caps_for(p, 1, ct, cp);
-    ctx->cap_theta = ct;
-    ctx->cap_phi = cp;
-    cudaStream_t s = ctx->stream;
-    CK(ctx->io_params.ensure(sizeof(vag_params)));
-    CK(ctx->io_t.ensure(sizeof(double) * 2));
-    const double tt[2] = {t_min, t_max};
-    CK(cudaMemcpyAsync(ctx->io_params.p, p, sizeof(vag_params), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->io_t.p, tt, sizeof(tt), cudaMemcpyHostToDevice, s));
     BatchWs w;
-    int totals[TOT_N];
     long long cells = 0;
-    ctx->launches = 0;
-    if (int rc = run_front(ctx, w, static_cast<vag_params*>(ctx->io_params.p), 1, static_cast<double*>(ctx->io_t.p), 2,
-                           s, totals, &cells))
-        return rc;
+    if (int rc = details_front(ctx, p, t_min, t_max, w, &cells)) return rc;
+    cudaStream_t s = ctx->stream;
     const size_t nc = (size_t)cells;
     CK(ctx->io_out.ensure(sizeof(double) * VAG_IC_DETAIL_PLANES * std::max<size_t>(nc, 1)));
     double* d_out = static_cast<double*>(ctx->io_out.p);

@@ -9,7 +9,7 @@
 // the per-node log2-luminosities, and never written to HBM.
 //
 // The work of one CTA is expressed as barrier-separated phases, each an HD function of the
-// thread index, so the same code runs as a CUDA block (vag_kernels.cu) and as a sequential
+// thread index, so the same code runs as a CUDA block (vag_b200.cu) and as a sequential
 // host emulation in the CPU test-suite (oracle/hostemu).
 #pragma once
 

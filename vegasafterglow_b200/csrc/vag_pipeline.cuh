@@ -497,4 +497,35 @@ VAG_HD double chi2_term(double lnF_obs, double F_model, double sigma_ln, double 
     return wgt * d * d;
 }
 
+// ---- host only: batch planning shared by vag_b200.cu and the host emulation (oracle/hostemu/hostemu.cpp) -----
+struct Caps {
+    int theta, phi;
+};
+
+// capacity planning from host-side parameters (upper bounds of auto_grid's node counts,
+// src/core/grid-refinement.h:246-262,655,664-677)
+inline Caps caps_for(const vag_params* p, size_t n) {
+    Caps c{64, 8};
+    for (size_t i = 0; i < n; ++i) {
+        const bool r = p[i].has_rvs != 0;
+        const double th_res = p[i].theta_resol > 0 ? p[i].theta_resol : (r ? 0.2 : 0.15);
+        const double ph_res = p[i].phi_resol > 0 ? p[i].phi_resol : 0.06;
+        const double lg = std::log10(std::max(1.0, std::max(p[i].Gamma0, p[i].Gamma0_w) * 1.5708));
+        const int ct = 36 + (int)(90 * th_res) + (int)(std::max(0.0, lg - 1) * th_res * 55) + (int)(lg * th_res * 25) + 64;
+        const int cp = std::max((int)(360 * ph_res), 1) * 5 + 8;
+        c.theta = std::max(c.theta, ct);
+        c.phi = std::max(c.phi, cp);
+    }
+    return c;
+}
+
+// Banded series: the boundary luminosities of every (node, band) are staged once per row instead of two spectra per
+// (point, row): n_bands * n_t tile evaluations against 2 * n_points per-point ones.  Measured on the config-5 batch
+// (5 bands, ~100-node lattices, scripts/series_ab.py): 3.18 ms banded, flat in the number of points, against 1.97 ms
+// per 100 points -- the break-even is n_bands * n_t ~ 3 n_points.  n_bands: distinct frequencies of the request (0
+// when not banded at all), max_n_t: longest time lattice of the batch, series_mode as vag_set_series_mode.
+inline bool series_banded(int n_bands, int max_n_t, size_t n_points, int series_mode) {
+    return n_bands >= 1 && n_bands <= EATS_NU_TILE && (series_mode == 2 || (size_t)n_bands * max_n_t <= 3 * n_points);
+}
+
 }  // namespace vag
