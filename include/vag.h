@@ -180,6 +180,15 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
              const double* lnF_obs, const double* sigma_ln, const double* w, size_t n_points, const vag_band_obs* bands,
              size_t n_bands, double* chi2, int32_t* status);
 
+/* vag_chi2 with host-galaxy extinction fitted per model (Fitter with an extinction law, fitter.py:512-519): the point
+ * term compares model m with lnF_obs[i] + A_V[m] * ext_k[i] (product rounded, then sum) instead of lnF_obs[i]; band
+ * terms are unchanged.  ext_k[n_points] is in the order of the points (time-sorted) and must be finite; A_V[n_models]
+ * is not range-checked (a non-finite A_V gives chi2 = +inf).  ext_k and A_V are both NULL (exactly vag_chi2) or both
+ * set, and then n_points > 0.  Same launches as vag_chi2 on the same data. */
+int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
+                 const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
+                 const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status);
+
 /* ok[i] = 1 where vag_params_validate accepts params[i], else 0 (no error is raised for rejected sets). */
 int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok);
 

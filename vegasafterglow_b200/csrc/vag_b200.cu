@@ -475,15 +475,24 @@ __global__ void k_total(double* out, size_t n_models, size_t comp_sz) {
 // A model whose ODE exhausted Boost's 500 consecutive step rejections is an exception in the reference
 // (max_step_checker.hpp:99-106) that the samplers turn into logL = -inf (samplers.py:63-70): chi2 = +inf here.
 // accumulate: add to chi2[] (band terms after the point term, fitter.py:525-531).
+// ext (per point) with av (per model): host extinction F e^{-A_V k} shifts the observed value to lnF + A_V k.  The
+// explicit intrinsics round the product, then the sum, as numpy does; a contracted FMA would differ in the last bit.
 __global__ void k_chi2(const double* __restrict__ flux, size_t n_models, int n, const double* __restrict__ lnF,
-                       const double* __restrict__ sigma_ln, const double* __restrict__ wgt, double* chi2,
+                       const double* __restrict__ sigma_ln, const double* __restrict__ wgt,
+                       const double* __restrict__ av, const double* __restrict__ ext, double* chi2,
                        const int* __restrict__ status, int accumulate) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= (int)n_models) return;
     const double* F = flux + (size_t)warp * VAG_NCOMP * n;  // total
     double s = 0;
-    for (int i = lane; i < n; i += 32) s += chi2_term(lnF[i], F[i], sigma_ln[i], wgt[i]);
+    if (ext) {
+        const double a = av[warp];
+        for (int i = lane; i < n; i += 32)
+            s += chi2_term(__dadd_rn(lnF[i], __dmul_rn(a, ext[i])), F[i], sigma_ln[i], wgt[i]);
+    } else {
+        for (int i = lane; i < n; i += 32) s += chi2_term(lnF[i], F[i], sigma_ln[i], wgt[i]);
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     if (lane == 0) {
@@ -658,6 +667,8 @@ struct Request {
     size_t n_t, n_nu;
     bool nu_code_units = false;
     const double *d_lnF = nullptr, *d_sig = nullptr, *d_w = nullptr;  // [n_t] observations of a chi-squared series
+    const double* d_ext = nullptr;  // [n_t] extinction per point, or NULL
+    const double* d_av = nullptr;   // [n_models] A_V per model of the batch, set with d_ext (run_flux offsets it per pass)
 };
 
 int setup_models(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps) {
@@ -985,7 +996,7 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
     }
     if (d_chi2) {
         k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
-                                                                 d_chi2, w.status, 0);
+                                                                 rq_in.d_av, rq_in.d_ext, d_chi2, w.status, 0);
         ctx->launches++;
     }
     mark(ctx, 5, s);
@@ -1008,7 +1019,9 @@ int run_flux(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, 
     const size_t comp_sz = rq.series ? rq.n_t : rq.n_nu * rq.n_t;
     for (size_t lo = 0; lo < n; lo += MAX_MODELS_PER_PASS) {
         const size_t m = std::min(MAX_MODELS_PER_PASS, n - lo);
-        if (int rc = run_flux_pass(ctx, d_params + lo, m, caps, rq, d_out + lo * VAG_NCOMP * comp_sz,
+        Request rq_pass = rq;
+        if (rq.d_av) rq_pass.d_av = rq.d_av + lo;
+        if (int rc = run_flux_pass(ctx, d_params + lo, m, caps, rq_pass, d_out + lo * VAG_NCOMP * comp_sz,
                                    d_status ? d_status + lo : nullptr, d_chi2 ? d_chi2 + lo : nullptr, s))
             return rc;
     }
@@ -1516,13 +1529,19 @@ int vag_flux_band(vag_context* ctx, const vag_params* params, size_t n_models, c
 
 // Replaces Fitter._evaluate (VegasAfterglow/fitting/fitter.py:503-533) for a batch of parameter sets: the chi-squared of the
 // point data (flux_density series) plus one term per band-integrated data set (Model.flux), all in ln-flux space.
-int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
-             const double* lnF_obs, const double* sigma_ln, const double* w, size_t n_points, const vag_band_obs* bands,
-             size_t n_bands, double* chi2, int32_t* status) {
+// With ext_k / A_V, the observed ln-flux of point i for model m is lnF_obs[i] + A_V[m] ext_k[i] (host extinction).
+int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
+                 const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
+                 const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status) {
     if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
     if (n_points && (!t || !nu || !lnF_obs || !sigma_ln || !w)) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL");
     if (n_bands && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
     if (n_points == 0 && n_bands == 0) return fail(VAG_ERR_INVALID, "no data: n_points and n_bands are both 0");
+    const bool ext = ext_k != nullptr;
+    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (ext && n_points == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points > 0)");
+    for (size_t i = 0; ext && i < n_points; ++i)
+        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
     // every band is checked before any work is enqueued
     std::vector<BandGrid> grids(n_bands);
     size_t max_obs = n_points;
@@ -1539,13 +1558,17 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
         if (int rc = prepare_request(ctx, t, n_points, nu, n_points)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
-    // observation staging: chi2 [n_models], lnF / sigma_ln / w [max_obs] of the term in flight, status OR [n_models]
-    CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * max_obs) + sizeof(int32_t) * n_models));
+    // observation staging: chi2 [n_models], lnF / sigma_ln / w [max_obs] of the term in flight, with extinction ext_k
+    // [n_points] and A_V [n_models], status OR [n_models]
+    const size_t n_ext = ext ? n_points + n_models : 0;
+    CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * max_obs + n_ext) + sizeof(int32_t) * n_models));
     double* d_chi2 = static_cast<double*>(ctx->io_obs.p);
     double* d_lnF = d_chi2 + n_models;
     double* d_sig = d_lnF + max_obs;
     double* d_w = d_sig + max_obs;
-    int32_t* d_stat_or = reinterpret_cast<int32_t*>(d_w + max_obs);
+    double* d_ext = d_w + max_obs;
+    double* d_av = d_ext + n_points;
+    int32_t* d_stat_or = reinterpret_cast<int32_t*>(d_w + max_obs + n_ext);
     int32_t* d_status = static_cast<int32_t*>(ctx->io_status.p);
     auto upload = [&](const double* a, const double* b_, const double* c, size_t n) -> int {
         CK(cudaMemcpyAsync(d_lnF, a, sizeof(double) * n, cudaMemcpyHostToDevice, s));
@@ -1565,6 +1588,12 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
         rq.d_lnF = d_lnF;
         rq.d_sig = d_sig;
         rq.d_w = d_w;
+        if (ext) {
+            CK(cudaMemcpyAsync(d_ext, ext_k, sizeof(double) * n_points, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(d_av, A_V, sizeof(double) * n_models, cudaMemcpyHostToDevice, s));
+            rq.d_ext = d_ext;
+            rq.d_av = d_av;
+        }
         if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq,
                               static_cast<double*>(ctx->io_out.p), d_status, d_chi2, s))
             return rc;
@@ -1582,7 +1611,7 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
         double* d_band = nullptr;
         if (int rc = run_band(ctx, n_models, caps, B.n, grids[b], &d_band, s)) return rc;
         if (int rc = upload(B.lnF_obs, B.sigma_ln, B.w, B.n)) return rc;
-        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, d_lnF, d_sig, d_w, d_chi2, d_status, 1);
+        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, d_lnF, d_sig, d_w, nullptr, nullptr, d_chi2, d_status, 1);
         k_or_status<<<og, 256, 0, s>>>(d_stat_or, d_status, n_models);
         launches += ctx->launches + 2;
     }
@@ -1593,6 +1622,13 @@ int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const 
         CK(cudaMemcpyAsync(status, or_status ? d_stat_or : d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
+}
+
+int vag_chi2(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
+             const double* lnF_obs, const double* sigma_ln, const double* w, size_t n_points, const vag_band_obs* bands,
+             size_t n_bands, double* chi2, int32_t* status) {
+    return vag_chi2_ext(ctx, params, n_models, t, nu, lnF_obs, sigma_ln, w, nullptr, n_points, nullptr, bands, n_bands,
+                        chi2, status);
 }
 
 // per-parameter-set validation of a batch: ok[i] = 1 where vag_params_validate accepts params[i] (a sampler masks the

@@ -110,11 +110,13 @@ class Engine:
                                              chi2.ctypes.data, st.ctypes.data))
         return (chi2, st) if return_status else chi2
 
-    def chi2(self, params, points=None, bands=(), return_status=False):
+    def chi2(self, params, points=None, bands=(), return_status=False, extinction=None):
         """Batched ``Fitter._evaluate`` (fitter.py:503-533) -> chi2[n_models]: the point-data term (``points`` =
         (t, nu, lnF_obs, sigma_ln, w), times ascending, or None) plus one term per band-integrated data set
         (``bands``: dicts with t, lnF_obs, sigma_ln, w, nu_min, nu_max, num_nu -- ``Model.flux`` on each).
-        +inf where the sum is not finite or the model's ODE failed (include/vag.h vag_chi2)."""
+        ``extinction`` = (ext_k[n_points], A_V[n_models]): a fitted host extinction, which compares model m's point
+        fluxes with lnF_obs + A_V[m] * ext_k (band terms unchanged).
+        +inf where the sum is not finite or the model's ODE failed (include/vag.h vag_chi2, vag_chi2_ext)."""
         p = self._params(params)
         keep = []  # the arrays must outlive the call
         if points is not None:
@@ -124,6 +126,15 @@ class Engine:
             n_pt = pt[0].size
         else:
             pt, n_pt = [np.zeros(0)] * 5, 0
+        ext = av = None
+        if extinction is not None:
+            if points is None:
+                raise ValueError("extinction shifts the point data: it needs points")
+            ext, av = (_f64(a).reshape(-1) for a in extinction)
+            if ext.size != n_pt:
+                raise ValueError(f"ext_k has {ext.size} values for {n_pt} points")
+            if av.size != p.size:
+                raise ValueError(f"A_V has {av.size} values for {p.size} models")
         arr = (abi.BandObs * max(len(bands), 1))()
         for i, b in enumerate(bands):
             cols = [_f64(b[k]).reshape(-1) for k in ("t", "lnF_obs", "sigma_ln", "w")]
@@ -134,9 +145,11 @@ class Engine:
                                  cols[0].size, float(b["nu_min"]), float(b["nu_max"]), int(b["num_nu"]))
         out = np.empty(p.size)
         st = np.zeros(p.size, dtype=np.int32)
-        _lib.check(self._lib.vag_chi2(self._h, p.ctypes.data, p.size, *[a.ctypes.data if n_pt else None for a in pt], n_pt,
-                                      C.cast(arr, C.c_void_p) if len(bands) else None, len(bands), out.ctypes.data,
-                                      st.ctypes.data))
+        _lib.check(self._lib.vag_chi2_ext(self._h, p.ctypes.data, p.size, *[a.ctypes.data if n_pt else None for a in pt],
+                                          None if ext is None else ext.ctypes.data, n_pt,
+                                          None if av is None else av.ctypes.data,
+                                          C.cast(arr, C.c_void_p) if len(bands) else None, len(bands), out.ctypes.data,
+                                          st.ctypes.data))
         return (out, st) if return_status else out
 
     @staticmethod

@@ -29,13 +29,18 @@ _FIELDS = {
 }
 
 
+def time_order(t):
+    """The stable time sort of the point data (fitter.py:407-437); per-point columns follow it."""
+    return np.argsort(np.asarray(t, dtype=np.float64).reshape(-1), kind="stable")
+
+
 def consolidate_data(t, nu, flux, err, weights=None):
     """fitter.py:407-437: sort by time, normalise weights to sum N, ln-flux and relative error."""
     t, nu, flux, err = (np.asarray(a, dtype=np.float64).reshape(-1) for a in (t, nu, flux, err))
     w = np.ones_like(t) if weights is None else np.asarray(weights, dtype=np.float64).reshape(-1)
     if np.any(flux <= 0) or np.any(err <= 0):
         raise ValueError("flux and err must be positive")
-    order = np.argsort(t, kind="stable")
+    order = time_order(t)
     t, nu, flux, err, w = t[order], nu[order], flux[order], err[order], w[order]
     if w.sum() > 0:
         w = w * (len(w) / w.sum())
@@ -60,22 +65,35 @@ class BatchedLikelihood:
     names / log_scale describe the sampler-space columns (log10 parameters are exponentiated like
     ``_build_transformer``, fitting/utils.py:110-135); ``template`` is a 1-record ``vag_params``
     array carrying every fixed setting (jet/medium type, distance, redshift, switches).
+
+    A name ``"A_V"`` fits host-galaxy extinction: ``ext_kernel`` (per point, in the caller's order) is the
+    extinction law at each point, and a sample's point data are compared as ln F_obs + A_V * ext_kernel
+    (``Engine.chi2(extinction=...)``).  Band data are not shifted.
     """
 
     def __init__(self, engine, template, names: Sequence[str], log_scale: Sequence[bool], t, nu, flux, err,
                  weights=None, lower=None, upper=None, log_prior: Optional[Callable] = None,
-                 log_likelihood_fn: Callable = lambda chi2: -0.5 * chi2, distributed: bool = False, bands=()):
+                 log_likelihood_fn: Callable = lambda chi2: -0.5 * chi2, distributed: bool = False, bands=(),
+                 ext_kernel=None):
         self.engine = engine
         self.template = np.ascontiguousarray(template, dtype=abi.PARAMS_DTYPE).reshape(-1)[:1].copy()
         self.names = list(names)
         self.log_scale = np.asarray(log_scale, dtype=bool)
         for n in self.names:
-            if n not in _FIELDS:
-                raise ValueError(f"unknown parameter '{n}' (supported: {sorted(_FIELDS)})")
+            if n not in _FIELDS and n != "A_V":
+                raise ValueError(f"unknown parameter '{n}' (supported: {sorted(_FIELDS)} and A_V)")
+        if "A_V" in self.names and ext_kernel is None:
+            raise ValueError("fitting A_V needs ext_kernel, the extinction law at each point")
         if len(np.atleast_1d(t)):
             self.t, self.nu, self.lnF, self.sig, self.w = consolidate_data(t, nu, flux, err, weights)
         else:
             self.t = self.nu = self.lnF = self.sig = self.w = np.zeros(0)
+        self.ext_kernel = None
+        if ext_kernel is not None:
+            ext = np.asarray(ext_kernel, dtype=np.float64).reshape(-1)
+            if ext.size != self.t.size:
+                raise ValueError(f"ext_kernel has {ext.size} values for {self.t.size} points")
+            self.ext_kernel = ext[time_order(t)]
         # band-integrated data sets (Fitter.add_flux -> BandObs; fitter.py:525-531 evaluates Model.flux on each)
         self.bands = [band_obs(**b) for b in bands]
         if not self.t.size and not self.bands:
@@ -90,7 +108,9 @@ class BatchedLikelihood:
         samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
         P = np.repeat(self.template, samples.shape[0])
         for i, name in enumerate(self.names):
-            col = 10.0 ** samples[:, i] if self.log_scale[i] else samples[:, i]
+            if name == "A_V":  # not a model parameter: it shifts the observed point data (_evaluate)
+                continue
+            col = self._column(samples, i)
             path = _FIELDS[name]
             if len(path) == 1:
                 P[path[0]] = col
@@ -98,10 +118,15 @@ class BatchedLikelihood:
                 P[path[0]][path[1]] = col
         return P
 
-    def _evaluate(self, P: np.ndarray) -> np.ndarray:
-        if not self.bands:
-            return self.engine.chi2_series(P, self.t, self.nu, self.lnF, self.sig, self.w)
+    def _column(self, samples, i):
+        return 10.0 ** samples[:, i] if self.log_scale[i] else samples[:, i]
+
+    def _evaluate(self, P: np.ndarray, A_V=None) -> np.ndarray:
         pts = (self.t, self.nu, self.lnF, self.sig, self.w) if self.t.size else None
+        if A_V is not None:
+            return self.engine.chi2(P, pts, self.bands, extinction=(self.ext_kernel, A_V))
+        if not self.bands:
+            return self.engine.chi2_series(P, *pts)
         return self.engine.chi2(P, pts, self.bands)
 
     def chi2(self, samples: np.ndarray) -> np.ndarray:
@@ -110,17 +135,20 @@ class BatchedLikelihood:
         rank, BEFORE the ensemble is split: a rejected walker can therefore never desynchronise the collective."""
         from .engine import Engine
 
+        samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
         P = self.to_params(samples)
         ok = Engine.valid_mask(P)
+        # a fitted A_V shifts the point data; without point data there is nothing to shift
+        per_walker = (self._column(samples, self.names.index("A_V")),) if "A_V" in self.names and self.t.size else ()
         if self.distributed:
             from . import parallel
 
             tt = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
             return parallel.partitioned_chi2(self.engine, P, tt, self.nu, self.lnF, self.sig, self.w, evaluate=self._evaluate,
-                                             valid=ok)
+                                             valid=ok, per_walker=per_walker)
         out = np.full(P.size, np.inf)
         if ok.any():
-            out[ok] = self._evaluate(P[ok])
+            out[ok] = self._evaluate(P[ok], *(a[ok] for a in per_walker))
         return out
 
     def __call__(self, samples: np.ndarray) -> np.ndarray:

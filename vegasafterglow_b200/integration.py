@@ -4,8 +4,9 @@ replaces the thread pool of ``fit_emcee`` / ``fit_bilby`` (fitting/samplers.py:3
 The reference evaluates one walker per host thread: ``pool.map(eval_one, valid_samples)`` builds a ``Model`` per walker
 (``Fitter._build_model``, fitter.py:455-495) and sums its chi-squared (``Fitter._evaluate``, :503-533).  Here the same
 ``Fitter`` object -- its data, configuration flags and parameter transformer are used as they are -- is evaluated for a
-whole ensemble in ONE call of the C ABI (``vag_chi2``): point data + band-integrated data, on one GPU or partitioned by
-walker over the GPUs of the box (vegasafterglow_b200/parallel.py).
+whole ensemble in ONE call of the C ABI (``vag_chi2``, or ``vag_chi2_ext`` with a built-in extinction law and a per-walker
+``A_V``): point data + band-integrated data, on one GPU or partitioned by walker over the GPUs of the box
+(vegasafterglow_b200/parallel.py).
 
 * ``params_from_fitter(fitter, model_params)``   ModelParams namespaces -> ``vag_params`` records (what ``_build_model`` +
                                                  the default jet / medium factories, fitting/utils.py:31-70, construct)
@@ -98,8 +99,10 @@ class GpuFitterEvaluator:
         self.points = ((fitter._all_t, fitter._all_nu, fitter._all_log_flux, fitter._all_log_err, fitter._all_weights)
                        if self.has_points else None)
         self.bands = [band_obs(bd.t, bd.flux, bd.err, bd.nu_min, bd.nu_max, bd.num_points, bd.weights) for bd in fitter._band_obs]
-        # built-in host extinction: F -> F exp(-A_V k(lambda)) is a shift of ln F_obs per point (fitter.py:512-519)
-        self.ext_kernel = fitter._ext_kernel if fitter._ext_law is not None else None
+        # built-in host extinction: F -> F exp(-A_V k(lambda)) is a shift of ln F_obs per point (fitter.py:512-519),
+        # ln F_obs - ln(F e^{-A_V k}) = (ln F_obs + A_V k) - ln F, with a walker-dependent A_V.  Without point data
+        # there is nothing to shift.
+        self.ext_kernel = fitter._ext_kernel if fitter._ext_law is not None and self.has_points else None
 
     def chi2(self, thetas: np.ndarray) -> np.ndarray:
         thetas = np.atleast_2d(np.asarray(thetas, dtype=np.float64))
@@ -108,32 +111,26 @@ class GpuFitterEvaluator:
         from .engine import Engine
 
         ok = Engine.valid_mask(P)
-        A_V = np.array([getattr(p, "A_V", 0.0) for p in mp])
-        if self.ext_kernel is not None and np.any(A_V != 0.0):
-            # extinction makes the observed ln-flux walker dependent: ln F_obs - ln(F e^{-A_V k}) = (ln F_obs + A_V k) - ln F.
-            # Walkers are grouped by A_V (a fitted A_V gives one group per walker: the point term then runs per walker)
-            out = np.full(len(mp), np.inf)
-            for av in np.unique(A_V):
-                sel = ok & (A_V == av)
-                if sel.any():
-                    pts = (self.points[0], self.points[1], self.points[2] + av * self.ext_kernel, self.points[3], self.points[4])
-                    out[sel] = self._run(P[sel], pts)
-            return out
+        per_walker = ()
+        if self.ext_kernel is not None:
+            per_walker = (np.array([getattr(p, "A_V", 0.0) for p in mp], dtype=np.float64),)
         out = np.full(len(mp), np.inf)
         if ok.any():
             if self.distributed:
                 from . import parallel
 
                 tt = self.points[0] if self.has_points else self.bands[0]["t"]
-                return parallel.partitioned_chi2(self.engine, P, tt, None, None, None, None,
-                                                 evaluate=lambda B: self._run(B, self.points), valid=ok)
-            out[ok] = self._run(P[ok], self.points)
+                return parallel.partitioned_chi2(self.engine, P, tt, None, None, None, None, evaluate=self._run, valid=ok,
+                                                 per_walker=per_walker)
+            out[ok] = self._run(P[ok], *(a[ok] for a in per_walker))
         return out
 
-    def _run(self, P, pts):
+    def _run(self, P, A_V=None):
+        if A_V is not None:
+            return self.engine.chi2(P, self.points, self.bands, extinction=(self.ext_kernel, A_V))
         if not self.bands:
-            return self.engine.chi2_series(P, *pts)
-        return self.engine.chi2(P, pts, self.bands)
+            return self.engine.chi2_series(P, *self.points)
+        return self.engine.chi2(P, self.points, self.bands)
 
     def log_likelihoods(self, thetas, log_likelihood_fn: Callable) -> np.ndarray:
         chi2 = self.chi2(thetas)

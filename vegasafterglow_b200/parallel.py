@@ -102,7 +102,8 @@ def gather_indexed(local: np.ndarray, sets, n: int, device=None) -> np.ndarray:
     return out
 
 
-def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=True, valid=None) -> np.ndarray:
+def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=True, valid=None,
+                     per_walker=None) -> np.ndarray:
     """chi2 of the whole ensemble, each rank evaluating its share on its own GPU; ONE all-gather of float64[~n / world].
 
     * ``valid`` (bool[n], computed identically on every rank -- ``Engine.valid_mask`` is pure host code): walkers the
@@ -110,7 +111,9 @@ def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=
       shape whatever its own block contains (the reference maps that exception to logL = -inf, samplers.py:63-70);
     * ``balance``: split by the cost proxy (mixed tophat / structured ensembles) instead of contiguous blocks;
     * ``evaluate(params_block) -> chi2_block`` defaults to ``engine.chi2_series``; the CPU tests pass a host evaluator
-      to exercise the partition / gather logic under gloo."""
+      to exercise the partition / gather logic under gloo;
+    * ``per_walker``: a tuple of length-n arrays (e.g. a fitted A_V), sliced with the rank's walkers like ``params``
+      and passed to ``evaluate`` as extra arguments."""
     import torch.distributed as dist
 
     n = len(params)
@@ -126,5 +129,6 @@ def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=
     if evaluate is None:
         evaluate = lambda P: engine.chi2_series(P, t, nu, lnF, sig, w)  # noqa: E731
     mine = sets[rank]
-    local = evaluate(params[mine]) if len(mine) else np.zeros(0)
+    extra = [np.asarray(a)[mine] for a in per_walker or ()]
+    local = evaluate(params[mine], *extra) if len(mine) else np.zeros(0)
     return gather_indexed(local, sets, n)
