@@ -56,8 +56,10 @@ enum {
     VAG_ST_ODE_FAIL500 = 4,   /* boost max_step_checker.hpp:99-106 (reference throws)            */
     VAG_ST_GRID_NONFINITE = 8, /* grid-refinement.h:633-635                                      */
     VAG_ST_CAPACITY = 16,     /* grid / SSC lattice larger than compiled capacity; model output is NaN */
-    VAG_ST_IC_BAND = 32       /* an SSC query left the clamped output band (inverse-compton.h:622-635:
+    VAG_ST_IC_BAND = 32,      /* an SSC query left the clamped output band (inverse-compton.h:622-635:
                                  the reference would rebuild that cell's full-range spectrum)      */
+    VAG_ST_INVALID = 64       /* the entry points that plan on the device (vag_chi2_dev, vag_flux_band_dev): the
+                                 reference constructors reject this parameter set; flux NaN, chi2 +inf */
 };
 
 /* Radiation(eps_e, eps_B, p, xi_e=1, ssc=False, kn=False): pybind/pymodel.h:303-313 */
@@ -199,7 +201,9 @@ int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok);
  * cudaStream_t passed as void* (NULL = the context's own stream).  The calls are stream-ordered;
  * they synchronise the stream once internally (to size the ragged workspace after the grid
  * kernel) and return with the remaining kernels enqueued: call vag_synchronize / sync the stream
- * before reading the outputs.  t must be ascending (not checked on the device path). */
+ * before reading the outputs.  t must be ascending (not checked on the device path).
+ * vag_chi2_dev and vag_flux_band_dev below also plan on the device, which synchronises the stream
+ * once more, before the grid kernel. */
 int vag_flux_density_grid_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t,
                               size_t n_t, const double* d_nu, size_t n_nu, double* d_out, int32_t* d_status,
                               void* stream);
@@ -214,6 +218,34 @@ int vag_synchronize(vag_context* ctx);
  * points derive tight capacities from the parameters themselves.  A model that needs more nodes
  * than the capacity gets VAG_ST_CAPACITY and NaN output. */
 int vag_set_capacity(vag_context* ctx, int cap_theta, int cap_phi);
+
+/* ------------------------------------------------------------------------------------------- */
+/* DEVICE buffers, planned on the device: the likelihood of a sampler whose walkers stay in HBM  */
+/* ------------------------------------------------------------------------------------------- */
+/* Device counterpart of vag_params_validate_batch: d_ok[i] = 1 where vag_params_validate accepts d_params[i], else 0,
+ * and caps = {theta, phi} node capacities the accepted records need (the host path's capacities for them).  One kernel;
+ * synchronises `stream` to return caps. */
+int vag_params_validate_batch_dev(vag_context* ctx, const vag_params* d_params, size_t n, int32_t* d_ok, int caps[2],
+                                  void* stream);
+
+/* vag_flux_band and vag_chi2_ext on device buffers, each parameter set checked on the device as vag_params_validate
+ * checks it, and the grids sized from the parameters as the host-buffer entry points size them (not by
+ * vag_set_capacity).  A rejected set runs as a fixed valid stand-in (an on-axis tophat in ISM) and its results are then
+ * overwritten: status VAG_ST_INVALID, flux NaN, chi2 +inf -- the reference raises there, and its samplers map that to
+ * logL = -inf (samplers.py:63-70).  The stand-ins are members of the batch: series mode 0 (vag_set_series_mode) sees
+ * their lattices too.  Planning is one extra kernel before and one after the call's work, and one D2H of two ints with
+ * one more synchronisation of `stream`, before the grid kernel: the capacities size the workspaces on the host.
+ * Not checked on the device path: the time order of d_t and of every band's t, and the finiteness of d_ext_k.
+ * vag_flux_band_dev: d_out[n_models][VAG_NCOMP][n_t]; the band's frequency nodes and weights are made on the host.
+ * vag_chi2_dev: the terms and rules of vag_chi2_ext (ext_k / A_V both NULL or both set, and then n_points > 0; at least
+ * one term; status OR over terms only with band terms); `bands` is a host array whose t / lnF_obs / sigma_ln / w are
+ * device pointers. */
+int vag_flux_band_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t, size_t n_t,
+                      double nu_min, double nu_max, size_t num_nu, double* d_out, int32_t* d_status, void* stream);
+int vag_chi2_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t, const double* d_nu,
+                 const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k, size_t n_points,
+                 const double* d_A_V, const vag_band_obs* bands, size_t n_bands, double* d_chi2, int32_t* d_status,
+                 void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* introspection (tests, profiling): stage tables of ONE model, the analogue of                 */

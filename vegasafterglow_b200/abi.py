@@ -16,6 +16,7 @@ MEDIUM_ISM, MEDIUM_WIND = 0, 1
 NCOMP = 5
 COMPONENTS = ("total", "fwd_sync", "fwd_ssc", "rvs_sync", "rvs_ssc")
 ST_ODE_STEP_CAP, ST_ODE_STALLED, ST_ODE_FAIL500, ST_GRID_NONFINITE, ST_CAPACITY, ST_IC_BAND = 1, 2, 4, 8, 16, 32
+ST_INVALID = 64  # rejected by the parameter checks of the device-planned entry points (vag_chi2_dev, vag_flux_band_dev)
 
 RADIATION_DTYPE = np.dtype(
     [("eps_e", "f8"), ("eps_B", "f8"), ("p", "f8"), ("xi_e", "f8"), ("ssc", "i4"), ("kn", "i4")], align=True

@@ -574,6 +574,43 @@ __global__ void __launch_bounds__(256) k_fp64_peak(double* sink, int iters) {
     if (a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7 == 12345.678) sink[0] = a0;
 }
 
+// Planning of a batch whose parameters are on the device (thread / record): ok[i] = vag_params_validate accepts in[i],
+// caps[0..1] = max over the accepted records' bounds (zeroed by the caller), and, with run, the records that will run:
+// a rejected record is replaced by stand_in, so no kernel downstream meets a set the reference constructors refuse.
+__global__ void __launch_bounds__(256) k_plan(const vag_params* __restrict__ in, size_t n, vag_params stand_in,
+                                              vag_params* __restrict__ run, int32_t* __restrict__ ok, int* caps) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int ct = 0, cp = 0;
+    if (i < n) {
+        const bool good = params_check(in[i]) == PR_OK;
+        ok[i] = good ? 1 : 0;
+        if (good) {
+            const Caps c = caps_of(in[i]);
+            ct = c.theta;
+            cp = c.phi;
+        }
+        if (run) run[i] = good ? in[i] : stand_in;
+    }
+    ct = __reduce_max_sync(0xffffffffu, ct);
+    cp = __reduce_max_sync(0xffffffffu, cp);
+    if ((threadIdx.x & 31) == 0) {
+        atomicMax(caps, ct);
+        atomicMax(caps + 1, cp);
+    }
+}
+
+// After a planned run (block / model): a rejected record ran as the stand-in; its result becomes VAG_ST_INVALID,
+// chi2 = +inf (the reference raises, its samplers give logL = -inf, samplers.py:63-70) and NaN flux.
+__global__ void k_reject(const int32_t* __restrict__ ok, int32_t* status, double* chi2, double* out, size_t per_model) {
+    const size_t mi = blockIdx.x;
+    if (ok[mi]) return;
+    if (threadIdx.x == 0) {
+        if (status) status[mi] = VAG_ST_INVALID;
+        if (chi2) chi2[mi] = kInf;
+    }
+    for (size_t i = threadIdx.x; out && i < per_model; i += blockDim.x) out[mi * per_model + i] = NAN;
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -622,7 +659,9 @@ struct vag_context {
     cudaStream_t stream = nullptr;
     DevBuf model_buf, row_buf, cell_buf, obs_buf, ic_buf, lut_buf, sp_buf, geom_buf, split_buf, work_buf;
     DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs;  // staging of the host-buffer entry points
+    DevBuf plan_buf;                // device planning: the records that run, ok[], capacities
     int* h_totals = nullptr;        // pinned
+    int* h_caps = nullptr;          // pinned: capacities planned on the device
     long long* h_cells = nullptr;   // pinned
     int* h_bands = nullptr;         // pinned: distinct frequencies of the series request in flight
     int series_mode = 0;            // vag_set_series_mode: 0 auto, 1 per-point spectra always, 2 banded whenever possible
@@ -1028,8 +1067,6 @@ int run_flux(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, 
     return VAG_OK;
 }
 
-bool finite_pos(double x) { return std::isfinite(x) && x > 0; }
-
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -1056,70 +1093,45 @@ void vag_params_default(vag_params* p) {
 }
 
 int vag_params_validate(const vag_params* p) {
-    auto bad = [&](const std::string& m) { return fail(VAG_ERR_INVALID, m); };
-    auto rng_oi = [](double v, double lo, double hi) { return std::isfinite(v) && v > lo && v <= hi; };
-    if (p->jet_type < 0 || p->jet_type > 5) return bad("jet_type must be one of VAG_JET_* (0..5)");
-    if (p->medium_type < 0 || p->medium_type > 1) return bad("medium_type must be 0 (ISM) or 1 (wind)");
-    // PyTophatJet / PyGaussianJet / PyPowerLawJet: pybind/pymodel.cpp:47-95
-    if (!rng_oi(p->theta_c, 0.0, con::pi / 2)) return bad("theta_c must be in (0, pi/2]");
-    const bool has_core = p->jet_type != VAG_JET_POWERLAW_WING;
-    const bool has_wing = p->jet_type >= VAG_JET_TWO_COMPONENT;
-    if (has_core && !finite_pos(p->E_iso)) return bad("E_iso must be finite and > 0");
-    if (has_core && !(std::isfinite(p->Gamma0) && p->Gamma0 > 1.0)) return bad("Gamma0 must be > 1");
-    if (!finite_pos(p->duration)) return bad("duration must be finite and > 0");
-    if ((p->jet_type == VAG_JET_POWERLAW || p->jet_type == VAG_JET_STEP_POWERLAW || p->jet_type == VAG_JET_POWERLAW_WING) &&
-        (!finite_pos(p->k_e) || !finite_pos(p->k_g)))
-        return bad("k_e and k_g must be finite and > 0");
-    // PyTwoComponentJet / PyStepPowerLawJet / PyPowerLawWing: pybind/pymodel.cpp:97-146
-    if (has_wing) {
-        if (!finite_pos(p->E_iso_w)) return bad("E_iso_w must be finite and > 0");
-        if (!(std::isfinite(p->Gamma0_w) && p->Gamma0_w > 1.0)) return bad("Gamma0_w must be > 1");
+    static const char* const rad[4] = {"eps_e must be in (0, 1]", "eps_B must be in (0, 1]", "xi_e must be in (0, 1]",
+                                       "p must be > 1"};
+    const int r = params_check(*p);
+    const char* m = nullptr;
+    switch (r) {
+        case PR_OK: return VAG_OK;
+        case PR_JET_TYPE: m = "jet_type must be one of VAG_JET_* (0..5)"; break;
+        case PR_MEDIUM_TYPE: m = "medium_type must be 0 (ISM) or 1 (wind)"; break;
+        case PR_THETA_C: m = "theta_c must be in (0, pi/2]"; break;
+        case PR_E_ISO: m = "E_iso must be finite and > 0"; break;
+        case PR_GAMMA0: m = "Gamma0 must be > 1"; break;
+        case PR_DURATION: m = "duration must be finite and > 0"; break;
+        case PR_K_EG: m = "k_e and k_g must be finite and > 0"; break;
+        case PR_E_ISO_W: m = "E_iso_w must be finite and > 0"; break;
+        case PR_GAMMA0_W: m = "Gamma0_w must be > 1"; break;
+        case PR_THETA_W: m = "theta_w must be in (0, pi/2]"; break;
+        case PR_THETA_W_ORDER:
+            return fail(VAG_ERR_INVALID, "theta_w (wing angle) must be greater than theta_c (core angle), got theta_w=" +
+                                             std::to_string(p->theta_w) + ", theta_c=" + std::to_string(p->theta_c));
+        case PR_SIGMA0: m = "sigma0 must be finite and >= 0"; break;
+        case PR_MAG_L0: m = "L0 must be finite and > 0"; break;
+        case PR_MAG_T0: m = "t0 must be finite and > 0"; break;
+        case PR_MAG_Q: m = "q must be finite and > 0"; break;
+        case PR_MAG_WING: m = "PowerLawWing takes no magnetar (pybind/pybind.cpp:220-223)"; break;
+        case PR_N_ISM: m = "n_ism must be finite and >= 0"; break;
+        case PR_A_STAR: m = "A_star must be finite and > 0"; break;
+        case PR_N0: m = "n0 must be > 0 (or +inf for no floor)"; break;
+        case PR_K_M: m = "k_m must be finite and > 0"; break;
+        case PR_LUMI_DIST: m = "lumi_dist must be finite and > 0"; break;
+        case PR_Z: m = "z must be finite and >= 0"; break;
+        case PR_THETA_OBS: m = "theta_obs must be in [0, pi]"; break;
+        case PR_PHI_OBS: m = "phi_obs must be finite"; break;
+        case PR_RTOL: m = "rtol must be in (0, 1)"; break;
+        case PR_NONFINITE_RES: m = "resolutions and rtol must be finite"; break;
+        default:  // PyRadiation: PR_FWD_* / PR_RVS_*
+            return fail(VAG_ERR_INVALID, std::string(r < PR_RVS_EPS_E ? "fwd_rad." : "rvs_rad.") +
+                                             rad[(r - PR_FWD_EPS_E) % 4]);
     }
-    if (p->jet_type == VAG_JET_TWO_COMPONENT) {
-        if (!rng_oi(p->theta_w, 0.0, con::pi / 2)) return bad("theta_w must be in (0, pi/2]");
-        if (!(p->theta_w > p->theta_c))
-            return bad("theta_w (wing angle) must be greater than theta_c (core angle), got theta_w=" +
-                       std::to_string(p->theta_w) + ", theta_c=" + std::to_string(p->theta_c));
-    }
-    if (!(std::isfinite(p->sigma0) && p->sigma0 >= 0)) return bad("sigma0 must be finite and >= 0");
-    if (p->has_magnetar) {  // PyMagnetar: pybind/pymodel.h:45-49
-        if (!finite_pos(p->magnetar_L0)) return bad("L0 must be finite and > 0");
-        if (!finite_pos(p->magnetar_t0)) return bad("t0 must be finite and > 0");
-        if (!finite_pos(p->magnetar_q)) return bad("q must be finite and > 0");
-        if (p->jet_type == VAG_JET_POWERLAW_WING) return bad("PowerLawWing takes no magnetar (pybind/pybind.cpp:220-223)");
-    }
-    // PyISM / PyWind: pybind/pymodel.cpp:148-186
-    if (p->medium_type == VAG_MEDIUM_ISM) {
-        if (!(std::isfinite(p->n_ism) && p->n_ism >= 0)) return bad("n_ism must be finite and >= 0");
-    } else {
-        if (!finite_pos(p->A_star)) return bad("A_star must be finite and > 0");
-        if (!(std::isfinite(p->n_ism) && p->n_ism >= 0)) return bad("n_ism must be finite and >= 0");
-        if (!(p->n0 > 0)) return bad("n0 must be > 0 (or +inf for no floor)");
-        if (!(std::isfinite(p->wind_k_m))) return bad("k_m must be finite and > 0");
-    }
-    // PyObserver: pybind/pymodel.h:190-204
-    if (!finite_pos(p->lumi_dist)) return bad("lumi_dist must be finite and > 0");
-    if (!(std::isfinite(p->z) && p->z >= 0)) return bad("z must be finite and >= 0");
-    if (!(std::isfinite(p->theta_obs) && p->theta_obs >= 0 && p->theta_obs <= con::pi))
-        return bad("theta_obs must be in [0, pi]");
-    if (!std::isfinite(p->phi_obs)) return bad("phi_obs must be finite");
-    // PyRadiation: pybind/pymodel.h:303-313
-    auto chk_rad = [&](const vag_radiation& r, const char* who) -> int {
-        if (!rng_oi(r.eps_e, 0.0, 1.0)) return bad(std::string(who) + ".eps_e must be in (0, 1]");
-        if (!rng_oi(r.eps_B, 0.0, 1.0)) return bad(std::string(who) + ".eps_B must be in (0, 1]");
-        if (!rng_oi(r.xi_e, 0.0, 1.0)) return bad(std::string(who) + ".xi_e must be in (0, 1]");
-        if (!(std::isfinite(r.p) && r.p > 1.0)) return bad(std::string(who) + ".p must be > 1");
-        return VAG_OK;
-    };
-    if (int rc = chk_rad(p->fwd, "fwd_rad")) return rc;
-    if (p->has_rvs)
-        if (int rc = chk_rad(p->rvs, "rvs_rad")) return rc;
-    // PyModel ctor: pybind/pymodel.h:642-647 (a non-positive value selects the default)
-    if (p->rtol > 0 && !(p->rtol < 1)) return bad("rtol must be in (0, 1)");
-    if (!std::isfinite(p->rtol) || !std::isfinite(p->phi_resol) || !std::isfinite(p->theta_resol) ||
-        !std::isfinite(p->t_resol))
-        return bad("resolutions and rtol must be finite");
-    return VAG_OK;
+    return fail(VAG_ERR_INVALID, m);
 }
 
 int vag_create(int device, vag_context** out) {
@@ -1139,6 +1151,7 @@ int vag_create(int device, vag_context** out) {
     CK(cudaMallocHost(&c->h_totals, sizeof(int) * TOT_N));
     CK(cudaMallocHost(&c->h_cells, sizeof(long long)));
     CK(cudaMallocHost(&c->h_bands, sizeof(int)));
+    CK(cudaMallocHost(&c->h_caps, sizeof(int) * 2));
     for (auto& ev : c->ev) CK(cudaEventCreate(&ev));
     {
         std::vector<double> lut(SPL_DOUBLES);
@@ -1184,6 +1197,7 @@ void vag_destroy(vag_context* c) {
     if (c->h_totals) cudaFreeHost(c->h_totals);
     if (c->h_cells) cudaFreeHost(c->h_cells);
     if (c->h_bands) cudaFreeHost(c->h_bands);
+    if (c->h_caps) cudaFreeHost(c->h_caps);
     for (auto& ev : c->ev)
         if (ev) cudaEventDestroy(ev);
     cudaStreamDestroy(c->stream);
@@ -1307,11 +1321,17 @@ static int check_times(const double* t, size_t n_t) {
     return VAG_OK;
 }
 
+// times -> io_t, checked by the caller
+static int upload_times(vag_context* ctx, const double* t, size_t n_t) {
+    CK(ctx->io_t.ensure(sizeof(double) * n_t));
+    CK(cudaMemcpyAsync(ctx->io_t.p, t, sizeof(double) * n_t, cudaMemcpyHostToDevice, ctx->stream));
+    return VAG_OK;
+}
+
 // times -> io_t, frequencies -> io_nu, checked by the caller
 static int upload_request(vag_context* ctx, const double* t, size_t n_t, const double* nu, size_t n_nu) {
-    CK(ctx->io_t.ensure(sizeof(double) * n_t));
+    if (int rc = upload_times(ctx, t, n_t)) return rc;
     CK(ctx->io_nu.ensure(sizeof(double) * n_nu));
-    CK(cudaMemcpyAsync(ctx->io_t.p, t, sizeof(double) * n_t, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(ctx->io_nu.p, nu, sizeof(double) * n_nu, cudaMemcpyHostToDevice, ctx->stream));
     return VAG_OK;
 }
@@ -1485,22 +1505,22 @@ static int band_grid(double nu_min, double nu_max, size_t num_nu, BandGrid& g) {
     return VAG_OK;
 }
 
-// Band-integrated flux of a batch whose parameters, times (io_t) and band nodes g.nu (io_nu) are on the device: grid
-// evaluation on the band's frequency nodes, then the weighted sum over frequency.  *d_band -> [n_models][VAG_NCOMP][n_t]
-// inside io_out.
-static int run_band(vag_context* ctx, size_t n_models, Caps caps, size_t n_t, const BandGrid& g, double** d_band,
-                    cudaStream_t s) {
+// Band-integrated flux of a batch whose parameters and times d_t are on the device: grid evaluation on the band's
+// frequency nodes g.nu (uploaded to io_nu, the weights to io_w), then the weighted sum over frequency.
+// *d_band -> [n_models][VAG_NCOMP][n_t] inside io_out.
+static int run_band(vag_context* ctx, const vag_params* d_params, size_t n_models, Caps caps, const double* d_t, size_t n_t,
+                    const BandGrid& g, int32_t* d_status, double** d_band, cudaStream_t s) {
     const size_t num_nu = g.nu.size();
+    CK(ctx->io_nu.ensure(sizeof(double) * num_nu));
     CK(ctx->io_w.ensure(sizeof(double) * num_nu));
     const size_t grid_elems = n_models * VAG_NCOMP * num_nu * n_t;
     CK(ctx->io_out.ensure(sizeof(double) * (grid_elems + n_models * VAG_NCOMP * n_t)));
+    CK(cudaMemcpyAsync(ctx->io_nu.p, g.nu.data(), sizeof(double) * num_nu, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(ctx->io_w.p, g.wgt.data(), sizeof(double) * num_nu, cudaMemcpyHostToDevice, s));
     double* d_grid = static_cast<double*>(ctx->io_out.p);
     *d_band = d_grid + grid_elems;
-    Request rq{false, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_t, num_nu, true};
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq, d_grid,
-                          static_cast<int32_t*>(ctx->io_status.p), nullptr, s))
-        return rc;
+    Request rq{false, d_t, static_cast<double*>(ctx->io_nu.p), n_t, num_nu, true};
+    if (int rc = run_flux(ctx, d_params, n_models, caps, rq, d_grid, d_status, nullptr, s)) return rc;
     const size_t n_mc = n_models * VAG_NCOMP;
     k_band_reduce<<<(unsigned)((n_mc * n_t + 255) / 256), 256, 0, s>>>(d_grid, static_cast<double*>(ctx->io_w.p), *d_band,
                                                                      n_mc, (int)num_nu, (int)n_t);
@@ -1516,86 +1536,50 @@ int vag_flux_band(vag_context* ctx, const vag_params* params, size_t n_models, c
     if (int rc = band_grid(nu_min, nu_max, num_nu, g)) return rc;
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
-    if (int rc = prepare_request(ctx, t, n_t, g.nu.data(), num_nu)) return rc;
+    if (int rc = check_times(t, n_t)) return rc;
+    if (int rc = upload_times(ctx, t, n_t)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
     double* d_band = nullptr;
-    if (int rc = run_band(ctx, n_models, caps, n_t, g, &d_band, s)) return rc;
+    if (int rc = run_band(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, static_cast<double*>(ctx->io_t.p),
+                          n_t, g, static_cast<int32_t*>(ctx->io_status.p), &d_band, s))
+        return rc;
     CK(cudaMemcpyAsync(out, d_band, sizeof(double) * n_models * VAG_NCOMP * n_t, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
 }
 
-// Replaces Fitter._evaluate (VegasAfterglow/fitting/fitter.py:503-533) for a batch of parameter sets: the chi-squared of the
-// point data (flux_density series) plus one term per band-integrated data set (Model.flux), all in ln-flux space.
-// With ext_k / A_V, the observed ln-flux of point i for model m is lnF_obs[i] + A_V[m] ext_k[i] (host extinction).
-int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
-                 const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
-                 const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status) {
-    if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (n_points && (!t || !nu || !lnF_obs || !sigma_ln || !w)) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL");
-    if (n_bands && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
-    if (n_points == 0 && n_bands == 0) return fail(VAG_ERR_INVALID, "no data: n_points and n_bands are both 0");
-    const bool ext = ext_k != nullptr;
-    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
-    if (ext && n_points == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points > 0)");
-    for (size_t i = 0; ext && i < n_points; ++i)
-        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
-    // every band is checked before any work is enqueued
-    std::vector<BandGrid> grids(n_bands);
-    size_t max_obs = n_points;
-    for (size_t b = 0; b < n_bands; ++b) {
-        const vag_band_obs& B = bands[b];
-        if (B.n == 0 || !B.t || !B.lnF_obs || !B.sigma_ln || !B.w) return fail(VAG_ERR_INVALID, "band data arrays must be non-empty");
-        if (int rc = band_grid(B.nu_min, B.nu_max, B.num_nu, grids[b])) return rc;
-        if (int rc = check_times(B.t, B.n)) return rc;
-        max_obs = std::max(max_obs, B.n);
-    }
-    Caps caps;
-    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
-    if (n_points)
-        if (int rc = prepare_request(ctx, t, n_points, nu, n_points)) return rc;
-    if (n_models == 0) return VAG_OK;
-    cudaStream_t s = ctx->stream;
-    // observation staging: chi2 [n_models], lnF / sigma_ln / w [max_obs] of the term in flight, with extinction ext_k
-    // [n_points] and A_V [n_models], status OR [n_models]
-    const size_t n_ext = ext ? n_points + n_models : 0;
-    CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * max_obs + n_ext) + sizeof(int32_t) * n_models));
-    double* d_chi2 = static_cast<double*>(ctx->io_obs.p);
-    double* d_lnF = d_chi2 + n_models;
-    double* d_sig = d_lnF + max_obs;
-    double* d_w = d_sig + max_obs;
-    double* d_ext = d_w + max_obs;
-    double* d_av = d_ext + n_points;
-    int32_t* d_stat_or = reinterpret_cast<int32_t*>(d_w + max_obs + n_ext);
+// The likelihood's data on the device: the point series (n == 0: none; ext / av both set or both NULL) and the bands
+struct Chi2Points {
+    const double *t, *nu, *lnF, *sig, *w, *ext, *av;
+    size_t n;
+};
+struct BandTerm {
+    const double *t, *lnF, *sig, *w;
+    size_t n;
+    const BandGrid* g;
+};
+
+// chi2[n] of a batch whose parameters and data are on the device: the point term (k_chi2 inside run_flux writes chi2),
+// then per band Model.flux and an accumulating k_chi2.  The status of every run goes to io_status; with band terms it is
+// ORed into d_stat_or, which is then the call's status.  ctx->launches counts every launch of the call.
+static int chi2_run(vag_context* ctx, const vag_params* d_params, size_t n_models, Caps caps, const Chi2Points& pts,
+                    const BandTerm* bands, size_t n_bands, double* d_chi2, int32_t* d_stat_or, cudaStream_t s) {
     int32_t* d_status = static_cast<int32_t*>(ctx->io_status.p);
-    auto upload = [&](const double* a, const double* b_, const double* c, size_t n) -> int {
-        CK(cudaMemcpyAsync(d_lnF, a, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(d_sig, b_, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(d_w, c, sizeof(double) * n, cudaMemcpyHostToDevice, s));
-        return VAG_OK;
-    };
-    // with band terms, the status is the OR over every term's status; a lone point term's status is the status
     const bool or_status = n_bands > 0;
     const unsigned og = (unsigned)((n_models + 255) / 256), cg = (unsigned)((n_models * 32 + 127) / 128);
     if (or_status) CK(cudaMemsetAsync(d_stat_or, 0, sizeof(int32_t) * n_models, s));
     int launches = 0;
-    if (n_points) {  // the first term: run_flux writes chi2
-        if (int rc = upload(lnF_obs, sigma_ln, w, n_points)) return rc;
-        CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * n_points));
-        Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points, n_points};
-        rq.d_lnF = d_lnF;
-        rq.d_sig = d_sig;
-        rq.d_w = d_w;
-        if (ext) {
-            CK(cudaMemcpyAsync(d_ext, ext_k, sizeof(double) * n_points, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpyAsync(d_av, A_V, sizeof(double) * n_models, cudaMemcpyHostToDevice, s));
-            rq.d_ext = d_ext;
-            rq.d_av = d_av;
-        }
-        if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq,
-                              static_cast<double*>(ctx->io_out.p), d_status, d_chi2, s))
+    if (pts.n) {  // the first term: run_flux writes chi2
+        CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * pts.n));
+        Request rq{true, pts.t, pts.nu, pts.n, pts.n};
+        rq.d_lnF = pts.lnF;
+        rq.d_sig = pts.sig;
+        rq.d_w = pts.w;
+        rq.d_ext = pts.ext;
+        rq.d_av = pts.av;
+        if (int rc = run_flux(ctx, d_params, n_models, caps, rq, static_cast<double*>(ctx->io_out.p), d_status, d_chi2, s))
             return rc;
         launches += ctx->launches;
         if (or_status) {
@@ -1606,20 +1590,106 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
         CK(cudaMemsetAsync(d_chi2, 0, sizeof(double) * n_models, s));
     }
     for (size_t b = 0; b < n_bands; ++b) {
-        const vag_band_obs& B = bands[b];
-        if (int rc = upload_request(ctx, B.t, B.n, grids[b].nu.data(), grids[b].nu.size())) return rc;
+        const BandTerm& B = bands[b];
         double* d_band = nullptr;
-        if (int rc = run_band(ctx, n_models, caps, B.n, grids[b], &d_band, s)) return rc;
-        if (int rc = upload(B.lnF_obs, B.sigma_ln, B.w, B.n)) return rc;
-        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, d_lnF, d_sig, d_w, nullptr, nullptr, d_chi2, d_status, 1);
+        if (int rc = run_band(ctx, d_params, n_models, caps, B.t, B.n, *B.g, d_status, &d_band, s)) return rc;
+        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, B.lnF, B.sig, B.w, nullptr, nullptr, d_chi2, d_status, 1);
         k_or_status<<<og, 256, 0, s>>>(d_stat_or, d_status, n_models);
         launches += ctx->launches + 2;
     }
     ctx->launches = launches;
     CK(cudaGetLastError());
+    return VAG_OK;
+}
+
+// The checks of vag_chi2_ext and vag_chi2_dev, all before any work is enqueued: arguments, every band's grid and -- for
+// data in host memory (host_data) -- the values of ext_k and of the band times
+static int check_chi2_args(vag_context* ctx, const double* chi2, size_t n_points, bool point_ptrs, const double* ext_k,
+                           const double* A_V, const vag_band_obs* bands, size_t n_bands, bool host_data,
+                           std::vector<BandGrid>& grids) {
+    if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (n_points && !point_ptrs) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL");
+    if (n_bands && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
+    if (n_points == 0 && n_bands == 0) return fail(VAG_ERR_INVALID, "no data: n_points and n_bands are both 0");
+    const bool ext = ext_k != nullptr;
+    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (ext && n_points == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points > 0)");
+    for (size_t i = 0; host_data && ext && i < n_points; ++i)
+        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
+    grids.resize(n_bands);
+    for (size_t b = 0; b < n_bands; ++b) {
+        const vag_band_obs& B = bands[b];
+        if (B.n == 0 || !B.t || !B.lnF_obs || !B.sigma_ln || !B.w) return fail(VAG_ERR_INVALID, "band data arrays must be non-empty");
+        if (int rc = band_grid(B.nu_min, B.nu_max, B.num_nu, grids[b])) return rc;
+        if (host_data)
+            if (int rc = check_times(B.t, B.n)) return rc;
+    }
+    return VAG_OK;
+}
+
+// Replaces Fitter._evaluate (VegasAfterglow/fitting/fitter.py:503-533) for a batch of parameter sets: the chi-squared of the
+// point data (flux_density series) plus one term per band-integrated data set (Model.flux), all in ln-flux space.
+// With ext_k / A_V, the observed ln-flux of point i for model m is lnF_obs[i] + A_V[m] ext_k[i] (host extinction).
+int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
+                 const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
+                 const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status) {
+    std::vector<BandGrid> grids;
+    if (int rc = check_chi2_args(ctx, chi2, n_points, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, bands, n_bands, true,
+                                 grids))
+        return rc;
+    const bool ext = ext_k != nullptr;
+    size_t n_obs = n_models + 3 * n_points + (ext ? n_points + n_models : 0);
+    for (size_t b = 0; b < n_bands; ++b) n_obs += 4 * bands[b].n;
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_points)
+        if (int rc = prepare_request(ctx, t, n_points, nu, n_points)) return rc;
+    if (n_models == 0) return VAG_OK;
+    cudaStream_t s = ctx->stream;
+    // observation staging: chi2 [n_models]; lnF / sigma_ln / w of the points (with extinction ext_k [n_points] and A_V
+    // [n_models]); t / lnF / sigma_ln / w of every band; status OR [n_models]
+    CK(ctx->io_obs.ensure(sizeof(double) * n_obs + sizeof(int32_t) * n_models));
+    double* cur = static_cast<double*>(ctx->io_obs.p);
+    double* d_chi2 = cur;
+    cur += n_models;
+    cudaError_t ce = cudaSuccess;
+    auto stage = [&](const double* h, size_t n) {
+        double* d = cur;
+        cur += n;
+        if (ce == cudaSuccess) ce = cudaMemcpyAsync(d, h, sizeof(double) * n, cudaMemcpyHostToDevice, s);
+        return d;
+    };
+    Chi2Points pts{};
+    if (n_points) {
+        pts = Chi2Points{static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), nullptr, nullptr, nullptr,
+                         nullptr, nullptr, n_points};
+        pts.lnF = stage(lnF_obs, n_points);
+        pts.sig = stage(sigma_ln, n_points);
+        pts.w = stage(w, n_points);
+        if (ext) {
+            pts.ext = stage(ext_k, n_points);
+            pts.av = stage(A_V, n_models);
+        }
+    }
+    std::vector<BandTerm> terms(n_bands);
+    for (size_t b = 0; b < n_bands; ++b) {
+        const vag_band_obs& B = bands[b];
+        terms[b].t = stage(B.t, B.n);
+        terms[b].lnF = stage(B.lnF_obs, B.n);
+        terms[b].sig = stage(B.sigma_ln, B.n);
+        terms[b].w = stage(B.w, B.n);
+        terms[b].n = B.n;
+        terms[b].g = &grids[b];
+    }
+    if (ce != cudaSuccess) return fail(VAG_ERR_CUDA, std::string("staging the observations: ") + cudaGetErrorString(ce));
+    int32_t* d_stat_or = reinterpret_cast<int32_t*>(cur);
+    if (int rc = chi2_run(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, pts, terms.data(), n_bands, d_chi2,
+                          d_stat_or, s))
+        return rc;
     CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
     if (status)
-        CK(cudaMemcpyAsync(status, or_status ? d_stat_or : d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(status, n_bands ? d_stat_or : ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost,
+                           s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
 }
@@ -1646,6 +1716,136 @@ int vag_chi2_series(vag_context* ctx, const vag_params* params, size_t n_models,
     if (n == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
     if (!nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
     return vag_chi2(ctx, params, n_models, t, nu, lnF_obs, sigma_ln, w, n, nullptr, 0, chi2, status);
+}
+
+// ---- device-buffer entry points that plan on the device --------------------------------------------------------
+// The record that runs in place of a rejected one: an on-axis tophat in ISM (one ODE row, one phi row) with coarse theta
+// and time resolutions, so that its theta grid and time lattice stay below those of the batch's real models, which size
+// the EATS stage of the whole batch
+static vag_params stand_in_params() {
+    vag_params p;
+    vag_params_default(&p);
+    p.jet_type = VAG_JET_TOPHAT;
+    p.theta_c = 0.1;
+    p.E_iso = 1e52;
+    p.Gamma0 = 100.0;
+    p.medium_type = VAG_MEDIUM_ISM;
+    p.n_ism = 1.0;
+    p.lumi_dist = 1e28;
+    p.theta_resol = 0.05;
+    p.t_resol = 2.0;
+    return p;
+}
+
+// k_plan over n device records (run may be NULL) and the capacities of the accepted ones on the host (caps_for's floor
+// included): one D2H of two ints and one synchronisation of s, because setup_models sizes the workspaces on the host
+static int plan(vag_context* ctx, const vag_params* d_params, size_t n, vag_params* run, int32_t* ok, int* d_caps,
+                Caps* caps, cudaStream_t s) {
+    CK(cudaMemsetAsync(d_caps, 0, sizeof(int) * 2, s));
+    k_plan<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_params, n, stand_in_params(), run, ok, d_caps);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(ctx->h_caps, d_caps, sizeof(int) * 2, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    *caps = Caps{std::max(64, ctx->h_caps[0]), std::max(8, ctx->h_caps[1])};
+    return VAG_OK;
+}
+
+// The records that run (*d_run, rejected ones replaced by the stand-in), ok[] (*d_ok) and the capacities that cover both
+static int plan_run(vag_context* ctx, const vag_params* d_params, size_t n, cudaStream_t s, const vag_params** d_run,
+                    const int32_t** d_ok, Caps* caps) {
+    CK(ctx->plan_buf.ensure(carve_sz<vag_params>(n) + carve_sz<int32_t>(n) + carve_sz<int>(2)));
+    char* p = static_cast<char*>(ctx->plan_buf.p);
+    vag_params* run = carve<vag_params>(p, n);
+    int32_t* ok = carve<int32_t>(p, n);
+    int* d_caps = carve<int>(p, 2);
+    if (int rc = plan(ctx, d_params, n, run, ok, d_caps, caps, s)) return rc;
+    const vag_params sp = stand_in_params();
+    const Caps sc = caps_of(sp);
+    caps->theta = std::max(caps->theta, sc.theta);
+    caps->phi = std::max(caps->phi, sc.phi);
+    *d_run = run;
+    *d_ok = ok;
+    return VAG_OK;
+}
+
+int vag_params_validate_batch_dev(vag_context* ctx, const vag_params* d_params, size_t n, int32_t* d_ok, int caps[2],
+                                  void* stream) {
+    if (!ctx || !caps || (n && (!d_params || !d_ok))) return fail(VAG_ERR_INVALID, "NULL argument");
+    ctx->launches = 0;
+    if (n == 0) {
+        caps[0] = 64;
+        caps[1] = 8;
+        return VAG_OK;
+    }
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    CK(ctx->plan_buf.ensure(carve_sz<int>(2)));
+    Caps c;
+    if (int rc = plan(ctx, d_params, n, nullptr, d_ok, static_cast<int*>(ctx->plan_buf.p), &c, s)) return rc;
+    ctx->launches = 1;
+    caps[0] = c.theta;
+    caps[1] = c.phi;
+    return VAG_OK;
+}
+
+int vag_flux_band_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t, size_t n_t,
+                      double nu_min, double nu_max, size_t num_nu, double* d_out, int32_t* d_status, void* stream) {
+    if (!ctx || !d_out || (n_models && !d_params)) return fail(VAG_ERR_INVALID, "NULL argument");
+    BandGrid g;
+    if (int rc = band_grid(nu_min, nu_max, num_nu, g)) return rc;
+    if (n_t == 0 || !d_t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
+    if (n_models == 0) return VAG_OK;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    const vag_params* d_run = nullptr;
+    const int32_t* d_ok = nullptr;
+    Caps caps;
+    if (int rc = plan_run(ctx, d_params, n_models, s, &d_run, &d_ok, &caps)) return rc;
+    CK(ctx->io_status.ensure(sizeof(int32_t) * n_models));
+    double* d_band = nullptr;
+    if (int rc = run_band(ctx, d_run, n_models, caps, d_t, n_t, g, static_cast<int32_t*>(ctx->io_status.p), &d_band, s))
+        return rc;
+    const size_t per_model = VAG_NCOMP * n_t;
+    CK(cudaMemcpyAsync(d_out, d_band, sizeof(double) * n_models * per_model, cudaMemcpyDeviceToDevice, s));
+    if (d_status)
+        CK(cudaMemcpyAsync(d_status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToDevice, s));
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, nullptr, d_out, per_model);
+    ctx->launches += 2;  // k_plan, k_reject
+    CK(cudaGetLastError());
+    return VAG_OK;
+}
+
+int vag_chi2_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const double* d_t, const double* d_nu,
+                 const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k, size_t n_points,
+                 const double* d_A_V, const vag_band_obs* bands, size_t n_bands, double* d_chi2, int32_t* d_status,
+                 void* stream) {
+    std::vector<BandGrid> grids;
+    if (int rc = check_chi2_args(ctx, d_chi2, n_points, d_t && d_nu && d_lnF_obs && d_sigma_ln && d_w, d_ext_k, d_A_V,
+                                 bands, n_bands, false, grids))
+        return rc;
+    if (n_models && !d_params) return fail(VAG_ERR_INVALID, "params is NULL");
+    if (n_models == 0) return VAG_OK;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    const vag_params* d_run = nullptr;
+    const int32_t* d_ok = nullptr;
+    Caps caps;
+    if (int rc = plan_run(ctx, d_params, n_models, s, &d_run, &d_ok, &caps)) return rc;
+    CK(ctx->io_status.ensure(sizeof(int32_t) * n_models));
+    CK(ctx->io_obs.ensure(sizeof(int32_t) * n_models));  // status OR of the band terms
+    int32_t* d_stat_or = static_cast<int32_t*>(ctx->io_obs.p);
+    const Chi2Points pts{d_t, d_nu, d_lnF_obs, d_sigma_ln, d_w, d_ext_k, d_A_V, n_points};
+    std::vector<BandTerm> terms(n_bands);
+    for (size_t b = 0; b < n_bands; ++b)
+        terms[b] = BandTerm{bands[b].t, bands[b].lnF_obs, bands[b].sigma_ln, bands[b].w, bands[b].n, &grids[b]};
+    if (int rc = chi2_run(ctx, d_run, n_models, caps, pts, terms.data(), n_bands, d_chi2, d_stat_or, s)) return rc;
+    if (d_status)
+        CK(cudaMemcpyAsync(d_status, n_bands ? d_stat_or : ctx->io_status.p, sizeof(int32_t) * n_models,
+                           cudaMemcpyDeviceToDevice, s));
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, d_chi2, nullptr, 0);
+    ctx->launches += 2;  // k_plan, k_reject
+    CK(cudaGetLastError());
+    return VAG_OK;
 }
 
 // ---- introspection ---------------------------------------------------------------------------------

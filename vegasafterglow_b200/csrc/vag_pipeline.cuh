@@ -12,6 +12,8 @@
 // Each body is an HD function so the CPU test-suite can execute the identical code sequentially.
 #pragma once
 
+#include <climits>
+
 #include "vag_grid.cuh"
 #include "vag_ic.cuh"
 #include "vag_observer.cuh"
@@ -497,24 +499,122 @@ VAG_HD double chi2_term(double lnF_obs, double F_model, double sigma_ln, double 
     return wgt * d * d;
 }
 
-// ---- host only: batch planning shared by vag_b200.cu and the host emulation (oracle/hostemu/hostemu.cpp) -----
+// ---- parameter checks and capacity bounds: one definition for the host and for the device planning (k_plan) ----------
+// Why vag_params_validate rejects a parameter set; vag_b200.cu maps each reason to its message.  The order of the checks
+// decides which reason a set with several faults gets.
+enum ParamsReason {
+    PR_OK = 0, PR_JET_TYPE, PR_MEDIUM_TYPE, PR_THETA_C, PR_E_ISO, PR_GAMMA0, PR_DURATION, PR_K_EG, PR_E_ISO_W, PR_GAMMA0_W,
+    PR_THETA_W, PR_THETA_W_ORDER, PR_SIGMA0, PR_MAG_L0, PR_MAG_T0, PR_MAG_Q, PR_MAG_WING, PR_N_ISM, PR_A_STAR, PR_N0, PR_K_M,
+    PR_LUMI_DIST, PR_Z, PR_THETA_OBS, PR_PHI_OBS,
+    PR_FWD_EPS_E, PR_FWD_EPS_B, PR_FWD_XI_E, PR_FWD_P,  // the reverse shock's four follow in the same order
+    PR_RVS_EPS_E, PR_RVS_EPS_B, PR_RVS_XI_E, PR_RVS_P, PR_RTOL, PR_NONFINITE_RES
+};
+
+VAG_HD bool finite_pos(double x) { return isfinite(x) && x > 0; }
+VAG_HD bool in_open_closed(double v, double lo, double hi) { return isfinite(v) && v > lo && v <= hi; }
+
+// PyRadiation (pybind/pymodel.h:303-313); base = PR_FWD_EPS_E or PR_RVS_EPS_E
+VAG_HD int radiation_check(const vag_radiation& r, int base) {
+    if (!in_open_closed(r.eps_e, 0.0, 1.0)) return base;
+    if (!in_open_closed(r.eps_B, 0.0, 1.0)) return base + 1;
+    if (!in_open_closed(r.xi_e, 0.0, 1.0)) return base + 2;
+    if (!(isfinite(r.p) && r.p > 1.0)) return base + 3;
+    return PR_OK;
+}
+
+// The checks of the reference constructors (pybind/pymodel.cpp:47-186, pybind/pymodel.h:190-204,303-313,613-649)
+VAG_HD int params_check(const vag_params& p) {
+    if (p.jet_type < 0 || p.jet_type > 5) return PR_JET_TYPE;
+    if (p.medium_type < 0 || p.medium_type > 1) return PR_MEDIUM_TYPE;
+    // PyTophatJet / PyGaussianJet / PyPowerLawJet: pybind/pymodel.cpp:47-95
+    if (!in_open_closed(p.theta_c, 0.0, con::pi / 2)) return PR_THETA_C;
+    const bool has_core = p.jet_type != VAG_JET_POWERLAW_WING;
+    const bool has_wing = p.jet_type >= VAG_JET_TWO_COMPONENT;
+    if (has_core && !finite_pos(p.E_iso)) return PR_E_ISO;
+    if (has_core && !(isfinite(p.Gamma0) && p.Gamma0 > 1.0)) return PR_GAMMA0;
+    if (!finite_pos(p.duration)) return PR_DURATION;
+    if ((p.jet_type == VAG_JET_POWERLAW || p.jet_type == VAG_JET_STEP_POWERLAW || p.jet_type == VAG_JET_POWERLAW_WING) &&
+        (!finite_pos(p.k_e) || !finite_pos(p.k_g)))
+        return PR_K_EG;
+    // PyTwoComponentJet / PyStepPowerLawJet / PyPowerLawWing: pybind/pymodel.cpp:97-146
+    if (has_wing) {
+        if (!finite_pos(p.E_iso_w)) return PR_E_ISO_W;
+        if (!(isfinite(p.Gamma0_w) && p.Gamma0_w > 1.0)) return PR_GAMMA0_W;
+    }
+    if (p.jet_type == VAG_JET_TWO_COMPONENT) {
+        if (!in_open_closed(p.theta_w, 0.0, con::pi / 2)) return PR_THETA_W;
+        if (!(p.theta_w > p.theta_c)) return PR_THETA_W_ORDER;
+    }
+    if (!(isfinite(p.sigma0) && p.sigma0 >= 0)) return PR_SIGMA0;
+    if (p.has_magnetar) {  // PyMagnetar: pybind/pymodel.h:45-49
+        if (!finite_pos(p.magnetar_L0)) return PR_MAG_L0;
+        if (!finite_pos(p.magnetar_t0)) return PR_MAG_T0;
+        if (!finite_pos(p.magnetar_q)) return PR_MAG_Q;
+        if (p.jet_type == VAG_JET_POWERLAW_WING) return PR_MAG_WING;
+    }
+    // PyISM / PyWind: pybind/pymodel.cpp:148-186
+    if (p.medium_type == VAG_MEDIUM_ISM) {
+        if (!(isfinite(p.n_ism) && p.n_ism >= 0)) return PR_N_ISM;
+    } else {
+        if (!finite_pos(p.A_star)) return PR_A_STAR;
+        if (!(isfinite(p.n_ism) && p.n_ism >= 0)) return PR_N_ISM;
+        if (!(p.n0 > 0)) return PR_N0;
+        if (!isfinite(p.wind_k_m)) return PR_K_M;
+    }
+    // PyObserver: pybind/pymodel.h:190-204
+    if (!finite_pos(p.lumi_dist)) return PR_LUMI_DIST;
+    if (!(isfinite(p.z) && p.z >= 0)) return PR_Z;
+    if (!(isfinite(p.theta_obs) && p.theta_obs >= 0 && p.theta_obs <= con::pi)) return PR_THETA_OBS;
+    if (!isfinite(p.phi_obs)) return PR_PHI_OBS;
+    if (const int r = radiation_check(p.fwd, PR_FWD_EPS_E)) return r;
+    if (p.has_rvs)
+        if (const int r = radiation_check(p.rvs, PR_RVS_EPS_E)) return r;
+    // PyModel ctor: pybind/pymodel.h:642-647 (a non-positive value selects the default)
+    if (p.rtol > 0 && !(p.rtol < 1)) return PR_RTOL;
+    if (!isfinite(p.rtol) || !isfinite(p.phi_resol) || !isfinite(p.theta_resol) || !isfinite(p.t_resol))
+        return PR_NONFINITE_RES;
+    return PR_OK;
+}
+
 struct Caps {
     int theta, phi;
 };
 
-// capacity planning from host-side parameters (upper bounds of auto_grid's node counts,
-// src/core/grid-refinement.h:246-262,655,664-677)
+// (int)x as the x86-64 host converts it (cvttsd2si: truncation, INT_MIN for NaN and for values outside int's range) and
+// int sums that wrap.  The device's own conversion saturates: spelled out, the bound of a record with, e.g., an unused
+// Gamma0_w = inf is the same number on both sides.
+VAG_HD int host_int(double x) { return (x > -2147483649.0 && x < 2147483648.0) ? (int)x : INT_MIN; }
+VAG_HD int wrap_add(int a, int b) { return (int)((unsigned)a + (unsigned)b); }
+
+// Grid nodes one parameter set can need (upper bounds of auto_grid's node counts,
+// src/core/grid-refinement.h:246-262,655,664-677).  log10 is glibc's on the host and its bit-exact restatement on the
+// device (vag_libm.cuh): CUDA's log10 can differ by an ulp, which can move the integer bound at a boundary.
+VAG_HD Caps caps_of(const vag_params& p) {
+    const bool r = p.has_rvs != 0;
+    const double th_res = p.theta_resol > 0 ? p.theta_resol : (r ? 0.2 : 0.15);
+    const double ph_res = p.phi_resol > 0 ? p.phi_resol : 0.06;
+    const double g = vmax(1.0, vmax(p.Gamma0, p.Gamma0_w) * 1.5708);
+#if defined(__CUDA_ARCH__)
+    const double lg = gl::log10(g);
+#else
+    const double lg = std::log10(g);
+#endif
+    int ct = wrap_add(36, host_int(90 * th_res));
+    ct = wrap_add(ct, host_int(vmax(0.0, lg - 1) * th_res * 55));
+    ct = wrap_add(ct, host_int(lg * th_res * 25));
+    ct = wrap_add(ct, 64);
+    const int cp = wrap_add((int)((unsigned)imax(host_int(360 * ph_res), 1) * 5u), 8);
+    return Caps{ct, cp};
+}
+
+// ---- host only: batch planning shared by vag_b200.cu and the host emulation (oracle/hostemu/hostemu.cpp) -----
+// capacities of a batch from host-side parameters
 inline Caps caps_for(const vag_params* p, size_t n) {
     Caps c{64, 8};
     for (size_t i = 0; i < n; ++i) {
-        const bool r = p[i].has_rvs != 0;
-        const double th_res = p[i].theta_resol > 0 ? p[i].theta_resol : (r ? 0.2 : 0.15);
-        const double ph_res = p[i].phi_resol > 0 ? p[i].phi_resol : 0.06;
-        const double lg = std::log10(std::max(1.0, std::max(p[i].Gamma0, p[i].Gamma0_w) * 1.5708));
-        const int ct = 36 + (int)(90 * th_res) + (int)(std::max(0.0, lg - 1) * th_res * 55) + (int)(lg * th_res * 25) + 64;
-        const int cp = std::max((int)(360 * ph_res), 1) * 5 + 8;
-        c.theta = std::max(c.theta, ct);
-        c.phi = std::max(c.phi, cp);
+        const Caps b = caps_of(p[i]);
+        c.theta = std::max(c.theta, b.theta);
+        c.phi = std::max(c.phi, b.phi);
     }
     return c;
 }

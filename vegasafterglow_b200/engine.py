@@ -173,6 +173,33 @@ class Engine:
         _lib.check(self._lib.vag_chi2_series_dev(self._h, d_params, n_models, d_t, d_nu, d_lnF, d_sig, d_w, n, d_chi2,
                                                  d_status or None, stream or None))
 
+    def validate_dev(self, d_params, n, d_ok, stream=0):
+        """``vag_params_validate_batch_dev``: int32 ok flags into ``d_ok``; returns the planned (theta, phi) capacities.
+        Synchronises the stream."""
+        caps = (C.c_int * 2)()
+        _lib.check(self._lib.vag_params_validate_batch_dev(self._h, d_params, n, d_ok, caps, stream or None))
+        return int(caps[0]), int(caps[1])
+
+    def flux_band_dev(self, d_params, n_models, d_t, n_t, nu_min, nu_max, num_nu, d_out, d_status=0, stream=0):
+        """``vag_flux_band_dev``: ``Model.flux`` into d_out[n_models, 5, n_t]; parameters checked and grids sized on the
+        device (rejected sets: NaN, ``abi.ST_INVALID``)."""
+        _lib.check(self._lib.vag_flux_band_dev(self._h, d_params, n_models, d_t, n_t, float(nu_min), float(nu_max),
+                                               int(num_nu), d_out, d_status or None, stream or None))
+
+    def chi2_dev(self, d_params, n_models, points=None, bands=(), d_chi2=0, d_status=0, extinction=None, stream=0):
+        """``vag_chi2_dev``: the likelihood of ``chi2`` on device pointers.  ``points`` = (d_t, d_nu, d_lnF, d_sig, d_w,
+        n_points) or None; ``bands``: dicts like ``chi2``'s whose t, lnF_obs, sigma_ln, w are device pointers with their
+        length ``n``; ``extinction`` = (d_ext_k, d_A_V).  Rejected parameter sets give chi2 = +inf and ``abi.ST_INVALID``."""
+        pts, n_pt = ([None] * 5, 0) if points is None else (list(points[:5]), int(points[5]))
+        ext, av = (None, None) if extinction is None else extinction
+        arr = (abi.BandObs * max(len(bands), 1))()
+        for i, b in enumerate(bands):
+            arr[i] = abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], int(b["n"]), float(b["nu_min"]),
+                                 float(b["nu_max"]), int(b["num_nu"]))
+        _lib.check(self._lib.vag_chi2_dev(self._h, d_params, n_models, *pts, ext, n_pt, av,
+                                          C.cast(arr, C.c_void_p) if len(bands) else None, len(bands), d_chi2,
+                                          d_status or None, stream or None))
+
     def synchronize(self):
         _lib.check(self._lib.vag_synchronize(self._h))
 

@@ -170,3 +170,105 @@ class BatchedLikelihood:
             logp[idx] = ll
         return logp
 
+
+
+_CUDA_STREAM_LEGACY = 0x1  # cudaStreamLegacy (driver_types.h)
+
+
+def _field_offset(path):
+    """Byte offset of a float64 field of ``abi.PARAMS_DTYPE`` (``("fwd", "eps_e")`` for a nested one)."""
+    dt, off = abi.PARAMS_DTYPE, 0
+    for name in path:
+        dt, o = dt.fields[name][:2]
+        off += o
+    assert dt == np.float64 and off % 8 == 0
+    return off
+
+
+class DeviceLikelihood(BatchedLikelihood):
+    """``BatchedLikelihood`` with the data, the walkers and the result in HBM: the same constructor (``device``: where the
+    data live, default the engine's GPU) and the same ``__call__(samples[n, ndim]) -> logp[n]``.
+
+    The point data, ``ext_kernel`` and band arrays go to the device once, here.  Per call only the ``n x ndim`` sampler
+    columns are uploaded -- exponentiated on the host with ``BatchedLikelihood._column``'s numpy expression (a device
+    ``pow`` would not give the same bits, and the theta grid amplifies a last-bit difference).  The records are assembled
+    on the device from the template, and ONE ``vag_chi2_dev`` call on the current torch stream validates them (rejected
+    walkers: chi2 = +inf), sizes their grids and evaluates every term.  Distributed, each rank evaluates its share of the
+    host-side cost-balanced assignment and the chi2 tensors are gathered on the device."""
+
+    def __init__(self, engine, *args, device=None, **kwargs):
+        import torch
+
+        super().__init__(engine, *args, **kwargs)
+        self.device = torch.device("cuda", engine.device) if device is None else torch.device(device)
+
+        def dev(a):
+            return torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device=self.device)
+
+        self._pts = tuple(dev(a) for a in (self.t, self.nu, self.lnF, self.sig, self.w)) if self.t.size else None
+        self._ext = dev(self.ext_kernel) if self.ext_kernel is not None else None
+        self._bands = [dict(b, **{k: dev(b[k]) for k in ("t", "lnF_obs", "sigma_ln", "w")}) for b in self.bands]
+        self._template = torch.as_tensor(self.template.view(np.uint8), device=self.device)
+        model = [i for i, n in enumerate(self.names) if n != "A_V"]
+        self._cols = torch.as_tensor(model, dtype=torch.long, device=self.device)
+        self._slots = torch.as_tensor([_field_offset(_FIELDS[self.names[i]]) // 8 for i in model], dtype=torch.long,
+                                      device=self.device)
+        self._av = self.names.index("A_V") if "A_V" in self.names and self.t.size else None
+
+    def columns(self, samples: np.ndarray) -> np.ndarray:
+        """float64[n, ndim]: the sampler columns as the model sees them (log10 columns exponentiated)."""
+        samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
+        out = np.empty_like(samples)
+        for i in range(len(self.names)):
+            out[:, i] = self._column(samples, i)
+        return out
+
+    def records(self, cols):
+        """uint8[n * sizeof(vag_params)] on the device: the template repeated, the model columns of ``cols`` (float64
+        tensor [n, ndim] from ``columns``) scattered into a float64 view at their fields' offsets."""
+        import torch
+
+        n = cols.shape[0]
+        rec = self._template.repeat(n)
+        view = rec.view(torch.float64).view(n, abi.PARAMS_DTYPE.itemsize // 8)
+        view[:, self._slots] = cols[:, self._cols]
+        return rec
+
+    def _chi2_dev(self, cols):
+        import torch
+
+        n = cols.shape[0]
+        chi2 = torch.empty(n, dtype=torch.float64, device=self.device)
+        if n == 0:
+            return chi2
+        rec = self.records(cols)
+        points = None if self._pts is None else (*(a.data_ptr() for a in self._pts), self.t.size)
+        av = None if self._av is None else cols[:, self._av].contiguous()
+        extinction = None if av is None else (self._ext.data_ptr(), av.data_ptr())
+        bands = [dict(b, n=b["t"].numel(), **{k: b[k].data_ptr() for k in ("t", "lnF_obs", "sigma_ln", "w")})
+                 for b in self._bands]
+        stream = 0
+        if self.device.type == "cuda":
+            # A NULL stream would be the engine's own, unordered with the record assembly above.  torch's default
+            # stream has the handle 0 and is CUDA's legacy default stream, which the C ABI takes as cudaStreamLegacy.
+            stream = torch.cuda.current_stream(self.device).cuda_stream or _CUDA_STREAM_LEGACY
+        self.engine.chi2_dev(rec.data_ptr(), n, points, bands, chi2.data_ptr(), extinction=extinction, stream=stream)
+        return chi2
+
+    def chi2(self, samples: np.ndarray) -> np.ndarray:
+        """chi2 of every sample; +inf for a sample the model constructor rejects (checked on the device)."""
+        import torch
+
+        cols = torch.as_tensor(self.columns(samples), device=self.device)
+        if not self.distributed:
+            return self._chi2_dev(cols).cpu().numpy()
+        import torch.distributed as dist
+
+        from . import parallel
+
+        world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
+        tt = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
+        cost = parallel.cost_proxy(self.to_params(samples), float(np.min(tt)), float(np.max(tt)))
+        sets = parallel.balanced_assignment(cost, world)
+        mine = torch.as_tensor(sets[rank], dtype=torch.long, device=self.device)
+        return parallel.gather_indexed_tensor(self._chi2_dev(cols[mine]), sets, cols.shape[0]).cpu().numpy()

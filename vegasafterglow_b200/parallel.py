@@ -132,3 +132,24 @@ def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=
     extra = [np.asarray(a)[mine] for a in per_walker or ()]
     local = evaluate(params[mine], *extra) if len(mine) else np.zeros(0)
     return gather_indexed(local, sets, n)
+
+
+def gather_indexed_tensor(local, sets, n: int):
+    """``gather_indexed`` for a float64 tensor on the rank's device: the gather stays on that device (NCCL on GPUs, gloo
+    on the CPU) and the result is a length-``n`` tensor there, +inf where no rank wrote."""
+    import torch
+    import torch.distributed as dist
+
+    dev = local.device
+    out = torch.full((n,), float("inf"), dtype=torch.float64, device=dev)
+    if len(sets) == 1 or not (dist.is_available() and dist.is_initialized()):
+        out[torch.as_tensor(sets[0], dtype=torch.long, device=dev)] = local
+        return out
+    per = max(max(len(s) for s in sets), 1)
+    buf = torch.full((per,), float("inf"), dtype=torch.float64, device=dev)
+    buf[: local.numel()] = local
+    got = torch.empty(per * len(sets), dtype=torch.float64, device=dev)
+    dist.all_gather_into_tensor(got, buf)
+    for r, idx in enumerate(sets):
+        out[torch.as_tensor(idx, dtype=torch.long, device=dev)] = got[r * per: r * per + len(idx)]
+    return out
