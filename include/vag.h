@@ -191,6 +191,42 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
                  const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
                  const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status);
 
+/* ---- several light curves in one batch: every model has its own data set ------------------------------------------
+ * The points of all data sets are concatenated into t / nu (and lnF_obs / sigma_ln / w / ext_k) of n_points_total
+ * entries; data set d is the slice [sets[d].offset, sets[d].offset + sets[d].n), ascending in time.  Model m is
+ * evaluated on data set dataset_of[m] only: its grid window, time lattice and values are those that
+ * vag_flux_density_series / vag_chi2_series / vag_chi2_ext give for it on that data set alone (bit for bit when
+ * neither call splits the rows of a model over several CTAs -- i.e. from 2368 (model x shock) CTAs on 148 SMs -- and both
+ * stage the same number of rows per pass; otherwise to rounding).  An SSC model's tables span its own data set's band.
+ * Series modes (vag_set_series_mode) apply to the batch as a whole: it runs banded only when EVERY data set passes the
+ * banded test of a single request with the batch's longest time lattice -- mode 0: n_bands(d) <= 8 and
+ * n_bands(d) * max_n_t <= 3 n(d) for every d; 1: never; 2: whenever every data set has at most 8 distinct frequencies.
+ * Otherwise every model runs per point.
+ * Checks, all before any work is enqueued (VAG_ERR_INVALID, the message names the data set or the model): every set
+ * non-empty, inside the arrays, ascending, finite and > 0 in t, finite and > 0 in nu; 0 <= dataset_of[m] < n_sets;
+ * parameter sets as vag_params_validate.  A data set no model uses is allowed.  Batches over 32768 models run in
+ * passes as the other entry points do.  Launches: those of vag_chi2_series / vag_flux_density_series on the same
+ * total data, whatever n_sets (one CTA per data set inside the band search kernel).
+ * Not provided: band-integrated data per data set, a device-buffer (_dev) variant, per-model grid (t x nu) requests.
+ * The output mode (vag_set_output_mode) does not apply: every plane of `out` is written. */
+typedef struct vag_series_set {
+    size_t offset, n; /* slice of the concatenated points */
+} vag_series_set;
+
+/* out: model m's [VAG_NCOMP][n of its data set] block starts at element VAG_NCOMP * off[m], off[m] = the sum of the
+ * sizes of the data sets of models 0 .. m-1 (out has VAG_NCOMP * off[n_models] elements). */
+int vag_flux_density_series_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                  const vag_series_set* sets, size_t n_sets, const double* t, const double* nu,
+                                  size_t n_points_total, double* out, int32_t* status);
+
+/* chi2[m] of vag_chi2_series (ext_k / A_V NULL) or of vag_chi2_ext's point term (both set: ext_k[n_points_total] finite,
+ * in point order; A_V[n_models], a non-finite A_V gives +inf) for model m on its data set.  VAG_ST_ODE_FAIL500 gives
+ * +inf. */
+int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                   const vag_series_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                   const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total, const double* A_V,
+                   double* chi2, int32_t* status);
+
 /* ok[i] = 1 where vag_params_validate accepts params[i], else 0 (no error is raised for rejected sets). */
 int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok);
 

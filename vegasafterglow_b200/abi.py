@@ -88,6 +88,12 @@ class BandObs(C.Structure):
                 ("nu_min", C.c_double), ("nu_max", C.c_double), ("num_nu", C.c_size_t)]
 
 
+class SeriesSet(C.Structure):
+    """``vag_series_set`` (include/vag.h): one data set of a ragged series request, a slice of the concatenated points."""
+
+    _fields_ = [("offset", C.c_size_t), ("n", C.c_size_t)]
+
+
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
 

@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -311,9 +312,9 @@ __global__ void k_prep_obs(const double* __restrict__ t, int n_t, const double* 
 // Distinct frequencies of a series request (one CTA).  out_n = their number, or EATS_NU_TILE + 1 when there are more
 // (or a NaN); band_of[i] = index of point i's frequency in the list; the list is kept as log2 / linear / ^(2/3).
 // The list grows in order of first appearance: each round appends the unmatched point of lowest index.
-__global__ void __launch_bounds__(1024) k_series_bands(const double* __restrict__ lg2_nu, const double* __restrict__ nu_lin,
-                                                        const double* __restrict__ nu23, int n, int* band_of, double* b_lg2,
-                                                        double* b_lin, double* b_23, int* out_n) {
+__device__ __forceinline__ void series_bands_cta(const double* __restrict__ lg2_nu, const double* __restrict__ nu_lin,
+                                                 const double* __restrict__ nu23, int n, int* band_of, double* b_lg2,
+                                                 double* b_lin, double* b_23, int* out_n) {
     __shared__ double s_u[EATS_NU_TILE + 1];
     __shared__ int s_cnt, s_cand;
     if (threadIdx.x == 0) s_cnt = 0;
@@ -351,6 +352,11 @@ __global__ void __launch_bounds__(1024) k_series_bands(const double* __restrict_
         __syncthreads();
     }
     if (threadIdx.x == 0) *out_n = s_cnt;
+}
+__global__ void __launch_bounds__(1024) k_series_bands(const double* __restrict__ lg2_nu, const double* __restrict__ nu_lin,
+                                                        const double* __restrict__ nu23, int n, int* band_of, double* b_lg2,
+                                                        double* b_lin, double* b_23, int* out_n) {
+    series_bands_cta(lg2_nu, nu_lin, nu23, n, band_of, b_lg2, b_lin, b_23, out_n);
 }
 
 // Observer::flux (src/core/observer.h:555-567): band[m][c][j] = sum_i F[m][c][i][j] * w[i]
@@ -477,14 +483,11 @@ __global__ void k_total(double* out, size_t n_models, size_t comp_sz) {
 // accumulate: add to chi2[] (band terms after the point term, fitter.py:525-531).
 // ext (per point) with av (per model): host extinction F e^{-A_V k} shifts the observed value to lnF + A_V k.  The
 // explicit intrinsics round the product, then the sum, as numpy does; a contracted FMA would differ in the last bit.
-__global__ void k_chi2(const double* __restrict__ flux, size_t n_models, int n, const double* __restrict__ lnF,
-                       const double* __restrict__ sigma_ln, const double* __restrict__ wgt,
-                       const double* __restrict__ av, const double* __restrict__ ext, double* chi2,
-                       const int* __restrict__ status, int accumulate) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (warp >= (int)n_models) return;
-    const double* F = flux + (size_t)warp * VAG_NCOMP * n;  // total
+// (the warp of model `warp`: F its total plane, the data its point slice)
+__device__ __forceinline__ void chi2_warp(int warp, int lane, const double* __restrict__ F, int n, const double* __restrict__ lnF,
+                                          const double* __restrict__ sigma_ln, const double* __restrict__ wgt,
+                                          const double* __restrict__ av, const double* __restrict__ ext, double* chi2,
+                                          const int* __restrict__ status, int accumulate) {
     double s = 0;
     if (ext) {
         const double a = av[warp];
@@ -500,6 +503,16 @@ __global__ void k_chi2(const double* __restrict__ flux, size_t n_models, int n, 
         const bool fatal = status && (status[warp] & VAG_ST_ODE_FAIL500);
         chi2[warp] = (isfinite(s) && !fatal) ? s : kInf;
     }
+}
+__global__ void k_chi2(const double* __restrict__ flux, size_t n_models, int n, const double* __restrict__ lnF,
+                       const double* __restrict__ sigma_ln, const double* __restrict__ wgt,
+                       const double* __restrict__ av, const double* __restrict__ ext, double* chi2,
+                       const int* __restrict__ status, int accumulate) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (warp >= (int)n_models) return;
+    const double* F = flux + (size_t)warp * VAG_NCOMP * n;  // total
+    chi2_warp(warp, lane, F, n, lnF, sigma_ln, wgt, av, ext, chi2, status, accumulate);
 }
 
 // vag_details_ic: [VAG_IC_DETAIL_PLANES][n_cells] <- IcCell records
@@ -611,6 +624,227 @@ __global__ void k_reject(const int32_t* __restrict__ ok, int32_t* status, double
     for (size_t i = threadIdx.x; out && i < per_model; i += blockDim.x) out[mi * per_model + i] = NAN;
 }
 
+// ---- ragged series requests: every model has its own data set (vag_flux_density_series_multi, vag_chi2_multi) ----------
+// A data set is a slice of the concatenated points, sorted by time within the slice.  Its distinct frequencies (banded
+// runs) sit at [set * EATS_NU_TILE] of the band tables.  Model m's output is [VAG_NCOMP][n of its set] at point offset
+// out_off[m] - out_off[0] of the pass's output.  These kernels are the shared-request ones with the request rebased per
+// model; every model's arithmetic is that of the shared-request kernels on its own data set.
+struct SeriesSet {
+    int off, n;   // slice of the concatenated points
+    int n_bands;  // distinct frequencies of the slice (k_series_bands_sets)
+    int pad_;
+};
+struct SetsDev {
+    const int* set_of;         // [models of the pass] data set of each model
+    SeriesSet* sets;           // [n_sets]
+    const long long* out_off;  // [models of the pass] first output point of each model (prefix sums over the batch)
+};
+
+// K0 with each model's observation window taken from its own data set
+template <int G>
+__global__ void __launch_bounds__(128, GRID_MIN_BLOCKS) k_grid_sets(BatchWs w, const double* __restrict__ t_obs, SetsDev sd) {
+    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+    const int mi = gt / G;
+    if (mi >= w.n_models) return;  // whole groups exit together
+    const int lane = threadIdx.x & 31;
+    const int shift = lane & ~(G - 1);
+    const GroupPar<G> par{lane & (G - 1), (G == 32 ? 0xffffffffu : ((1u << (G & 31)) - 1u)) << shift, shift};
+    const SeriesSet s = sd.sets[sd.set_of[mi]];
+    k0_grid_body(par, w, mi, t_obs[s.off], t_obs[s.off + s.n - 1]);
+}
+
+// k_series_bands per data set (CTA / set) into sets[].n_bands and the set's band table.  red[0] = max over the sets of
+// n_bands, red[1] = min over the sets of floor(3 n / n_bands): the batch is banded when every set passes series_banded
+// (see series_banded_sets).  red is preset to {0, INT_MAX} by the caller.
+__global__ void __launch_bounds__(256) k_series_bands_sets(const double* __restrict__ lg2_nu, const double* __restrict__ nu_lin,
+                                                           const double* __restrict__ nu23, SeriesSet* sets, int* band_of,
+                                                           double* b_lg2, double* b_lin, double* b_23, int* red) {
+    const int d = blockIdx.x;
+    const int off = sets[d].off, n = sets[d].n;
+    const size_t b = (size_t)d * EATS_NU_TILE;
+    series_bands_cta(lg2_nu + off, nu_lin + off, nu23 + off, n, band_of + off, b_lg2 + b, b_lin + b, b_23 + b,
+                     &sets[d].n_bands);
+    if (threadIdx.x == 0) {
+        const int nb = sets[d].n_bands;
+        atomicMax(red, nb);
+        atomicMin(red + 1, (int)min(3LL * n / max(nb, 1), (long long)INT_MAX));
+    }
+}
+
+// k_nu_range per model (warp / model): out[2 m], out[2 m + 1] = log2 of the smallest / largest frequency of its data set
+__global__ void k_nu_range_sets(const double* __restrict__ lg2_nu, SetsDev sd, int n_models, double* out) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (warp >= n_models) return;
+    const SeriesSet s = sd.sets[sd.set_of[warp]];
+    double lo = kInf, hi = -kInf;
+    for (int i = lane; i < s.n; i += 32) {
+        lo = fmin(lo, lg2_nu[s.off + i]);
+        hi = fmax(hi, lg2_nu[s.off + i]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if (lane == 0) {
+        out[2 * warp] = lo;
+        out[2 * warp + 1] = hi;
+    }
+}
+
+// K2b with each model's SSC tables sized by its own data set's band (nu_range_of: k_nu_range_sets)
+__global__ void __launch_bounds__(128) k_ic_spectrum_sets(BatchWs w, int n_rows, int n_warps, const double* __restrict__ nu_range_of) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const WarpPar par{(int)(threadIdx.x & 31)};
+    double* scratch = w.ic_scratch + (size_t)warp * IC_SCRATCH_DOUBLES;
+    BatchWs wm = w;
+    for (long long g = warp; g < w.n_cells; g += n_warps) {
+        int lo = 0, hi = n_rows;
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (w.row_cell_off[mid] <= g)
+                lo = mid;
+            else
+                hi = mid;
+        }
+        const int row = lo;
+        const int k = (int)(g - w.row_cell_off[row]);
+        const int mi = w.row_model[row];
+        const ModelCfg& cfg = w.cfg[mi];
+        wm.nu_range = nu_range_of + 2 * (size_t)mi;
+        for (int which = 0; which < 2; ++which) {
+            if (which && !cfg.has_rvs) continue;
+            if (!(which ? cfg.rvs : cfg.fwd).ssc) continue;
+            const int st = k2b_ic_spectrum_cell(par, wm, row, k, which, scratch);
+            if (st && par.lane == 0) atomicOr(&w.status[mi], st);
+        }
+    }
+}
+
+// K3 on a ragged request: k_eats with the CTA's request rebased on its model's data set (KIND: EATS_POINT or EATS_BANDED)
+// and the model's [VAG_NCOMP][n] block written at its output offset.  A copy of k_eats' CTA rather than a shared body:
+// the existing instantiations keep their code exactly (a shared inline body changed their instruction schedule).
+template <int MODE, int KIND>
+__global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats_sets(BatchWs w, EatsRequest rq0, SetsDev sd,
+                                                 double* __restrict__ out, int n_split, int row_chunk, int max_n_t,
+                                                 int nu_tile, size_t split_stride) {
+    extern __shared__ __align__(16) double smem[];
+    const int mi = blockIdx.x;
+    const int split = blockIdx.y;
+    const int which = (int)blockIdx.z + (MODE == 2 ? 2 : 0);  // 0 fwd sync, 1 rvs sync, 2 fwd ssc, 3 rvs ssc
+    {
+        const ModelCfg& cfg = w.cfg[mi];
+        if ((which & 1) && !cfg.has_rvs) return;
+        const bool ssc = ((which & 1) ? cfg.rvs : cfg.fwd).ssc != 0;
+        if ((MODE == 0) == ssc) return;  // MODE 0 handles the shocks without ssc, MODE 1/2 those with
+    }
+    if (w.status[mi] & VAG_ST_CAPACITY) return;
+    EatsModel M = make_eats_model(w, mi, which);
+    M.breach = &w.status[mi];
+    {
+        // log2_softplus table -> head of the dynamic shared memory (16-byte aligned rows)
+        for (int a = threadIdx.x; a < SPL_DOUBLES; a += blockDim.x) smem[a] = w.sp_lut[a];
+        M.sp_lut = smem;
+    }
+    const int n_t = M.h->n_t;
+    const int erows = M.h->n_theta * M.h->n_phi_eff;
+    constexpr bool series = KIND != EATS_GRID;
+    constexpr bool banded = KIND == EATS_BANDED;  // series points read a (node, band) tile staged as in grid mode
+    double* acc = smem + SPL_DOUBLES;     // [acc_cols][acc_stride]
+    const int acc_stride = rq0.acc_stride;
+    const int acc_cols = series ? 1 : nu_tile;
+    EatsShared sh = eats_carve(acc + acc_cols * acc_stride, max_n_t, series && !banded, row_chunk, nu_tile);
+    EatsRequest rq = rq0;
+    const int set = sd.set_of[mi];
+    const SeriesSet ds = sd.sets[set];
+    {
+        rq.n_t_obs = rq.n_nu = ds.n;
+        rq.lg2_t_obs += ds.off;
+        rq.t_obs_lin += ds.off;
+        const size_t nu_off = KIND == EATS_BANDED ? (size_t)set * EATS_NU_TILE : (size_t)ds.off;  // band table / points
+        rq.lg2_nu_obs += nu_off;
+        rq.nu_obs_lin += nu_off;
+        rq.nu23_obs += nu_off;
+        rq.n_bands = KIND == EATS_BANDED ? ds.n_bands : 0;
+        rq.band_of += ds.off;
+    }
+    const int tid = threadIdx.x, nthr = blockDim.x;
+    const int comp = which == 0 ? VAG_C_FWD_SYNC : which == 1 ? VAG_C_RVS_SYNC : which == 2 ? VAG_C_FWD_SSC : VAG_C_RVS_SSC;
+    const size_t comp_sz = series ? (size_t)rq.n_t_obs : (size_t)rq.n_nu * rq.n_t_obs;
+    // row-split batches (n_split > 1, small batches): each split owns a slab of `out` (= the partial buffer) and
+    // k_sum_splits adds the slabs in split order -- deterministic, unlike an atomicAdd into one cell
+    double* dst = out + (size_t)split * split_stride + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP + comp * comp_sz;
+    const int n_nu_tiles = series ? 1 : (rq.n_nu + nu_tile - 1) / nu_tile;
+    const RowGeom* rowg = w.rowgeom + (size_t)mi * w.max_erows;
+    // rows per pass: this model's lattice may be shorter than the batch maximum the buffers are sized for
+    const int rpp = eats_rows_per_pass(n_t, row_chunk, nthr);
+    for (int tile = 0; tile < n_nu_tiles; ++tile) {
+        const int l0 = tile * nu_tile;
+        const int nl = series ? (banded ? rq.n_bands : 1) : imin(nu_tile, rq.n_nu - l0);
+        for (int i0 = 0; i0 < rq.n_t_obs; i0 += EATS_T_BLOCK) {
+            rq.i0 = i0;
+            rq.ni = imin(EATS_T_BLOCK, rq.n_t_obs - i0);
+            // zeroed by the thread that accumulates into and finally reads the column (ii == tid mod nthr): no barrier is
+            // needed even when this split has no pass to run (compute-sanitizer racecheck, profiles/r02_sanitize.txt)
+            for (int ii = tid; ii < rq.ni; ii += nthr)
+                for (int l = 0; l < acc_cols; ++l) acc[l * acc_stride + ii] = 0.0;
+            for (int q0 = split * rpp; q0 < erows; q0 += n_split * rpp) {
+                const int nrows = imin(rpp, erows - q0);
+                sh.rowg = rowg + q0;
+                __syncthreads();  // previous pass finished reading the staged rows (and the table is loaded)
+                eats_phase1<MODE, KIND == EATS_POINT>(M, rq, sh, nrows, l0, nl, tid, nthr);
+                __syncthreads();
+                if (banded)
+                    eats_phase2_banded(M, rq, sh, nrows, acc, tid, nthr);
+                else if (series)
+                    eats_phase2_series<MODE>(M, rq, sh, nrows, acc, tid, nthr);
+                else
+                    eats_phase2_grid(M, rq, sh, nrows, nl, acc, tid, nthr);
+            }
+            // accumulator columns are thread-owned (ii == tid mod nthr): no barrier needed here
+            for (int ii = tid; ii < rq.ni; ii += nthr) {
+                for (int l = 0; l < (series ? 1 : nl); ++l) {
+                    const double v = flux_scale(M, acc[l * acc_stride + ii]);
+                    double* p = series ? (dst + i0 + ii) : (dst + (size_t)(l0 + l) * rq.n_t_obs + i0 + ii);
+                    *p = v;
+                }
+            }
+            __syncthreads();
+        }
+    }
+}
+
+// k_total on a ragged output (CTA / model)
+__global__ void k_total_sets(double* out, SetsDev sd) {
+    const int mi = blockIdx.x;
+    const size_t cs = (size_t)sd.sets[sd.set_of[mi]].n;
+    double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
+    for (size_t e = threadIdx.x; e < cs; e += blockDim.x)
+        o[e] = o[VAG_C_FWD_SYNC * cs + e] + o[VAG_C_FWD_SSC * cs + e] + o[VAG_C_RVS_SYNC * cs + e] + o[VAG_C_RVS_SSC * cs + e];
+}
+
+// k_nan_capacity on a ragged output (CTA / model)
+__global__ void k_nan_capacity_sets(BatchWs w, double* out, SetsDev sd) {
+    const int mi = blockIdx.x;
+    if (!(w.status[mi] & VAG_ST_CAPACITY)) return;
+    const size_t per_model = (size_t)VAG_NCOMP * sd.sets[sd.set_of[mi]].n;
+    double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
+    for (size_t i = threadIdx.x; i < per_model; i += blockDim.x) o[i] = NAN;
+}
+
+// K4 on a ragged request: the warp of model m reads its total plane and its data set's slice of the data (ext: of ext_k)
+__global__ void k_chi2_sets(const double* __restrict__ flux, size_t n_models, SetsDev sd, const double* __restrict__ lnF,
+                            const double* __restrict__ sigma_ln, const double* __restrict__ wgt, const double* __restrict__ av,
+                            const double* __restrict__ ext, double* chi2, const int* __restrict__ status) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (warp >= (int)n_models) return;
+    const SeriesSet s = sd.sets[sd.set_of[warp]];
+    const double* F = flux + (size_t)(sd.out_off[warp] - sd.out_off[0]) * VAG_NCOMP;  // total
+    chi2_warp(warp, lane, F, s.n, lnF + s.off, sigma_ln + s.off, wgt + s.off, av, ext ? ext + s.off : nullptr, chi2, status, 0);
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -658,12 +892,12 @@ struct vag_context {
     int device = 0;
     cudaStream_t stream = nullptr;
     DevBuf model_buf, row_buf, cell_buf, obs_buf, ic_buf, lut_buf, sp_buf, geom_buf, split_buf, work_buf;
-    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs;  // staging of the host-buffer entry points
+    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs, io_sets;  // staging of the host-buffer entry points
     DevBuf plan_buf;                // device planning: the records that run, ok[], capacities
     int* h_totals = nullptr;        // pinned
     int* h_caps = nullptr;          // pinned: capacities planned on the device
     long long* h_cells = nullptr;   // pinned
-    int* h_bands = nullptr;         // pinned: distinct frequencies of the series request in flight
+    int* h_bands = nullptr;         // pinned [2]: distinct frequencies of the series request in flight (ragged: see k_series_bands_sets)
     int series_mode = 0;            // vag_set_series_mode: 0 auto, 1 per-point spectra always, 2 banded whenever possible
     int grid_lanes = 0;             // vag_set_grid_lanes: 0 by batch size, else k_grid<grid_lanes> for every batch
     int cap_theta = 384, cap_phi = 128;  // vag_set_capacity: what the *_dev entry points run with (host calls size each batch)
@@ -708,6 +942,13 @@ struct Request {
     const double *d_lnF = nullptr, *d_sig = nullptr, *d_w = nullptr;  // [n_t] observations of a chi-squared series
     const double* d_ext = nullptr;  // [n_t] extinction per point, or NULL
     const double* d_av = nullptr;   // [n_models] A_V per model of the batch, set with d_ext (run_flux offsets it per pass)
+    // A ragged series request (every model its own data set; d_t ... d_ext concatenated over the sets): the device
+    // tables (run_flux slices set_of and out_off per pass), the host prefix sums of the models' output points
+    // [n_models + 1], the number of sets and the size of the largest
+    const SetsDev* sets = nullptr;
+    const long long* h_off = nullptr;
+    int n_sets = 0;
+    size_t max_set = 0;
 };
 
 int setup_models(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps) {
@@ -808,6 +1049,10 @@ constexpr int EATS_MODES = 3, EATS_KINDS = 3;
 // (defined after run_front: the cubin lists the kernel templates in the order the source first names them)
 GridKernel grid_kernel(int lanes);
 EatsKernel eats_kernel(int mode, int kind);
+using GridSetsKernel = void (*)(BatchWs, const double*, SetsDev);
+using EatsSetsKernel = void (*)(BatchWs, EatsRequest, SetsDev, double*, int, int, int, int, size_t);
+GridSetsKernel grid_sets_kernel(int lanes);
+EatsSetsKernel eats_sets_kernel(int mode, bool banded);
 
 // Lanes per model of k_grid: the widest group whose launch fits into one wave of resident CTAs (GRID_MIN_BLOCKS CTAs of
 // 128 threads per SM).  Narrower groups only pay once a wider launch would need a second wave: the models of one warp
@@ -823,13 +1068,17 @@ int grid_lanes_for(size_t n, int sm_count) {
 }
 
 // grid + dynamics + radiation for a batch; fills w and the totals
+// (sets: each model's observation window from its own data set of d_t)
 int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps, const double* d_t,
-              size_t n_t, cudaStream_t s, int* totals_out, long long* cells_out) {
+              size_t n_t, cudaStream_t s, int* totals_out, long long* cells_out, const SetsDev* sets = nullptr) {
     int rc = setup_models(ctx, w, d_params, n, caps);
     if (rc) return rc;
     mark(ctx, 0, s);
     const int lanes = ctx->grid_lanes ? ctx->grid_lanes : grid_lanes_for(n, ctx->sm_count);
-    grid_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
+    if (sets)
+        grid_sets_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, *sets);
+    else
+        grid_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
     k_scan<<<1, 1024, 0, s>>>(w);
     ctx->launches += 2;
     CK(cudaMemcpyAsync(ctx->h_totals, w.totals, sizeof(int) * TOT_N, cudaMemcpyDeviceToHost, s));
@@ -909,12 +1158,31 @@ EatsKernel eats_kernel(int mode, int kind) {
     return k[mode][kind];
 }
 
+GridSetsKernel grid_sets_kernel(int lanes) {
+    switch (lanes) {
+        case 4: return k_grid_sets<4>;
+        case 8: return k_grid_sets<8>;
+        case 16: return k_grid_sets<16>;
+        default: return k_grid_sets<32>;
+    }
+}
+
+EatsSetsKernel eats_sets_kernel(int mode, bool banded) {
+    static const EatsSetsKernel k[EATS_MODES][2] = {{k_eats_sets<0, EATS_POINT>, k_eats_sets<0, EATS_BANDED>},
+                                                    {k_eats_sets<1, EATS_POINT>, k_eats_sets<1, EATS_BANDED>},
+                                                    {k_eats_sets<2, EATS_POINT>, k_eats_sets<2, EATS_BANDED>}};
+    return k[mode][banded ? 1 : 0];
+}
+
 // flux of a batch into d_out [n][VAG_NCOMP][comp]; with d_chi2, also the chi-squared of the series against rq_in's data
 int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, const Request& rq_in, double* d_out,
                   int32_t* d_status, double* d_chi2, cudaStream_t s) {
     const size_t n_t = rq_in.n_t, n_nu = rq_in.n_nu;
-    // observation arrays
-    CK(ctx->obs_buf.ensure(sizeof(double) * (2 * n_t + 3 * n_nu + 8 + 3 * EATS_NU_TILE) + sizeof(int) * (n_t + 2)));
+    const SetsDev* sets = rq_in.sets;
+    // observation arrays (a ragged request: one band table per data set, the SSC band of every model)
+    const size_t n_tables = sets ? (size_t)rq_in.n_sets : 1, n_ranges = sets ? 2 * n : 0;
+    CK(ctx->obs_buf.ensure(sizeof(double) * (2 * n_t + 3 * n_nu + 8 + 3 * EATS_NU_TILE * n_tables + n_ranges) +
+                           sizeof(int) * (n_t + 2)));
     double* lg2_t = static_cast<double*>(ctx->obs_buf.p);
     double* t_lin = lg2_t + n_t;
     double* lg2_nu = t_lin + n_t;
@@ -922,9 +1190,10 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
     double* nu23 = nu_lin + n_nu;
     double* nu_range = nu23 + n_nu;
     double* band_lg2 = nu_range + 8;
-    double* band_lin = band_lg2 + EATS_NU_TILE;
-    double* band_23 = band_lin + EATS_NU_TILE;
-    int* band_of = reinterpret_cast<int*>(band_23 + EATS_NU_TILE);
+    double* band_lin = band_lg2 + EATS_NU_TILE * n_tables;
+    double* band_23 = band_lin + EATS_NU_TILE * n_tables;
+    double* nu_range_of = band_23 + EATS_NU_TILE * n_tables;
+    int* band_of = reinterpret_cast<int*>(nu_range_of + n_ranges);
     int* d_n_bands = band_of + n_t;
     {
         const size_t m = std::max(n_t, n_nu);
@@ -935,40 +1204,62 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
     *ctx->h_bands = 0;
     if (rq_in.series && ctx->series_mode != 1) {
         // distinct frequencies of the request; the count reaches the host with run_front's synchronisation
-        k_series_bands<<<1, 1024, 0, s>>>(lg2_nu, nu_lin, nu23, (int)n_nu, band_of, band_lg2, band_lin, band_23, d_n_bands);
-        CK(cudaMemcpyAsync(ctx->h_bands, d_n_bands, sizeof(int), cudaMemcpyDeviceToHost, s));
+        if (sets) {
+            CK(cudaMemsetAsync(d_n_bands, 0, sizeof(int), s));
+            CK(cudaMemsetAsync(d_n_bands + 1, 0x7f, sizeof(int), s));
+            k_series_bands_sets<<<(unsigned)rq_in.n_sets, 256, 0, s>>>(lg2_nu, nu_lin, nu23, sets->sets, band_of, band_lg2,
+                                                                       band_lin, band_23, d_n_bands);
+            CK(cudaMemcpyAsync(ctx->h_bands, d_n_bands, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
+        } else {
+            k_series_bands<<<1, 1024, 0, s>>>(lg2_nu, nu_lin, nu23, (int)n_nu, band_of, band_lg2, band_lin, band_23, d_n_bands);
+            CK(cudaMemcpyAsync(ctx->h_bands, d_n_bands, sizeof(int), cudaMemcpyDeviceToHost, s));
+        }
         ctx->launches++;
     }
     BatchWs w;
     int totals[TOT_N];
     long long cells = 0;
-    int rc = run_front(ctx, w, d_params, n, caps, rq_in.d_t, n_t, s, totals, &cells);
+    int rc = run_front(ctx, w, d_params, n, caps, rq_in.d_t, n_t, s, totals, &cells, sets);
     if (rc) return rc;
 
     if (w.any_ssc && totals[TOT_ROWS] > 0) {
         // SSC tables: observation band -> per-row line-of-sight cosines -> per-k Doppler extrema -> tables
+        // (a ragged request: each model's band is its own data set's, as its shared-request call would see it)
         w.nu_range = nu_range;
-        k_nu_range<<<1, 256, 0, s>>>(lg2_nu, (int)n_nu, nu_range);
+        if (sets)
+            k_nu_range_sets<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(lg2_nu, *sets, (int)n, nu_range_of);
+        else
+            k_nu_range<<<1, 256, 0, s>>>(lg2_nu, (int)n_nu, nu_range);
         k_rowcos<<<dim3((unsigned)((w.max_erows + 127) / 128), (unsigned)n), 128, 0, s>>>(w);
         k_dop_extrema<<<dim3((unsigned)((w.max_n_t + 63) / 64), (unsigned)n), 64, 0, s>>>(w);
         const int n_ic_warps = (int)std::min<long long>(std::max<long long>(cells, 1), (long long)ctx->sm_count * ctx->ic_warps_per_sm);
-        k_ic_spectrum<<<(unsigned)((n_ic_warps * 32 + 127) / 128), 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps);
+        const unsigned ic_blocks = (unsigned)((n_ic_warps * 32 + 127) / 128);
+        if (sets)
+            k_ic_spectrum_sets<<<ic_blocks, 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps, nu_range_of);
+        else
+            k_ic_spectrum<<<ic_blocks, 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps);
         ctx->launches += 4;
     }
+    // points per component plane of a model (shared request), and the elements of the pass's output
     const size_t comp_sz = rq_in.series ? n_t : n_nu * n_t;
-    CK(cudaMemsetAsync(d_out, 0, sizeof(double) * n * VAG_NCOMP * comp_sz, s));
+    const size_t elems = sets ? (size_t)VAG_NCOMP * (rq_in.h_off[n] - rq_in.h_off[0]) : n * VAG_NCOMP * comp_sz;
+    CK(cudaMemsetAsync(d_out, 0, sizeof(double) * elems, s));
     const int max_n_t = std::max(totals[TOT_MAX_NT], 2);
     const int max_erows = std::max(totals[TOT_MAX_EROWS], 1);
     if (totals[TOT_ROWS] > 0) {
         // shared-memory budget -> rows staged per pass
         const size_t budget = EATS_SMEM_BUDGET;
         int row_chunk = EATS_ROW_CHUNK;
+        // a ragged request: h_bands = the largest set's distinct frequencies and min floor(3 n / n_bands) over the sets
         const int n_bands_req = rq_in.series ? *ctx->h_bands : 0;
-        const bool banded = series_banded(n_bands_req, max_n_t, n_t, ctx->series_mode);
+        const bool banded = sets ? ctx->series_mode != 1 && series_banded_sets(n_bands_req, ctx->h_bands[1], max_n_t,
+                                                                               ctx->series_mode)
+                                 : series_banded(n_bands_req, max_n_t, n_t, ctx->series_mode);
         const int nu_tile = rq_in.series ? (banded ? n_bands_req : 1) : (int)std::min<size_t>(EATS_NU_TILE, n_nu);
         const int acc_cols = rq_in.series ? 1 : nu_tile;
+        const int acc_n = (int)(sets ? rq_in.max_set : n_t);  // accumulator columns: the longest request of the batch
         auto smem_bytes = [&](int rc_) {
-            return sizeof(double) * (acc_cols * eats_acc_stride((int)n_t) +
+            return sizeof(double) * (acc_cols * eats_acc_stride(acc_n) +
                                      eats_shared_doubles(max_n_t, rq_in.series && !banded, rc_, nu_tile) + SPL_DOUBLES);
         };
         // fewer staged rows per pass while that buys residency: 8 CTAs / SM need <= 27 KB each (227 KB per SM,
@@ -987,7 +1278,7 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         const size_t target_ctas = (size_t)ctx->sm_count * EATS_MIN_BLOCKS * 2;
         const size_t have = n * (size_t)n_shock;
         int n_split = (have < target_ctas) ? (int)std::min<size_t>(chunks, (target_ctas + have - 1) / have) : 1;
-        const size_t slab_bytes = sizeof(double) * n * VAG_NCOMP * comp_sz;
+        const size_t slab_bytes = sizeof(double) * elems;
         while (n_split > 1 && slab_bytes * n_split > ((size_t)1 << 30)) --n_split;  // <= 1 GiB of slabs
         n_split = std::max(n_split, 1);
         const size_t sb = smem_bytes(row_chunk);  // <= EATS_SMEM_BUDGET, the opt-in limit set once in vag_create
@@ -1002,9 +1293,8 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         rq.n_bands = banded ? n_bands_req : 0;
         rq.band_of = band_of;
         rq.t_obs_lin = t_lin;
-        rq.acc_stride = eats_acc_stride((int)n_t);
+        rq.acc_stride = eats_acc_stride(acc_n);
         const dim3 eg((unsigned)n, (unsigned)n_split, (unsigned)n_shock);  // no reverse shock in the batch: no z = 1 CTAs
-        const size_t elems = n * VAG_NCOMP * comp_sz;
         double* eats_out = d_out;
         if (n_split > 1) {
             CK(ctx->split_buf.ensure(sizeof(double) * elems * n_split));
@@ -1013,8 +1303,13 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         }
         const int kind = !rq_in.series ? EATS_GRID : banded ? EATS_BANDED : EATS_POINT;
         const int n_modes = w.any_ssc ? EATS_MODES : 1;
-        for (int mode = 0; mode < n_modes; ++mode)
-            eats_kernel(mode, kind)<<<eg, 128, sb, s>>>(w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
+        for (int mode = 0; mode < n_modes; ++mode) {
+            if (sets)
+                eats_sets_kernel(mode, banded)<<<eg, 128, sb, s>>>(w, rq, *sets, eats_out, n_split, row_chunk, max_n_t,
+                                                                   nu_tile, elems);
+            else
+                eats_kernel(mode, kind)<<<eg, 128, sb, s>>>(w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
+        }
         ctx->launches += n_modes;
         if (n_split > 1) {
             k_sum_splits<<<(unsigned)((elems + 255) / 256), 256, 0, s>>>(d_out, eats_out, n_split, elems);
@@ -1024,18 +1319,28 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
     mark(ctx, 4, s);
     {
         const size_t tot = n * comp_sz;
-        k_total<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(d_out, n, comp_sz);
+        if (sets)
+            k_total_sets<<<(unsigned)n, 128, 0, s>>>(d_out, *sets);
+        else
+            k_total<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(d_out, n, comp_sz);
         ctx->launches++;
         // the SSC lattices can overflow later than the grid (k_ic_spectrum sets the bit after k_scan read the OR):
         // with ssc shocks in the batch the kernel runs unconditionally and tests each model's bit on the device
         if ((totals[TOT_STATUS_OR] & VAG_ST_CAPACITY) || w.any_ssc) {
-            k_nan_capacity<<<(unsigned)n, 128, 0, s>>>(w, d_out, VAG_NCOMP * comp_sz);
+            if (sets)
+                k_nan_capacity_sets<<<(unsigned)n, 128, 0, s>>>(w, d_out, *sets);
+            else
+                k_nan_capacity<<<(unsigned)n, 128, 0, s>>>(w, d_out, VAG_NCOMP * comp_sz);
             ctx->launches++;
         }
     }
     if (d_chi2) {
-        k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
-                                                                 rq_in.d_av, rq_in.d_ext, d_chi2, w.status, 0);
+        if (sets)
+            k_chi2_sets<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, *sets, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
+                                                                          rq_in.d_av, rq_in.d_ext, d_chi2, w.status);
+        else
+            k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
+                                                                     rq_in.d_av, rq_in.d_ext, d_chi2, w.status, 0);
         ctx->launches++;
     }
     mark(ctx, 5, s);
@@ -1060,7 +1365,14 @@ int run_flux(vag_context* ctx, const vag_params* d_params, size_t n, Caps caps, 
         const size_t m = std::min(MAX_MODELS_PER_PASS, n - lo);
         Request rq_pass = rq;
         if (rq.d_av) rq_pass.d_av = rq.d_av + lo;
-        if (int rc = run_flux_pass(ctx, d_params + lo, m, caps, rq_pass, d_out + lo * VAG_NCOMP * comp_sz,
+        SetsDev sets_pass{};
+        if (rq.sets) {
+            sets_pass = SetsDev{rq.sets->set_of + lo, rq.sets->sets, rq.sets->out_off + lo};
+            rq_pass.sets = &sets_pass;
+            rq_pass.h_off = rq.h_off + lo;
+        }
+        const size_t out_lo = rq.sets ? (size_t)rq.h_off[lo] * VAG_NCOMP : lo * VAG_NCOMP * comp_sz;
+        if (int rc = run_flux_pass(ctx, d_params + lo, m, caps, rq_pass, d_out + out_lo,
                                    d_status ? d_status + lo : nullptr, d_chi2 ? d_chi2 + lo : nullptr, s))
             return rc;
     }
@@ -1150,7 +1462,7 @@ int vag_create(int device, vag_context** out) {
     CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     CK(cudaMallocHost(&c->h_totals, sizeof(int) * TOT_N));
     CK(cudaMallocHost(&c->h_cells, sizeof(long long)));
-    CK(cudaMallocHost(&c->h_bands, sizeof(int)));
+    CK(cudaMallocHost(&c->h_bands, 2 * sizeof(int)));
     CK(cudaMallocHost(&c->h_caps, sizeof(int) * 2));
     for (auto& ev : c->ev) CK(cudaEventCreate(&ev));
     {
@@ -1181,6 +1493,11 @@ int vag_create(int device, vag_context** out) {
     for (int mode = 0; mode < EATS_MODES; ++mode)
         for (int kind = 0; kind < EATS_KINDS; ++kind)
             CK(cudaFuncSetAttribute(eats_kernel(mode, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET));
+    for (int lanes : GRID_LANES) cudaFuncSetCacheConfig(grid_sets_kernel(lanes), cudaFuncCachePreferL1);
+    for (int mode = 0; mode < EATS_MODES; ++mode)
+        for (bool banded : {false, true})
+            CK(cudaFuncSetAttribute(eats_sets_kernel(mode, banded), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)EATS_SMEM_BUDGET));
     {
         int blocks = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum, 128, 0) == cudaSuccess && blocks > 0)
@@ -1716,6 +2033,125 @@ int vag_chi2_series(vag_context* ctx, const vag_params* params, size_t n_models,
     if (n == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
     if (!nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
     return vag_chi2(ctx, params, n_models, t, nu, lnF_obs, sigma_ln, w, n, nullptr, 0, chi2, status);
+}
+
+// ---- ragged series requests: several data sets in one batch --------------------------------------------------------
+// The checks of vag_flux_density_series_multi and vag_chi2_multi that concern the data sets (before any work is enqueued)
+static int check_sets(size_t n_models, const int32_t* dataset_of, const vag_series_set* sets, size_t n_sets, const double* t,
+                      const double* nu, size_t n_points) {
+    if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no data sets: sets is NULL or n_sets is 0");
+    if (!t || !nu || n_points == 0) return fail(VAG_ERR_INVALID, "time and frequency arrays must be non-empty");
+    if (n_points > (size_t)INT_MAX || n_sets > (size_t)INT_MAX)
+        return fail(VAG_ERR_INVALID, "n_points_total and n_sets must fit in a 32-bit int");
+    if (n_models && !dataset_of) return fail(VAG_ERR_INVALID, "dataset_of is NULL");
+    for (size_t d = 0; d < n_sets; ++d) {
+        const std::string name = "data set " + std::to_string(d) + ": ";
+        const size_t off = sets[d].offset, n = sets[d].n;
+        if (n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
+        if (off > n_points || n > n_points - off)
+            return fail(VAG_ERR_INVALID, name + "points [" + std::to_string(off) + ", " + std::to_string(off) + " + " +
+                                             std::to_string(n) + ") lie outside the " + std::to_string(n_points) + " points");
+        if (check_times(t + off, n)) return fail(VAG_ERR_INVALID, name + g_err);
+        for (size_t i = off; i < off + n; ++i)
+            if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
+    }
+    for (size_t m = 0; m < n_models; ++m)
+        if (dataset_of[m] < 0 || (size_t)dataset_of[m] >= n_sets)
+            return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": dataset_of = " + std::to_string(dataset_of[m]) +
+                                             " is not a data set index (n_sets = " + std::to_string(n_sets) + ")");
+    return VAG_OK;
+}
+
+// The series flux (out != NULL) or the chi-squared (chi2 != NULL; data lnF / sig / w [/ ext] over the concatenated points,
+// A_V per model) of a ragged request from host buffers; arguments checked by the caller.  out: model m's
+// [VAG_NCOMP][n of its set] block at m's offset, the prefix sum of the sizes of the data sets of models 0 .. m-1.
+static int sets_host(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                     const vag_series_set* sets, size_t n_sets, const double* t, const double* nu, size_t n_points,
+                     const double* const* data, const double* ext_k, const double* A_V, double* out, double* chi2,
+                     int32_t* status) {
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) return VAG_OK;
+    std::vector<SeriesSet> hs(n_sets);
+    size_t max_set = 0;
+    for (size_t d = 0; d < n_sets; ++d) {
+        hs[d] = SeriesSet{(int)sets[d].offset, (int)sets[d].n, 0, 0};
+        max_set = std::max(max_set, sets[d].n);
+    }
+    std::vector<long long> off(n_models + 1, 0);
+    for (size_t m = 0; m < n_models; ++m) off[m + 1] = off[m] + (long long)sets[dataset_of[m]].n;
+    const size_t n_out = (size_t)off[n_models] * VAG_NCOMP;
+    cudaStream_t s = ctx->stream;
+    if (int rc = upload_request(ctx, t, n_points, nu, n_points)) return rc;
+    CK(ctx->io_sets.ensure(carve_sz<int>(n_models) + carve_sz<SeriesSet>(n_sets) + carve_sz<long long>(n_models)));
+    char* p = static_cast<char*>(ctx->io_sets.p);
+    int* d_set_of = carve<int>(p, n_models);
+    SeriesSet* d_sets = carve<SeriesSet>(p, n_sets);
+    long long* d_off = carve<long long>(p, n_models);
+    CK(cudaMemcpyAsync(d_set_of, dataset_of, sizeof(int) * n_models, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d_sets, hs.data(), sizeof(SeriesSet) * n_sets, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * n_models, cudaMemcpyHostToDevice, s));
+    const SetsDev sd{d_set_of, d_sets, d_off};
+    Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points, n_points};
+    rq.sets = &sd;
+    rq.h_off = off.data();
+    rq.n_sets = (int)n_sets;
+    rq.max_set = max_set;
+    double* d_chi2 = nullptr;
+    if (chi2) {
+        // observation staging: chi2 [n_models], lnF / sigma_ln / w [n_points] (with extinction ext_k [n_points], A_V [n_models])
+        CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * n_points + (ext_k ? n_points + n_models : 0))));
+        double* cur = static_cast<double*>(ctx->io_obs.p);
+        d_chi2 = cur;
+        cur += n_models;
+        auto stage = [&](const double* h, size_t n) -> const double* {
+            double* dv = cur;
+            cur += n;
+            return cudaMemcpyAsync(dv, h, sizeof(double) * n, cudaMemcpyHostToDevice, s) == cudaSuccess ? dv : nullptr;
+        };
+        rq.d_lnF = stage(data[0], n_points);
+        rq.d_sig = stage(data[1], n_points);
+        rq.d_w = stage(data[2], n_points);
+        if (ext_k) {
+            rq.d_ext = stage(ext_k, n_points);
+            rq.d_av = stage(A_V, n_models);
+        }
+        if (!rq.d_lnF || !rq.d_sig || !rq.d_w || (ext_k && (!rq.d_ext || !rq.d_av)))
+            return fail(VAG_ERR_CUDA, "staging the observations failed");
+    }
+    CK(ctx->io_out.ensure(sizeof(double) * std::max<size_t>(n_out, 1)));
+    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq, static_cast<double*>(ctx->io_out.p),
+                          static_cast<int32_t*>(ctx->io_status.p), d_chi2, s))
+        return rc;
+    if (out) CK(cudaMemcpyAsync(out, ctx->io_out.p, sizeof(double) * n_out, cudaMemcpyDeviceToHost, s));
+    if (chi2) CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
+    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
+}
+
+int vag_flux_density_series_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                  const vag_series_set* sets, size_t n_sets, const double* t, const double* nu,
+                                  size_t n_points_total, double* out, int32_t* status) {
+    if (!ctx || !out) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (int rc = check_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total)) return rc;
+    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, n_points_total, nullptr, nullptr, nullptr, out,
+                     nullptr, status);
+}
+
+int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                   const vag_series_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                   const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total, const double* A_V,
+                   double* chi2, int32_t* status) {
+    if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (!lnF_obs || !sigma_ln || !w) return fail(VAG_ERR_INVALID, "data arrays must not be NULL");
+    if ((ext_k != nullptr) != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (int rc = check_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total)) return rc;
+    for (size_t i = 0; ext_k && i < n_points_total; ++i)
+        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
+    const double* data[3] = {lnF_obs, sigma_ln, w};
+    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, n_points_total, data, ext_k, A_V, nullptr, chi2,
+                     status);
 }
 
 // ---- device-buffer entry points that plan on the device --------------------------------------------------------

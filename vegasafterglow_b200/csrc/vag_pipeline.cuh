@@ -628,4 +628,11 @@ inline bool series_banded(int n_bands, int max_n_t, size_t n_points, int series_
     return n_bands >= 1 && n_bands <= EATS_NU_TILE && (series_mode == 2 || (size_t)n_bands * max_n_t <= 3 * n_points);
 }
 
+// A ragged request (several data sets, vag_chi2_multi) runs banded when every data set passes series_banded with the
+// batch's max_n_t.  With max_bands = the largest count of distinct frequencies of a set and min_q = the smallest
+// floor(3 n / n_bands) of a set, that is this test: n_bands * max_n_t <= 3 n  <=>  max_n_t <= floor(3 n / n_bands).
+inline bool series_banded_sets(int max_bands, int min_q, int max_n_t, int series_mode) {
+    return max_bands >= 1 && max_bands <= EATS_NU_TILE && (series_mode == 2 || max_n_t <= min_q);
+}
+
 }  // namespace vag

@@ -152,6 +152,81 @@ class Engine:
                                           st.ctypes.data))
         return (out, st) if return_status else out
 
+    # ---- several data sets in one batch (include/vag.h vag_flux_density_series_multi, vag_chi2_multi) -------------------
+    @staticmethod
+    def _concat_sets(datasets, names):
+        """Per-data-set column tuples -> (the columns concatenated over the sets, ``abi.SeriesSet`` array, their number)."""
+        cols, sizes = [[] for _ in names], []
+        for d, ds in enumerate(datasets):
+            arrs = [_f64(a).reshape(-1) for a in ds]
+            if len(arrs) != len(names) or len({a.size for a in arrs}) != 1:
+                raise ValueError(f"data set {d} must be ({', '.join(names)}) of one size")
+            for c, a in zip(cols, arrs):
+                c.append(a)
+            sizes.append(arrs[0].size)
+        if not sizes:
+            raise ValueError("no data sets")
+        sets = (abi.SeriesSet * len(sizes))()
+        offsets = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
+        for d, (o, n) in enumerate(zip(offsets, sizes)):
+            sets[d] = abi.SeriesSet(int(o), int(n))
+        return [np.concatenate(c) for c in cols], sets, np.asarray(sizes, dtype=np.int64)
+
+    @staticmethod
+    def _dataset_of(dataset_of, n_models):
+        ds = np.asarray(dataset_of).reshape(-1)
+        if ds.size != n_models:
+            raise ValueError(f"dataset_of has {ds.size} entries for {n_models} models")
+        if ds.size and not (np.issubdtype(ds.dtype, np.integer) and ds.min() >= -2**31 and ds.max() < 2**31):
+            raise ValueError("dataset_of must hold int32 data-set indices")
+        return np.ascontiguousarray(ds, dtype=np.int32)
+
+    def flux_density_series_multi(self, params, datasets, dataset_of, return_status=False):
+        """``flux_density_series`` of model m on its own data set ``datasets[dataset_of[m]]`` = (t, nu), t ascending,
+        all in one batch.  Returns a list with one float64[5, n_d] array per model (n_d: the size of its data set); the
+        arrays are views into one buffer in model order (``vag_flux_density_series_multi``)."""
+        p = self._params(params)
+        (t, nu), sets, sizes = self._concat_sets(datasets, ("t", "nu"))
+        ds = self._dataset_of(dataset_of, p.size)
+        n_m = sizes[ds] if p.size else np.zeros(0, dtype=np.int64)
+        off = np.concatenate([[0], np.cumsum(n_m)]).astype(np.int64)
+        buf = np.empty(abi.NCOMP * int(off[-1]))
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_flux_density_series_multi(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p),
+                                                           len(sets), t.ctypes.data, nu.ctypes.data, t.size, buf.ctypes.data,
+                                                           st.ctypes.data))
+        out = [buf[abi.NCOMP * off[m]:abi.NCOMP * off[m + 1]].reshape(abi.NCOMP, int(n_m[m])) for m in range(p.size)]
+        return (out, st) if return_status else out
+
+    def chi2_multi(self, params, datasets, dataset_of, extinction=None, return_status=False):
+        """``chi2_series`` of model m on its own data set ``datasets[dataset_of[m]]`` = (t, nu, lnF_obs, sigma_ln, w), t
+        ascending, all in one batch -> chi2[n_models].  ``extinction`` = (ext_k, A_V): one ext_k array per data set (in the
+        order of its points) and A_V[n_models]; model m's points are then compared as lnF_obs + A_V[m] * ext_k
+        (``vag_chi2_multi``, the rules of ``chi2(extinction=...)``)."""
+        p = self._params(params)
+        (t, nu, lnF, sig, w), sets, sizes = self._concat_sets(datasets, ("t", "nu", "lnF_obs", "sigma_ln", "w"))
+        ds = self._dataset_of(dataset_of, p.size)
+        ext = av = None
+        if extinction is not None:
+            ext_sets, av = extinction
+            if len(ext_sets) != len(sizes):
+                raise ValueError(f"extinction has {len(ext_sets)} ext_k arrays for {len(sizes)} data sets")
+            ext = [_f64(e).reshape(-1) for e in ext_sets]
+            for d, (e, n) in enumerate(zip(ext, sizes)):
+                if e.size != n:
+                    raise ValueError(f"data set {d}: ext_k has {e.size} values for {n} points")
+            ext = np.concatenate(ext)
+            av = _f64(av).reshape(-1)
+            if av.size != p.size:
+                raise ValueError(f"A_V has {av.size} values for {p.size} models")
+        out = np.empty(p.size)
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_chi2_multi(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p), len(sets),
+                                            t.ctypes.data, nu.ctypes.data, lnF.ctypes.data, sig.ctypes.data, w.ctypes.data,
+                                            None if ext is None else ext.ctypes.data, t.size,
+                                            None if av is None else av.ctypes.data, out.ctypes.data, st.ctypes.data))
+        return (out, st) if return_status else out
+
     @staticmethod
     def valid_mask(params):
         """bool[n]: which parameter sets pass the constructor checks of the reference (vag_params_validate_batch)."""

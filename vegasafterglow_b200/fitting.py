@@ -151,24 +151,30 @@ class BatchedLikelihood:
             out[ok] = self._evaluate(P[ok], *(a[ok] for a in per_walker))
         return out
 
-    def __call__(self, samples: np.ndarray) -> np.ndarray:
-        samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
-        n = samples.shape[0]
-        in_bounds = np.ones(n, dtype=bool)
+    def _in_bounds(self, samples: np.ndarray) -> np.ndarray:
+        """Indices of the samples inside [lower, upper]."""
+        in_bounds = np.ones(samples.shape[0], dtype=bool)
         if self.lower is not None:
             in_bounds &= np.all(samples >= self.lower, axis=1)
         if self.upper is not None:
             in_bounds &= np.all(samples <= self.upper, axis=1)
-        logp = np.full(n, -np.inf)
-        idx = np.nonzero(in_bounds)[0]
+        return np.nonzero(in_bounds)[0]
+
+    def _log_prob(self, samples: np.ndarray, idx: np.ndarray, chi2: np.ndarray) -> np.ndarray:
+        """logp of every sample from the chi2 of the in-bounds ones (``idx``); -inf elsewhere and where not finite."""
+        logp = np.full(samples.shape[0], -np.inf)
         if idx.size:
-            chi2 = self.chi2(samples[idx])
             ll = np.where(np.isfinite(chi2), self.log_likelihood_fn(chi2), -np.inf)
             ll[~np.isfinite(ll)] = -np.inf
             if self.log_prior is not None:
                 ll = ll + self.log_prior(samples[idx])
             logp[idx] = ll
         return logp
+
+    def __call__(self, samples: np.ndarray) -> np.ndarray:
+        samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
+        idx = self._in_bounds(samples)
+        return self._log_prob(samples, idx, self.chi2(samples[idx]) if idx.size else np.zeros(0))
 
 
 
@@ -272,3 +278,66 @@ class DeviceLikelihood(BatchedLikelihood):
         sets = parallel.balanced_assignment(cost, world)
         mine = torch.as_tensor(sets[rank], dtype=torch.long, device=self.device)
         return parallel.gather_indexed_tensor(self._chi2_dev(cols[mine]), sets, cols.shape[0]).cpu().numpy()
+
+
+class LikelihoodStack:
+    """K independent fits evaluated together: ``__call__([samples_1, ..., samples_K]) -> [logp_1, ..., logp_K]`` with ONE
+    ``Engine.chi2_multi`` call, where each ``BatchedLikelihood`` called alone would make K calls.  Meant for many small
+    ensembles -- K emcee samplers stepped in lockstep, a catalogue of light curves, injection-recovery runs -- which
+    fill the GPU together where one alone would not.
+
+    Each likelihood keeps its own template, names, point data, bounds, prior, ``log_likelihood_fn`` and optional fitted
+    ``A_V``; fit k's walkers are evaluated on fit k's data set.  Bounds, rejected parameter sets and non-finite chi2 give
+    -inf as in ``BatchedLikelihood.__call__``.  When only some fits sample ``A_V``, the others run with ext_k = 0 and
+    A_V = 0, and lnF_obs + 0 * 0 is lnF_obs exactly.  The engine is the first likelihood's.
+    Not supported (``NotImplementedError``): band-integrated data, ``distributed=True`` and ``DeviceLikelihood``."""
+
+    def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
+        self.likelihoods = list(likelihoods)
+        if not self.likelihoods:
+            raise ValueError("LikelihoodStack needs at least one likelihood")
+        for k, lk in enumerate(self.likelihoods):
+            if isinstance(lk, DeviceLikelihood):
+                raise NotImplementedError(f"likelihood {k}: a DeviceLikelihood cannot be stacked (its data live in HBM)")
+            if lk.bands or not lk.t.size:
+                raise NotImplementedError(f"likelihood {k}: band-integrated data cannot be stacked (point data only)")
+            if lk.distributed:
+                raise NotImplementedError(f"likelihood {k}: distributed=True cannot be stacked")
+        self.engine = self.likelihoods[0].engine
+        self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) for lk in self.likelihoods]
+        self.fits_av = ["A_V" in lk.names for lk in self.likelihoods]
+
+    def chi2(self, samples):
+        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject."""
+        from .engine import Engine
+
+        P, ds, av, ok = [], [], [], []
+        for k, (lk, s) in enumerate(zip(self.likelihoods, samples)):
+            s = np.atleast_2d(np.asarray(s, dtype=np.float64))
+            p = lk.to_params(s)
+            good = Engine.valid_mask(p)
+            ok.append(good)
+            P.append(p[good])
+            ds.append(np.full(int(good.sum()), k, dtype=np.int32))
+            av.append(lk._column(s, lk.names.index("A_V"))[good] if self.fits_av[k] else np.zeros(int(good.sum())))
+        P, ds = np.concatenate(P), np.concatenate(ds)
+        extinction = None
+        if any(self.fits_av):
+            ext = [lk.ext_kernel if fit else np.zeros(lk.t.size) for lk, fit in zip(self.likelihoods, self.fits_av)]
+            extinction = (ext, np.concatenate(av))
+        flat = self.engine.chi2_multi(P, self.datasets, ds, extinction=extinction) if P.size else np.zeros(0)
+        out, lo = [], 0
+        for good in ok:
+            c = np.full(good.size, np.inf)
+            c[good] = flat[lo:lo + int(good.sum())]
+            lo += int(good.sum())
+            out.append(c)
+        return out
+
+    def __call__(self, samples):
+        if len(samples) != len(self.likelihoods):
+            raise ValueError(f"{len(samples)} sample arrays for {len(self.likelihoods)} likelihoods")
+        samples = [np.atleast_2d(np.asarray(s, dtype=np.float64)) for s in samples]
+        idx = [lk._in_bounds(s) for lk, s in zip(self.likelihoods, samples)]
+        chi2 = self.chi2([s[i] for s, i in zip(samples, idx)])
+        return [lk._log_prob(s, i, c) for lk, s, i, c in zip(self.likelihoods, samples, idx, chi2)]
