@@ -9,7 +9,9 @@ synchronisation) after a warm-up of each arm:
   sequential  K Engine.chi2_series calls, one per fit, on one engine
   threads     the same K calls spread over 4 engines (one CUDA stream each), one host thread per engine
   multi       one Engine.chi2_multi call on the K data sets
-Series mode 0 (the default) in every arm.  Check: the multi result against per-fit chi2_series calls padded to 2368
+Series mode 0 (the default) in every arm.  A second batch times one chi2_multi call on 8 of these fits whose odd
+fits are SSC+KN forward-shock draws instead (configs.random_draw(..., ssc=True, kn=True)), in series modes 0 and 2: the
+FS+RS fits never run the SSC kernels (k_ic_spectrum, k_eats MODE 2), and mode 0 never runs them banded.  Check: the multi result against per-fit chi2_series calls padded to 2368
 models (37 copies of the 64 walkers, so that neither call splits rows) in series mode 1 -- bit for bit where both calls
 stage the same rows per pass (include/vag.h) -- and the largest relative difference to the unpadded sequential arm.
 Prints the card's name and power limit, then one JSON line per arm and K and one for the check.
@@ -99,6 +101,26 @@ for K in args.k:
         print(json.dumps({"arm": a, "K": K, "walkers_per_fit": args.walkers, "ms_median": round(float(np.median(ms)), 3),
                           "ms_min": round(float(ms.min()), 3), "ms_per_fit": round(float(np.median(ms)) / K, 3),
                           "reps": args.reps}), flush=True)
+
+# ---- mixed batch with SSC+KN fits ---------------------------------------------------------------------------------------
+K_SSC = 8
+SSC_FITS = [(configs.random_draw(args.walkers, seed=3000 + k, ssc=True, kn=True) if k % 2 else
+             configs.random_draw(args.walkers, seed=2000 + k, rvs=True), light_curve(k)) for k in range(K_SSC)]
+P_SSC = np.concatenate([P for P, _ in SSC_FITS])
+DS_SSC = np.repeat(np.arange(K_SSC, dtype=np.int32), args.walkers)
+for mode in (0, 2):  # 0 picks per-point EATS on these light curves, 2 forces the banded one
+    engines[0].set_series_mode(mode)
+    engines[0].chi2_multi(P_SSC, [data for _, data in SSC_FITS], DS_SSC)  # warm-up
+    ms = []
+    for r in range(args.reps):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        engines[0].chi2_multi(P_SSC, [data for _, data in SSC_FITS], DS_SSC)
+        ms.append((time.perf_counter() - t0) * 1e3)
+    print(json.dumps({"arm": "multi_ssc_kn_mixed", "K": K_SSC, "walkers_per_fit": args.walkers, "series_mode": mode,
+                      "ms_median": round(float(np.median(ms)), 3), "ms_min": round(float(np.min(ms)), 3),
+                      "reps": args.reps}), flush=True)
+engines[0].set_series_mode(0)
 
 # ---- check ---------------------------------------------------------------------------------------------------------------
 K = K_MAX

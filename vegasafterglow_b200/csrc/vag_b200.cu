@@ -33,21 +33,46 @@ static_assert(sizeof(vag_params) == 320, "vag_params layout must match vegasafte
 // ------------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------------
+// A ragged series request (vag_flux_density_series_multi, vag_chi2_multi) gives every model its own data set: a slice
+// of the concatenated points, sorted by time within the slice.  Its distinct frequencies (banded runs) sit at
+// [set * EATS_NU_TILE] of the band tables.  Model m's output is [VAG_NCOMP][n of its set] at point offset
+// out_off[m] - out_off[0] of the pass's output.  The kernels that take `bool RAGGED` run either request: their ragged
+// instantiation rebases the request on the model's data set, so every model's arithmetic is that of the shared-request
+// kernel on its own data set.  The table (SetsDev sd) is their last parameter: placed earlier, it would move the
+// parameter offsets of the shared instantiations and change their code.
+struct SeriesSet {
+    int off, n;   // slice of the concatenated points
+    int n_bands;  // distinct frequencies of the slice (k_series_bands_sets)
+    int pad_;
+};
+struct SetsDev {
+    const int* set_of;         // [models of the pass] data set of each model
+    SeriesSet* sets;           // [n_sets]
+    const long long* out_off;  // [models of the pass] first output point of each model (prefix sums over the batch)
+};
+
 // K0: G lanes per model (vag_grid.cuh GroupPar), 32 / G models per warp, 4 warps per CTA.  Narrow groups
 // share the scalar instruction stream between more models (throughput, large batches); wide groups
-// finish one model sooner (latency, small batches).
+// finish one model sooner (latency, small batches).  The observation window is the request's, or (RAGGED) the
+// model's data set's.
 #ifndef GRID_MIN_BLOCKS
 #define GRID_MIN_BLOCKS 4
 #endif
-template <int G>
-__global__ void __launch_bounds__(128, GRID_MIN_BLOCKS) k_grid(BatchWs w, const double* __restrict__ t_obs, int n_t_obs) {
+template <int G, bool RAGGED>
+__global__ void __launch_bounds__(128, GRID_MIN_BLOCKS) k_grid(BatchWs w, const double* __restrict__ t_obs, int n_t_obs,
+                                                               SetsDev sd) {
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
     const int mi = gt / G;
     if (mi >= w.n_models) return;  // whole groups exit together
     const int lane = threadIdx.x & 31;
     const int shift = lane & ~(G - 1);
     const GroupPar<G> par{lane & (G - 1), (G == 32 ? 0xffffffffu : ((1u << (G & 31)) - 1u)) << shift, shift};
-    k0_grid_body(par, w, mi, t_obs[0], t_obs[n_t_obs - 1]);
+    if constexpr (RAGGED) {
+        const SeriesSet s = sd.sets[sd.set_of[mi]];
+        k0_grid_body(par, w, mi, t_obs[s.off], t_obs[s.off + s.n - 1]);
+    } else {
+        k0_grid_body(par, w, mi, t_obs[0], t_obs[n_t_obs - 1]);
+    }
 }
 
 // K0b: exclusive scan of the ragged row / cell counts over the models of the batch + totals.
@@ -262,11 +287,15 @@ __global__ void k_dop_extrema(BatchWs w) {
     k_dop_extrema_body(w, mi, k);
 }
 
-// K2b: SSC spectrum tables, one warp per unique cell (both shocks); warps stride over the batch's cells
+// K2b: SSC spectrum tables, one warp per unique cell (both shocks); warps stride over the batch's cells.
+// RAGGED: each model's tables are sized by its own data set's band, w.nu_range[2 m .. 2 m + 1] (k_nu_range_sets).  The
+// table comes in w rather than as a parameter of its own: an added parameter changes the code of k_ic_spectrum<false>.
+template <bool RAGGED>
 __global__ void __launch_bounds__(128) k_ic_spectrum(BatchWs w, int n_rows, int n_warps) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const WarpPar par{(int)(threadIdx.x & 31)};
     double* scratch = w.ic_scratch + (size_t)warp * IC_SCRATCH_DOUBLES;
+    BatchWs wm = w;  // RAGGED: w with the band of the cell's model
     for (long long g = warp; g < w.n_cells; g += n_warps) {
         // row of global cell g: last row whose first cell is <= g
         int lo = 0, hi = n_rows;
@@ -281,10 +310,11 @@ __global__ void __launch_bounds__(128) k_ic_spectrum(BatchWs w, int n_rows, int 
         const int k = (int)(g - w.row_cell_off[row]);
         const int mi = w.row_model[row];
         const ModelCfg& cfg = w.cfg[mi];
+        if constexpr (RAGGED) wm.nu_range = w.nu_range + 2 * (size_t)mi;
         for (int which = 0; which < 2; ++which) {
             if (which && !cfg.has_rvs) continue;
             if (!(which ? cfg.rvs : cfg.fwd).ssc) continue;
-            const int st = k2b_ic_spectrum_cell(par, w, row, k, which, scratch);
+            const int st = k2b_ic_spectrum_cell(par, RAGGED ? wm : w, row, k, which, scratch);
             if (st && par.lane == 0) atomicOr(&w.status[mi], st);
         }
     }
@@ -382,9 +412,11 @@ __global__ void k_band_reduce(const double* __restrict__ F, const double* __rest
 enum { EATS_GRID = 0, EATS_POINT = 1, EATS_BANDED = 2 };
 // MODE 1 (synchrotron with the inverse-Compton correction) carries the IC record of the cell next to the tile state: at
 // 64 registers it spilled 120 M local loads per config-4 batch; 5 CTAs / SM (90 registers) hold it without spills.
-template <int MODE, int KIND>
+// RAGGED (KIND EATS_POINT or EATS_BANDED): the CTA's request is rebased on its model's data set and the model's
+// [VAG_NCOMP][n] block is written at its output offset.
+template <int MODE, int KIND, bool RAGGED>
 __global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats(BatchWs w, EatsRequest rq0, double* __restrict__ out, int n_split,
-                                                 int row_chunk, int max_n_t, int nu_tile, size_t split_stride) {
+                                                 int row_chunk, int max_n_t, int nu_tile, size_t split_stride, SetsDev sd) {
     extern __shared__ __align__(16) double smem[];
     const int mi = blockIdx.x;
     const int split = blockIdx.y;
@@ -412,12 +444,27 @@ __global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats(B
     const int acc_cols = series ? 1 : nu_tile;
     EatsShared sh = eats_carve(acc + acc_cols * acc_stride, max_n_t, series && !banded, row_chunk, nu_tile);
     EatsRequest rq = rq0;
+    if constexpr (RAGGED) {
+        const int set = sd.set_of[mi];
+        const SeriesSet ds = sd.sets[set];
+        rq.n_t_obs = rq.n_nu = ds.n;
+        rq.lg2_t_obs += ds.off;
+        rq.t_obs_lin += ds.off;
+        const size_t nu_off = banded ? (size_t)set * EATS_NU_TILE : (size_t)ds.off;  // band table / points
+        rq.lg2_nu_obs += nu_off;
+        rq.nu_obs_lin += nu_off;
+        rq.nu23_obs += nu_off;
+        rq.n_bands = banded ? ds.n_bands : 0;
+        rq.band_of += ds.off;
+    }
     const int tid = threadIdx.x, nthr = blockDim.x;
     const int comp = which == 0 ? VAG_C_FWD_SYNC : which == 1 ? VAG_C_RVS_SYNC : which == 2 ? VAG_C_FWD_SSC : VAG_C_RVS_SSC;
     const size_t comp_sz = series ? (size_t)rq.n_t_obs : (size_t)rq.n_nu * rq.n_t_obs;
     // row-split batches (n_split > 1, small batches): each split owns a slab of `out` (= the partial buffer) and
     // k_sum_splits adds the slabs in split order -- deterministic, unlike an atomicAdd into one cell
-    double* dst = out + (size_t)split * split_stride + ((size_t)mi * VAG_NCOMP + comp) * comp_sz;
+    double* dst =
+        RAGGED ? out + (size_t)split * split_stride + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP + comp * comp_sz
+               : out + (size_t)split * split_stride + ((size_t)mi * VAG_NCOMP + comp) * comp_sz;
     const int n_nu_tiles = series ? 1 : (rq.n_nu + nu_tile - 1) / nu_tile;
     const RowGeom* rowg = w.rowgeom + (size_t)mi * w.max_erows;
     // rows per pass: this model's lattice may be shorter than the batch maximum the buffers are sized for
@@ -504,15 +551,24 @@ __device__ __forceinline__ void chi2_warp(int warp, int lane, const double* __re
         chi2[warp] = (isfinite(s) && !fatal) ? s : kInf;
     }
 }
+// RAGGED: the warp of model m reads its total plane and its data set's slice of the data (ext: of ext_k)
+template <bool RAGGED>
 __global__ void k_chi2(const double* __restrict__ flux, size_t n_models, int n, const double* __restrict__ lnF,
                        const double* __restrict__ sigma_ln, const double* __restrict__ wgt,
                        const double* __restrict__ av, const double* __restrict__ ext, double* chi2,
-                       const int* __restrict__ status, int accumulate) {
+                       const int* __restrict__ status, int accumulate, SetsDev sd) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= (int)n_models) return;
-    const double* F = flux + (size_t)warp * VAG_NCOMP * n;  // total
-    chi2_warp(warp, lane, F, n, lnF, sigma_ln, wgt, av, ext, chi2, status, accumulate);
+    if constexpr (RAGGED) {
+        const SeriesSet s = sd.sets[sd.set_of[warp]];
+        const double* F = flux + (size_t)(sd.out_off[warp] - sd.out_off[0]) * VAG_NCOMP;  // total
+        chi2_warp(warp, lane, F, s.n, lnF + s.off, sigma_ln + s.off, wgt + s.off, av, ext ? ext + s.off : nullptr, chi2,
+                  status, accumulate);
+    } else {
+        const double* F = flux + (size_t)warp * VAG_NCOMP * n;  // total
+        chi2_warp(warp, lane, F, n, lnF, sigma_ln, wgt, av, ext, chi2, status, accumulate);
+    }
 }
 
 // vag_details_ic: [VAG_IC_DETAIL_PLANES][n_cells] <- IcCell records
@@ -548,11 +604,19 @@ __global__ void k_or_status(int32_t* acc, const int32_t* __restrict__ st, size_t
     if (i < n) acc[i] |= st[i];
 }
 
-__global__ void k_nan_capacity(BatchWs w, double* out, size_t comp_sz_total) {
-    // models whose grid exceeded the compiled capacity produce NaN, never a silent partial result
+// models whose grid exceeded the compiled capacity produce NaN, never a silent partial result (CTA / model; RAGGED: the
+// model's block of the ragged output)
+template <bool RAGGED>
+__global__ void k_nan_capacity(BatchWs w, double* out, size_t comp_sz_total, SetsDev sd) {
     const int mi = blockIdx.x;
     if (!(w.status[mi] & VAG_ST_CAPACITY)) return;
-    for (size_t i = threadIdx.x; i < comp_sz_total; i += blockDim.x) out[(size_t)mi * comp_sz_total + i] = NAN;
+    if constexpr (RAGGED) {
+        const size_t per_model = (size_t)VAG_NCOMP * sd.sets[sd.set_of[mi]].n;
+        double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
+        for (size_t i = threadIdx.x; i < per_model; i += blockDim.x) o[i] = NAN;
+    } else {
+        for (size_t i = threadIdx.x; i < comp_sz_total; i += blockDim.x) out[(size_t)mi * comp_sz_total + i] = NAN;
+    }
 }
 
 // Self-test of vag_libm.cuh on the device: out[i] = gl::fn(x[i] [, y[i]]) (fn as in vag_selftest_libm, include/vag.h)
@@ -624,34 +688,10 @@ __global__ void k_reject(const int32_t* __restrict__ ok, int32_t* status, double
     for (size_t i = threadIdx.x; out && i < per_model; i += blockDim.x) out[mi * per_model + i] = NAN;
 }
 
-// ---- ragged series requests: every model has its own data set (vag_flux_density_series_multi, vag_chi2_multi) ----------
-// A data set is a slice of the concatenated points, sorted by time within the slice.  Its distinct frequencies (banded
-// runs) sit at [set * EATS_NU_TILE] of the band tables.  Model m's output is [VAG_NCOMP][n of its set] at point offset
-// out_off[m] - out_off[0] of the pass's output.  These kernels are the shared-request ones with the request rebased per
-// model; every model's arithmetic is that of the shared-request kernels on its own data set.
-struct SeriesSet {
-    int off, n;   // slice of the concatenated points
-    int n_bands;  // distinct frequencies of the slice (k_series_bands_sets)
-    int pad_;
-};
-struct SetsDev {
-    const int* set_of;         // [models of the pass] data set of each model
-    SeriesSet* sets;           // [n_sets]
-    const long long* out_off;  // [models of the pass] first output point of each model (prefix sums over the batch)
-};
-
-// K0 with each model's observation window taken from its own data set
-template <int G>
-__global__ void __launch_bounds__(128, GRID_MIN_BLOCKS) k_grid_sets(BatchWs w, const double* __restrict__ t_obs, SetsDev sd) {
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int mi = gt / G;
-    if (mi >= w.n_models) return;  // whole groups exit together
-    const int lane = threadIdx.x & 31;
-    const int shift = lane & ~(G - 1);
-    const GroupPar<G> par{lane & (G - 1), (G == 32 ? 0xffffffffu : ((1u << (G & 31)) - 1u)) << shift, shift};
-    const SeriesSet s = sd.sets[sd.set_of[mi]];
-    k0_grid_body(par, w, mi, t_obs[s.off], t_obs[s.off + s.n - 1]);
-}
+// ---- ragged series requests (see SeriesSet): the kernels that stay apart from their shared-request ones ----------
+// k_series_bands_sets shares series_bands_cta with k_series_bands, but runs one CTA per set and reduces over the sets.
+// k_nu_range_sets (a warp per model) and k_nu_range (one CTA per batch) compute different things.  k_total_sets (a CTA
+// per model) and k_total (a thread per element) have different launch geometries: a fold would change k_total's launch.
 
 // k_series_bands per data set (CTA / set) into sets[].n_bands and the set's band table.  red[0] = max over the sets of
 // n_bands, red[1] = min over the sets of floor(3 n / n_bands): the batch is banded when every set passes series_banded
@@ -693,128 +733,6 @@ __global__ void k_nu_range_sets(const double* __restrict__ lg2_nu, SetsDev sd, i
     }
 }
 
-// K2b with each model's SSC tables sized by its own data set's band (nu_range_of: k_nu_range_sets)
-__global__ void __launch_bounds__(128) k_ic_spectrum_sets(BatchWs w, int n_rows, int n_warps, const double* __restrict__ nu_range_of) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const WarpPar par{(int)(threadIdx.x & 31)};
-    double* scratch = w.ic_scratch + (size_t)warp * IC_SCRATCH_DOUBLES;
-    BatchWs wm = w;
-    for (long long g = warp; g < w.n_cells; g += n_warps) {
-        int lo = 0, hi = n_rows;
-        while (hi - lo > 1) {
-            const int mid = (lo + hi) >> 1;
-            if (w.row_cell_off[mid] <= g)
-                lo = mid;
-            else
-                hi = mid;
-        }
-        const int row = lo;
-        const int k = (int)(g - w.row_cell_off[row]);
-        const int mi = w.row_model[row];
-        const ModelCfg& cfg = w.cfg[mi];
-        wm.nu_range = nu_range_of + 2 * (size_t)mi;
-        for (int which = 0; which < 2; ++which) {
-            if (which && !cfg.has_rvs) continue;
-            if (!(which ? cfg.rvs : cfg.fwd).ssc) continue;
-            const int st = k2b_ic_spectrum_cell(par, wm, row, k, which, scratch);
-            if (st && par.lane == 0) atomicOr(&w.status[mi], st);
-        }
-    }
-}
-
-// K3 on a ragged request: k_eats with the CTA's request rebased on its model's data set (KIND: EATS_POINT or EATS_BANDED)
-// and the model's [VAG_NCOMP][n] block written at its output offset.  A copy of k_eats' CTA rather than a shared body:
-// the existing instantiations keep their code exactly (a shared inline body changed their instruction schedule).
-template <int MODE, int KIND>
-__global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats_sets(BatchWs w, EatsRequest rq0, SetsDev sd,
-                                                 double* __restrict__ out, int n_split, int row_chunk, int max_n_t,
-                                                 int nu_tile, size_t split_stride) {
-    extern __shared__ __align__(16) double smem[];
-    const int mi = blockIdx.x;
-    const int split = blockIdx.y;
-    const int which = (int)blockIdx.z + (MODE == 2 ? 2 : 0);  // 0 fwd sync, 1 rvs sync, 2 fwd ssc, 3 rvs ssc
-    {
-        const ModelCfg& cfg = w.cfg[mi];
-        if ((which & 1) && !cfg.has_rvs) return;
-        const bool ssc = ((which & 1) ? cfg.rvs : cfg.fwd).ssc != 0;
-        if ((MODE == 0) == ssc) return;  // MODE 0 handles the shocks without ssc, MODE 1/2 those with
-    }
-    if (w.status[mi] & VAG_ST_CAPACITY) return;
-    EatsModel M = make_eats_model(w, mi, which);
-    M.breach = &w.status[mi];
-    {
-        // log2_softplus table -> head of the dynamic shared memory (16-byte aligned rows)
-        for (int a = threadIdx.x; a < SPL_DOUBLES; a += blockDim.x) smem[a] = w.sp_lut[a];
-        M.sp_lut = smem;
-    }
-    const int n_t = M.h->n_t;
-    const int erows = M.h->n_theta * M.h->n_phi_eff;
-    constexpr bool series = KIND != EATS_GRID;
-    constexpr bool banded = KIND == EATS_BANDED;  // series points read a (node, band) tile staged as in grid mode
-    double* acc = smem + SPL_DOUBLES;     // [acc_cols][acc_stride]
-    const int acc_stride = rq0.acc_stride;
-    const int acc_cols = series ? 1 : nu_tile;
-    EatsShared sh = eats_carve(acc + acc_cols * acc_stride, max_n_t, series && !banded, row_chunk, nu_tile);
-    EatsRequest rq = rq0;
-    const int set = sd.set_of[mi];
-    const SeriesSet ds = sd.sets[set];
-    {
-        rq.n_t_obs = rq.n_nu = ds.n;
-        rq.lg2_t_obs += ds.off;
-        rq.t_obs_lin += ds.off;
-        const size_t nu_off = KIND == EATS_BANDED ? (size_t)set * EATS_NU_TILE : (size_t)ds.off;  // band table / points
-        rq.lg2_nu_obs += nu_off;
-        rq.nu_obs_lin += nu_off;
-        rq.nu23_obs += nu_off;
-        rq.n_bands = KIND == EATS_BANDED ? ds.n_bands : 0;
-        rq.band_of += ds.off;
-    }
-    const int tid = threadIdx.x, nthr = blockDim.x;
-    const int comp = which == 0 ? VAG_C_FWD_SYNC : which == 1 ? VAG_C_RVS_SYNC : which == 2 ? VAG_C_FWD_SSC : VAG_C_RVS_SSC;
-    const size_t comp_sz = series ? (size_t)rq.n_t_obs : (size_t)rq.n_nu * rq.n_t_obs;
-    // row-split batches (n_split > 1, small batches): each split owns a slab of `out` (= the partial buffer) and
-    // k_sum_splits adds the slabs in split order -- deterministic, unlike an atomicAdd into one cell
-    double* dst = out + (size_t)split * split_stride + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP + comp * comp_sz;
-    const int n_nu_tiles = series ? 1 : (rq.n_nu + nu_tile - 1) / nu_tile;
-    const RowGeom* rowg = w.rowgeom + (size_t)mi * w.max_erows;
-    // rows per pass: this model's lattice may be shorter than the batch maximum the buffers are sized for
-    const int rpp = eats_rows_per_pass(n_t, row_chunk, nthr);
-    for (int tile = 0; tile < n_nu_tiles; ++tile) {
-        const int l0 = tile * nu_tile;
-        const int nl = series ? (banded ? rq.n_bands : 1) : imin(nu_tile, rq.n_nu - l0);
-        for (int i0 = 0; i0 < rq.n_t_obs; i0 += EATS_T_BLOCK) {
-            rq.i0 = i0;
-            rq.ni = imin(EATS_T_BLOCK, rq.n_t_obs - i0);
-            // zeroed by the thread that accumulates into and finally reads the column (ii == tid mod nthr): no barrier is
-            // needed even when this split has no pass to run (compute-sanitizer racecheck, profiles/r02_sanitize.txt)
-            for (int ii = tid; ii < rq.ni; ii += nthr)
-                for (int l = 0; l < acc_cols; ++l) acc[l * acc_stride + ii] = 0.0;
-            for (int q0 = split * rpp; q0 < erows; q0 += n_split * rpp) {
-                const int nrows = imin(rpp, erows - q0);
-                sh.rowg = rowg + q0;
-                __syncthreads();  // previous pass finished reading the staged rows (and the table is loaded)
-                eats_phase1<MODE, KIND == EATS_POINT>(M, rq, sh, nrows, l0, nl, tid, nthr);
-                __syncthreads();
-                if (banded)
-                    eats_phase2_banded(M, rq, sh, nrows, acc, tid, nthr);
-                else if (series)
-                    eats_phase2_series<MODE>(M, rq, sh, nrows, acc, tid, nthr);
-                else
-                    eats_phase2_grid(M, rq, sh, nrows, nl, acc, tid, nthr);
-            }
-            // accumulator columns are thread-owned (ii == tid mod nthr): no barrier needed here
-            for (int ii = tid; ii < rq.ni; ii += nthr) {
-                for (int l = 0; l < (series ? 1 : nl); ++l) {
-                    const double v = flux_scale(M, acc[l * acc_stride + ii]);
-                    double* p = series ? (dst + i0 + ii) : (dst + (size_t)(l0 + l) * rq.n_t_obs + i0 + ii);
-                    *p = v;
-                }
-            }
-            __syncthreads();
-        }
-    }
-}
-
 // k_total on a ragged output (CTA / model)
 __global__ void k_total_sets(double* out, SetsDev sd) {
     const int mi = blockIdx.x;
@@ -822,27 +740,6 @@ __global__ void k_total_sets(double* out, SetsDev sd) {
     double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
     for (size_t e = threadIdx.x; e < cs; e += blockDim.x)
         o[e] = o[VAG_C_FWD_SYNC * cs + e] + o[VAG_C_FWD_SSC * cs + e] + o[VAG_C_RVS_SYNC * cs + e] + o[VAG_C_RVS_SSC * cs + e];
-}
-
-// k_nan_capacity on a ragged output (CTA / model)
-__global__ void k_nan_capacity_sets(BatchWs w, double* out, SetsDev sd) {
-    const int mi = blockIdx.x;
-    if (!(w.status[mi] & VAG_ST_CAPACITY)) return;
-    const size_t per_model = (size_t)VAG_NCOMP * sd.sets[sd.set_of[mi]].n;
-    double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
-    for (size_t i = threadIdx.x; i < per_model; i += blockDim.x) o[i] = NAN;
-}
-
-// K4 on a ragged request: the warp of model m reads its total plane and its data set's slice of the data (ext: of ext_k)
-__global__ void k_chi2_sets(const double* __restrict__ flux, size_t n_models, SetsDev sd, const double* __restrict__ lnF,
-                            const double* __restrict__ sigma_ln, const double* __restrict__ wgt, const double* __restrict__ av,
-                            const double* __restrict__ ext, double* chi2, const int* __restrict__ status) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (warp >= (int)n_models) return;
-    const SeriesSet s = sd.sets[sd.set_of[warp]];
-    const double* F = flux + (size_t)(sd.out_off[warp] - sd.out_off[0]) * VAG_NCOMP;  // total
-    chi2_warp(warp, lane, F, s.n, lnF + s.off, sigma_ln + s.off, wgt + s.off, av, ext ? ext + s.off : nullptr, chi2, status, 0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1041,18 +938,14 @@ void mark(vag_context* ctx, int i, cudaStream_t s) {
 }
 
 // The kernel variants: the launch sites and vag_create's function attributes take them from here
-using GridKernel = void (*)(BatchWs, const double*, int);
-using EatsKernel = void (*)(BatchWs, EatsRequest, double*, int, int, int, int, size_t);
+using GridKernel = void (*)(BatchWs, const double*, int, SetsDev);
+using EatsKernel = void (*)(BatchWs, EatsRequest, double*, int, int, int, int, size_t, SetsDev);
 constexpr int GRID_LANES[] = {4, 8, 16, 32};
 constexpr int EATS_MODES = 3, EATS_KINDS = 3;
 
 // (defined after run_front: the cubin lists the kernel templates in the order the source first names them)
-GridKernel grid_kernel(int lanes);
-EatsKernel eats_kernel(int mode, int kind);
-using GridSetsKernel = void (*)(BatchWs, const double*, SetsDev);
-using EatsSetsKernel = void (*)(BatchWs, EatsRequest, SetsDev, double*, int, int, int, int, size_t);
-GridSetsKernel grid_sets_kernel(int lanes);
-EatsSetsKernel eats_sets_kernel(int mode, bool banded);
+GridKernel grid_kernel(int lanes, bool ragged);
+EatsKernel eats_kernel(int mode, int kind, bool ragged);  // ragged: nullptr for EATS_GRID
 
 // Lanes per model of k_grid: the widest group whose launch fits into one wave of resident CTAs (GRID_MIN_BLOCKS CTAs of
 // 128 threads per SM).  Narrower groups only pay once a wider launch would need a second wave: the models of one warp
@@ -1075,10 +968,8 @@ int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n
     if (rc) return rc;
     mark(ctx, 0, s);
     const int lanes = ctx->grid_lanes ? ctx->grid_lanes : grid_lanes_for(n, ctx->sm_count);
-    if (sets)
-        grid_sets_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, *sets);
-    else
-        grid_kernel(lanes)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t);
+    grid_kernel(lanes, sets != nullptr)<<<(unsigned)((n * lanes + 127) / 128), 128, 0, s>>>(w, d_t, (int)n_t,
+                                                                                          sets ? *sets : SetsDev{});
     k_scan<<<1, 1024, 0, s>>>(w);
     ctx->launches += 2;
     CK(cudaMemcpyAsync(ctx->h_totals, w.totals, sizeof(int) * TOT_N, cudaMemcpyDeviceToHost, s));
@@ -1141,37 +1032,24 @@ int run_front(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n
     return VAG_OK;
 }
 
-GridKernel grid_kernel(int lanes) {
+GridKernel grid_kernel(int lanes, bool ragged) {
     switch (lanes) {
-        case 4: return k_grid<4>;
-        case 8: return k_grid<8>;
-        case 16: return k_grid<16>;
-        default: return k_grid<32>;
+        case 4: return ragged ? k_grid<4, true> : k_grid<4, false>;
+        case 8: return ragged ? k_grid<8, true> : k_grid<8, false>;
+        case 16: return ragged ? k_grid<16, true> : k_grid<16, false>;
+        default: return ragged ? k_grid<32, true> : k_grid<32, false>;
     }
 }
 
-EatsKernel eats_kernel(int mode, int kind) {
-    static const EatsKernel k[EATS_MODES][EATS_KINDS] = {
-        {k_eats<0, EATS_GRID>, k_eats<0, EATS_POINT>, k_eats<0, EATS_BANDED>},
-        {k_eats<1, EATS_GRID>, k_eats<1, EATS_POINT>, k_eats<1, EATS_BANDED>},
-        {k_eats<2, EATS_GRID>, k_eats<2, EATS_POINT>, k_eats<2, EATS_BANDED>}};
-    return k[mode][kind];
-}
-
-GridSetsKernel grid_sets_kernel(int lanes) {
-    switch (lanes) {
-        case 4: return k_grid_sets<4>;
-        case 8: return k_grid_sets<8>;
-        case 16: return k_grid_sets<16>;
-        default: return k_grid_sets<32>;
-    }
-}
-
-EatsSetsKernel eats_sets_kernel(int mode, bool banded) {
-    static const EatsSetsKernel k[EATS_MODES][2] = {{k_eats_sets<0, EATS_POINT>, k_eats_sets<0, EATS_BANDED>},
-                                                    {k_eats_sets<1, EATS_POINT>, k_eats_sets<1, EATS_BANDED>},
-                                                    {k_eats_sets<2, EATS_POINT>, k_eats_sets<2, EATS_BANDED>}};
-    return k[mode][banded ? 1 : 0];
+EatsKernel eats_kernel(int mode, int kind, bool ragged) {
+    static const EatsKernel k[2][EATS_MODES][EATS_KINDS] = {
+        {{k_eats<0, EATS_GRID, false>, k_eats<0, EATS_POINT, false>, k_eats<0, EATS_BANDED, false>},
+         {k_eats<1, EATS_GRID, false>, k_eats<1, EATS_POINT, false>, k_eats<1, EATS_BANDED, false>},
+         {k_eats<2, EATS_GRID, false>, k_eats<2, EATS_POINT, false>, k_eats<2, EATS_BANDED, false>}},
+        {{nullptr, k_eats<0, EATS_POINT, true>, k_eats<0, EATS_BANDED, true>},
+         {nullptr, k_eats<1, EATS_POINT, true>, k_eats<1, EATS_BANDED, true>},
+         {nullptr, k_eats<2, EATS_POINT, true>, k_eats<2, EATS_BANDED, true>}}};
+    return k[ragged][mode][kind];
 }
 
 // flux of a batch into d_out [n][VAG_NCOMP][comp]; with d_chi2, also the chi-squared of the series against rq_in's data
@@ -1225,7 +1103,7 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
     if (w.any_ssc && totals[TOT_ROWS] > 0) {
         // SSC tables: observation band -> per-row line-of-sight cosines -> per-k Doppler extrema -> tables
         // (a ragged request: each model's band is its own data set's, as its shared-request call would see it)
-        w.nu_range = nu_range;
+        w.nu_range = sets ? nu_range_of : nu_range;
         if (sets)
             k_nu_range_sets<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(lg2_nu, *sets, (int)n, nu_range_of);
         else
@@ -1234,10 +1112,7 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         k_dop_extrema<<<dim3((unsigned)((w.max_n_t + 63) / 64), (unsigned)n), 64, 0, s>>>(w);
         const int n_ic_warps = (int)std::min<long long>(std::max<long long>(cells, 1), (long long)ctx->sm_count * ctx->ic_warps_per_sm);
         const unsigned ic_blocks = (unsigned)((n_ic_warps * 32 + 127) / 128);
-        if (sets)
-            k_ic_spectrum_sets<<<ic_blocks, 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps, nu_range_of);
-        else
-            k_ic_spectrum<<<ic_blocks, 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps);
+        (sets ? k_ic_spectrum<true> : k_ic_spectrum<false>)<<<ic_blocks, 128, 0, s>>>(w, totals[TOT_ROWS], n_ic_warps);
         ctx->launches += 4;
     }
     // points per component plane of a model (shared request), and the elements of the pass's output
@@ -1303,13 +1178,9 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         }
         const int kind = !rq_in.series ? EATS_GRID : banded ? EATS_BANDED : EATS_POINT;
         const int n_modes = w.any_ssc ? EATS_MODES : 1;
-        for (int mode = 0; mode < n_modes; ++mode) {
-            if (sets)
-                eats_sets_kernel(mode, banded)<<<eg, 128, sb, s>>>(w, rq, *sets, eats_out, n_split, row_chunk, max_n_t,
-                                                                   nu_tile, elems);
-            else
-                eats_kernel(mode, kind)<<<eg, 128, sb, s>>>(w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile, elems);
-        }
+        for (int mode = 0; mode < n_modes; ++mode)
+            eats_kernel(mode, kind, sets != nullptr)<<<eg, 128, sb, s>>>(w, rq, eats_out, n_split, row_chunk, max_n_t, nu_tile,
+                                                                         elems, sets ? *sets : SetsDev{});
         ctx->launches += n_modes;
         if (n_split > 1) {
             k_sum_splits<<<(unsigned)((elems + 255) / 256), 256, 0, s>>>(d_out, eats_out, n_split, elems);
@@ -1327,20 +1198,15 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         // the SSC lattices can overflow later than the grid (k_ic_spectrum sets the bit after k_scan read the OR):
         // with ssc shocks in the batch the kernel runs unconditionally and tests each model's bit on the device
         if ((totals[TOT_STATUS_OR] & VAG_ST_CAPACITY) || w.any_ssc) {
-            if (sets)
-                k_nan_capacity_sets<<<(unsigned)n, 128, 0, s>>>(w, d_out, *sets);
-            else
-                k_nan_capacity<<<(unsigned)n, 128, 0, s>>>(w, d_out, VAG_NCOMP * comp_sz);
+            (sets ? k_nan_capacity<true> : k_nan_capacity<false>)<<<(unsigned)n, 128, 0, s>>>(w, d_out, VAG_NCOMP * comp_sz,
+                                                                                              sets ? *sets : SetsDev{});
             ctx->launches++;
         }
     }
     if (d_chi2) {
-        if (sets)
-            k_chi2_sets<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, *sets, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
-                                                                          rq_in.d_av, rq_in.d_ext, d_chi2, w.status);
-        else
-            k_chi2<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w,
-                                                                     rq_in.d_av, rq_in.d_ext, d_chi2, w.status, 0);
+        (sets ? k_chi2<true> : k_chi2<false>)<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(
+            d_out, n, (int)n_t, rq_in.d_lnF, rq_in.d_sig, rq_in.d_w, rq_in.d_av, rq_in.d_ext, d_chi2, w.status, 0,
+            sets ? *sets : SetsDev{});
         ctx->launches++;
     }
     mark(ctx, 5, s);
@@ -1486,21 +1352,19 @@ int vag_create(int device, vag_context** out) {
     }
     // k_grid spills its scratch to local memory: prefer L1.  k_dynamics keeps its dopri5 stage vectors
     // in shared memory (23 KB per 32-row CTA): give it the full carve-out so several CTAs share an SM.
-    for (int lanes : GRID_LANES) cudaFuncSetCacheConfig(grid_kernel(lanes), cudaFuncCachePreferL1);
+    for (bool ragged : {false, true})
+        for (int lanes : GRID_LANES) cudaFuncSetCacheConfig(grid_kernel(lanes, ragged), cudaFuncCachePreferL1);
     cudaFuncSetAttribute(k_dynamics<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     // per-function process state: set once, to the largest request run_flux can make (not per call, where two contexts
     // with different request shapes would race on it)
-    for (int mode = 0; mode < EATS_MODES; ++mode)
-        for (int kind = 0; kind < EATS_KINDS; ++kind)
-            CK(cudaFuncSetAttribute(eats_kernel(mode, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET));
-    for (int lanes : GRID_LANES) cudaFuncSetCacheConfig(grid_sets_kernel(lanes), cudaFuncCachePreferL1);
-    for (int mode = 0; mode < EATS_MODES; ++mode)
-        for (bool banded : {false, true})
-            CK(cudaFuncSetAttribute(eats_sets_kernel(mode, banded), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)EATS_SMEM_BUDGET));
+    for (bool ragged : {false, true})
+        for (int mode = 0; mode < EATS_MODES; ++mode)
+            for (int kind = 0; kind < EATS_KINDS; ++kind)
+                if (EatsKernel k = eats_kernel(mode, kind, ragged))
+                    CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET));
     {
         int blocks = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum, 128, 0) == cudaSuccess && blocks > 0)
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum<false>, 128, 0) == cudaSuccess && blocks > 0)
             c->ic_warps_per_sm = std::min(blocks, 8) * 4;
     }
     *out = c;
@@ -1910,7 +1774,8 @@ static int chi2_run(vag_context* ctx, const vag_params* d_params, size_t n_model
         const BandTerm& B = bands[b];
         double* d_band = nullptr;
         if (int rc = run_band(ctx, d_params, n_models, caps, B.t, B.n, *B.g, d_status, &d_band, s)) return rc;
-        k_chi2<<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, B.lnF, B.sig, B.w, nullptr, nullptr, d_chi2, d_status, 1);
+        k_chi2<false><<<cg, 128, 0, s>>>(d_band, n_models, (int)B.n, B.lnF, B.sig, B.w, nullptr, nullptr, d_chi2, d_status, 1,
+                                         SetsDev{});
         k_or_status<<<og, 256, 0, s>>>(d_stat_or, d_status, n_models);
         launches += ctx->launches + 2;
     }

@@ -74,7 +74,7 @@ struct BatchWs {
     double* dop_max;
     const KnLut* lut;
     double* ic_scratch;       // [n_ic_warps][IC_SCRATCH_DOUBLES]
-    const double* nu_range;   // [2] log2 of min / max observation frequency (code units)
+    const double* nu_range;   // [2] log2 of min / max observation frequency (code units); ragged request: [n_models][2]
     const double* sp_lut;     // [SPL_DOUBLES] log2_softplus table (vag_math.cuh)
     RowGeom* rowgeom;         // [n_models][max_erows] EATS row constants (k_rowgeom)
 };
