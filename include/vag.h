@@ -207,7 +207,8 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
  * parameter sets as vag_params_validate.  A data set no model uses is allowed.  Batches over 32768 models run in
  * passes as the other entry points do.  Launches: those of vag_chi2_series / vag_flux_density_series on the same
  * total data, whatever n_sets (one CTA per data set inside the band search kernel).
- * Not provided: band-integrated data per data set, a device-buffer (_dev) variant, per-model grid (t x nu) requests.
+ * Not provided here: band-integrated data per data set (vag_flux_band_multi, vag_chi2_multi_bands below), a
+ * device-buffer (_dev) variant, a public per-model grid (t x nu) request.
  * The output mode (vag_set_output_mode) does not apply: every plane of `out` is written. */
 typedef struct vag_series_set {
     size_t offset, n; /* slice of the concatenated points */
@@ -226,6 +227,50 @@ int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, 
                    const vag_series_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
                    const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total, const double* A_V,
                    double* chi2, int32_t* status);
+
+/* ---- band-integrated data in a batch of several light curves ------------------------------------------------------
+ * Every (model, band) pair of a call is one evaluation of a single ragged grid request: its own band times x its own
+ * frequency nodes (band_grid of vag_flux_band), run through the pipeline once for all evaluations and reduced with each
+ * band's weights.  Model m's values are those of vag_flux_band / vag_chi2_ext for that model on that band (data set)
+ * alone: bit for bit when neither call splits the rows of a model over several CTAs (from 2368 (evaluation x shock)
+ * CTAs on 148 SMs) and both stage the same number of rows per pass; otherwise to rounding.  The pass sizes its
+ * shared-memory stage from the longest band and widest node set of the batch: that can lower the rows staged per pass
+ * (long lattices), never the frequency tiles -- a model tiles its own num_nu nodes by min(8, widest num_nu) >=
+ * min(8, its num_nu), which gives the tiles of its own call (one of num_nu nodes when num_nu <= 8, of 8 and the
+ * remainder otherwise), so the same eats_phase2_grid instantiation sums the same terms.  An SSC model's tables span its
+ * own band's nodes.  Batches over 32768 evaluations run in passes.  Checks, all before any work is enqueued
+ * (VAG_ERR_INVALID, messages name the data set, the band or the model; a failed call leaves the context usable): every
+ * band n > 0, t ascending, finite and > 0, nu_min / nu_max / num_nu as vag_flux_band; indices in range; parameter sets
+ * as vag_params_validate.  Bands and data sets no model uses are allowed.  The output mode does not apply. */
+
+/* Model.flux of model m on bands[band_of[m]]: only t, n, nu_min, nu_max and num_nu of a band are read (the data
+ * pointers may be NULL).  out: model m's [VAG_NCOMP][n of its band] block starts at element VAG_NCOMP * off[m], off[m] =
+ * the sum of the sizes of the bands of models 0 .. m-1 (the layout of vag_flux_density_series_multi).  Launches: those
+ * of vag_flux_band on one band. */
+int vag_flux_band_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* band_of,
+                        const vag_band_obs* bands, size_t n_bands, double* out, int32_t* status);
+
+/* One data set of vag_chi2_multi_bands: a slice of the concatenated points (n = 0: no point data) and its band-integrated
+ * data bands[band0 .. band0 + n_bands), in this order.  n > 0 or n_bands > 0. */
+typedef struct vag_multi_set {
+    size_t offset, n;
+    size_t band0, n_bands;
+} vag_multi_set;
+
+/* chi2[m] and status[m] of vag_chi2_ext (vag_chi2 when ext_k and A_V are NULL) for model m on its data set's points and
+ * bands alone: the point term (0 without points), then each band's term in the set's order, added as band + chi2 with
+ * the band sum sum_i F(nu_i) w_i in node order; VAG_ST_ODE_FAIL500 of the run a term came from gives +inf.  status = the
+ * OR over the terms when the set has bands, the point run's status otherwise.  Point arrays as vag_chi2_multi (NULL
+ * only when n_points_total == 0; every set with points passes vag_chi2_multi's checks, and those sets alone decide its
+ * series mode); ext_k / A_V as vag_chi2_multi, and A_V[m] is not read for a model whose set has no points.  Band data
+ * pointers must be set.  Launches, whatever n_sets and the number of bands: L(points) + L(bands) + 2, where L(points) =
+ * those of vag_chi2_multi on the models with points (0 when none has one), L(bands) = those of vag_flux_band_multi on
+ * all evaluations (0 when no model has a band), and the 2 are the device gather of the evaluations' parameter records
+ * from the models' and the band chi-squared (a warp per model). */
+int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                         const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                         const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
+                         const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status);
 
 /* ok[i] = 1 where vag_params_validate accepts params[i], else 0 (no error is raised for rejected sets). */
 int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok);

@@ -94,6 +94,13 @@ class SeriesSet(C.Structure):
     _fields_ = [("offset", C.c_size_t), ("n", C.c_size_t)]
 
 
+class MultiSet(C.Structure):
+    """``vag_multi_set`` (include/vag.h): one data set of ``vag_chi2_multi_bands`` -- a slice of the concatenated points
+    (n = 0: none) and its band-integrated data ``bands[band0 .. band0 + n_bands)``."""
+
+    _fields_ = [("offset", C.c_size_t), ("n", C.c_size_t), ("band0", C.c_size_t), ("n_bands", C.c_size_t)]
+
+
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
 

@@ -36,20 +36,26 @@ static_assert(sizeof(vag_params) == 320, "vag_params layout must match vegasafte
 // A ragged series request (vag_flux_density_series_multi, vag_chi2_multi) gives every model its own data set: a slice
 // of the concatenated points, sorted by time within the slice.  Its distinct frequencies (banded runs) sit at
 // [set * EATS_NU_TILE] of the band tables.  Model m's output is [VAG_NCOMP][n of its set] at point offset
-// out_off[m] - out_off[0] of the pass's output.  The kernels that take `bool RAGGED` run either request: their ragged
-// instantiation rebases the request on the model's data set, so every model's arithmetic is that of the shared-request
-// kernel on its own data set.  The table (SetsDev sd) is their last parameter: placed earlier, it would move the
-// parameter offsets of the shared instantiations and change their code.
+// out_off[m] - out_off[0] of the pass's output.  A ragged grid request (the band pass of vag_flux_band_multi and
+// vag_chi2_multi_bands) gives every model a slice of the concatenated times and one of the concatenated frequency nodes;
+// its output is [VAG_NCOMP][n_nu][n] at out_off[m] - out_off[0], out_off counting (time x node) points.  The kernels that
+// take `bool RAGGED` run either request: their ragged instantiation rebases the request on the model's data set, so
+// every model's arithmetic is that of the shared-request kernel on its own data set.  The table (SetsDev sd) is their
+// last parameter: placed earlier, it would move the parameter offsets of the shared instantiations and change their code.
 struct SeriesSet {
-    int off, n;   // slice of the concatenated points
-    int n_bands;  // distinct frequencies of the slice (k_series_bands_sets)
-    int pad_;
+    int off, n;  // slice of the concatenated points (grid request: of the concatenated times)
+    int n_nu;    // series: distinct frequencies of the slice (k_series_bands_sets); grid: frequency nodes of the slice
+    int nu_off;  // grid: first node of the slice in the concatenated nodes
 };
 struct SetsDev {
     const int* set_of;         // [models of the pass] data set of each model
     SeriesSet* sets;           // [n_sets]
-    const long long* out_off;  // [models of the pass] first output point of each model (prefix sums over the batch)
+    const long long* out_off;  // [models of the pass + 1] first output point of each model (prefix sums over the batch)
 };
+// points of model mi's ragged output block, per component
+__device__ __forceinline__ size_t ragged_comp_size(const SetsDev& sd, int mi) {
+    return (size_t)(sd.out_off[mi + 1] - sd.out_off[mi]);
+}
 
 // K0: G lanes per model (vag_grid.cuh GroupPar), 32 / G models per warp, 4 warps per CTA.  Narrow groups
 // share the scalar instruction stream between more models (throughput, large batches); wide groups
@@ -412,8 +418,10 @@ __global__ void k_band_reduce(const double* __restrict__ F, const double* __rest
 enum { EATS_GRID = 0, EATS_POINT = 1, EATS_BANDED = 2 };
 // MODE 1 (synchrotron with the inverse-Compton correction) carries the IC record of the cell next to the tile state: at
 // 64 registers it spilled 120 M local loads per config-4 batch; 5 CTAs / SM (90 registers) hold it without spills.
-// RAGGED (KIND EATS_POINT or EATS_BANDED): the CTA's request is rebased on its model's data set and the model's
-// [VAG_NCOMP][n] block is written at its output offset.
+// RAGGED: the CTA's request is rebased on its model's data set and the model's [VAG_NCOMP][n] (series) or
+// [VAG_NCOMP][n_nu][n] (grid) block is written at its output offset.  A grid CTA tiles its own n_nu with the batch's
+// nu_tile: a tile is min(nu_tile, n_nu - l0) wide, and as nu_tile = min(EATS_NU_TILE, widest n_nu) >= min(EATS_NU_TILE,
+// own n_nu), the tiles are those of the model's own call; nu_tile itself only sets strides (staged tile, accumulators).
 template <int MODE, int KIND, bool RAGGED>
 __global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats(BatchWs w, EatsRequest rq0, double* __restrict__ out, int n_split,
                                                  int row_chunk, int max_n_t, int nu_tile, size_t split_stride, SetsDev sd) {
@@ -444,7 +452,7 @@ __global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats(B
     const int acc_cols = series ? 1 : nu_tile;
     EatsShared sh = eats_carve(acc + acc_cols * acc_stride, max_n_t, series && !banded, row_chunk, nu_tile);
     EatsRequest rq = rq0;
-    if constexpr (RAGGED) {
+    if constexpr (RAGGED && series) {
         const int set = sd.set_of[mi];
         const SeriesSet ds = sd.sets[set];
         rq.n_t_obs = rq.n_nu = ds.n;
@@ -454,8 +462,17 @@ __global__ void __launch_bounds__(128, MODE == 1 ? 5 : EATS_MIN_BLOCKS) k_eats(B
         rq.lg2_nu_obs += nu_off;
         rq.nu_obs_lin += nu_off;
         rq.nu23_obs += nu_off;
-        rq.n_bands = banded ? ds.n_bands : 0;
+        rq.n_bands = banded ? ds.n_nu : 0;
         rq.band_of += ds.off;
+    } else if constexpr (RAGGED) {  // grid: the set's times x its frequency nodes, tiled by nu_tile as a call of its own
+        const SeriesSet ds = sd.sets[sd.set_of[mi]];
+        rq.n_t_obs = ds.n;
+        rq.n_nu = ds.n_nu;
+        rq.lg2_t_obs += ds.off;
+        rq.t_obs_lin += ds.off;
+        rq.lg2_nu_obs += ds.nu_off;
+        rq.nu_obs_lin += ds.nu_off;
+        rq.nu23_obs += ds.nu_off;
     }
     const int tid = threadIdx.x, nthr = blockDim.x;
     const int comp = which == 0 ? VAG_C_FWD_SYNC : which == 1 ? VAG_C_RVS_SYNC : which == 2 ? VAG_C_FWD_SSC : VAG_C_RVS_SSC;
@@ -611,7 +628,7 @@ __global__ void k_nan_capacity(BatchWs w, double* out, size_t comp_sz_total, Set
     const int mi = blockIdx.x;
     if (!(w.status[mi] & VAG_ST_CAPACITY)) return;
     if constexpr (RAGGED) {
-        const size_t per_model = (size_t)VAG_NCOMP * sd.sets[sd.set_of[mi]].n;
+        const size_t per_model = VAG_NCOMP * ragged_comp_size(sd, mi);
         double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
         for (size_t i = threadIdx.x; i < per_model; i += blockDim.x) o[i] = NAN;
     } else {
@@ -693,7 +710,7 @@ __global__ void k_reject(const int32_t* __restrict__ ok, int32_t* status, double
 // k_nu_range_sets (a warp per model) and k_nu_range (one CTA per batch) compute different things.  k_total_sets (a CTA
 // per model) and k_total (a thread per element) have different launch geometries: a fold would change k_total's launch.
 
-// k_series_bands per data set (CTA / set) into sets[].n_bands and the set's band table.  red[0] = max over the sets of
+// k_series_bands per data set (CTA / set) into sets[].n_nu and the set's band table.  red[0] = max over the sets of
 // n_bands, red[1] = min over the sets of floor(3 n / n_bands): the batch is banded when every set passes series_banded
 // (see series_banded_sets).  red is preset to {0, INT_MAX} by the caller.
 __global__ void __launch_bounds__(256) k_series_bands_sets(const double* __restrict__ lg2_nu, const double* __restrict__ nu_lin,
@@ -703,24 +720,27 @@ __global__ void __launch_bounds__(256) k_series_bands_sets(const double* __restr
     const int off = sets[d].off, n = sets[d].n;
     const size_t b = (size_t)d * EATS_NU_TILE;
     series_bands_cta(lg2_nu + off, nu_lin + off, nu23 + off, n, band_of + off, b_lg2 + b, b_lin + b, b_23 + b,
-                     &sets[d].n_bands);
+                     &sets[d].n_nu);
     if (threadIdx.x == 0) {
-        const int nb = sets[d].n_bands;
+        const int nb = sets[d].n_nu;
         atomicMax(red, nb);
         atomicMin(red + 1, (int)min(3LL * n / max(nb, 1), (long long)INT_MAX));
     }
 }
 
 // k_nu_range per model (warp / model): out[2 m], out[2 m + 1] = log2 of the smallest / largest frequency of its data set
+// (GRID: of its slice of the frequency nodes)
+template <bool GRID>
 __global__ void k_nu_range_sets(const double* __restrict__ lg2_nu, SetsDev sd, int n_models, double* out) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= n_models) return;
     const SeriesSet s = sd.sets[sd.set_of[warp]];
+    const int off = GRID ? s.nu_off : s.off, n = GRID ? s.n_nu : s.n;
     double lo = kInf, hi = -kInf;
-    for (int i = lane; i < s.n; i += 32) {
-        lo = fmin(lo, lg2_nu[s.off + i]);
-        hi = fmax(hi, lg2_nu[s.off + i]);
+    for (int i = lane; i < n; i += 32) {
+        lo = fmin(lo, lg2_nu[off + i]);
+        hi = fmax(hi, lg2_nu[off + i]);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
@@ -736,10 +756,62 @@ __global__ void k_nu_range_sets(const double* __restrict__ lg2_nu, SetsDev sd, i
 // k_total on a ragged output (CTA / model)
 __global__ void k_total_sets(double* out, SetsDev sd) {
     const int mi = blockIdx.x;
-    const size_t cs = (size_t)sd.sets[sd.set_of[mi]].n;
+    const size_t cs = ragged_comp_size(sd, mi);
     double* o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
     for (size_t e = threadIdx.x; e < cs; e += blockDim.x)
         o[e] = o[VAG_C_FWD_SYNC * cs + e] + o[VAG_C_FWD_SSC * cs + e] + o[VAG_C_RVS_SYNC * cs + e] + o[VAG_C_RVS_SSC * cs + e];
+}
+
+// ---- band-integrated data in a ragged batch (vag_flux_band_multi, vag_chi2_multi_bands) ----------------------------
+// An evaluation is one (model, band): a model of the ragged grid request whose set is the band (its times, its nodes).
+
+// dst[i] = src[idx[i]]: the parameter record of every evaluation, gathered from the records of the models
+__global__ void k_gather_params(const vag_params* __restrict__ src, const int* __restrict__ idx, size_t n, vag_params* dst) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) dst[i] = src[idx[i]];
+}
+
+// k_band_reduce per evaluation (CTA / evaluation): its [VAG_NCOMP][n_nu][n] grid block (sd.out_off counts from the first
+// evaluation of the call) -> [VAG_NCOMP][n] at VAG_NCOMP * red_off[e], with the weights of its node slice, summed in
+// k_band_reduce's order
+__global__ void k_band_reduce_sets(const double* __restrict__ F, const double* __restrict__ wgt, double* __restrict__ out,
+                                   const long long* __restrict__ red_off, SetsDev sd) {
+    const int e = blockIdx.x;
+    const SeriesSet b = sd.sets[sd.set_of[e]];
+    const double* f0 = F + (size_t)sd.out_off[e] * VAG_NCOMP;
+    const double* wb = wgt + b.nu_off;
+    double* o = out + (size_t)red_off[e] * VAG_NCOMP;
+    for (int q = threadIdx.x; q < VAG_NCOMP * b.n; q += blockDim.x) {
+        const int c = q / b.n, j = q - c * b.n;
+        const double* f = f0 + (size_t)c * b.n_nu * b.n + j;
+        double s = 0;
+        for (int i = 0; i < b.n_nu; ++i) s += f[(size_t)i * b.n] * wb[i];
+        o[q] = s;
+    }
+}
+
+// Band terms of vag_chi2_multi_bands (warp / model).  Model m starts from its point term (pt_of[m] >= 0: the point pass's
+// chi2_pts / st_pts; otherwise 0 and no status) and adds the band terms of its evaluations e0[m] .. e0[m + 1] - 1 in band
+// order through chi2_warp with accumulate, each one's fatal test on its own band run's status st_eval[e], as vag_chi2's
+// k_chi2 launches do.  status[m] = the OR over the terms.  The band data lnF / sig / wgt sit at the band times' offsets.
+__global__ void k_chi2_bands(const double* __restrict__ band, const long long* __restrict__ red_off, SetsDev sd,
+                             const double* __restrict__ lnF, const double* __restrict__ sig, const double* __restrict__ wgt,
+                             const int* __restrict__ st_eval, const int* __restrict__ e0, const int* __restrict__ pt_of,
+                             const double* __restrict__ chi2_pts, const int* __restrict__ st_pts, size_t n_models,
+                             double* chi2, int32_t* status) {
+    const int m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (m >= (int)n_models) return;
+    const int p = pt_of[m];
+    int st = p >= 0 ? st_pts[p] : 0;
+    if (lane == 0) chi2[m] = p >= 0 ? chi2_pts[p] : 0.0;  // read back by lane 0 only (chi2_warp)
+    for (int e = e0[m]; e < e0[m + 1]; ++e) {
+        const SeriesSet b = sd.sets[sd.set_of[e]];
+        chi2_warp(0, lane, band + (size_t)red_off[e] * VAG_NCOMP, b.n, lnF + b.off, sig + b.off, wgt + b.off, nullptr,
+                  nullptr, chi2 + m, st_eval + e, 1);
+        st |= st_eval[e];
+    }
+    if (lane == 0) status[m] = st;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -789,7 +861,7 @@ struct vag_context {
     int device = 0;
     cudaStream_t stream = nullptr;
     DevBuf model_buf, row_buf, cell_buf, obs_buf, ic_buf, lut_buf, sp_buf, geom_buf, split_buf, work_buf;
-    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs, io_sets;  // staging of the host-buffer entry points
+    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs, io_sets, io_bands;  // staging of the host-buffer entry points
     DevBuf plan_buf;                // device planning: the records that run, ok[], capacities
     int* h_totals = nullptr;        // pinned
     int* h_caps = nullptr;          // pinned: capacities planned on the device
@@ -825,6 +897,28 @@ size_t carve_sz(size_t n) {
     return ((n * sizeof(T) + 255) / 256) * 256;
 }
 
+// Host arrays packed for one upload, in 256-byte aligned slices (carve's layout); put() returns the slice's byte offset
+struct Pack {
+    std::vector<char> h;
+    template <class T>
+    size_t put(const T* p, size_t n) {
+        const size_t o = h.size();
+        const char* b = reinterpret_cast<const char*>(p);
+        if (n) h.insert(h.end(), b, b + sizeof(T) * n);
+        h.resize(o + carve_sz<T>(n));
+        return o;
+    }
+    template <class T>
+    size_t put(const std::vector<T>& v) {
+        return put(v.data(), v.size());
+    }
+};
+template <class T>
+T* at(void* base, size_t off) {
+    return reinterpret_cast<T*>(static_cast<char*>(base) + off);
+}
+
+
 constexpr size_t EATS_SMEM_BUDGET = 200 * 1024;  // dynamic shared memory k_eats may ask for
 // models per pipeline pass: k_rowgeom / k_rowcos / k_dop_extrema index the model with gridDim.y (<= 65535), and the
 // per-model workspaces of a pass stay below a few GB; larger batches are processed in consecutive passes
@@ -839,13 +933,14 @@ struct Request {
     const double *d_lnF = nullptr, *d_sig = nullptr, *d_w = nullptr;  // [n_t] observations of a chi-squared series
     const double* d_ext = nullptr;  // [n_t] extinction per point, or NULL
     const double* d_av = nullptr;   // [n_models] A_V per model of the batch, set with d_ext (run_flux offsets it per pass)
-    // A ragged series request (every model its own data set; d_t ... d_ext concatenated over the sets): the device
-    // tables (run_flux slices set_of and out_off per pass), the host prefix sums of the models' output points
-    // [n_models + 1], the number of sets and the size of the largest
+    // A ragged request (every model its own data set; d_t ... d_ext concatenated over the sets; a grid request: d_t and
+    // d_nu): the device tables (run_flux slices set_of and out_off per pass), the host prefix sums of the models' output
+    // points [n_models + 1], the number of sets, the size of the largest (grid: the most times) and, for a grid request,
+    // the most frequency nodes of a model
     const SetsDev* sets = nullptr;
     const long long* h_off = nullptr;
     int n_sets = 0;
-    size_t max_set = 0;
+    size_t max_set = 0, max_nu = 0;
 };
 
 int setup_models(vag_context* ctx, BatchWs& w, const vag_params* d_params, size_t n, Caps caps) {
@@ -945,7 +1040,7 @@ constexpr int EATS_MODES = 3, EATS_KINDS = 3;
 
 // (defined after run_front: the cubin lists the kernel templates in the order the source first names them)
 GridKernel grid_kernel(int lanes, bool ragged);
-EatsKernel eats_kernel(int mode, int kind, bool ragged);  // ragged: nullptr for EATS_GRID
+EatsKernel eats_kernel(int mode, int kind, bool ragged);
 
 // Lanes per model of k_grid: the widest group whose launch fits into one wave of resident CTAs (GRID_MIN_BLOCKS CTAs of
 // 128 threads per SM).  Narrower groups only pay once a wider launch would need a second wave: the models of one warp
@@ -1046,9 +1141,9 @@ EatsKernel eats_kernel(int mode, int kind, bool ragged) {
         {{k_eats<0, EATS_GRID, false>, k_eats<0, EATS_POINT, false>, k_eats<0, EATS_BANDED, false>},
          {k_eats<1, EATS_GRID, false>, k_eats<1, EATS_POINT, false>, k_eats<1, EATS_BANDED, false>},
          {k_eats<2, EATS_GRID, false>, k_eats<2, EATS_POINT, false>, k_eats<2, EATS_BANDED, false>}},
-        {{nullptr, k_eats<0, EATS_POINT, true>, k_eats<0, EATS_BANDED, true>},
-         {nullptr, k_eats<1, EATS_POINT, true>, k_eats<1, EATS_BANDED, true>},
-         {nullptr, k_eats<2, EATS_POINT, true>, k_eats<2, EATS_BANDED, true>}}};
+        {{k_eats<0, EATS_GRID, true>, k_eats<0, EATS_POINT, true>, k_eats<0, EATS_BANDED, true>},
+         {k_eats<1, EATS_GRID, true>, k_eats<1, EATS_POINT, true>, k_eats<1, EATS_BANDED, true>},
+         {k_eats<2, EATS_GRID, true>, k_eats<2, EATS_POINT, true>, k_eats<2, EATS_BANDED, true>}}};
     return k[ragged][mode][kind];
 }
 
@@ -1105,7 +1200,8 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         // (a ragged request: each model's band is its own data set's, as its shared-request call would see it)
         w.nu_range = sets ? nu_range_of : nu_range;
         if (sets)
-            k_nu_range_sets<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(lg2_nu, *sets, (int)n, nu_range_of);
+            (rq_in.series ? k_nu_range_sets<false> : k_nu_range_sets<true>)<<<(unsigned)((n * 32 + 127) / 128), 128, 0, s>>>(
+                lg2_nu, *sets, (int)n, nu_range_of);
         else
             k_nu_range<<<1, 256, 0, s>>>(lg2_nu, (int)n_nu, nu_range);
         k_rowcos<<<dim3((unsigned)((w.max_erows + 127) / 128), (unsigned)n), 128, 0, s>>>(w);
@@ -1130,7 +1226,9 @@ int run_flux_pass(vag_context* ctx, const vag_params* d_params, size_t n, Caps c
         const bool banded = sets ? ctx->series_mode != 1 && series_banded_sets(n_bands_req, ctx->h_bands[1], max_n_t,
                                                                                ctx->series_mode)
                                  : series_banded(n_bands_req, max_n_t, n_t, ctx->series_mode);
-        const int nu_tile = rq_in.series ? (banded ? n_bands_req : 1) : (int)std::min<size_t>(EATS_NU_TILE, n_nu);
+        // (a ragged grid request: the widest node set of the batch; each CTA tiles its own, see k_eats)
+        const int nu_tile = rq_in.series ? (banded ? n_bands_req : 1)
+                                         : (int)std::min<size_t>(EATS_NU_TILE, sets ? rq_in.max_nu : n_nu);
         const int acc_cols = rq_in.series ? 1 : nu_tile;
         const int acc_n = (int)(sets ? rq_in.max_set : n_t);  // accumulator columns: the longest request of the batch
         auto smem_bytes = [&](int rc_) {
@@ -1360,8 +1458,8 @@ int vag_create(int device, vag_context** out) {
     for (bool ragged : {false, true})
         for (int mode = 0; mode < EATS_MODES; ++mode)
             for (int kind = 0; kind < EATS_KINDS; ++kind)
-                if (EatsKernel k = eats_kernel(mode, kind, ragged))
-                    CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EATS_SMEM_BUDGET));
+                CK(cudaFuncSetAttribute(eats_kernel(mode, kind, ragged), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)EATS_SMEM_BUDGET));
     {
         int blocks = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum<false>, 128, 0) == cudaSuccess && blocks > 0)
@@ -1948,14 +2046,14 @@ static int sets_host(vag_context* ctx, const vag_params* params, size_t n_models
     const size_t n_out = (size_t)off[n_models] * VAG_NCOMP;
     cudaStream_t s = ctx->stream;
     if (int rc = upload_request(ctx, t, n_points, nu, n_points)) return rc;
-    CK(ctx->io_sets.ensure(carve_sz<int>(n_models) + carve_sz<SeriesSet>(n_sets) + carve_sz<long long>(n_models)));
+    CK(ctx->io_sets.ensure(carve_sz<int>(n_models) + carve_sz<SeriesSet>(n_sets) + carve_sz<long long>(n_models + 1)));
     char* p = static_cast<char*>(ctx->io_sets.p);
     int* d_set_of = carve<int>(p, n_models);
     SeriesSet* d_sets = carve<SeriesSet>(p, n_sets);
-    long long* d_off = carve<long long>(p, n_models);
+    long long* d_off = carve<long long>(p, n_models + 1);
     CK(cudaMemcpyAsync(d_set_of, dataset_of, sizeof(int) * n_models, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(d_sets, hs.data(), sizeof(SeriesSet) * n_sets, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * n_models, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * (n_models + 1), cudaMemcpyHostToDevice, s));
     const SetsDev sd{d_set_of, d_sets, d_off};
     Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points, n_points};
     rq.sets = &sd;
@@ -2017,6 +2115,284 @@ int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, 
     const double* data[3] = {lnF_obs, sigma_ln, w};
     return sets_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, n_points_total, data, ext_k, A_V, nullptr, chi2,
                      status);
+}
+
+// ---- band-integrated data in a ragged batch ----------------------------------------------------------------------
+// The checks of one band (data: lnF_obs / sigma_ln / w too) and its frequency grid
+static int check_band(const vag_band_obs& B, size_t b, bool data, BandGrid& g) {
+    const std::string name = "band " + std::to_string(b) + ": ";
+    if (B.n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
+    if (data && (!B.lnF_obs || !B.sigma_ln || !B.w)) return fail(VAG_ERR_INVALID, name + "data arrays must not be NULL");
+    if (check_times(B.t, B.n)) return fail(VAG_ERR_INVALID, name + g_err);
+    if (band_grid(B.nu_min, B.nu_max, B.num_nu, g)) return fail(VAG_ERR_INVALID, name + g_err);
+    return VAG_OK;
+}
+
+// Every band checked, its grid built, and the concatenated times and nodes within a 32-bit int
+static int check_bands(const vag_band_obs* bands, size_t n_bands, bool data, std::vector<BandGrid>& grids) {
+    grids.resize(n_bands);
+    size_t n_t = 0, n_nu = 0;
+    for (size_t b = 0; b < n_bands; ++b) {
+        if (int rc = check_band(bands[b], b, data, grids[b])) return rc;
+        n_t += bands[b].n;
+        n_nu += bands[b].num_nu;
+    }
+    if (n_t > (size_t)INT_MAX || n_nu > (size_t)INT_MAX)
+        return fail(VAG_ERR_INVALID, "the band times and frequency nodes of all bands must fit in a 32-bit int");
+    return VAG_OK;
+}
+
+// vag_params_validate with the model named
+static int check_models(const vag_params* params, size_t n_models) {
+    if (!params && n_models) return fail(VAG_ERR_INVALID, "params is NULL");
+    for (size_t m = 0; m < n_models; ++m)
+        if (vag_params_validate(&params[m])) return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": " + g_err);
+    return VAG_OK;
+}
+
+// The band pass: evaluation e evaluates record e of d_params on band band_of[e], all as one ragged grid request through
+// run_flux (passes of 32768 evaluations), then k_band_reduce_sets.  Times, frequency nodes (code units) and weights are
+// concatenated over the bands, and with `data` lnF_obs / sigma_ln / w at the times' offsets.  Its tables go to io_bands,
+// the grid and the band fluxes to io_out.  ctx->launches: run_flux's + 1.
+struct BandPass {
+    SetsDev sd;                      // every evaluation: its band, the band table, its grid block's offset
+    const long long* red_off;        // [n_eval + 1] first band-flux point of each evaluation
+    const double *lnF, *sig, *w;     // with data
+    double* red;                     // [VAG_NCOMP * h_red_off[n_eval]] band fluxes
+    std::vector<long long> h_red_off;
+};
+static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval, Caps caps, const int32_t* band_of,
+                     const vag_band_obs* bands, size_t n_bands, const std::vector<BandGrid>& grids, bool data,
+                     int32_t* d_status, BandPass& bp, cudaStream_t s) {
+    std::vector<SeriesSet> tab(n_bands);
+    std::vector<double> t, nu, wgt, lnF, sig, w;
+    for (size_t b = 0; b < n_bands; ++b) {
+        const vag_band_obs& B = bands[b];
+        const BandGrid& g = grids[b];
+        tab[b] = SeriesSet{(int)t.size(), (int)B.n, (int)g.nu.size(), (int)nu.size()};
+        t.insert(t.end(), B.t, B.t + B.n);
+        nu.insert(nu.end(), g.nu.begin(), g.nu.end());
+        wgt.insert(wgt.end(), g.wgt.begin(), g.wgt.end());
+        if (data) {
+            lnF.insert(lnF.end(), B.lnF_obs, B.lnF_obs + B.n);
+            sig.insert(sig.end(), B.sigma_ln, B.sigma_ln + B.n);
+            w.insert(w.end(), B.w, B.w + B.n);
+        }
+    }
+    std::vector<long long> grid_off(n_eval + 1, 0);
+    bp.h_red_off.assign(n_eval + 1, 0);
+    size_t max_n = 0, max_nu = 0;
+    for (size_t e = 0; e < n_eval; ++e) {
+        const SeriesSet& B = tab[band_of[e]];
+        grid_off[e + 1] = grid_off[e] + (long long)B.n * B.n_nu;
+        bp.h_red_off[e + 1] = bp.h_red_off[e] + B.n;
+        max_n = std::max(max_n, (size_t)B.n);
+        max_nu = std::max(max_nu, (size_t)B.n_nu);
+    }
+    Pack pk;
+    const size_t o_t = pk.put(t), o_nu = pk.put(nu), o_wgt = pk.put(wgt), o_tab = pk.put(tab), o_of = pk.put(band_of, n_eval),
+                 o_go = pk.put(grid_off), o_ro = pk.put(bp.h_red_off), o_lnF = pk.put(lnF), o_sig = pk.put(sig),
+                 o_w = pk.put(w);
+    CK(ctx->io_bands.ensure(pk.h.size()));
+    void* base = ctx->io_bands.p;
+    CK(cudaMemcpyAsync(base, pk.h.data(), pk.h.size(), cudaMemcpyHostToDevice, s));
+    bp.sd = SetsDev{at<int>(base, o_of), at<SeriesSet>(base, o_tab), at<long long>(base, o_go)};
+    bp.red_off = at<long long>(base, o_ro);
+    bp.lnF = data ? at<double>(base, o_lnF) : nullptr;
+    bp.sig = data ? at<double>(base, o_sig) : nullptr;
+    bp.w = data ? at<double>(base, o_w) : nullptr;
+    const size_t grid_elems = (size_t)grid_off[n_eval] * VAG_NCOMP, red_elems = (size_t)bp.h_red_off[n_eval] * VAG_NCOMP;
+    CK(ctx->io_out.ensure(sizeof(double) * (grid_elems + red_elems)));
+    double* d_grid = static_cast<double*>(ctx->io_out.p);
+    bp.red = d_grid + grid_elems;
+    Request rq{false, at<double>(base, o_t), at<double>(base, o_nu), t.size(), nu.size(), true};
+    rq.sets = &bp.sd;
+    rq.h_off = grid_off.data();
+    rq.n_sets = (int)n_bands;
+    rq.max_set = max_n;
+    rq.max_nu = max_nu;
+    if (int rc = run_flux(ctx, d_params, n_eval, caps, rq, d_grid, d_status, nullptr, s)) return rc;
+    k_band_reduce_sets<<<(unsigned)n_eval, 128, 0, s>>>(d_grid, at<double>(base, o_wgt), bp.red, bp.red_off, bp.sd);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    return VAG_OK;
+}
+
+int vag_flux_band_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* band_of,
+                        const vag_band_obs* bands, size_t n_bands, double* out, int32_t* status) {
+    if (!ctx || !out) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (!bands || n_bands == 0) return fail(VAG_ERR_INVALID, "no bands: bands is NULL or n_bands is 0");
+    if (n_models && !band_of) return fail(VAG_ERR_INVALID, "band_of is NULL");
+    if (n_models > (size_t)INT_MAX) return fail(VAG_ERR_INVALID, "n_models must fit in a 32-bit int");
+    std::vector<BandGrid> grids;
+    if (int rc = check_bands(bands, n_bands, false, grids)) return rc;
+    for (size_t m = 0; m < n_models; ++m)
+        if (band_of[m] < 0 || (size_t)band_of[m] >= n_bands)
+            return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": band_of = " + std::to_string(band_of[m]) +
+                                             " is not a band index (n_bands = " + std::to_string(n_bands) + ")");
+    if (int rc = check_models(params, n_models)) return rc;
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) return VAG_OK;
+    cudaStream_t s = ctx->stream;
+    BandPass bp;
+    if (int rc = band_pass(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, band_of, bands, n_bands, grids,
+                           false, static_cast<int32_t*>(ctx->io_status.p), bp, s))
+        return rc;
+    CK(cudaMemcpyAsync(out, bp.red, sizeof(double) * VAG_NCOMP * bp.h_red_off[n_models], cudaMemcpyDeviceToHost, s));
+    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
+}
+
+// The checks of vag_chi2_multi_bands that concern the data sets and the points (before any work is enqueued)
+static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const vag_multi_set* sets, size_t n_sets,
+                            const double* t, const double* nu, size_t n_points, size_t n_bands) {
+    if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no data sets: sets is NULL or n_sets is 0");
+    if (n_points > (size_t)INT_MAX || n_sets > (size_t)INT_MAX || n_models > (size_t)INT_MAX)
+        return fail(VAG_ERR_INVALID, "n_points_total, n_sets and n_models must fit in a 32-bit int");
+    if (n_models && !dataset_of) return fail(VAG_ERR_INVALID, "dataset_of is NULL");
+    for (size_t d = 0; d < n_sets; ++d) {
+        const std::string name = "data set " + std::to_string(d) + ": ";
+        const vag_multi_set& S = sets[d];
+        if (S.n == 0 && S.n_bands == 0) return fail(VAG_ERR_INVALID, name + "no data (n = 0 and n_bands = 0)");
+        if (S.offset > n_points || S.n > n_points - S.offset)
+            return fail(VAG_ERR_INVALID, name + "points [" + std::to_string(S.offset) + ", " + std::to_string(S.offset) +
+                                             " + " + std::to_string(S.n) + ") lie outside the " + std::to_string(n_points) +
+                                             " points");
+        if (S.band0 > n_bands || S.n_bands > n_bands - S.band0)
+            return fail(VAG_ERR_INVALID, name + "bands [" + std::to_string(S.band0) + ", " + std::to_string(S.band0) + " + " +
+                                             std::to_string(S.n_bands) + ") lie outside the " + std::to_string(n_bands) +
+                                             " bands");
+        if (S.n == 0) continue;
+        if (check_times(t + S.offset, S.n)) return fail(VAG_ERR_INVALID, name + g_err);
+        for (size_t i = S.offset; i < S.offset + S.n; ++i)
+            if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
+    }
+    for (size_t m = 0; m < n_models; ++m)
+        if (dataset_of[m] < 0 || (size_t)dataset_of[m] >= n_sets)
+            return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": dataset_of = " + std::to_string(dataset_of[m]) +
+                                             " is not a data set index (n_sets = " + std::to_string(n_sets) + ")");
+    return VAG_OK;
+}
+
+// 1. the ragged point pass over the models whose set has points (vag_chi2_multi's, on those models and the sets with
+// points), 2. the band pass over every (model, band) evaluation, model-major, 3. its reduction, 4. k_chi2_bands.  The
+// records of both passes are gathered on the device from the models' (k_gather_params, one launch for both lists).
+int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                         const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                         const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
+                         const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status) {
+    if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (n_points_total && (!t || !nu || !lnF_obs || !sigma_ln || !w))
+        return fail(VAG_ERR_INVALID, "point data arrays must not be NULL when n_points_total > 0");
+    if (n_bands_total && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
+    const bool ext = ext_k != nullptr;
+    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (ext && n_points_total == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points_total > 0)");
+    if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total, n_bands_total)) return rc;
+    for (size_t i = 0; ext && i < n_points_total; ++i)
+        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
+    std::vector<BandGrid> grids;
+    if (int rc = check_bands(bands, n_bands_total, true, grids)) return rc;
+    if (int rc = check_models(params, n_models)) return rc;
+    // the two lists: models with points (pt_of[m] = index in the point pass, or -1), evaluations (model, band) model-major
+    std::vector<int> gather, pt_of(n_models, -1), e0(n_models + 1, 0), eval_band;
+    std::vector<int> set_idx(n_sets, -1);  // point-pass index of each set with points
+    std::vector<SeriesSet> pt_sets;
+    size_t max_set = 0;
+    for (size_t d = 0; d < n_sets; ++d)
+        if (sets[d].n) {
+            set_idx[d] = (int)pt_sets.size();
+            pt_sets.push_back(SeriesSet{(int)sets[d].offset, (int)sets[d].n, 0, 0});
+            max_set = std::max(max_set, sets[d].n);
+        }
+    std::vector<int> pt_set_of;
+    std::vector<long long> pt_off(1, 0);
+    std::vector<double> pt_av;
+    for (size_t m = 0; m < n_models; ++m) {
+        const vag_multi_set& S = sets[dataset_of[m]];
+        if (!S.n) continue;
+        pt_of[m] = (int)gather.size();
+        gather.push_back((int)m);
+        pt_set_of.push_back(set_idx[dataset_of[m]]);
+        pt_off.push_back(pt_off.back() + (long long)S.n);
+        if (ext) pt_av.push_back(A_V[m]);
+    }
+    const size_t n_pt = gather.size();
+    for (size_t m = 0; m < n_models; ++m) {
+        const vag_multi_set& S = sets[dataset_of[m]];
+        for (size_t j = 0; j < S.n_bands; ++j) {
+            gather.push_back((int)m);
+            eval_band.push_back((int)(S.band0 + j));
+        }
+        e0[m + 1] = (int)eval_band.size();
+        if (eval_band.size() > (size_t)INT_MAX - n_pt)
+            return fail(VAG_ERR_INVALID, "the (model, band) evaluations must fit in a 32-bit int");
+    }
+    const size_t n_eval = eval_band.size();
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) return VAG_OK;
+    cudaStream_t s = ctx->stream;
+    if (n_pt)
+        if (int rc = upload_request(ctx, t, n_points_total, nu, n_points_total)) return rc;
+    // one upload: the lists, the point pass's tables and data; then room for the records and results on the device
+    Pack pk;
+    const size_t o_gather = pk.put(gather), o_pt_of = pk.put(pt_of), o_e0 = pk.put(e0), o_sets = pk.put(pt_sets),
+                 o_set_of = pk.put(pt_set_of), o_off = pk.put(pt_off), o_lnF = pk.put(lnF_obs, n_pt ? n_points_total : 0),
+                 o_sig = pk.put(sigma_ln, n_pt ? n_points_total : 0), o_w = pk.put(w, n_pt ? n_points_total : 0),
+                 o_ext = pk.put(ext_k, ext && n_pt ? n_points_total : 0), o_av = pk.put(pt_av);
+    const size_t up = pk.h.size();
+    const size_t o_rec = up, o_chi2_pts = o_rec + carve_sz<vag_params>(n_pt + n_eval),
+                 o_st_pts = o_chi2_pts + carve_sz<double>(n_pt), o_st_eval = o_st_pts + carve_sz<int>(n_pt),
+                 o_chi2 = o_st_eval + carve_sz<int>(n_eval), o_status = o_chi2 + carve_sz<double>(n_models),
+                 end = o_status + carve_sz<int>(n_models);
+    CK(ctx->io_sets.ensure(end));
+    void* base = ctx->io_sets.p;
+    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
+    vag_params* d_rec = at<vag_params>(base, o_rec);
+    k_gather_params<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(static_cast<vag_params*>(ctx->io_params.p),
+                                                                           at<int>(base, o_gather), n_pt + n_eval, d_rec);
+    int launches = 1;
+    if (n_pt) {
+        const SetsDev sd{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)};
+        Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points_total, n_points_total};
+        rq.sets = &sd;
+        rq.h_off = pt_off.data();
+        rq.n_sets = (int)pt_sets.size();
+        rq.max_set = max_set;
+        rq.d_lnF = at<double>(base, o_lnF);
+        rq.d_sig = at<double>(base, o_sig);
+        rq.d_w = at<double>(base, o_w);
+        if (ext) {
+            rq.d_ext = at<double>(base, o_ext);
+            rq.d_av = at<double>(base, o_av);
+        }
+        CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (size_t)pt_off[n_pt]));
+        if (int rc = run_flux(ctx, d_rec, n_pt, caps, rq, static_cast<double*>(ctx->io_out.p), at<int32_t>(base, o_st_pts),
+                              at<double>(base, o_chi2_pts), s))
+            return rc;
+        launches += ctx->launches;
+    }
+    BandPass bp{};
+    if (n_eval) {
+        if (int rc = band_pass(ctx, d_rec + n_pt, n_eval, caps, eval_band.data(), bands, n_bands_total, grids, true,
+                               at<int32_t>(base, o_st_eval), bp, s))
+            return rc;
+        launches += ctx->launches;
+    }
+    double* d_chi2 = at<double>(base, o_chi2);
+    int32_t* d_status = at<int32_t>(base, o_status);
+    k_chi2_bands<<<(unsigned)((n_models * 32 + 127) / 128), 128, 0, s>>>(
+        bp.red, bp.red_off, bp.sd, bp.lnF, bp.sig, bp.w, at<int>(base, o_st_eval), at<int>(base, o_e0), at<int>(base, o_pt_of),
+        at<double>(base, o_chi2_pts), at<int>(base, o_st_pts), n_models, d_chi2, d_status);
+    ctx->launches = launches + 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
+    if (status) CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
 }
 
 // ---- device-buffer entry points that plan on the device --------------------------------------------------------

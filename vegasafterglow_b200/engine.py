@@ -227,6 +227,93 @@ class Engine:
                                             None if av is None else av.ctypes.data, out.ctypes.data, st.ctypes.data))
         return (out, st) if return_status else out
 
+    # ---- band-integrated data in a batch of several light curves (vag_flux_band_multi, vag_chi2_multi_bands) ------------
+    @staticmethod
+    def _band_array(bands, data):
+        """``abi.BandObs`` array of band dicts (t, nu_min, nu_max, num_nu; with ``data`` also lnF_obs, sigma_ln, w) and the
+        float64 arrays it points into, which must outlive the call."""
+        names = ("t", "lnF_obs", "sigma_ln", "w") if data else ("t",)
+        arr, keep = (abi.BandObs * max(len(bands), 1))(), []
+        for b, band in enumerate(bands):
+            cols = [_f64(band[k]).reshape(-1) for k in names]
+            if len({a.size for a in cols}) != 1:
+                raise ValueError(f"band {b}: arrays {', '.join(names)} must have the same size")
+            keep.append(cols)
+            ptrs = [a.ctypes.data for a in cols] + [None] * (4 - len(cols))
+            arr[b] = abi.BandObs(*ptrs, cols[0].size, float(band["nu_min"]), float(band["nu_max"]), int(band["num_nu"]))
+        return arr, keep
+
+    def flux_band_multi(self, params, bands, band_of, return_status=False):
+        """``flux_band`` of model m on its own band ``bands[band_of[m]]`` (a dict with t, nu_min, nu_max, num_nu), all in
+        one batch.  Returns a list with one float64[5, n_t] array per model (n_t: its band's epochs); the arrays are views
+        into one buffer in model order (``vag_flux_band_multi``)."""
+        p = self._params(params)
+        arr, keep = self._band_array(bands, data=False)
+        bo = self._dataset_of(band_of, p.size)
+        n_m = np.asarray([keep[b][0].size for b in bo] if p.size and bo.min() >= 0 and bo.max() < len(bands) else
+                         np.zeros(p.size), dtype=np.int64)
+        off = np.concatenate([[0], np.cumsum(n_m)]).astype(np.int64)
+        buf = np.empty(abi.NCOMP * int(off[-1]))
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_flux_band_multi(self._h, p.ctypes.data, p.size, bo.ctypes.data, C.cast(arr, C.c_void_p),
+                                                 len(bands), buf.ctypes.data, st.ctypes.data))
+        out = [buf[abi.NCOMP * off[m]:abi.NCOMP * off[m + 1]].reshape(abi.NCOMP, int(n_m[m])) for m in range(p.size)]
+        return (out, st) if return_status else out
+
+    def chi2_multi_bands(self, params, datasets, bands, dataset_of, extinction=None, return_status=False):
+        """``chi2`` of model m on its own data set, all in one batch -> chi2[n_models].  Data set d is its point data
+        ``datasets[d]`` = (t, nu, lnF_obs, sigma_ln, w), t ascending, or None when it has none, and its band-integrated data
+        ``bands[d]``, a list of ``fitting.band_obs`` dicts (may be empty when it has points).  ``extinction`` = (ext_k, A_V):
+        ext_k a list with one array per data set (None for a set without points), A_V[n_models]; model m's points are then
+        compared as lnF_obs + A_V[m] * ext_k, its band terms unchanged (``vag_chi2_multi_bands``)."""
+        p = self._params(params)
+        if len(bands) != len(datasets):
+            raise ValueError(f"{len(bands)} band lists for {len(datasets)} data sets")
+        cols, n_pts = [[] for _ in range(5)], np.zeros(len(datasets), dtype=np.int64)
+        for d, dset in enumerate(datasets):
+            if dset is None:
+                continue
+            arrs = [_f64(a).reshape(-1) for a in dset]
+            if len(arrs) != 5 or len({a.size for a in arrs}) != 1:
+                raise ValueError(f"data set {d} must be (t, nu, lnF_obs, sigma_ln, w) of one size, or None")
+            for c, a in zip(cols, arrs):
+                c.append(a)
+            n_pts[d] = arrs[0].size
+        t, nu, lnF, sig, w = (np.concatenate(c) if c else np.zeros(0) for c in cols)
+        pt_off = np.concatenate([[0], np.cumsum(n_pts)]).astype(np.int64)
+        flat = [b for bl in bands for b in bl]
+        arr, _keep = self._band_array(flat, data=True)
+        sets = (abi.MultiSet * max(len(datasets), 1))()
+        b0 = 0
+        for d in range(len(datasets)):
+            sets[d] = abi.MultiSet(int(pt_off[d]), int(n_pts[d]), b0, len(bands[d]))
+            b0 += len(bands[d])
+        ds = self._dataset_of(dataset_of, p.size)
+        ext = av = None
+        if extinction is not None:
+            ext_sets, av = extinction
+            if len(ext_sets) != len(datasets):
+                raise ValueError(f"extinction has {len(ext_sets)} ext_k entries for {len(datasets)} data sets")
+            ext = []
+            for d, e in enumerate(ext_sets):
+                e = np.zeros(0) if e is None else _f64(e).reshape(-1)
+                if e.size != n_pts[d]:
+                    raise ValueError(f"data set {d}: ext_k has {e.size} values for {n_pts[d]} points")
+                ext.append(e)
+            ext = np.concatenate(ext)
+            av = _f64(av).reshape(-1)
+            if av.size != p.size:
+                raise ValueError(f"A_V has {av.size} values for {p.size} models")
+        out = np.empty(p.size)
+        st = np.zeros(p.size, dtype=np.int32)
+        pts = [a.ctypes.data if t.size else None for a in (t, nu, lnF, sig, w)]
+        _lib.check(self._lib.vag_chi2_multi_bands(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p),
+                                                  len(datasets), *pts, None if ext is None else ext.ctypes.data, t.size,
+                                                  None if av is None else av.ctypes.data,
+                                                  C.cast(arr, C.c_void_p) if flat else None, len(flat), out.ctypes.data,
+                                                  st.ctypes.data))
+        return (out, st) if return_status else out
+
     @staticmethod
     def valid_mask(params):
         """bool[n]: which parameter sets pass the constructor checks of the reference (vag_params_validate_batch)."""

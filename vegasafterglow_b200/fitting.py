@@ -290,7 +290,8 @@ class LikelihoodStack:
     ``A_V``; fit k's walkers are evaluated on fit k's data set.  Bounds, rejected parameter sets and non-finite chi2 give
     -inf as in ``BatchedLikelihood.__call__``.  When only some fits sample ``A_V``, the others run with ext_k = 0 and
     A_V = 0, and lnF_obs + 0 * 0 is lnF_obs exactly.  The engine is the first likelihood's.
-    Not supported (``NotImplementedError``): band-integrated data, ``distributed=True`` and ``DeviceLikelihood``."""
+    Not supported (``NotImplementedError``): band-integrated data (stack such fits with ``BandLikelihoodStack``),
+    ``distributed=True`` and ``DeviceLikelihood``."""
 
     def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
         self.likelihoods = list(likelihoods)
@@ -307,8 +308,9 @@ class LikelihoodStack:
         self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) for lk in self.likelihoods]
         self.fits_av = ["A_V" in lk.names for lk in self.likelihoods]
 
-    def chi2(self, samples):
-        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject."""
+    def _walkers(self, samples):
+        """The valid walkers of every fit as one batch: (records, fit of each, A_V of each (0 where the fit has none),
+        the validity mask of every fit)."""
         from .engine import Engine
 
         P, ds, av, ok = [], [], [], []
@@ -320,12 +322,11 @@ class LikelihoodStack:
             P.append(p[good])
             ds.append(np.full(int(good.sum()), k, dtype=np.int32))
             av.append(lk._column(s, lk.names.index("A_V"))[good] if self.fits_av[k] else np.zeros(int(good.sum())))
-        P, ds = np.concatenate(P), np.concatenate(ds)
-        extinction = None
-        if any(self.fits_av):
-            ext = [lk.ext_kernel if fit else np.zeros(lk.t.size) for lk, fit in zip(self.likelihoods, self.fits_av)]
-            extinction = (ext, np.concatenate(av))
-        flat = self.engine.chi2_multi(P, self.datasets, ds, extinction=extinction) if P.size else np.zeros(0)
+        return np.concatenate(P), np.concatenate(ds), np.concatenate(av), ok
+
+    @staticmethod
+    def _split(flat, ok):
+        """chi2 of the valid walkers back per fit, +inf for the rejected ones."""
         out, lo = [], 0
         for good in ok:
             c = np.full(good.size, np.inf)
@@ -334,6 +335,16 @@ class LikelihoodStack:
             out.append(c)
         return out
 
+    def chi2(self, samples):
+        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject."""
+        P, ds, av, ok = self._walkers(samples)
+        extinction = None
+        if any(self.fits_av):
+            ext = [lk.ext_kernel if fit else np.zeros(lk.t.size) for lk, fit in zip(self.likelihoods, self.fits_av)]
+            extinction = (ext, av)
+        flat = self.engine.chi2_multi(P, self.datasets, ds, extinction=extinction) if P.size else np.zeros(0)
+        return self._split(flat, ok)
+
     def __call__(self, samples):
         if len(samples) != len(self.likelihoods):
             raise ValueError(f"{len(samples)} sample arrays for {len(self.likelihoods)} likelihoods")
@@ -341,3 +352,38 @@ class LikelihoodStack:
         idx = [lk._in_bounds(s) for lk, s in zip(self.likelihoods, samples)]
         chi2 = self.chi2([s[i] for s, i in zip(samples, idx)])
         return [lk._log_prob(s, i, c) for lk, s, i, c in zip(self.likelihoods, samples, idx, chi2)]
+
+
+class BandLikelihoodStack(LikelihoodStack):
+    """``LikelihoodStack`` for fits with band-integrated data: fits with points and bands, bands only, or points only, all
+    evaluated with ONE ``Engine.chi2_multi_bands`` call -- the points of every fit in one ragged pass and every band of
+    every fit in one more, where each ``BatchedLikelihood`` alone makes 1 + (its bands) pipeline runs.  Fit k's walkers
+    get fit k's point term and then its band terms in its own order; ``__call__``, the bounds and the -inf rules are
+    ``LikelihoodStack``'s.  A bands-only fit that names ``A_V`` ignores it, as ``BatchedLikelihood`` does without points.
+    Not supported (``NotImplementedError``): ``distributed=True`` and ``DeviceLikelihood``."""
+
+    def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
+        self.likelihoods = list(likelihoods)
+        if not self.likelihoods:
+            raise ValueError("BandLikelihoodStack needs at least one likelihood")
+        for k, lk in enumerate(self.likelihoods):
+            if isinstance(lk, DeviceLikelihood):
+                raise NotImplementedError(f"likelihood {k}: a DeviceLikelihood cannot be stacked (its data live in HBM)")
+            if lk.distributed:
+                raise NotImplementedError(f"likelihood {k}: distributed=True cannot be stacked")
+        self.engine = self.likelihoods[0].engine
+        self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) if lk.t.size else None for lk in self.likelihoods]
+        self.bands = [lk.bands for lk in self.likelihoods]
+        self.fits_av = ["A_V" in lk.names and lk.t.size > 0 for lk in self.likelihoods]
+
+    def chi2(self, samples):
+        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject."""
+        P, ds, av, ok = self._walkers(samples)
+        extinction = None
+        if any(self.fits_av):
+            ext = [None if not lk.t.size else lk.ext_kernel if fit else np.zeros(lk.t.size)
+                   for lk, fit in zip(self.likelihoods, self.fits_av)]
+            extinction = (ext, av)
+        flat = (self.engine.chi2_multi_bands(P, self.datasets, self.bands, ds, extinction=extinction) if P.size
+                else np.zeros(0))
+        return self._split(flat, ok)
