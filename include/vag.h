@@ -207,8 +207,9 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
  * parameter sets as vag_params_validate.  A data set no model uses is allowed.  Batches over 32768 models run in
  * passes as the other entry points do.  Launches: those of vag_chi2_series / vag_flux_density_series on the same
  * total data, whatever n_sets (one CTA per data set inside the band search kernel).
- * Not provided here: band-integrated data per data set (vag_flux_band_multi, vag_chi2_multi_bands below), a
- * device-buffer (_dev) variant, a public per-model grid (t x nu) request.
+ * Band-integrated data per data set: vag_flux_band_multi, vag_chi2_multi_bands below; on device buffers, planned on the
+ * device: vag_chi2_multi_bands_dev (further below).  Not provided here: a device-buffer (_dev) variant of the two flux
+ * calls, a public per-model grid (t x nu) request.
  * The output mode (vag_set_output_mode) does not apply: every plane of `out` is written. */
 typedef struct vag_series_set {
     size_t offset, n; /* slice of the concatenated points */
@@ -327,6 +328,36 @@ int vag_chi2_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, 
                  const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k, size_t n_points,
                  const double* d_A_V, const vag_band_obs* bands, size_t n_bands, double* d_chi2, int32_t* d_status,
                  void* stream);
+
+/* vag_chi2_multi_bands on device buffers, planned on the device: several light curves with points and bands in one batch
+ * whose records, data and results stay in HBM.  d_params, d_t ... d_ext_k, d_A_V, d_chi2 and d_status (may be NULL) are
+ * device pointers; dataset_of, sets and `bands` are host arrays, read only during the call, and the bands' t / lnF_obs /
+ * sigma_ln / w are device pointers (vag_chi2_dev's convention).  The output offsets, the point and evaluation lists and
+ * the passes of 32768 models are planned on the host, as in vag_chi2_multi_bands.
+ * Planning: k_plan checks every record as vag_params_validate does and takes the capacities of the accepted ones; one D2H
+ * brings back the two capacities and the ok flags, with one synchronisation of `stream`.  A rejected record is left out
+ * of the batch, not run as a stand-in (unlike vag_chi2_dev): the lists hold the accepted models only, and a final k_reject
+ * writes chi2 = +inf and status VAG_ST_INVALID for the rejected ones.  For every accepted model, chi2 and status equal
+ * those of vag_chi2_multi_bands called on the accepted models alone with host copies of the same arrays, bit for bit, in
+ * every series mode: it is the same batch, and the plan's capacities are the host's.  The result does not depend on what
+ * the rejected records contain.
+ * The accepted models' records, and the point models' A_V, are gathered from d_params / d_A_V on the device (one launch);
+ * every band's t / lnF_obs / sigma_ln / w are copied into the concatenated band workspace by one more launch (a CTA per
+ * band); the bands' frequency nodes and weights are made on the host.
+ * Launches: 2 when no record is accepted (k_plan, k_reject); otherwise L + 2 + (1 when any accepted model has a band),
+ * where L = the launches of vag_chi2_multi_bands on the accepted models (L(points) + L(bands) + 2, see there) -- whatever
+ * the number of data sets, bands or models.  Synchronisations: those of vag_chi2_multi_bands plus the plan's; the call
+ * returns with its work enqueued on `stream`.  n_models == 0: VAG_OK, nothing enqueued.
+ * Checks before any work (VAG_ERR_INVALID, messages name the data set, the band or the model; a failed call leaves the
+ * context usable): the structural checks of vag_chi2_multi_bands -- set and band ranges, dataset_of in range, n > 0 or
+ * n_bands > 0 per set, nu_min / nu_max / num_nu, NULL pointers, the 32-bit limits, ext_k / A_V both set or both NULL and
+ * then points.  Not checked on the device path: the time order and finiteness of d_t, d_nu and the band times, and the
+ * finiteness of d_ext_k. */
+int vag_chi2_multi_bands_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const int32_t* dataset_of,
+                             const vag_multi_set* sets, size_t n_sets, const double* d_t, const double* d_nu,
+                             const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k,
+                             size_t n_points_total, const double* d_A_V, const vag_band_obs* bands, size_t n_bands_total,
+                             double* d_chi2, int32_t* d_status, void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* introspection (tests, profiling): stage tables of ONE model, the analogue of                 */

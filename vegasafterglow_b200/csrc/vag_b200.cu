@@ -814,6 +814,30 @@ __global__ void k_chi2_bands(const double* __restrict__ band, const long long* _
     if (lane == 0) status[m] = st;
 }
 
+// ---- the ragged call planned on the device (vag_chi2_multi_bands_dev) --------------------------------------------
+// k_gather_params, and for the first n_av entries (the point pass's models) their A_V as well: av_dst[i] = av_src[idx[i]]
+__global__ void k_gather_params_av(const vag_params* __restrict__ src, const int* __restrict__ idx, size_t n, vag_params* dst,
+                                   const double* __restrict__ av_src, size_t n_av, double* av_dst) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int j = idx[i];
+    dst[i] = src[j];
+    if (i < n_av) av_dst[i] = av_src[j];
+}
+
+// The band data into the concatenated band workspace (CTA / band): plane k of dst (t, lnF_obs, sigma_ln, w; `stride`
+// doubles each) receives band b's device array src[4 b + k] at the band's time offset tab[b].off
+__global__ void k_gather_bands(const double* const* __restrict__ src, const SeriesSet* __restrict__ tab, size_t stride,
+                               double* dst) {
+    const int b = blockIdx.x;
+    const SeriesSet B = tab[b];
+    for (int k = 0; k < 4; ++k) {
+        const double* __restrict__ a = src[4 * (size_t)b + k];
+        double* d = dst + k * stride + B.off;
+        for (int i = threadIdx.x; i < B.n; i += blockDim.x) d[i] = a[i];
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -865,6 +889,8 @@ struct vag_context {
     DevBuf plan_buf;                // device planning: the records that run, ok[], capacities
     int* h_totals = nullptr;        // pinned
     int* h_caps = nullptr;          // pinned: capacities planned on the device
+    char* h_plan = nullptr;         // pinned, grown on demand: ok[] and the capacities of vag_chi2_multi_bands_dev's plan
+    size_t h_plan_cap = 0;
     long long* h_cells = nullptr;   // pinned
     int* h_bands = nullptr;         // pinned [2]: distinct frequencies of the series request in flight (ragged: see k_series_bands_sets)
     int series_mode = 0;            // vag_set_series_mode: 0 auto, 1 per-point spectra always, 2 banded whenever possible
@@ -1477,6 +1503,7 @@ void vag_destroy(vag_context* c) {
     if (c->h_cells) cudaFreeHost(c->h_cells);
     if (c->h_bands) cudaFreeHost(c->h_bands);
     if (c->h_caps) cudaFreeHost(c->h_caps);
+    if (c->h_plan) cudaFreeHost(c->h_plan);
     for (auto& ev : c->ev)
         if (ev) cudaEventDestroy(ev);
     cudaStreamDestroy(c->stream);
@@ -2118,22 +2145,28 @@ int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, 
 }
 
 // ---- band-integrated data in a ragged batch ----------------------------------------------------------------------
-// The checks of one band (data: lnF_obs / sigma_ln / w too) and its frequency grid
-static int check_band(const vag_band_obs& B, size_t b, bool data, BandGrid& g) {
+// The checks of one band (data: lnF_obs / sigma_ln / w too) and its frequency grid; with `device` its arrays are device
+// memory, whose values are not read (only t != NULL is checked)
+static int check_band(const vag_band_obs& B, size_t b, bool data, BandGrid& g, bool device) {
     const std::string name = "band " + std::to_string(b) + ": ";
     if (B.n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
     if (data && (!B.lnF_obs || !B.sigma_ln || !B.w)) return fail(VAG_ERR_INVALID, name + "data arrays must not be NULL");
-    if (check_times(B.t, B.n)) return fail(VAG_ERR_INVALID, name + g_err);
+    if (device) {
+        if (!B.t) return fail(VAG_ERR_INVALID, name + "time array must not be NULL");
+    } else if (check_times(B.t, B.n)) {
+        return fail(VAG_ERR_INVALID, name + g_err);
+    }
     if (band_grid(B.nu_min, B.nu_max, B.num_nu, g)) return fail(VAG_ERR_INVALID, name + g_err);
     return VAG_OK;
 }
 
 // Every band checked, its grid built, and the concatenated times and nodes within a 32-bit int
-static int check_bands(const vag_band_obs* bands, size_t n_bands, bool data, std::vector<BandGrid>& grids) {
+static int check_bands(const vag_band_obs* bands, size_t n_bands, bool data, std::vector<BandGrid>& grids,
+                       bool device = false) {
     grids.resize(n_bands);
     size_t n_t = 0, n_nu = 0;
     for (size_t b = 0; b < n_bands; ++b) {
-        if (int rc = check_band(bands[b], b, data, grids[b])) return rc;
+        if (int rc = check_band(bands[b], b, data, grids[b], device)) return rc;
         n_t += bands[b].n;
         n_nu += bands[b].num_nu;
     }
@@ -2153,7 +2186,9 @@ static int check_models(const vag_params* params, size_t n_models) {
 // The band pass: evaluation e evaluates record e of d_params on band band_of[e], all as one ragged grid request through
 // run_flux (passes of 32768 evaluations), then k_band_reduce_sets.  Times, frequency nodes (code units) and weights are
 // concatenated over the bands, and with `data` lnF_obs / sigma_ln / w at the times' offsets.  Its tables go to io_bands,
-// the grid and the band fluxes to io_out.  ctx->launches: run_flux's + 1.
+// the grid and the band fluxes to io_out.  ctx->launches: run_flux's + 1.  With `device` (implies data) the bands' t /
+// lnF_obs / sigma_ln / w are device pointers: the host uploads a table of them with the other tables, and k_gather_bands
+// (one more launch) copies the arrays into the concatenated workspace behind that upload.
 struct BandPass {
     SetsDev sd;                      // every evaluation: its band, the band table, its grid block's offset
     const long long* red_off;        // [n_eval + 1] first band-flux point of each evaluation
@@ -2163,16 +2198,23 @@ struct BandPass {
 };
 static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval, Caps caps, const int32_t* band_of,
                      const vag_band_obs* bands, size_t n_bands, const std::vector<BandGrid>& grids, bool data,
-                     int32_t* d_status, BandPass& bp, cudaStream_t s) {
+                     int32_t* d_status, BandPass& bp, cudaStream_t s, bool device = false) {
     std::vector<SeriesSet> tab(n_bands);
     std::vector<double> t, nu, wgt, lnF, sig, w;
+    std::vector<const double*> src;  // device: [n_bands][4] t, lnF_obs, sigma_ln, w
+    size_t n_t = 0;
     for (size_t b = 0; b < n_bands; ++b) {
         const vag_band_obs& B = bands[b];
         const BandGrid& g = grids[b];
-        tab[b] = SeriesSet{(int)t.size(), (int)B.n, (int)g.nu.size(), (int)nu.size()};
-        t.insert(t.end(), B.t, B.t + B.n);
+        tab[b] = SeriesSet{(int)n_t, (int)B.n, (int)g.nu.size(), (int)nu.size()};
+        n_t += B.n;
         nu.insert(nu.end(), g.nu.begin(), g.nu.end());
         wgt.insert(wgt.end(), g.wgt.begin(), g.wgt.end());
+        if (device) {
+            src.insert(src.end(), {B.t, B.lnF_obs, B.sigma_ln, B.w});
+            continue;
+        }
+        t.insert(t.end(), B.t, B.t + B.n);
         if (data) {
             lnF.insert(lnF.end(), B.lnF_obs, B.lnF_obs + B.n);
             sig.insert(sig.end(), B.sigma_ln, B.sigma_ln + B.n);
@@ -2192,20 +2234,30 @@ static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval
     Pack pk;
     const size_t o_t = pk.put(t), o_nu = pk.put(nu), o_wgt = pk.put(wgt), o_tab = pk.put(tab), o_of = pk.put(band_of, n_eval),
                  o_go = pk.put(grid_off), o_ro = pk.put(bp.h_red_off), o_lnF = pk.put(lnF), o_sig = pk.put(sig),
-                 o_w = pk.put(w);
-    CK(ctx->io_bands.ensure(pk.h.size()));
+                 o_w = pk.put(w), o_src = pk.put(src);
+    const size_t up = pk.h.size(), plane = device ? carve_sz<double>(n_t) / sizeof(double) : 0;
+    CK(ctx->io_bands.ensure(up + 4 * sizeof(double) * plane));
     void* base = ctx->io_bands.p;
-    CK(cudaMemcpyAsync(base, pk.h.data(), pk.h.size(), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
     bp.sd = SetsDev{at<int>(base, o_of), at<SeriesSet>(base, o_tab), at<long long>(base, o_go)};
     bp.red_off = at<long long>(base, o_ro);
+    const double* d_t = at<double>(base, o_t);
     bp.lnF = data ? at<double>(base, o_lnF) : nullptr;
     bp.sig = data ? at<double>(base, o_sig) : nullptr;
     bp.w = data ? at<double>(base, o_w) : nullptr;
+    if (device) {
+        double* planes = at<double>(base, up);
+        k_gather_bands<<<(unsigned)n_bands, 128, 0, s>>>(at<const double*>(base, o_src), bp.sd.sets, plane, planes);
+        d_t = planes;
+        bp.lnF = planes + plane;
+        bp.sig = planes + 2 * plane;
+        bp.w = planes + 3 * plane;
+    }
     const size_t grid_elems = (size_t)grid_off[n_eval] * VAG_NCOMP, red_elems = (size_t)bp.h_red_off[n_eval] * VAG_NCOMP;
     CK(ctx->io_out.ensure(sizeof(double) * (grid_elems + red_elems)));
     double* d_grid = static_cast<double*>(ctx->io_out.p);
     bp.red = d_grid + grid_elems;
-    Request rq{false, at<double>(base, o_t), at<double>(base, o_nu), t.size(), nu.size(), true};
+    Request rq{false, d_t, at<double>(base, o_nu), n_t, nu.size(), true};
     rq.sets = &bp.sd;
     rq.h_off = grid_off.data();
     rq.n_sets = (int)n_bands;
@@ -2213,7 +2265,7 @@ static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval
     rq.max_nu = max_nu;
     if (int rc = run_flux(ctx, d_params, n_eval, caps, rq, d_grid, d_status, nullptr, s)) return rc;
     k_band_reduce_sets<<<(unsigned)n_eval, 128, 0, s>>>(d_grid, at<double>(base, o_wgt), bp.red, bp.red_off, bp.sd);
-    ctx->launches++;
+    ctx->launches += device ? 2 : 1;  // (k_gather_bands ran before run_flux, which restarts the count)
     CK(cudaGetLastError());
     return VAG_OK;
 }
@@ -2245,9 +2297,10 @@ int vag_flux_band_multi(vag_context* ctx, const vag_params* params, size_t n_mod
     return VAG_OK;
 }
 
-// The checks of vag_chi2_multi_bands that concern the data sets and the points (before any work is enqueued)
+// The checks of vag_chi2_multi_bands that concern the data sets and the points (before any work is enqueued); with
+// `device` the points are device memory, whose values are not read
 static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const vag_multi_set* sets, size_t n_sets,
-                            const double* t, const double* nu, size_t n_points, size_t n_bands) {
+                            const double* t, const double* nu, size_t n_points, size_t n_bands, bool device = false) {
     if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no data sets: sets is NULL or n_sets is 0");
     if (n_points > (size_t)INT_MAX || n_sets > (size_t)INT_MAX || n_models > (size_t)INT_MAX)
         return fail(VAG_ERR_INVALID, "n_points_total, n_sets and n_models must fit in a 32-bit int");
@@ -2264,7 +2317,7 @@ static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const va
             return fail(VAG_ERR_INVALID, name + "bands [" + std::to_string(S.band0) + ", " + std::to_string(S.band0) + " + " +
                                              std::to_string(S.n_bands) + ") lie outside the " + std::to_string(n_bands) +
                                              " bands");
-        if (S.n == 0) continue;
+        if (S.n == 0 || device) continue;
         if (check_times(t + S.offset, S.n)) return fail(VAG_ERR_INVALID, name + g_err);
         for (size_t i = S.offset; i < S.offset + S.n; ++i)
             if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
@@ -2273,6 +2326,104 @@ static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const va
         if (dataset_of[m] < 0 || (size_t)dataset_of[m] >= n_sets)
             return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": dataset_of = " + std::to_string(dataset_of[m]) +
                                              " is not a data set index (n_sets = " + std::to_string(n_sets) + ")");
+    return VAG_OK;
+}
+
+// The two lists of vag_chi2_multi_bands(_dev), over the models m with ok[m] (every model when ok is NULL): the models whose
+// set has points (pt_of[m] = index in the point pass, or -1) and the (model, band) evaluations, model-major; gather = the
+// model of every entry of both, the point pass first.  The point pass's data sets are all the sets with points, whether a
+// model uses them or not.
+struct MultiLists {
+    std::vector<int> gather, pt_of, e0, eval_band, pt_set_of;
+    std::vector<SeriesSet> pt_sets;
+    std::vector<long long> pt_off{0};
+    size_t max_set = 0, n_pt = 0, n_eval = 0;
+};
+static void multi_lists(size_t n_models, const int32_t* dataset_of, const vag_multi_set* sets, size_t n_sets,
+                        const int32_t* ok, MultiLists& L) {
+    L.pt_of.assign(n_models, -1);
+    L.e0.assign(n_models + 1, 0);
+    std::vector<int> set_idx(n_sets, -1);  // point-pass index of each set with points
+    for (size_t d = 0; d < n_sets; ++d)
+        if (sets[d].n) {
+            set_idx[d] = (int)L.pt_sets.size();
+            L.pt_sets.push_back(SeriesSet{(int)sets[d].offset, (int)sets[d].n, 0, 0});
+            L.max_set = std::max(L.max_set, sets[d].n);
+        }
+    for (size_t m = 0; m < n_models; ++m) {
+        const vag_multi_set& S = sets[dataset_of[m]];
+        if (!S.n || (ok && !ok[m])) continue;
+        L.pt_of[m] = (int)L.gather.size();
+        L.gather.push_back((int)m);
+        L.pt_set_of.push_back(set_idx[dataset_of[m]]);
+        L.pt_off.push_back(L.pt_off.back() + (long long)S.n);
+    }
+    L.n_pt = L.gather.size();
+    for (size_t m = 0; m < n_models; ++m) {
+        const vag_multi_set& S = sets[dataset_of[m]];
+        for (size_t j = 0; (!ok || ok[m]) && j < S.n_bands; ++j) {
+            L.gather.push_back((int)m);
+            L.eval_band.push_back((int)(S.band0 + j));
+        }
+        L.e0[m + 1] = (int)L.eval_band.size();
+    }
+    L.n_eval = L.eval_band.size();
+}
+
+// The entries of both lists over all models within a 32-bit int (sets and dataset_of checked)
+static int check_multi_count(size_t n_models, const int32_t* dataset_of, const vag_multi_set* sets) {
+    size_t n = 0;
+    for (size_t m = 0; m < n_models; ++m) {
+        const vag_multi_set& S = sets[dataset_of[m]];
+        n += S.n_bands + (S.n ? 1 : 0);
+        if (n > (size_t)INT_MAX) return fail(VAG_ERR_INVALID, "the (model, band) evaluations must fit in a 32-bit int");
+    }
+    return VAG_OK;
+}
+
+// L's tables and the intermediate results on the device
+struct MultiDev {
+    const int *pt_of, *e0;
+    SetsDev pt_sd;              // the point pass: its models' data sets, the sets, the output offsets
+    double* chi2_pts;           // [n_pt]
+    int32_t *st_pts, *st_eval;  // [n_pt], [n_eval]
+};
+
+// Steps 1, 2 (with 3) and 4 below on the records d_rec gathered for L (the point models', then the evaluations'): the point
+// pass on pts (pts.av: the A_V of each point model), the band pass (device: its data are device pointers), and
+// k_chi2_bands over all n_models.  *launches: the launches of the three.
+static int multi_passes(vag_context* ctx, const vag_params* d_rec, const MultiLists& L, Caps caps, const Chi2Points& pts,
+                        const MultiDev& tb, const vag_band_obs* bands, size_t n_bands, const std::vector<BandGrid>& grids,
+                        bool device, size_t n_models, double* d_chi2, int32_t* d_status, cudaStream_t s, int* launches) {
+    *launches = 0;
+    if (L.n_pt) {
+        Request rq{true, pts.t, pts.nu, pts.n, pts.n};
+        rq.sets = &tb.pt_sd;
+        rq.h_off = L.pt_off.data();
+        rq.n_sets = (int)L.pt_sets.size();
+        rq.max_set = L.max_set;
+        rq.d_lnF = pts.lnF;
+        rq.d_sig = pts.sig;
+        rq.d_w = pts.w;
+        rq.d_ext = pts.ext;
+        rq.d_av = pts.av;
+        CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (size_t)L.pt_off[L.n_pt]));
+        if (int rc = run_flux(ctx, d_rec, L.n_pt, caps, rq, static_cast<double*>(ctx->io_out.p), tb.st_pts, tb.chi2_pts, s))
+            return rc;
+        *launches += ctx->launches;
+    }
+    BandPass bp{};
+    if (L.n_eval) {
+        if (int rc = band_pass(ctx, d_rec + L.n_pt, L.n_eval, caps, L.eval_band.data(), bands, n_bands, grids, true,
+                               tb.st_eval, bp, s, device))
+            return rc;
+        *launches += ctx->launches;
+    }
+    k_chi2_bands<<<(unsigned)((n_models * 32 + 127) / 128), 128, 0, s>>>(bp.red, bp.red_off, bp.sd, bp.lnF, bp.sig, bp.w,
+                                                                         tb.st_eval, tb.e0, tb.pt_of, tb.chi2_pts, tb.st_pts,
+                                                                         n_models, d_chi2, d_status);
+    *launches += 1;
+    CK(cudaGetLastError());
     return VAG_OK;
 }
 
@@ -2296,41 +2447,12 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
     std::vector<BandGrid> grids;
     if (int rc = check_bands(bands, n_bands_total, true, grids)) return rc;
     if (int rc = check_models(params, n_models)) return rc;
-    // the two lists: models with points (pt_of[m] = index in the point pass, or -1), evaluations (model, band) model-major
-    std::vector<int> gather, pt_of(n_models, -1), e0(n_models + 1, 0), eval_band;
-    std::vector<int> set_idx(n_sets, -1);  // point-pass index of each set with points
-    std::vector<SeriesSet> pt_sets;
-    size_t max_set = 0;
-    for (size_t d = 0; d < n_sets; ++d)
-        if (sets[d].n) {
-            set_idx[d] = (int)pt_sets.size();
-            pt_sets.push_back(SeriesSet{(int)sets[d].offset, (int)sets[d].n, 0, 0});
-            max_set = std::max(max_set, sets[d].n);
-        }
-    std::vector<int> pt_set_of;
-    std::vector<long long> pt_off(1, 0);
+    if (int rc = check_multi_count(n_models, dataset_of, sets)) return rc;
+    MultiLists L;
+    multi_lists(n_models, dataset_of, sets, n_sets, nullptr, L);
+    const size_t n_pt = L.n_pt, n_eval = L.n_eval;
     std::vector<double> pt_av;
-    for (size_t m = 0; m < n_models; ++m) {
-        const vag_multi_set& S = sets[dataset_of[m]];
-        if (!S.n) continue;
-        pt_of[m] = (int)gather.size();
-        gather.push_back((int)m);
-        pt_set_of.push_back(set_idx[dataset_of[m]]);
-        pt_off.push_back(pt_off.back() + (long long)S.n);
-        if (ext) pt_av.push_back(A_V[m]);
-    }
-    const size_t n_pt = gather.size();
-    for (size_t m = 0; m < n_models; ++m) {
-        const vag_multi_set& S = sets[dataset_of[m]];
-        for (size_t j = 0; j < S.n_bands; ++j) {
-            gather.push_back((int)m);
-            eval_band.push_back((int)(S.band0 + j));
-        }
-        e0[m + 1] = (int)eval_band.size();
-        if (eval_band.size() > (size_t)INT_MAX - n_pt)
-            return fail(VAG_ERR_INVALID, "the (model, band) evaluations must fit in a 32-bit int");
-    }
-    const size_t n_eval = eval_band.size();
+    for (size_t i = 0; ext && i < n_pt; ++i) pt_av.push_back(A_V[L.gather[i]]);
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
     if (n_models == 0) return VAG_OK;
@@ -2339,8 +2461,8 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
         if (int rc = upload_request(ctx, t, n_points_total, nu, n_points_total)) return rc;
     // one upload: the lists, the point pass's tables and data; then room for the records and results on the device
     Pack pk;
-    const size_t o_gather = pk.put(gather), o_pt_of = pk.put(pt_of), o_e0 = pk.put(e0), o_sets = pk.put(pt_sets),
-                 o_set_of = pk.put(pt_set_of), o_off = pk.put(pt_off), o_lnF = pk.put(lnF_obs, n_pt ? n_points_total : 0),
+    const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0), o_sets = pk.put(L.pt_sets),
+                 o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off), o_lnF = pk.put(lnF_obs, n_pt ? n_points_total : 0),
                  o_sig = pk.put(sigma_ln, n_pt ? n_points_total : 0), o_w = pk.put(w, n_pt ? n_points_total : 0),
                  o_ext = pk.put(ext_k, ext && n_pt ? n_points_total : 0), o_av = pk.put(pt_av);
     const size_t up = pk.h.size();
@@ -2354,41 +2476,19 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
     vag_params* d_rec = at<vag_params>(base, o_rec);
     k_gather_params<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(static_cast<vag_params*>(ctx->io_params.p),
                                                                            at<int>(base, o_gather), n_pt + n_eval, d_rec);
-    int launches = 1;
-    if (n_pt) {
-        const SetsDev sd{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)};
-        Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points_total, n_points_total};
-        rq.sets = &sd;
-        rq.h_off = pt_off.data();
-        rq.n_sets = (int)pt_sets.size();
-        rq.max_set = max_set;
-        rq.d_lnF = at<double>(base, o_lnF);
-        rq.d_sig = at<double>(base, o_sig);
-        rq.d_w = at<double>(base, o_w);
-        if (ext) {
-            rq.d_ext = at<double>(base, o_ext);
-            rq.d_av = at<double>(base, o_av);
-        }
-        CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (size_t)pt_off[n_pt]));
-        if (int rc = run_flux(ctx, d_rec, n_pt, caps, rq, static_cast<double*>(ctx->io_out.p), at<int32_t>(base, o_st_pts),
-                              at<double>(base, o_chi2_pts), s))
-            return rc;
-        launches += ctx->launches;
-    }
-    BandPass bp{};
-    if (n_eval) {
-        if (int rc = band_pass(ctx, d_rec + n_pt, n_eval, caps, eval_band.data(), bands, n_bands_total, grids, true,
-                               at<int32_t>(base, o_st_eval), bp, s))
-            return rc;
-        launches += ctx->launches;
-    }
+    const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
+                      SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
+                      at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
+    const Chi2Points pts{static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), at<double>(base, o_lnF),
+                         at<double>(base, o_sig), at<double>(base, o_w), ext ? at<double>(base, o_ext) : nullptr,
+                         ext ? at<double>(base, o_av) : nullptr, n_points_total};
     double* d_chi2 = at<double>(base, o_chi2);
     int32_t* d_status = at<int32_t>(base, o_status);
-    k_chi2_bands<<<(unsigned)((n_models * 32 + 127) / 128), 128, 0, s>>>(
-        bp.red, bp.red_off, bp.sd, bp.lnF, bp.sig, bp.w, at<int>(base, o_st_eval), at<int>(base, o_e0), at<int>(base, o_pt_of),
-        at<double>(base, o_chi2_pts), at<int>(base, o_st_pts), n_models, d_chi2, d_status);
-    ctx->launches = launches + 1;
-    CK(cudaGetLastError());
+    int launches = 0;
+    if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands_total, grids, false, n_models, d_chi2, d_status, s,
+                              &launches))
+        return rc;
+    ctx->launches = 1 + launches;  // k_gather_params
     CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -2521,6 +2621,99 @@ int vag_chi2_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, 
                            cudaMemcpyDeviceToDevice, s));
     k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, d_chi2, nullptr, 0);
     ctx->launches += 2;  // k_plan, k_reject
+    CK(cudaGetLastError());
+    return VAG_OK;
+}
+
+// k_plan without stand-ins, and ok[] with the capacities on the host: ok[] and the two capacities sit back to back in
+// plan_buf, so one D2H into the pinned h_plan (grown on demand) and one synchronisation of s bring back both
+static int plan_ok(vag_context* ctx, const vag_params* d_params, size_t n, const int32_t** d_ok, const int32_t** h_ok,
+                   Caps* caps, cudaStream_t s) {
+    const size_t ok_bytes = carve_sz<int32_t>(n), bytes = ok_bytes + sizeof(int) * 2;
+    CK(ctx->plan_buf.ensure(bytes));
+    if (bytes > ctx->h_plan_cap) {
+        if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
+        ctx->h_plan = nullptr;
+        ctx->h_plan_cap = 0;
+        const size_t want = bytes + bytes / 4;
+        CK(cudaMallocHost(&ctx->h_plan, want));
+        ctx->h_plan_cap = want;
+    }
+    int32_t* ok = static_cast<int32_t*>(ctx->plan_buf.p);
+    int* d_caps = at<int>(ctx->plan_buf.p, ok_bytes);
+    CK(cudaMemsetAsync(d_caps, 0, sizeof(int) * 2, s));
+    k_plan<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_params, n, stand_in_params(), nullptr, ok, d_caps);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(ctx->h_plan, ok, bytes, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    const int* hc = at<int>(ctx->h_plan, ok_bytes);
+    *caps = Caps{std::max(64, hc[0]), std::max(8, hc[1])};
+    *d_ok = ok;
+    *h_ok = reinterpret_cast<const int32_t*>(ctx->h_plan);
+    return VAG_OK;
+}
+
+// vag_chi2_multi_bands on device buffers, planned on the device: k_plan, then the lists of the accepted models alone
+// (multi_lists with ok[]), the gather of their records and A_V (k_gather_params_av), the passes of the host call with
+// the band data gathered on the device (k_gather_bands), and k_reject for the rejected models
+int vag_chi2_multi_bands_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const int32_t* dataset_of,
+                             const vag_multi_set* sets, size_t n_sets, const double* d_t, const double* d_nu,
+                             const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k,
+                             size_t n_points_total, const double* d_A_V, const vag_band_obs* bands, size_t n_bands_total,
+                             double* d_chi2, int32_t* d_status, void* stream) {
+    if (!ctx || (n_models && !d_chi2)) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (n_models && !d_params) return fail(VAG_ERR_INVALID, "params is NULL");
+    if (n_points_total && (!d_t || !d_nu || !d_lnF_obs || !d_sigma_ln || !d_w))
+        return fail(VAG_ERR_INVALID, "point data arrays must not be NULL when n_points_total > 0");
+    if (n_bands_total && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
+    const bool ext = d_ext_k != nullptr;
+    if (ext != (d_A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (ext && n_points_total == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points_total > 0)");
+    if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, d_t, d_nu, n_points_total, n_bands_total, true))
+        return rc;
+    std::vector<BandGrid> grids;
+    if (int rc = check_bands(bands, n_bands_total, true, grids, true)) return rc;
+    if (int rc = check_multi_count(n_models, dataset_of, sets)) return rc;
+    if (n_models == 0) return VAG_OK;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    const int32_t *d_ok = nullptr, *h_ok = nullptr;
+    Caps caps;
+    if (int rc = plan_ok(ctx, d_params, n_models, &d_ok, &h_ok, &caps, s)) return rc;
+    MultiLists L;
+    multi_lists(n_models, dataset_of, sets, n_sets, h_ok, L);
+    const size_t n_pt = L.n_pt, n_eval = L.n_eval;
+    int launches = 1;  // k_plan
+    if (n_pt + n_eval) {
+        // one upload: the lists and the point pass's tables; then room for the records, A_V and the results
+        Pack pk;
+        const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0),
+                     o_sets = pk.put(L.pt_sets), o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off);
+        const size_t up = pk.h.size();
+        const size_t n_av = ext ? n_pt : 0;
+        const size_t o_rec = up, o_av = o_rec + carve_sz<vag_params>(n_pt + n_eval), o_chi2_pts = o_av + carve_sz<double>(n_av),
+                     o_st_pts = o_chi2_pts + carve_sz<double>(n_pt), o_st_eval = o_st_pts + carve_sz<int>(n_pt),
+                     o_status = o_st_eval + carve_sz<int>(n_eval), end = o_status + (d_status ? 0 : carve_sz<int>(n_models));
+        CK(ctx->io_sets.ensure(end));
+        void* base = ctx->io_sets.p;
+        CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
+        vag_params* d_rec = at<vag_params>(base, o_rec);
+        k_gather_params_av<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(
+            d_params, at<int>(base, o_gather), n_pt + n_eval, d_rec, d_A_V, n_av, at<double>(base, o_av));
+        const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
+                          SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
+                          at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
+        const Chi2Points pts{d_t, d_nu, d_lnF_obs, d_sigma_ln, d_w, d_ext_k, ext ? at<double>(base, o_av) : nullptr,
+                             n_points_total};
+        int passes = 0;
+        if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands_total, grids, true, n_models, d_chi2,
+                                  d_status ? d_status : at<int32_t>(base, o_status), s, &passes))
+            return rc;
+        launches += 1 + passes;  // k_gather_params_av
+    }
+    // k_chi2_bands gave the rejected models (no point term, no band) chi2 = 0 and status 0; k_reject overwrites them
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, d_chi2, nullptr, 0);
+    ctx->launches = launches + 1;
     CK(cudaGetLastError());
     return VAG_OK;
 }

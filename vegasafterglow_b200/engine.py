@@ -362,6 +362,33 @@ class Engine:
                                           C.cast(arr, C.c_void_p) if len(bands) else None, len(bands), d_chi2,
                                           d_status or None, stream or None))
 
+    def chi2_multi_bands_dev(self, d_params, n_models, dataset_of, sets, points, bands, d_chi2, d_status=0, extinction=None,
+                             stream=0):
+        """``vag_chi2_multi_bands_dev``: ``chi2_multi_bands`` on device pointers, each record checked on the device
+        (rejected ones: chi2 = +inf, ``abi.ST_INVALID``; they are left out of the batch).  ``dataset_of`` (int32 per
+        model) and ``sets`` -- ``(offset, n, band0, n_bands)`` tuples or an ``abi.MultiSet`` array -- are host arrays;
+        ``points`` = (d_t, d_nu, d_lnF, d_sig, d_w, n_points_total) of the concatenated points, or None; ``bands``: the
+        concatenated band dicts of all sets, as ``chi2_dev``'s (device pointers t, lnF_obs, sigma_ln, w and their length
+        ``n``); ``extinction`` = (d_ext_k, d_A_V).  Returns with the work enqueued on ``stream``."""
+        pts, n_pt = ([None] * 5, 0) if points is None else (list(points[:5]), int(points[5]))
+        ext, av = (None, None) if extinction is None else extinction
+        if isinstance(sets, C.Array) and sets._type_ is abi.MultiSet:
+            arr_sets, n_sets = sets, len(sets)
+        else:
+            sets = list(sets)
+            arr_sets, n_sets = (abi.MultiSet * max(len(sets), 1))(), len(sets)
+            for d, s in enumerate(sets):
+                arr_sets[d] = abi.MultiSet(*(int(v) for v in s))
+        ds = self._dataset_of(dataset_of, int(n_models))
+        arr = (abi.BandObs * max(len(bands), 1))()
+        for i, b in enumerate(bands):
+            arr[i] = abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], int(b["n"]), float(b["nu_min"]),
+                                 float(b["nu_max"]), int(b["num_nu"]))
+        _lib.check(self._lib.vag_chi2_multi_bands_dev(self._h, d_params, int(n_models), ds.ctypes.data,
+                                                      C.cast(arr_sets, C.c_void_p) if n_sets else None, n_sets, *pts, ext,
+                                                      n_pt, av, C.cast(arr, C.c_void_p) if len(bands) else None, len(bands),
+                                                      d_chi2, d_status or None, stream or None))
+
     def synchronize(self):
         _lib.check(self._lib.vag_synchronize(self._h))
 

@@ -387,3 +387,145 @@ class BandLikelihoodStack(LikelihoodStack):
         flat = (self.engine.chi2_multi_bands(P, self.datasets, self.bands, ds, extinction=extinction) if P.size
                 else np.zeros(0))
         return self._split(flat, ok)
+
+
+class DeviceLikelihoodStack(LikelihoodStack):
+    """K ``DeviceLikelihood`` fits evaluated together with ONE ``Engine.chi2_multi_bands_dev`` call: the stack of
+    ``BandLikelihoodStack`` with the data, the walkers and the result in HBM, and -- with ``distributed=True`` -- spread
+    over the GPUs of a box.  Fits may have points, bands or both, with or without a fitted ``A_V``; ``__call__``, ``chi2``,
+    the bounds, the per-fit prior and ``log_likelihood_fn`` and the -inf rules are ``LikelihoodStack``'s.
+
+    The members' device point arrays are concatenated once, in fit order (ext_k = 0 for a fit with points and no ``A_V``,
+    and lnF_obs + 0 * 0 is lnF_obs exactly), their band arrays stay where they are, and the records' template of every fit
+    is a row of one [K, sizeof(vag_params) / 8] float64 table on the device.  Per call the host exponentiates the columns
+    (``DeviceLikelihood.columns``) and packs every in-bounds walker into one [n, max_ndim + 1] float64 matrix -- the last
+    column is ``A_V``, 0 where a fit has none -- uploaded with the walkers' fits in one copy.  The records are assembled on
+    the device by a few launches whatever K: the template rows gathered by fit, then one scatter through a per-fit slot
+    table whose padding points at a scratch column.  The call validates the records on the device (rejected: chi2 = +inf).
+
+    ``distributed=True``: every rank gets the same samples, splits all fits' in-bounds walkers with
+    ``parallel.balanced_assignment`` of ``parallel.cost_proxy`` (each fit over its own points' and bands' time window),
+    evaluates its share with one call and takes part in one ``parallel.gather_indexed_tensor``, even with an empty share.
+    The members must share one engine and one device and be built with ``distributed=False``: the stack's flag decides."""
+
+    def __init__(self, likelihoods: Sequence["DeviceLikelihood"], distributed: bool = False):
+        import torch
+
+        self.likelihoods = list(likelihoods)
+        if not self.likelihoods:
+            raise ValueError("DeviceLikelihoodStack needs at least one likelihood")
+        first = self.likelihoods[0]
+        for k, lk in enumerate(self.likelihoods):
+            if not isinstance(lk, DeviceLikelihood):
+                raise ValueError(f"likelihood {k}: DeviceLikelihoodStack stacks DeviceLikelihood fits only")
+            if lk.engine is not first.engine or lk.device != first.device:
+                raise ValueError(f"likelihood {k}: every fit of the stack must use the first fit's engine and device")
+            if lk.distributed:
+                raise ValueError(f"likelihood {k}: built with distributed=True; the stack's own flag decides")
+        self.engine, self.device, self.distributed = first.engine, first.device, distributed
+        lks = self.likelihoods
+        self.fits_av = [lk._av is not None for lk in lks]
+        with_pts = [lk for lk in lks if lk._pts is not None]
+        self.n_points = sum(lk.t.size for lk in with_pts)
+        self._pts = tuple(torch.cat([lk._pts[i] for lk in with_pts]) for i in range(5)) if with_pts else None
+        self._ext = None
+        if any(self.fits_av):
+            self._ext = torch.cat([lk._ext if fit else torch.zeros(lk.t.size, dtype=torch.float64, device=self.device)
+                                   for lk, fit in zip(lks, self.fits_av) if lk._pts is not None])
+        self._bands = [dict(b, n=b["t"].numel(), **{k: b[k].data_ptr() for k in ("t", "lnF_obs", "sigma_ln", "w")})
+                       for lk in lks for b in lk._bands]
+        self.sets = (abi.MultiSet * len(lks))()
+        off = b0 = 0
+        for k, lk in enumerate(lks):
+            self.sets[k] = abi.MultiSet(off, lk.t.size, b0, len(lk._bands))
+            off, b0 = off + lk.t.size, b0 + len(lk._bands)
+        # each fit's time window (points and bands), for the cost proxy of the distributed split
+        self._window = []
+        for lk in lks:
+            tt = np.concatenate([lk.t] + [b["t"] for b in lk.bands])
+            self._window.append((float(np.min(tt)), float(np.max(tt))))
+        # records: template table [K, W], per-fit slot table [K, max_ndim + 1] into a row of W + 1 (W: the scratch column)
+        self._width = abi.PARAMS_DTYPE.itemsize // 8
+        self._ncol = max(len(lk.names) for lk in lks) + 1
+        self._templates = torch.as_tensor(np.stack([lk.template.view(np.float64) for lk in lks]), device=self.device)
+        slots = np.full((len(lks), self._ncol), self._width, dtype=np.int64)
+        for k, lk in enumerate(lks):
+            for i, name in enumerate(lk.names):
+                if name != "A_V":
+                    slots[k, i] = _field_offset(_FIELDS[name]) // 8
+        self._slots = torch.as_tensor(slots, device=self.device)
+
+    def records(self, X, fit_of):
+        """uint8[n * sizeof(vag_params)] on the device from the packed columns ``X`` ([n, max_ndim + 1] float64) and the
+        fit of every walker (int64 [n]): each fit's template with its model columns at their fields' offsets."""
+        import torch
+
+        n = X.shape[0]
+        rec = torch.empty((n, self._width + 1), dtype=torch.float64, device=self.device)
+        rec[:, :self._width] = self._templates[fit_of]
+        rec.scatter_(1, self._slots[fit_of], X)
+        return rec[:, :self._width].contiguous().view(torch.uint8).view(-1)
+
+    def _pack(self, samples):
+        """(the packed columns and the walkers' fits in one float64 host buffer, their number, the fits as int32)"""
+        n_k = [s.shape[0] for s in samples]
+        n = sum(n_k)
+        buf = np.zeros(n * self._ncol + n)
+        X = buf[:n * self._ncol].reshape(n, self._ncol)
+        fit_of = np.repeat(np.arange(len(n_k), dtype=np.int64), n_k)
+        buf[n * self._ncol:] = fit_of.view(np.float64)
+        lo = 0
+        for k, (lk, s) in enumerate(zip(self.likelihoods, samples)):
+            if s.shape[0]:
+                X[lo:lo + s.shape[0], :len(lk.names)] = lk.columns(s)  # an A_V column's slot is the scratch column
+                if self.fits_av[k]:
+                    X[lo:lo + s.shape[0], -1] = lk._column(s, lk._av)
+            lo += s.shape[0]
+        return buf, n, fit_of.astype(np.int32)
+
+    def _chi2_dev(self, X, fit_of, dataset_of):
+        import torch
+
+        n = X.shape[0]
+        chi2 = torch.empty(n, dtype=torch.float64, device=self.device)
+        if n == 0:
+            return chi2
+        rec = self.records(X, fit_of)
+        points = None if self._pts is None else (*(a.data_ptr() for a in self._pts), self.n_points)
+        av = X[:, -1].contiguous() if self._ext is not None else None
+        extinction = None if av is None else (self._ext.data_ptr(), av.data_ptr())
+        stream = 0
+        if self.device.type == "cuda":  # as DeviceLikelihood._chi2_dev: ordered after the record assembly
+            stream = torch.cuda.current_stream(self.device).cuda_stream or _CUDA_STREAM_LEGACY
+        self.engine.chi2_multi_bands_dev(rec.data_ptr(), n, dataset_of, self.sets, points, self._bands, chi2.data_ptr(),
+                                         extinction=extinction, stream=stream)
+        return chi2
+
+    def chi2(self, samples):
+        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject (checked
+        on the device)."""
+        import torch
+
+        samples = [np.atleast_2d(np.asarray(s, dtype=np.float64)) for s in samples]
+        buf, n, ds = self._pack(samples)
+        up = torch.as_tensor(buf, device=self.device)  # the one H2D copy of the call
+        X, fit_of = up[:n * self._ncol].view(n, self._ncol), up[n * self._ncol:].view(torch.int64)
+        if not self.distributed:
+            flat = self._chi2_dev(X, fit_of, ds).cpu().numpy()
+        else:
+            import torch.distributed as dist
+
+            from . import parallel
+
+            world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
+            cost = np.concatenate([parallel.cost_proxy(lk.to_params(s), *win) if s.shape[0] else np.zeros(0)
+                                   for lk, s, win in zip(self.likelihoods, samples, self._window)])
+            sets = parallel.balanced_assignment(cost, world)
+            mine = sets[rank]
+            idx = torch.as_tensor(mine, dtype=torch.long, device=self.device)
+            flat = parallel.gather_indexed_tensor(self._chi2_dev(X[idx], fit_of[idx], ds[mine]), sets, n).cpu().numpy()
+        out, lo = [], 0
+        for s in samples:
+            out.append(flat[lo:lo + s.shape[0]])
+            lo += s.shape[0]
+        return out
