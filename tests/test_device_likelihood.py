@@ -370,6 +370,48 @@ def test_chi2_dev_equals_chi2_ext(engine, terms, series_mode):
 
 
 @pytest.mark.gpu
+def test_chi2_dev_arguments_are_checked_before_any_work(engine):
+    import torch
+
+    P = configs.random_draw(4, seed=1)
+    t = np.array([1e3, 1e4, 1e5])
+    keep = [_dev(a) for a in (t, np.full(t.size, 1e9), np.zeros(t.size), np.ones(t.size), np.ones(t.size), np.zeros(t.size),
+                              np.zeros(P.size))]
+    d_t, d_nu, d_lnF, d_sig, d_w, d_ext, d_av = (a.data_ptr() for a in keep)
+    rec = _records(P)
+    xb = dict(t=d_t, lnF_obs=d_lnF, sigma_ln=d_sig, w=d_w, n=t.size, nu_min=7.25e16, nu_max=2.4e18, num_nu=5)
+
+    def call(n_points=t.size, ext=None, A_V=None, **band):
+        b = dict(xb, **band)
+        arr = (abi.BandObs * 1)(abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], b["n"], b["nu_min"], b["nu_max"],
+                                            b["num_nu"]))
+        chi2 = torch.full((P.size,), 7.0, dtype=torch.float64, device="cuda:0")
+        st = torch.full((P.size,), 99, dtype=torch.int32, device="cuda:0")
+        rc = engine._lib.vag_chi2_dev(engine._h, rec.data_ptr(), P.size, d_t, d_nu, d_lnF, d_sig, d_w, ext, n_points, A_V,
+                                      C.cast(arr, C.c_void_p), 1, chi2.data_ptr(), st.data_ptr(), None)
+        engine.synchronize()
+        return rc, bool((chi2.cpu().numpy() == 7.0).all() and (st.cpu().numpy() == 99).all())
+
+    assert call() == (abi.VAG_OK, False)
+    # word in the message -> arguments
+    cases = {
+        "band 0: empty (n = 0)": dict(n=0),
+        "band 0: data arrays must not be NULL": dict(sigma_ln=None),
+        "band 0: time array must not be NULL": dict(t=None),
+        "band 0: nu_max": dict(nu_max=1e16),
+        "band 0: num_nu": dict(num_nu=1),
+        "both": dict(ext=d_ext),
+        "extinction needs point data": dict(n_points=0, ext=d_ext, A_V=d_av),
+    }
+    for word, kw in cases.items():
+        rc, untouched = call(**kw)
+        assert rc == abi.VAG_ERR_INVALID, word
+        assert untouched, word
+        msg = engine._lib.vag_last_error().decode()
+        assert word in msg, (word, msg)
+
+
+@pytest.mark.gpu
 def test_chi2_dev_across_the_pass_boundary(engine):
     n = 32768 + 64
     P = configs.random_draw(n, seed=21)

@@ -133,6 +133,51 @@ def test_extinction_arguments_are_validated(engine):
 
 
 @pytest.mark.gpu
+def test_chi2_ext_arguments_are_checked_before_any_work(engine):
+    import ctypes as C
+
+    P = np.ascontiguousarray(configs.random_draw(3, seed=1), dtype=abi.PARAMS_DTYPE)
+    pts, ext = _points()
+    pts = [np.ascontiguousarray(a, dtype=np.float64) for a in pts]
+    A_V = np.ones(P.size)
+    bad_ext = ext.copy()
+    bad_ext[7] = np.inf
+    bt, bl, bs, bw = np.array([1e3, 1e4]), np.zeros(2), np.ones(2), np.ones(2)
+    xb = dict(t=bt.ctypes.data, lnF_obs=bl.ctypes.data, sigma_ln=bs.ctypes.data, w=bw.ctypes.data, n=bt.size,
+              nu_min=7.25e16, nu_max=2.4e18, num_nu=5)
+
+    def call(n_points=pts[0].size, ext=None, A_V=None, **band):
+        b = dict(xb, **band)
+        arr = (abi.BandObs * 1)(abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], b["n"], b["nu_min"], b["nu_max"],
+                                            b["num_nu"]))
+        chi2 = np.full(P.size, 7.0)
+        st = np.full(P.size, 99, dtype=np.int32)
+        rc = engine._lib.vag_chi2_ext(engine._h, P.ctypes.data, P.size, *[a.ctypes.data for a in pts],
+                                      None if ext is None else ext.ctypes.data, n_points,
+                                      None if A_V is None else A_V.ctypes.data, C.cast(arr, C.c_void_p), 1, chi2.ctypes.data,
+                                      st.ctypes.data)
+        return rc, bool((chi2 == 7.0).all() and (st == 99).all())
+
+    assert call(ext=ext, A_V=A_V) == (abi.VAG_OK, False)
+    # word in the message -> arguments
+    cases = {
+        "band 0: empty (n = 0)": dict(n=0),
+        "band 0: data arrays must not be NULL": dict(lnF_obs=None),
+        "band 0: nu_max": dict(nu_max=1e16),
+        "band 0: num_nu": dict(num_nu=1),
+        "both": dict(ext=ext),
+        "extinction needs point data": dict(n_points=0, ext=ext, A_V=A_V),
+        "finite": dict(ext=bad_ext, A_V=A_V),
+    }
+    for word, kw in cases.items():
+        rc, untouched = call(**kw)
+        assert rc == abi.VAG_ERR_INVALID, word
+        assert untouched, word
+        msg = engine._lib.vag_last_error().decode()
+        assert word in msg, (word, msg)
+
+
+@pytest.mark.gpu
 def test_extinction_across_the_pass_boundary(engine):
     # 32768 models per pass: the second pass must read A_V from its own offset
     n = 32768 + 64

@@ -765,12 +765,6 @@ __global__ void k_total_sets(double* out, SetsDev sd) {
 // ---- band-integrated data in a ragged batch (vag_flux_band_multi, vag_chi2_multi_bands) ----------------------------
 // An evaluation is one (model, band): a model of the ragged grid request whose set is the band (its times, its nodes).
 
-// dst[i] = src[idx[i]]: the parameter record of every evaluation, gathered from the records of the models
-__global__ void k_gather_params(const vag_params* __restrict__ src, const int* __restrict__ idx, size_t n, vag_params* dst) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = src[idx[i]];
-}
-
 // k_band_reduce per evaluation (CTA / evaluation): its [VAG_NCOMP][n_nu][n] grid block (sd.out_off counts from the first
 // evaluation of the call) -> [VAG_NCOMP][n] at VAG_NCOMP * red_off[e], with the weights of its node slice, summed in
 // k_band_reduce's order
@@ -814,8 +808,9 @@ __global__ void k_chi2_bands(const double* __restrict__ band, const long long* _
     if (lane == 0) status[m] = st;
 }
 
-// ---- the ragged call planned on the device (vag_chi2_multi_bands_dev) --------------------------------------------
-// k_gather_params, and for the first n_av entries (the point pass's models) their A_V as well: av_dst[i] = av_src[idx[i]]
+// ---- the gathers of vag_chi2_multi_bands(_dev) ------------------------------------------------------------------
+// dst[i] = src[idx[i]]: the parameter record of every entry of the lists, gathered from the records of the models, and
+// for the first n_av entries (the point pass's models) their A_V as well: av_dst[i] = av_src[idx[i]]
 __global__ void k_gather_params_av(const vag_params* __restrict__ src, const int* __restrict__ idx, size_t n, vag_params* dst,
                                    const double* __restrict__ av_src, size_t n_av, double* av_dst) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -885,11 +880,10 @@ struct vag_context {
     int device = 0;
     cudaStream_t stream = nullptr;
     DevBuf model_buf, row_buf, cell_buf, obs_buf, ic_buf, lut_buf, sp_buf, geom_buf, split_buf, work_buf;
-    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_obs, io_sets, io_bands;  // staging of the host-buffer entry points
-    DevBuf plan_buf;                // device planning: the records that run, ok[], capacities
+    DevBuf io_params, io_status, io_t, io_nu, io_w, io_out, io_sets, io_bands;  // staging of the host-buffer entry points
+    DevBuf plan_buf;                // device planning: ok[], the capacities, the records that run
     int* h_totals = nullptr;        // pinned
-    int* h_caps = nullptr;          // pinned: capacities planned on the device
-    char* h_plan = nullptr;         // pinned, grown on demand: ok[] and the capacities of vag_chi2_multi_bands_dev's plan
+    char* h_plan = nullptr;         // pinned, grown on demand: the capacities planned on the device, with ok[] ahead of them
     size_t h_plan_cap = 0;
     long long* h_cells = nullptr;   // pinned
     int* h_bands = nullptr;         // pinned [2]: distinct frequencies of the series request in flight (ragged: see k_series_bands_sets)
@@ -1453,7 +1447,6 @@ int vag_create(int device, vag_context** out) {
     CK(cudaMallocHost(&c->h_totals, sizeof(int) * TOT_N));
     CK(cudaMallocHost(&c->h_cells, sizeof(long long)));
     CK(cudaMallocHost(&c->h_bands, 2 * sizeof(int)));
-    CK(cudaMallocHost(&c->h_caps, sizeof(int) * 2));
     for (auto& ev : c->ev) CK(cudaEventCreate(&ev));
     {
         std::vector<double> lut(SPL_DOUBLES);
@@ -1502,7 +1495,6 @@ void vag_destroy(vag_context* c) {
     if (c->h_totals) cudaFreeHost(c->h_totals);
     if (c->h_cells) cudaFreeHost(c->h_cells);
     if (c->h_bands) cudaFreeHost(c->h_bands);
-    if (c->h_caps) cudaFreeHost(c->h_caps);
     if (c->h_plan) cudaFreeHost(c->h_plan);
     for (auto& ev : c->ev)
         if (ev) cudaEventDestroy(ev);
@@ -1651,14 +1643,21 @@ static int prepare_request(vag_context* ctx, const double* t, size_t n_t, const 
 }
 
 // ---- device-buffer entry points ----------------------------------------------------------------
+// makes the context's device current and picks the stream of a _dev call: the caller's, or the context's when NULL
+static int dev_stream(vag_context* ctx, void* stream, cudaStream_t* s) {
+    CK(cudaSetDevice(ctx->device));
+    *s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    return VAG_OK;
+}
+
 // the caller's buffers and stream, the capacities of vag_set_capacity; with d_chi2 the series flux is scratch
 static int flux_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const Request& rq, double* d_out,
                     int32_t* d_status, double* d_chi2, void* stream) {
     if (!ctx) return fail(VAG_ERR_INVALID, "ctx is NULL");
     if (rq.n_t == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
     if (rq.n_nu == 0) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t s;
+    if (int rc = dev_stream(ctx, stream, &s)) return rc;
     if (d_chi2) {
         CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * rq.n_t));
         d_out = static_cast<double*>(ctx->io_out.p);
@@ -1867,6 +1866,23 @@ struct BandTerm {
     const BandGrid* g;
 };
 
+// The series request of pts (lnF ... av NULL: the flux alone); with sd a ragged one on the n_sets data sets of sd, the
+// largest of max_set points, whose models' output points have the host prefix sums h_off
+static Request points_request(const Chi2Points& pts, const SetsDev* sd = nullptr, const long long* h_off = nullptr,
+                              size_t n_sets = 0, size_t max_set = 0) {
+    Request rq{true, pts.t, pts.nu, pts.n, pts.n};
+    rq.d_lnF = pts.lnF;
+    rq.d_sig = pts.sig;
+    rq.d_w = pts.w;
+    rq.d_ext = pts.ext;
+    rq.d_av = pts.av;
+    rq.sets = sd;
+    rq.h_off = h_off;
+    rq.n_sets = (int)n_sets;
+    rq.max_set = max_set;
+    return rq;
+}
+
 // chi2[n] of a batch whose parameters and data are on the device: the point term (k_chi2 inside run_flux writes chi2),
 // then per band Model.flux and an accumulating k_chi2.  The status of every run goes to io_status; with band terms it is
 // ORed into d_stat_or, which is then the call's status.  ctx->launches counts every launch of the call.
@@ -1879,13 +1895,8 @@ static int chi2_run(vag_context* ctx, const vag_params* d_params, size_t n_model
     int launches = 0;
     if (pts.n) {  // the first term: run_flux writes chi2
         CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * pts.n));
-        Request rq{true, pts.t, pts.nu, pts.n, pts.n};
-        rq.d_lnF = pts.lnF;
-        rq.d_sig = pts.sig;
-        rq.d_w = pts.w;
-        rq.d_ext = pts.ext;
-        rq.d_av = pts.av;
-        if (int rc = run_flux(ctx, d_params, n_models, caps, rq, static_cast<double*>(ctx->io_out.p), d_status, d_chi2, s))
+        if (int rc = run_flux(ctx, d_params, n_models, caps, points_request(pts), static_cast<double*>(ctx->io_out.p), d_status,
+                              d_chi2, s))
             return rc;
         launches += ctx->launches;
         if (or_status) {
@@ -1909,28 +1920,45 @@ static int chi2_run(vag_context* ctx, const vag_params* d_params, size_t n_model
     return VAG_OK;
 }
 
-// The checks of vag_chi2_ext and vag_chi2_dev, all before any work is enqueued: arguments, every band's grid and -- for
-// data in host memory (host_data) -- the values of ext_k and of the band times
+// The rules of every chi-squared entry point for point data and fitted extinction (before any work is enqueued): with
+// points all their arrays are set (`arrays`), ext_k and A_V are both set or both NULL, extinction needs points, and ext_k
+// in host memory (!device) is finite
+static int check_points(size_t n_points, bool arrays, const double* ext_k, const double* A_V, bool device) {
+    if (n_points && !arrays) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL when there are points");
+    if ((ext_k != nullptr) != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
+    if (ext_k && n_points == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (no points)");
+    for (size_t i = 0; ext_k && !device && i < n_points; ++i)
+        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
+    return VAG_OK;
+}
+
+// The checks of one band (data: lnF_obs / sigma_ln / w too) and its frequency grid; with `device` its arrays are device
+// memory, whose values are not read (only t != NULL is checked)
+static int check_band(const vag_band_obs& B, size_t b, bool data, BandGrid& g, bool device) {
+    const std::string name = "band " + std::to_string(b) + ": ";
+    if (B.n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
+    if (data && (!B.lnF_obs || !B.sigma_ln || !B.w)) return fail(VAG_ERR_INVALID, name + "data arrays must not be NULL");
+    if (device) {
+        if (!B.t) return fail(VAG_ERR_INVALID, name + "time array must not be NULL");
+    } else if (check_times(B.t, B.n)) {
+        return fail(VAG_ERR_INVALID, name + g_err);
+    }
+    if (band_grid(B.nu_min, B.nu_max, B.num_nu, g)) return fail(VAG_ERR_INVALID, name + g_err);
+    return VAG_OK;
+}
+
+// The checks of vag_chi2_ext and vag_chi2_dev, all before any work is enqueued: the arguments, the point data and
+// extinction, and every band with its grid; with `device` the data are device memory, whose values are not read
 static int check_chi2_args(vag_context* ctx, const double* chi2, size_t n_points, bool point_ptrs, const double* ext_k,
-                           const double* A_V, const vag_band_obs* bands, size_t n_bands, bool host_data,
+                           const double* A_V, const vag_band_obs* bands, size_t n_bands, bool device,
                            std::vector<BandGrid>& grids) {
     if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (n_points && !point_ptrs) return fail(VAG_ERR_INVALID, "point data arrays must not be NULL");
     if (n_bands && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
     if (n_points == 0 && n_bands == 0) return fail(VAG_ERR_INVALID, "no data: n_points and n_bands are both 0");
-    const bool ext = ext_k != nullptr;
-    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
-    if (ext && n_points == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points > 0)");
-    for (size_t i = 0; host_data && ext && i < n_points; ++i)
-        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
+    if (int rc = check_points(n_points, point_ptrs, ext_k, A_V, device)) return rc;
     grids.resize(n_bands);
-    for (size_t b = 0; b < n_bands; ++b) {
-        const vag_band_obs& B = bands[b];
-        if (B.n == 0 || !B.t || !B.lnF_obs || !B.sigma_ln || !B.w) return fail(VAG_ERR_INVALID, "band data arrays must be non-empty");
-        if (int rc = band_grid(B.nu_min, B.nu_max, B.num_nu, grids[b])) return rc;
-        if (host_data)
-            if (int rc = check_times(B.t, B.n)) return rc;
-    }
+    for (size_t b = 0; b < n_bands; ++b)
+        if (int rc = check_band(bands[b], b, true, grids[b], device)) return rc;
     return VAG_OK;
 }
 
@@ -1941,55 +1969,41 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
                  const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k, size_t n_points,
                  const double* A_V, const vag_band_obs* bands, size_t n_bands, double* chi2, int32_t* status) {
     std::vector<BandGrid> grids;
-    if (int rc = check_chi2_args(ctx, chi2, n_points, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, bands, n_bands, true,
+    if (int rc = check_chi2_args(ctx, chi2, n_points, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, bands, n_bands, false,
                                  grids))
         return rc;
-    const bool ext = ext_k != nullptr;
-    size_t n_obs = n_models + 3 * n_points + (ext ? n_points + n_models : 0);
-    for (size_t b = 0; b < n_bands; ++b) n_obs += 4 * bands[b].n;
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
     if (n_points)
         if (int rc = prepare_request(ctx, t, n_points, nu, n_points)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
-    // observation staging: chi2 [n_models]; lnF / sigma_ln / w of the points (with extinction ext_k [n_points] and A_V
-    // [n_models]); t / lnF / sigma_ln / w of every band; status OR [n_models]
-    CK(ctx->io_obs.ensure(sizeof(double) * n_obs + sizeof(int32_t) * n_models));
-    double* cur = static_cast<double*>(ctx->io_obs.p);
-    double* d_chi2 = cur;
-    cur += n_models;
-    cudaError_t ce = cudaSuccess;
-    auto stage = [&](const double* h, size_t n) {
-        double* d = cur;
-        cur += n;
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(d, h, sizeof(double) * n, cudaMemcpyHostToDevice, s);
-        return d;
-    };
+    // one upload: lnF / sigma_ln / w of the points (with extinction ext_k [n_points] and A_V [n_models]) and t / lnF /
+    // sigma_ln / w of every band; then room for chi2 and the status OR [n_models]
+    const size_t n_ext = ext_k ? n_points : 0;
+    Pack pk;
+    const size_t o_lnF = pk.put(lnF_obs, n_points), o_sig = pk.put(sigma_ln, n_points), o_w = pk.put(w, n_points),
+                 o_ext = pk.put(ext_k, n_ext), o_av = pk.put(A_V, n_ext ? n_models : 0);
+    std::vector<size_t> o_band;  // [n_bands][4]
+    for (size_t b = 0; b < n_bands; ++b)
+        for (const double* a : {bands[b].t, bands[b].lnF_obs, bands[b].sigma_ln, bands[b].w}) o_band.push_back(pk.put(a, bands[b].n));
+    const size_t up = pk.h.size(), o_or = up + carve_sz<double>(n_models);
+    CK(ctx->io_sets.ensure(o_or + carve_sz<int32_t>(n_models)));
+    void* base = ctx->io_sets.p;
+    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
     Chi2Points pts{};
-    if (n_points) {
-        pts = Chi2Points{static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), nullptr, nullptr, nullptr,
-                         nullptr, nullptr, n_points};
-        pts.lnF = stage(lnF_obs, n_points);
-        pts.sig = stage(sigma_ln, n_points);
-        pts.w = stage(w, n_points);
-        if (ext) {
-            pts.ext = stage(ext_k, n_points);
-            pts.av = stage(A_V, n_models);
-        }
-    }
+    if (n_points)
+        pts = Chi2Points{static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), at<double>(base, o_lnF),
+                         at<double>(base, o_sig), at<double>(base, o_w), n_ext ? at<double>(base, o_ext) : nullptr,
+                         n_ext ? at<double>(base, o_av) : nullptr, n_points};
     std::vector<BandTerm> terms(n_bands);
     for (size_t b = 0; b < n_bands; ++b) {
-        const vag_band_obs& B = bands[b];
-        terms[b].t = stage(B.t, B.n);
-        terms[b].lnF = stage(B.lnF_obs, B.n);
-        terms[b].sig = stage(B.sigma_ln, B.n);
-        terms[b].w = stage(B.w, B.n);
-        terms[b].n = B.n;
-        terms[b].g = &grids[b];
+        const size_t* o = &o_band[4 * b];
+        terms[b] = BandTerm{at<double>(base, o[0]), at<double>(base, o[1]), at<double>(base, o[2]), at<double>(base, o[3]),
+                            bands[b].n, &grids[b]};
     }
-    if (ce != cudaSuccess) return fail(VAG_ERR_CUDA, std::string("staging the observations: ") + cudaGetErrorString(ce));
-    int32_t* d_stat_or = reinterpret_cast<int32_t*>(cur);
+    double* d_chi2 = at<double>(base, up);
+    int32_t* d_stat_or = at<int32_t>(base, o_or);
     if (int rc = chi2_run(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, pts, terms.data(), n_bands, d_chi2,
                           d_stat_or, s))
         return rc;
@@ -2019,30 +2033,41 @@ int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok) {
 int vag_chi2_series(vag_context* ctx, const vag_params* params, size_t n_models, const double* t, const double* nu,
                     const double* lnF_obs, const double* sigma_ln, const double* w, size_t n, double* chi2,
                     int32_t* status) {
-    if (!lnF_obs || !sigma_ln || !w || !chi2) return fail(VAG_ERR_INVALID, "data arrays must not be NULL");
-    if (n == 0 || !t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
-    if (!nu) return fail(VAG_ERR_INVALID, "frequency array must be non-empty");
     return vag_chi2(ctx, params, n_models, t, nu, lnF_obs, sigma_ln, w, n, nullptr, 0, chi2, status);
 }
 
 // ---- ragged series requests: several data sets in one batch --------------------------------------------------------
-// The checks of vag_flux_density_series_multi and vag_chi2_multi that concern the data sets (before any work is enqueued)
-static int check_sets(size_t n_models, const int32_t* dataset_of, const vag_series_set* sets, size_t n_sets, const double* t,
-                      const double* nu, size_t n_points) {
+extern "C++" {  // a template over the set type
+static size_t band0_of(const vag_series_set&) { return 0; }
+static size_t band0_of(const vag_multi_set& S) { return S.band0; }
+static size_t n_bands_of(const vag_series_set&) { return 0; }
+static size_t n_bands_of(const vag_multi_set& S) { return S.n_bands; }
+
+// The checks of the ragged calls that concern the data sets (before any work is enqueued): a vag_series_set is the
+// vag_multi_set of its points and no band.  With `device` the points are device memory, whose values are not read.  The
+// number of models is not limited here: the calls with bands bound it through check_multi_count.
+template <class Set>
+static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const Set* sets, size_t n_sets, const double* t,
+                            const double* nu, size_t n_points, size_t n_bands, bool device = false) {
     if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no data sets: sets is NULL or n_sets is 0");
-    if (!t || !nu || n_points == 0) return fail(VAG_ERR_INVALID, "time and frequency arrays must be non-empty");
     if (n_points > (size_t)INT_MAX || n_sets > (size_t)INT_MAX)
         return fail(VAG_ERR_INVALID, "n_points_total and n_sets must fit in a 32-bit int");
     if (n_models && !dataset_of) return fail(VAG_ERR_INVALID, "dataset_of is NULL");
     for (size_t d = 0; d < n_sets; ++d) {
         const std::string name = "data set " + std::to_string(d) + ": ";
-        const size_t off = sets[d].offset, n = sets[d].n;
-        if (n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
-        if (off > n_points || n > n_points - off)
-            return fail(VAG_ERR_INVALID, name + "points [" + std::to_string(off) + ", " + std::to_string(off) + " + " +
-                                             std::to_string(n) + ") lie outside the " + std::to_string(n_points) + " points");
-        if (check_times(t + off, n)) return fail(VAG_ERR_INVALID, name + g_err);
-        for (size_t i = off; i < off + n; ++i)
+        const Set& S = sets[d];
+        const size_t band0 = band0_of(S), nb = n_bands_of(S);
+        if (S.n == 0 && nb == 0) return fail(VAG_ERR_INVALID, name + "no data: empty (n = 0 and n_bands = 0)");
+        if (S.offset > n_points || S.n > n_points - S.offset)
+            return fail(VAG_ERR_INVALID, name + "points [" + std::to_string(S.offset) + ", " + std::to_string(S.offset) +
+                                             " + " + std::to_string(S.n) + ") lie outside the " + std::to_string(n_points) +
+                                             " points");
+        if (band0 > n_bands || nb > n_bands - band0)
+            return fail(VAG_ERR_INVALID, name + "bands [" + std::to_string(band0) + ", " + std::to_string(band0) + " + " +
+                                             std::to_string(nb) + ") lie outside the " + std::to_string(n_bands) + " bands");
+        if (S.n == 0 || device) continue;
+        if (check_times(t + S.offset, S.n)) return fail(VAG_ERR_INVALID, name + g_err);
+        for (size_t i = S.offset; i < S.offset + S.n; ++i)
             if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
     }
     for (size_t m = 0; m < n_models; ++m)
@@ -2051,13 +2076,13 @@ static int check_sets(size_t n_models, const int32_t* dataset_of, const vag_seri
                                              " is not a data set index (n_sets = " + std::to_string(n_sets) + ")");
     return VAG_OK;
 }
+}  // extern "C++"
 
-// The series flux (out != NULL) or the chi-squared (chi2 != NULL; data lnF / sig / w [/ ext] over the concatenated points,
-// A_V per model) of a ragged request from host buffers; arguments checked by the caller.  out: model m's
-// [VAG_NCOMP][n of its set] block at m's offset, the prefix sum of the sizes of the data sets of models 0 .. m-1.
+// The series flux (out != NULL) or the chi-squared (chi2 != NULL) of a ragged request from host buffers, arguments checked
+// by the caller: the concatenated points pts (with chi2 their lnF / sig / w [/ ext] and A_V per model in pts.av).  out:
+// model m's [VAG_NCOMP][n of its set] block at m's offset, the prefix sum of the sizes of the data sets of models 0 .. m-1.
 static int sets_host(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
-                     const vag_series_set* sets, size_t n_sets, const double* t, const double* nu, size_t n_points,
-                     const double* const* data, const double* ext_k, const double* A_V, double* out, double* chi2,
+                     const vag_series_set* sets, size_t n_sets, const Chi2Points& pts, double* out, double* chi2,
                      int32_t* status) {
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
@@ -2072,45 +2097,24 @@ static int sets_host(vag_context* ctx, const vag_params* params, size_t n_models
     for (size_t m = 0; m < n_models; ++m) off[m + 1] = off[m] + (long long)sets[dataset_of[m]].n;
     const size_t n_out = (size_t)off[n_models] * VAG_NCOMP;
     cudaStream_t s = ctx->stream;
-    if (int rc = upload_request(ctx, t, n_points, nu, n_points)) return rc;
-    CK(ctx->io_sets.ensure(carve_sz<int>(n_models) + carve_sz<SeriesSet>(n_sets) + carve_sz<long long>(n_models + 1)));
-    char* p = static_cast<char*>(ctx->io_sets.p);
-    int* d_set_of = carve<int>(p, n_models);
-    SeriesSet* d_sets = carve<SeriesSet>(p, n_sets);
-    long long* d_off = carve<long long>(p, n_models + 1);
-    CK(cudaMemcpyAsync(d_set_of, dataset_of, sizeof(int) * n_models, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_sets, hs.data(), sizeof(SeriesSet) * n_sets, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * (n_models + 1), cudaMemcpyHostToDevice, s));
-    const SetsDev sd{d_set_of, d_sets, d_off};
-    Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_points, n_points};
-    rq.sets = &sd;
-    rq.h_off = off.data();
-    rq.n_sets = (int)n_sets;
-    rq.max_set = max_set;
-    double* d_chi2 = nullptr;
-    if (chi2) {
-        // observation staging: chi2 [n_models], lnF / sigma_ln / w [n_points] (with extinction ext_k [n_points], A_V [n_models])
-        CK(ctx->io_obs.ensure(sizeof(double) * (n_models + 3 * n_points + (ext_k ? n_points + n_models : 0))));
-        double* cur = static_cast<double*>(ctx->io_obs.p);
-        d_chi2 = cur;
-        cur += n_models;
-        auto stage = [&](const double* h, size_t n) -> const double* {
-            double* dv = cur;
-            cur += n;
-            return cudaMemcpyAsync(dv, h, sizeof(double) * n, cudaMemcpyHostToDevice, s) == cudaSuccess ? dv : nullptr;
-        };
-        rq.d_lnF = stage(data[0], n_points);
-        rq.d_sig = stage(data[1], n_points);
-        rq.d_w = stage(data[2], n_points);
-        if (ext_k) {
-            rq.d_ext = stage(ext_k, n_points);
-            rq.d_av = stage(A_V, n_models);
-        }
-        if (!rq.d_lnF || !rq.d_sig || !rq.d_w || (ext_k && (!rq.d_ext || !rq.d_av)))
-            return fail(VAG_ERR_CUDA, "staging the observations failed");
-    }
+    // one upload: the points (with chi2 their data), the tables; then room for chi2 [n_models]
+    const size_t n = pts.n, n_data = chi2 ? n : 0, n_ext = chi2 && pts.ext ? n : 0;
+    Pack pk;
+    const size_t o_t = pk.put(pts.t, n), o_nu = pk.put(pts.nu, n), o_lnF = pk.put(pts.lnF, n_data),
+                 o_sig = pk.put(pts.sig, n_data), o_w = pk.put(pts.w, n_data), o_ext = pk.put(pts.ext, n_ext),
+                 o_av = pk.put(pts.av, n_ext ? n_models : 0), o_set_of = pk.put(dataset_of, n_models), o_sets = pk.put(hs),
+                 o_off = pk.put(off), up = pk.h.size();
+    CK(ctx->io_sets.ensure(up + carve_sz<double>(n_models)));
+    void* base = ctx->io_sets.p;
+    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
+    auto dev = [&](size_t o, size_t n_up) -> const double* { return n_up ? at<double>(base, o) : nullptr; };
+    const Chi2Points d{at<double>(base, o_t), at<double>(base, o_nu), dev(o_lnF, n_data), dev(o_sig, n_data),
+                       dev(o_w, n_data), dev(o_ext, n_ext), dev(o_av, n_ext), n};
+    const SetsDev sd{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)};
+    double* d_chi2 = chi2 ? at<double>(base, up) : nullptr;
     CK(ctx->io_out.ensure(sizeof(double) * std::max<size_t>(n_out, 1)));
-    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq, static_cast<double*>(ctx->io_out.p),
+    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps,
+                          points_request(d, &sd, off.data(), n_sets, max_set), static_cast<double*>(ctx->io_out.p),
                           static_cast<int32_t*>(ctx->io_status.p), d_chi2, s))
         return rc;
     if (out) CK(cudaMemcpyAsync(out, ctx->io_out.p, sizeof(double) * n_out, cudaMemcpyDeviceToHost, s));
@@ -2124,9 +2128,10 @@ int vag_flux_density_series_multi(vag_context* ctx, const vag_params* params, si
                                   const vag_series_set* sets, size_t n_sets, const double* t, const double* nu,
                                   size_t n_points_total, double* out, int32_t* status) {
     if (!ctx || !out) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (int rc = check_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total)) return rc;
-    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, n_points_total, nullptr, nullptr, nullptr, out,
-                     nullptr, status);
+    if (int rc = check_points(n_points_total, t && nu, nullptr, nullptr, false)) return rc;
+    if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total, 0)) return rc;
+    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets,
+                     Chi2Points{t, nu, nullptr, nullptr, nullptr, nullptr, nullptr, n_points_total}, out, nullptr, status);
 }
 
 int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
@@ -2134,32 +2139,13 @@ int vag_chi2_multi(vag_context* ctx, const vag_params* params, size_t n_models, 
                    const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total, const double* A_V,
                    double* chi2, int32_t* status) {
     if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (!lnF_obs || !sigma_ln || !w) return fail(VAG_ERR_INVALID, "data arrays must not be NULL");
-    if ((ext_k != nullptr) != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
-    if (int rc = check_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total)) return rc;
-    for (size_t i = 0; ext_k && i < n_points_total; ++i)
-        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
-    const double* data[3] = {lnF_obs, sigma_ln, w};
-    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, n_points_total, data, ext_k, A_V, nullptr, chi2,
-                     status);
+    if (int rc = check_points(n_points_total, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, false)) return rc;
+    if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total, 0)) return rc;
+    return sets_host(ctx, params, n_models, dataset_of, sets, n_sets,
+                     Chi2Points{t, nu, lnF_obs, sigma_ln, w, ext_k, A_V, n_points_total}, nullptr, chi2, status);
 }
 
 // ---- band-integrated data in a ragged batch ----------------------------------------------------------------------
-// The checks of one band (data: lnF_obs / sigma_ln / w too) and its frequency grid; with `device` its arrays are device
-// memory, whose values are not read (only t != NULL is checked)
-static int check_band(const vag_band_obs& B, size_t b, bool data, BandGrid& g, bool device) {
-    const std::string name = "band " + std::to_string(b) + ": ";
-    if (B.n == 0) return fail(VAG_ERR_INVALID, name + "empty (n = 0)");
-    if (data && (!B.lnF_obs || !B.sigma_ln || !B.w)) return fail(VAG_ERR_INVALID, name + "data arrays must not be NULL");
-    if (device) {
-        if (!B.t) return fail(VAG_ERR_INVALID, name + "time array must not be NULL");
-    } else if (check_times(B.t, B.n)) {
-        return fail(VAG_ERR_INVALID, name + g_err);
-    }
-    if (band_grid(B.nu_min, B.nu_max, B.num_nu, g)) return fail(VAG_ERR_INVALID, name + g_err);
-    return VAG_OK;
-}
-
 // Every band checked, its grid built, and the concatenated times and nodes within a 32-bit int
 static int check_bands(const vag_band_obs* bands, size_t n_bands, bool data, std::vector<BandGrid>& grids,
                        bool device = false) {
@@ -2297,38 +2283,6 @@ int vag_flux_band_multi(vag_context* ctx, const vag_params* params, size_t n_mod
     return VAG_OK;
 }
 
-// The checks of vag_chi2_multi_bands that concern the data sets and the points (before any work is enqueued); with
-// `device` the points are device memory, whose values are not read
-static int check_multi_sets(size_t n_models, const int32_t* dataset_of, const vag_multi_set* sets, size_t n_sets,
-                            const double* t, const double* nu, size_t n_points, size_t n_bands, bool device = false) {
-    if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no data sets: sets is NULL or n_sets is 0");
-    if (n_points > (size_t)INT_MAX || n_sets > (size_t)INT_MAX || n_models > (size_t)INT_MAX)
-        return fail(VAG_ERR_INVALID, "n_points_total, n_sets and n_models must fit in a 32-bit int");
-    if (n_models && !dataset_of) return fail(VAG_ERR_INVALID, "dataset_of is NULL");
-    for (size_t d = 0; d < n_sets; ++d) {
-        const std::string name = "data set " + std::to_string(d) + ": ";
-        const vag_multi_set& S = sets[d];
-        if (S.n == 0 && S.n_bands == 0) return fail(VAG_ERR_INVALID, name + "no data (n = 0 and n_bands = 0)");
-        if (S.offset > n_points || S.n > n_points - S.offset)
-            return fail(VAG_ERR_INVALID, name + "points [" + std::to_string(S.offset) + ", " + std::to_string(S.offset) +
-                                             " + " + std::to_string(S.n) + ") lie outside the " + std::to_string(n_points) +
-                                             " points");
-        if (S.band0 > n_bands || S.n_bands > n_bands - S.band0)
-            return fail(VAG_ERR_INVALID, name + "bands [" + std::to_string(S.band0) + ", " + std::to_string(S.band0) + " + " +
-                                             std::to_string(S.n_bands) + ") lie outside the " + std::to_string(n_bands) +
-                                             " bands");
-        if (S.n == 0 || device) continue;
-        if (check_times(t + S.offset, S.n)) return fail(VAG_ERR_INVALID, name + g_err);
-        for (size_t i = S.offset; i < S.offset + S.n; ++i)
-            if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
-    }
-    for (size_t m = 0; m < n_models; ++m)
-        if (dataset_of[m] < 0 || (size_t)dataset_of[m] >= n_sets)
-            return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": dataset_of = " + std::to_string(dataset_of[m]) +
-                                             " is not a data set index (n_sets = " + std::to_string(n_sets) + ")");
-    return VAG_OK;
-}
-
 // The two lists of vag_chi2_multi_bands(_dev), over the models m with ok[m] (every model when ok is NULL): the models whose
 // set has points (pt_of[m] = index in the point pass, or -1) and the (model, band) evaluations, model-major; gather = the
 // model of every entry of both, the point pass first.  The point pass's data sets are all the sets with points, whether a
@@ -2397,18 +2351,10 @@ static int multi_passes(vag_context* ctx, const vag_params* d_rec, const MultiLi
                         bool device, size_t n_models, double* d_chi2, int32_t* d_status, cudaStream_t s, int* launches) {
     *launches = 0;
     if (L.n_pt) {
-        Request rq{true, pts.t, pts.nu, pts.n, pts.n};
-        rq.sets = &tb.pt_sd;
-        rq.h_off = L.pt_off.data();
-        rq.n_sets = (int)L.pt_sets.size();
-        rq.max_set = L.max_set;
-        rq.d_lnF = pts.lnF;
-        rq.d_sig = pts.sig;
-        rq.d_w = pts.w;
-        rq.d_ext = pts.ext;
-        rq.d_av = pts.av;
         CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (size_t)L.pt_off[L.n_pt]));
-        if (int rc = run_flux(ctx, d_rec, L.n_pt, caps, rq, static_cast<double*>(ctx->io_out.p), tb.st_pts, tb.chi2_pts, s))
+        if (int rc = run_flux(ctx, d_rec, L.n_pt, caps, points_request(pts, &tb.pt_sd, L.pt_off.data(), L.pt_sets.size(),
+                                                                       L.max_set),
+                              static_cast<double*>(ctx->io_out.p), tb.st_pts, tb.chi2_pts, s))
             return rc;
         *launches += ctx->launches;
     }
@@ -2427,68 +2373,76 @@ static int multi_passes(vag_context* ctx, const vag_params* d_rec, const MultiLi
     return VAG_OK;
 }
 
+// The body of vag_chi2_multi_bands(_dev) on the lists L of the models that run and their records d_params[n_models] on
+// the device: one upload of the lists and the point pass's tables -- and, from host memory (`host`), of the points pts and
+// A_V[n_models] -- then room for the gathered records, the point models' A_V and the results.  k_gather_params_av gathers
+// the records of both lists and the A_V, and multi_passes runs steps 1 to 4.  chi2 / status [n_models]: device outputs,
+// or NULL to place them in io_sets.  *launches: k_gather_params_av's and multi_passes'.
+static int multi_chi2(vag_context* ctx, const vag_params* d_params, size_t n_models, const MultiLists& L, Caps caps,
+                      Chi2Points pts, const double* A_V, bool host, const vag_band_obs* bands, size_t n_bands,
+                      const std::vector<BandGrid>& grids, double*& chi2, int32_t*& status, cudaStream_t s, int* launches) {
+    const size_t n_pt = L.n_pt, n_eval = L.n_eval, n_up = host && n_pt ? pts.n : 0, n_av = A_V ? n_pt : 0;
+    Pack pk;
+    const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0), o_sets = pk.put(L.pt_sets),
+                 o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off), o_t = pk.put(pts.t, n_up),
+                 o_nu = pk.put(pts.nu, n_up), o_lnF = pk.put(pts.lnF, n_up), o_sig = pk.put(pts.sig, n_up),
+                 o_w = pk.put(pts.w, n_up), o_ext = pk.put(pts.ext, pts.ext ? n_up : 0),
+                 o_A_V = pk.put(A_V, host && A_V ? n_models : 0);
+    const size_t up = pk.h.size(), o_rec = up, o_av = o_rec + carve_sz<vag_params>(n_pt + n_eval),
+                 o_chi2_pts = o_av + carve_sz<double>(n_av), o_st_pts = o_chi2_pts + carve_sz<double>(n_pt),
+                 o_st_eval = o_st_pts + carve_sz<int>(n_pt), o_chi2 = o_st_eval + carve_sz<int>(n_eval),
+                 o_status = o_chi2 + (chi2 ? 0 : carve_sz<double>(n_models)),
+                 end = o_status + (status ? 0 : carve_sz<int>(n_models));
+    CK(ctx->io_sets.ensure(end));
+    void* base = ctx->io_sets.p;
+    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
+    if (host)
+        pts = Chi2Points{at<double>(base, o_t), at<double>(base, o_nu), at<double>(base, o_lnF), at<double>(base, o_sig),
+                         at<double>(base, o_w), pts.ext ? at<double>(base, o_ext) : nullptr, nullptr, pts.n};
+    pts.av = A_V ? at<double>(base, o_av) : nullptr;
+    if (!chi2) chi2 = at<double>(base, o_chi2);
+    if (!status) status = at<int32_t>(base, o_status);
+    vag_params* d_rec = at<vag_params>(base, o_rec);
+    k_gather_params_av<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(
+        d_params, at<int>(base, o_gather), n_pt + n_eval, d_rec, host && A_V ? at<double>(base, o_A_V) : A_V, n_av, at<double>(base, o_av));
+    const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
+                      SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
+                      at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
+    if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands, grids, !host, n_models, chi2, status, s, launches))
+        return rc;
+    *launches += 1;  // k_gather_params_av
+    return VAG_OK;
+}
+
 // 1. the ragged point pass over the models whose set has points (vag_chi2_multi's, on those models and the sets with
-// points), 2. the band pass over every (model, band) evaluation, model-major, 3. its reduction, 4. k_chi2_bands.  The
-// records of both passes are gathered on the device from the models' (k_gather_params, one launch for both lists).
+// points), 2. the band pass over every (model, band) evaluation, model-major, 3. its reduction, 4. k_chi2_bands, through
+// multi_chi2 on the records uploaded by prepare_params
 int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
                          const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
                          const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
                          const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status) {
     if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
-    if (n_points_total && (!t || !nu || !lnF_obs || !sigma_ln || !w))
-        return fail(VAG_ERR_INVALID, "point data arrays must not be NULL when n_points_total > 0");
     if (n_bands_total && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
-    const bool ext = ext_k != nullptr;
-    if (ext != (A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
-    if (ext && n_points_total == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points_total > 0)");
+    if (int rc = check_points(n_points_total, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, false)) return rc;
     if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, t, nu, n_points_total, n_bands_total)) return rc;
-    for (size_t i = 0; ext && i < n_points_total; ++i)
-        if (!std::isfinite(ext_k[i])) return fail(VAG_ERR_INVALID, "extinction coefficients ext_k must be finite");
     std::vector<BandGrid> grids;
     if (int rc = check_bands(bands, n_bands_total, true, grids)) return rc;
     if (int rc = check_models(params, n_models)) return rc;
     if (int rc = check_multi_count(n_models, dataset_of, sets)) return rc;
     MultiLists L;
     multi_lists(n_models, dataset_of, sets, n_sets, nullptr, L);
-    const size_t n_pt = L.n_pt, n_eval = L.n_eval;
-    std::vector<double> pt_av;
-    for (size_t i = 0; ext && i < n_pt; ++i) pt_av.push_back(A_V[L.gather[i]]);
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
     if (n_models == 0) return VAG_OK;
     cudaStream_t s = ctx->stream;
-    if (n_pt)
-        if (int rc = upload_request(ctx, t, n_points_total, nu, n_points_total)) return rc;
-    // one upload: the lists, the point pass's tables and data; then room for the records and results on the device
-    Pack pk;
-    const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0), o_sets = pk.put(L.pt_sets),
-                 o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off), o_lnF = pk.put(lnF_obs, n_pt ? n_points_total : 0),
-                 o_sig = pk.put(sigma_ln, n_pt ? n_points_total : 0), o_w = pk.put(w, n_pt ? n_points_total : 0),
-                 o_ext = pk.put(ext_k, ext && n_pt ? n_points_total : 0), o_av = pk.put(pt_av);
-    const size_t up = pk.h.size();
-    const size_t o_rec = up, o_chi2_pts = o_rec + carve_sz<vag_params>(n_pt + n_eval),
-                 o_st_pts = o_chi2_pts + carve_sz<double>(n_pt), o_st_eval = o_st_pts + carve_sz<int>(n_pt),
-                 o_chi2 = o_st_eval + carve_sz<int>(n_eval), o_status = o_chi2 + carve_sz<double>(n_models),
-                 end = o_status + carve_sz<int>(n_models);
-    CK(ctx->io_sets.ensure(end));
-    void* base = ctx->io_sets.p;
-    CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
-    vag_params* d_rec = at<vag_params>(base, o_rec);
-    k_gather_params<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(static_cast<vag_params*>(ctx->io_params.p),
-                                                                           at<int>(base, o_gather), n_pt + n_eval, d_rec);
-    const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
-                      SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
-                      at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
-    const Chi2Points pts{static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), at<double>(base, o_lnF),
-                         at<double>(base, o_sig), at<double>(base, o_w), ext ? at<double>(base, o_ext) : nullptr,
-                         ext ? at<double>(base, o_av) : nullptr, n_points_total};
-    double* d_chi2 = at<double>(base, o_chi2);
-    int32_t* d_status = at<int32_t>(base, o_status);
+    double* d_chi2 = nullptr;
+    int32_t* d_status = nullptr;
     int launches = 0;
-    if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands_total, grids, false, n_models, d_chi2, d_status, s,
-                              &launches))
+    if (int rc = multi_chi2(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, L, caps,
+                            Chi2Points{t, nu, lnF_obs, sigma_ln, w, ext_k, nullptr, n_points_total}, A_V, true, bands,
+                            n_bands_total, grids, d_chi2, d_status, s, &launches))
         return rc;
-    ctx->launches = 1 + launches;  // k_gather_params
+    ctx->launches = launches;
     CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -2514,34 +2468,48 @@ static vag_params stand_in_params() {
     return p;
 }
 
-// k_plan over n device records (run may be NULL) and the capacities of the accepted ones on the host (caps_for's floor
-// included): one D2H of two ints and one synchronisation of s, because setup_models sizes the workspaces on the host
-static int plan(vag_context* ctx, const vag_params* d_params, size_t n, vag_params* run, int32_t* ok, int* d_caps,
-                Caps* caps, cudaStream_t s) {
+// k_plan over the n device records d_params and the capacities of the accepted ones on the host (caps_for's floor
+// included), because setup_models sizes the workspaces on the host.  In plan_buf ok[] (unless the caller's d_ok takes it)
+// and the two capacities sit back to back, so one D2H into the pinned h_plan (grown on demand) -- of the capacities, or
+// with `host_ok` of ok[] and the capacities -- and one synchronisation of s bring them back.  With `stand_ins` the records
+// that run follow (P.run: a rejected one replaced by stand_in_params()), and the capacities cover the stand-in too.
+struct Plan {
+    const int32_t* ok;       // device ok[]
+    const int32_t* h_ok;     // host_ok: ok[] on the host, until the context's next plan
+    const vag_params* run;   // stand_ins: the records that run
+    Caps caps;
+};
+static int plan(vag_context* ctx, const vag_params* d_params, size_t n, int32_t* d_ok, bool stand_ins, bool host_ok,
+                cudaStream_t s, Plan* P) {
+    const size_t ok_bytes = d_ok ? 0 : carve_sz<int32_t>(n), caps_at = ok_bytes, run_at = caps_at + carve_sz<int>(2);
+    const size_t back = host_ok ? ok_bytes : 0, bytes = back + sizeof(int) * 2;  // h_plan: [ok[]] capacities
+    CK(ctx->plan_buf.ensure(run_at + (stand_ins ? carve_sz<vag_params>(n) : 0)));
+    if (bytes > ctx->h_plan_cap) {
+        if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
+        ctx->h_plan = nullptr;
+        ctx->h_plan_cap = 0;
+        const size_t want = bytes + bytes / 4;
+        CK(cudaMallocHost(&ctx->h_plan, want));
+        ctx->h_plan_cap = want;
+    }
+    void* base = ctx->plan_buf.p;
+    int32_t* ok = d_ok ? d_ok : at<int32_t>(base, 0);
+    int* d_caps = at<int>(base, caps_at);
+    vag_params* run = stand_ins ? at<vag_params>(base, run_at) : nullptr;
     CK(cudaMemsetAsync(d_caps, 0, sizeof(int) * 2, s));
     k_plan<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_params, n, stand_in_params(), run, ok, d_caps);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(ctx->h_caps, d_caps, sizeof(int) * 2, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(ctx->h_plan, at<char>(base, caps_at - back), bytes, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    *caps = Caps{std::max(64, ctx->h_caps[0]), std::max(8, ctx->h_caps[1])};
-    return VAG_OK;
-}
-
-// The records that run (*d_run, rejected ones replaced by the stand-in), ok[] (*d_ok) and the capacities that cover both
-static int plan_run(vag_context* ctx, const vag_params* d_params, size_t n, cudaStream_t s, const vag_params** d_run,
-                    const int32_t** d_ok, Caps* caps) {
-    CK(ctx->plan_buf.ensure(carve_sz<vag_params>(n) + carve_sz<int32_t>(n) + carve_sz<int>(2)));
-    char* p = static_cast<char*>(ctx->plan_buf.p);
-    vag_params* run = carve<vag_params>(p, n);
-    int32_t* ok = carve<int32_t>(p, n);
-    int* d_caps = carve<int>(p, 2);
-    if (int rc = plan(ctx, d_params, n, run, ok, d_caps, caps, s)) return rc;
-    const vag_params sp = stand_in_params();
-    const Caps sc = caps_of(sp);
-    caps->theta = std::max(caps->theta, sc.theta);
-    caps->phi = std::max(caps->phi, sc.phi);
-    *d_run = run;
-    *d_ok = ok;
+    const int* hc = at<int>(ctx->h_plan, back);
+    P->caps = Caps{std::max(64, hc[0]), std::max(8, hc[1])};
+    if (stand_ins) {
+        const Caps sc = caps_of(stand_in_params());
+        P->caps = Caps{std::max(P->caps.theta, sc.theta), std::max(P->caps.phi, sc.phi)};
+    }
+    P->ok = ok;
+    P->h_ok = host_ok ? reinterpret_cast<const int32_t*>(ctx->h_plan) : nullptr;
+    P->run = run;
     return VAG_OK;
 }
 
@@ -2554,14 +2522,13 @@ int vag_params_validate_batch_dev(vag_context* ctx, const vag_params* d_params, 
         caps[1] = 8;
         return VAG_OK;
     }
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    CK(ctx->plan_buf.ensure(carve_sz<int>(2)));
-    Caps c;
-    if (int rc = plan(ctx, d_params, n, nullptr, d_ok, static_cast<int*>(ctx->plan_buf.p), &c, s)) return rc;
+    cudaStream_t s;
+    if (int rc = dev_stream(ctx, stream, &s)) return rc;
+    Plan P;
+    if (int rc = plan(ctx, d_params, n, d_ok, false, false, s, &P)) return rc;
     ctx->launches = 1;
-    caps[0] = c.theta;
-    caps[1] = c.phi;
+    caps[0] = P.caps.theta;
+    caps[1] = P.caps.phi;
     return VAG_OK;
 }
 
@@ -2572,21 +2539,19 @@ int vag_flux_band_dev(vag_context* ctx, const vag_params* d_params, size_t n_mod
     if (int rc = band_grid(nu_min, nu_max, num_nu, g)) return rc;
     if (n_t == 0 || !d_t) return fail(VAG_ERR_INVALID, "time array must be non-empty");
     if (n_models == 0) return VAG_OK;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    const vag_params* d_run = nullptr;
-    const int32_t* d_ok = nullptr;
-    Caps caps;
-    if (int rc = plan_run(ctx, d_params, n_models, s, &d_run, &d_ok, &caps)) return rc;
+    cudaStream_t s;
+    if (int rc = dev_stream(ctx, stream, &s)) return rc;
+    Plan P;
+    if (int rc = plan(ctx, d_params, n_models, nullptr, true, false, s, &P)) return rc;
     CK(ctx->io_status.ensure(sizeof(int32_t) * n_models));
     double* d_band = nullptr;
-    if (int rc = run_band(ctx, d_run, n_models, caps, d_t, n_t, g, static_cast<int32_t*>(ctx->io_status.p), &d_band, s))
+    if (int rc = run_band(ctx, P.run, n_models, P.caps, d_t, n_t, g, static_cast<int32_t*>(ctx->io_status.p), &d_band, s))
         return rc;
     const size_t per_model = VAG_NCOMP * n_t;
     CK(cudaMemcpyAsync(d_out, d_band, sizeof(double) * n_models * per_model, cudaMemcpyDeviceToDevice, s));
     if (d_status)
         CK(cudaMemcpyAsync(d_status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToDevice, s));
-    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, nullptr, d_out, per_model);
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(P.ok, d_status, nullptr, d_out, per_model);
     ctx->launches += 2;  // k_plan, k_reject
     CK(cudaGetLastError());
     return VAG_OK;
@@ -2598,64 +2563,34 @@ int vag_chi2_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, 
                  void* stream) {
     std::vector<BandGrid> grids;
     if (int rc = check_chi2_args(ctx, d_chi2, n_points, d_t && d_nu && d_lnF_obs && d_sigma_ln && d_w, d_ext_k, d_A_V,
-                                 bands, n_bands, false, grids))
+                                 bands, n_bands, true, grids))
         return rc;
     if (n_models && !d_params) return fail(VAG_ERR_INVALID, "params is NULL");
     if (n_models == 0) return VAG_OK;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    const vag_params* d_run = nullptr;
-    const int32_t* d_ok = nullptr;
-    Caps caps;
-    if (int rc = plan_run(ctx, d_params, n_models, s, &d_run, &d_ok, &caps)) return rc;
+    cudaStream_t s;
+    if (int rc = dev_stream(ctx, stream, &s)) return rc;
+    Plan P;
+    if (int rc = plan(ctx, d_params, n_models, nullptr, true, false, s, &P)) return rc;
     CK(ctx->io_status.ensure(sizeof(int32_t) * n_models));
-    CK(ctx->io_obs.ensure(sizeof(int32_t) * n_models));  // status OR of the band terms
-    int32_t* d_stat_or = static_cast<int32_t*>(ctx->io_obs.p);
+    CK(ctx->io_sets.ensure(sizeof(int32_t) * n_models));  // status OR of the band terms
+    int32_t* d_stat_or = static_cast<int32_t*>(ctx->io_sets.p);
     const Chi2Points pts{d_t, d_nu, d_lnF_obs, d_sigma_ln, d_w, d_ext_k, d_A_V, n_points};
     std::vector<BandTerm> terms(n_bands);
     for (size_t b = 0; b < n_bands; ++b)
         terms[b] = BandTerm{bands[b].t, bands[b].lnF_obs, bands[b].sigma_ln, bands[b].w, bands[b].n, &grids[b]};
-    if (int rc = chi2_run(ctx, d_run, n_models, caps, pts, terms.data(), n_bands, d_chi2, d_stat_or, s)) return rc;
+    if (int rc = chi2_run(ctx, P.run, n_models, P.caps, pts, terms.data(), n_bands, d_chi2, d_stat_or, s)) return rc;
     if (d_status)
         CK(cudaMemcpyAsync(d_status, n_bands ? d_stat_or : ctx->io_status.p, sizeof(int32_t) * n_models,
                            cudaMemcpyDeviceToDevice, s));
-    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, d_chi2, nullptr, 0);
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(P.ok, d_status, d_chi2, nullptr, 0);
     ctx->launches += 2;  // k_plan, k_reject
     CK(cudaGetLastError());
     return VAG_OK;
 }
 
-// k_plan without stand-ins, and ok[] with the capacities on the host: ok[] and the two capacities sit back to back in
-// plan_buf, so one D2H into the pinned h_plan (grown on demand) and one synchronisation of s bring back both
-static int plan_ok(vag_context* ctx, const vag_params* d_params, size_t n, const int32_t** d_ok, const int32_t** h_ok,
-                   Caps* caps, cudaStream_t s) {
-    const size_t ok_bytes = carve_sz<int32_t>(n), bytes = ok_bytes + sizeof(int) * 2;
-    CK(ctx->plan_buf.ensure(bytes));
-    if (bytes > ctx->h_plan_cap) {
-        if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
-        ctx->h_plan = nullptr;
-        ctx->h_plan_cap = 0;
-        const size_t want = bytes + bytes / 4;
-        CK(cudaMallocHost(&ctx->h_plan, want));
-        ctx->h_plan_cap = want;
-    }
-    int32_t* ok = static_cast<int32_t*>(ctx->plan_buf.p);
-    int* d_caps = at<int>(ctx->plan_buf.p, ok_bytes);
-    CK(cudaMemsetAsync(d_caps, 0, sizeof(int) * 2, s));
-    k_plan<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_params, n, stand_in_params(), nullptr, ok, d_caps);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(ctx->h_plan, ok, bytes, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    const int* hc = at<int>(ctx->h_plan, ok_bytes);
-    *caps = Caps{std::max(64, hc[0]), std::max(8, hc[1])};
-    *d_ok = ok;
-    *h_ok = reinterpret_cast<const int32_t*>(ctx->h_plan);
-    return VAG_OK;
-}
-
 // vag_chi2_multi_bands on device buffers, planned on the device: k_plan, then the lists of the accepted models alone
-// (multi_lists with ok[]), the gather of their records and A_V (k_gather_params_av), the passes of the host call with
-// the band data gathered on the device (k_gather_bands), and k_reject for the rejected models
+// (multi_lists with ok[]), multi_chi2 on device data (the band data gathered on the device by k_gather_bands), and
+// k_reject for the rejected models
 int vag_chi2_multi_bands_dev(vag_context* ctx, const vag_params* d_params, size_t n_models, const int32_t* dataset_of,
                              const vag_multi_set* sets, size_t n_sets, const double* d_t, const double* d_nu,
                              const double* d_lnF_obs, const double* d_sigma_ln, const double* d_w, const double* d_ext_k,
@@ -2663,57 +2598,31 @@ int vag_chi2_multi_bands_dev(vag_context* ctx, const vag_params* d_params, size_
                              double* d_chi2, int32_t* d_status, void* stream) {
     if (!ctx || (n_models && !d_chi2)) return fail(VAG_ERR_INVALID, "NULL argument");
     if (n_models && !d_params) return fail(VAG_ERR_INVALID, "params is NULL");
-    if (n_points_total && (!d_t || !d_nu || !d_lnF_obs || !d_sigma_ln || !d_w))
-        return fail(VAG_ERR_INVALID, "point data arrays must not be NULL when n_points_total > 0");
     if (n_bands_total && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
-    const bool ext = d_ext_k != nullptr;
-    if (ext != (d_A_V != nullptr)) return fail(VAG_ERR_INVALID, "ext_k and A_V must both be NULL or both be set");
-    if (ext && n_points_total == 0) return fail(VAG_ERR_INVALID, "extinction needs point data (n_points_total > 0)");
+    if (int rc = check_points(n_points_total, d_t && d_nu && d_lnF_obs && d_sigma_ln && d_w, d_ext_k, d_A_V, true)) return rc;
     if (int rc = check_multi_sets(n_models, dataset_of, sets, n_sets, d_t, d_nu, n_points_total, n_bands_total, true))
         return rc;
     std::vector<BandGrid> grids;
     if (int rc = check_bands(bands, n_bands_total, true, grids, true)) return rc;
     if (int rc = check_multi_count(n_models, dataset_of, sets)) return rc;
     if (n_models == 0) return VAG_OK;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    const int32_t *d_ok = nullptr, *h_ok = nullptr;
-    Caps caps;
-    if (int rc = plan_ok(ctx, d_params, n_models, &d_ok, &h_ok, &caps, s)) return rc;
+    cudaStream_t s;
+    if (int rc = dev_stream(ctx, stream, &s)) return rc;
+    Plan P;
+    if (int rc = plan(ctx, d_params, n_models, nullptr, false, true, s, &P)) return rc;
     MultiLists L;
-    multi_lists(n_models, dataset_of, sets, n_sets, h_ok, L);
-    const size_t n_pt = L.n_pt, n_eval = L.n_eval;
-    int launches = 1;  // k_plan
-    if (n_pt + n_eval) {
-        // one upload: the lists and the point pass's tables; then room for the records, A_V and the results
-        Pack pk;
-        const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0),
-                     o_sets = pk.put(L.pt_sets), o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off);
-        const size_t up = pk.h.size();
-        const size_t n_av = ext ? n_pt : 0;
-        const size_t o_rec = up, o_av = o_rec + carve_sz<vag_params>(n_pt + n_eval), o_chi2_pts = o_av + carve_sz<double>(n_av),
-                     o_st_pts = o_chi2_pts + carve_sz<double>(n_pt), o_st_eval = o_st_pts + carve_sz<int>(n_pt),
-                     o_status = o_st_eval + carve_sz<int>(n_eval), end = o_status + (d_status ? 0 : carve_sz<int>(n_models));
-        CK(ctx->io_sets.ensure(end));
-        void* base = ctx->io_sets.p;
-        CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
-        vag_params* d_rec = at<vag_params>(base, o_rec);
-        k_gather_params_av<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(
-            d_params, at<int>(base, o_gather), n_pt + n_eval, d_rec, d_A_V, n_av, at<double>(base, o_av));
-        const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
-                          SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
-                          at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
-        const Chi2Points pts{d_t, d_nu, d_lnF_obs, d_sigma_ln, d_w, d_ext_k, ext ? at<double>(base, o_av) : nullptr,
-                             n_points_total};
-        int passes = 0;
-        if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands_total, grids, true, n_models, d_chi2,
-                                  d_status ? d_status : at<int32_t>(base, o_status), s, &passes))
+    multi_lists(n_models, dataset_of, sets, n_sets, P.h_ok, L);
+    int launches = 0;
+    double* chi2 = d_chi2;
+    int32_t* status = d_status;  // NULL: scratch for k_chi2_bands
+    if (L.n_pt + L.n_eval)
+        if (int rc = multi_chi2(ctx, d_params, n_models, L, P.caps,
+                                Chi2Points{d_t, d_nu, d_lnF_obs, d_sigma_ln, d_w, d_ext_k, nullptr, n_points_total}, d_A_V,
+                                false, bands, n_bands_total, grids, chi2, status, s, &launches))
             return rc;
-        launches += 1 + passes;  // k_gather_params_av
-    }
     // k_chi2_bands gave the rejected models (no point term, no band) chi2 = 0 and status 0; k_reject overwrites them
-    k_reject<<<(unsigned)n_models, 128, 0, s>>>(d_ok, d_status, d_chi2, nullptr, 0);
-    ctx->launches = launches + 1;
+    k_reject<<<(unsigned)n_models, 128, 0, s>>>(P.ok, d_status, d_chi2, nullptr, 0);
+    ctx->launches = launches + 2;  // k_plan, k_reject
     CK(cudaGetLastError());
     return VAG_OK;
 }

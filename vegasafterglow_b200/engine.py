@@ -118,7 +118,6 @@ class Engine:
         fluxes with lnF_obs + A_V[m] * ext_k (band terms unchanged).
         +inf where the sum is not finite or the model's ODE failed (include/vag.h vag_chi2, vag_chi2_ext)."""
         p = self._params(params)
-        keep = []  # the arrays must outlive the call
         if points is not None:
             pt = [_f64(a).reshape(-1) for a in points]
             if len(pt) != 5 or len({a.size for a in pt}) != 1:
@@ -135,14 +134,7 @@ class Engine:
                 raise ValueError(f"ext_k has {ext.size} values for {n_pt} points")
             if av.size != p.size:
                 raise ValueError(f"A_V has {av.size} values for {p.size} models")
-        arr = (abi.BandObs * max(len(bands), 1))()
-        for i, b in enumerate(bands):
-            cols = [_f64(b[k]).reshape(-1) for k in ("t", "lnF_obs", "sigma_ln", "w")]
-            if len({a.size for a in cols}) != 1:
-                raise ValueError("band arrays t, lnF_obs, sigma_ln, w must have the same size")
-            keep.append(cols)
-            arr[i] = abi.BandObs(cols[0].ctypes.data, cols[1].ctypes.data, cols[2].ctypes.data, cols[3].ctypes.data,
-                                 cols[0].size, float(b["nu_min"]), float(b["nu_max"]), int(b["num_nu"]))
+        arr, _keep = self._band_array(bands, data=True)
         out = np.empty(p.size)
         st = np.zeros(p.size, dtype=np.int32)
         _lib.check(self._lib.vag_chi2_ext(self._h, p.ctypes.data, p.size, *[a.ctypes.data if n_pt else None for a in pt],
@@ -181,6 +173,24 @@ class Engine:
             raise ValueError("dataset_of must hold int32 data-set indices")
         return np.ascontiguousarray(ds, dtype=np.int32)
 
+    @staticmethod
+    def _extinction(extinction, sizes, n_models):
+        """``extinction`` = (ext_k, A_V) of a batch of several data sets -> (ext_k concatenated over the sets, A_V) as float64
+        arrays, or (None, None).  ext_k holds one array per data set, None for a set without points; A_V[n_models]."""
+        if extinction is None:
+            return None, None
+        ext_sets, av = extinction
+        if len(ext_sets) != len(sizes):
+            raise ValueError(f"extinction has {len(ext_sets)} ext_k entries for {len(sizes)} data sets")
+        ext = [np.zeros(0) if e is None else _f64(e).reshape(-1) for e in ext_sets]
+        for d, (e, n) in enumerate(zip(ext, sizes)):
+            if e.size != n:
+                raise ValueError(f"data set {d}: ext_k has {e.size} values for {n} points")
+        av = _f64(av).reshape(-1)
+        if av.size != n_models:
+            raise ValueError(f"A_V has {av.size} values for {n_models} models")
+        return np.concatenate(ext), av
+
     def flux_density_series_multi(self, params, datasets, dataset_of, return_status=False):
         """``flux_density_series`` of model m on its own data set ``datasets[dataset_of[m]]`` = (t, nu), t ascending,
         all in one batch.  Returns a list with one float64[5, n_d] array per model (n_d: the size of its data set); the
@@ -206,19 +216,7 @@ class Engine:
         p = self._params(params)
         (t, nu, lnF, sig, w), sets, sizes = self._concat_sets(datasets, ("t", "nu", "lnF_obs", "sigma_ln", "w"))
         ds = self._dataset_of(dataset_of, p.size)
-        ext = av = None
-        if extinction is not None:
-            ext_sets, av = extinction
-            if len(ext_sets) != len(sizes):
-                raise ValueError(f"extinction has {len(ext_sets)} ext_k arrays for {len(sizes)} data sets")
-            ext = [_f64(e).reshape(-1) for e in ext_sets]
-            for d, (e, n) in enumerate(zip(ext, sizes)):
-                if e.size != n:
-                    raise ValueError(f"data set {d}: ext_k has {e.size} values for {n} points")
-            ext = np.concatenate(ext)
-            av = _f64(av).reshape(-1)
-            if av.size != p.size:
-                raise ValueError(f"A_V has {av.size} values for {p.size} models")
+        ext, av = self._extinction(extinction, sizes, p.size)
         out = np.empty(p.size)
         st = np.zeros(p.size, dtype=np.int32)
         _lib.check(self._lib.vag_chi2_multi(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p), len(sets),
@@ -289,21 +287,7 @@ class Engine:
             sets[d] = abi.MultiSet(int(pt_off[d]), int(n_pts[d]), b0, len(bands[d]))
             b0 += len(bands[d])
         ds = self._dataset_of(dataset_of, p.size)
-        ext = av = None
-        if extinction is not None:
-            ext_sets, av = extinction
-            if len(ext_sets) != len(datasets):
-                raise ValueError(f"extinction has {len(ext_sets)} ext_k entries for {len(datasets)} data sets")
-            ext = []
-            for d, e in enumerate(ext_sets):
-                e = np.zeros(0) if e is None else _f64(e).reshape(-1)
-                if e.size != n_pts[d]:
-                    raise ValueError(f"data set {d}: ext_k has {e.size} values for {n_pts[d]} points")
-                ext.append(e)
-            ext = np.concatenate(ext)
-            av = _f64(av).reshape(-1)
-            if av.size != p.size:
-                raise ValueError(f"A_V has {av.size} values for {p.size} models")
+        ext, av = self._extinction(extinction, n_pts, p.size)
         out = np.empty(p.size)
         st = np.zeros(p.size, dtype=np.int32)
         pts = [a.ctypes.data if t.size else None for a in (t, nu, lnF, sig, w)]
@@ -348,16 +332,22 @@ class Engine:
         _lib.check(self._lib.vag_flux_band_dev(self._h, d_params, n_models, d_t, n_t, float(nu_min), float(nu_max),
                                                int(num_nu), d_out, d_status or None, stream or None))
 
+    @staticmethod
+    def _band_array_dev(bands):
+        """``abi.BandObs`` array of band dicts whose t, lnF_obs, sigma_ln, w are device pointers of length ``n``."""
+        arr = (abi.BandObs * max(len(bands), 1))()
+        for i, b in enumerate(bands):
+            arr[i] = abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], int(b["n"]), float(b["nu_min"]),
+                                 float(b["nu_max"]), int(b["num_nu"]))
+        return arr
+
     def chi2_dev(self, d_params, n_models, points=None, bands=(), d_chi2=0, d_status=0, extinction=None, stream=0):
         """``vag_chi2_dev``: the likelihood of ``chi2`` on device pointers.  ``points`` = (d_t, d_nu, d_lnF, d_sig, d_w,
         n_points) or None; ``bands``: dicts like ``chi2``'s whose t, lnF_obs, sigma_ln, w are device pointers with their
         length ``n``; ``extinction`` = (d_ext_k, d_A_V).  Rejected parameter sets give chi2 = +inf and ``abi.ST_INVALID``."""
         pts, n_pt = ([None] * 5, 0) if points is None else (list(points[:5]), int(points[5]))
         ext, av = (None, None) if extinction is None else extinction
-        arr = (abi.BandObs * max(len(bands), 1))()
-        for i, b in enumerate(bands):
-            arr[i] = abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], int(b["n"]), float(b["nu_min"]),
-                                 float(b["nu_max"]), int(b["num_nu"]))
+        arr = self._band_array_dev(bands)
         _lib.check(self._lib.vag_chi2_dev(self._h, d_params, n_models, *pts, ext, n_pt, av,
                                           C.cast(arr, C.c_void_p) if len(bands) else None, len(bands), d_chi2,
                                           d_status or None, stream or None))
@@ -380,10 +370,7 @@ class Engine:
             for d, s in enumerate(sets):
                 arr_sets[d] = abi.MultiSet(*(int(v) for v in s))
         ds = self._dataset_of(dataset_of, int(n_models))
-        arr = (abi.BandObs * max(len(bands), 1))()
-        for i, b in enumerate(bands):
-            arr[i] = abi.BandObs(b["t"], b["lnF_obs"], b["sigma_ln"], b["w"], int(b["n"]), float(b["nu_min"]),
-                                 float(b["nu_max"]), int(b["num_nu"]))
+        arr = self._band_array_dev(bands)
         _lib.check(self._lib.vag_chi2_multi_bands_dev(self._h, d_params, int(n_models), ds.ctypes.data,
                                                       C.cast(arr_sets, C.c_void_p) if n_sets else None, n_sets, *pts, ext,
                                                       n_pt, av, C.cast(arr, C.c_void_p) if len(bands) else None, len(bands),
