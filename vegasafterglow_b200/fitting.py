@@ -59,6 +59,38 @@ def band_obs(t, flux, err, nu_min, nu_max, num_points=5, weights=None):
             "nu_min": float(nu_min), "nu_max": float(nu_max), "num_nu": int(num_points)}
 
 
+def _chi2_batch(engine, P, points, bands, ext_kernel=None, A_V=None):
+    """chi2 of the records ``P`` in one engine call: ``chi2_series`` for points alone, ``chi2`` with bands, and
+    ``chi2(extinction=(ext_kernel, A_V))`` with a per-walker A_V.  The stored arrays are passed as they are."""
+    if A_V is not None:
+        return engine.chi2(P, points, bands, extinction=(ext_kernel, A_V))
+    if not bands:
+        return engine.chi2_series(P, *points)
+    return engine.chi2(P, points, bands)
+
+
+def _ensemble_chi2(engine, P, points, bands, ext_kernel=None, A_V=None, window=None):
+    """chi2 of every record of ``P``; +inf for a record the model constructor rejects (the reference maps that exception
+    to logL = -inf, samplers.py:63-70).  ``A_V`` (per walker) shifts the point data and is dropped without points.
+    ``window``: None evaluates every walker here; else the ensemble is split over the ranks by the cost proxy over the
+    span of these times.  The validity mask is computed from the parameters alone, identically on every rank, BEFORE the
+    split, and every rank joins the gather even with an empty share: a rejected walker can never desynchronise it."""
+    from .engine import Engine
+
+    ok = Engine.valid_mask(P)
+    per_walker = (A_V,) if A_V is not None and points is not None else ()
+    evaluate = lambda Q, *av: _chi2_batch(engine, Q, points, bands, ext_kernel, *av)  # noqa: E731
+    if window is not None:
+        from . import parallel
+
+        return parallel.partitioned_chi2(engine, P, window, None, None, None, None, evaluate=evaluate, valid=ok,
+                                         per_walker=per_walker)
+    out = np.full(P.size, np.inf)
+    if ok.any():
+        out[ok] = evaluate(P[ok], *(a[ok] for a in per_walker))
+    return out
+
+
 class BatchedLikelihood:
     """``log_prob_batch(samples[n, ndim]) -> logp[n]`` on the GPU.
 
@@ -98,6 +130,8 @@ class BatchedLikelihood:
         self.bands = [band_obs(**b) for b in bands]
         if not self.t.size and not self.bands:
             raise ValueError("no data")
+        # the times of the distributed split's cost proxy: the points', or every band's without points
+        self._cost_times = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
         self.lower = None if lower is None else np.asarray(lower, dtype=np.float64)
         self.upper = None if upper is None else np.asarray(upper, dtype=np.float64)
         self.log_prior = log_prior
@@ -108,7 +142,7 @@ class BatchedLikelihood:
         samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
         P = np.repeat(self.template, samples.shape[0])
         for i, name in enumerate(self.names):
-            if name == "A_V":  # not a model parameter: it shifts the observed point data (_evaluate)
+            if name == "A_V":  # not a model parameter: it shifts the observed point data (_chi2_batch)
                 continue
             col = self._column(samples, i)
             path = _FIELDS[name]
@@ -121,35 +155,13 @@ class BatchedLikelihood:
     def _column(self, samples, i):
         return 10.0 ** samples[:, i] if self.log_scale[i] else samples[:, i]
 
-    def _evaluate(self, P: np.ndarray, A_V=None) -> np.ndarray:
-        pts = (self.t, self.nu, self.lnF, self.sig, self.w) if self.t.size else None
-        if A_V is not None:
-            return self.engine.chi2(P, pts, self.bands, extinction=(self.ext_kernel, A_V))
-        if not self.bands:
-            return self.engine.chi2_series(P, *pts)
-        return self.engine.chi2(P, pts, self.bands)
-
     def chi2(self, samples: np.ndarray) -> np.ndarray:
-        """chi2 of every sample; +inf for a sample the model constructor rejects (the reference maps that exception to
-        logL = -inf, samplers.py:63-70).  The validity mask is computed from the parameters alone, identically on every
-        rank, BEFORE the ensemble is split: a rejected walker can therefore never desynchronise the collective."""
-        from .engine import Engine
-
+        """chi2 of every sample; +inf for a sample the model constructor rejects (``_ensemble_chi2``)."""
         samples = np.atleast_2d(np.asarray(samples, dtype=np.float64))
-        P = self.to_params(samples)
-        ok = Engine.valid_mask(P)
-        # a fitted A_V shifts the point data; without point data there is nothing to shift
-        per_walker = (self._column(samples, self.names.index("A_V")),) if "A_V" in self.names and self.t.size else ()
-        if self.distributed:
-            from . import parallel
-
-            tt = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
-            return parallel.partitioned_chi2(self.engine, P, tt, self.nu, self.lnF, self.sig, self.w, evaluate=self._evaluate,
-                                             valid=ok, per_walker=per_walker)
-        out = np.full(P.size, np.inf)
-        if ok.any():
-            out[ok] = self._evaluate(P[ok], *(a[ok] for a in per_walker))
-        return out
+        pts = (self.t, self.nu, self.lnF, self.sig, self.w) if self.t.size else None
+        A_V = self._column(samples, self.names.index("A_V")) if "A_V" in self.names else None
+        return _ensemble_chi2(self.engine, self.to_params(samples), pts, self.bands, self.ext_kernel, A_V,
+                              self._cost_times if self.distributed else None)
 
     def _in_bounds(self, samples: np.ndarray) -> np.ndarray:
         """Indices of the samples inside [lower, upper]."""
@@ -177,8 +189,34 @@ class BatchedLikelihood:
         return self._log_prob(samples, idx, self.chi2(samples[idx]) if idx.size else np.zeros(0))
 
 
-
 _CUDA_STREAM_LEGACY = 0x1  # cudaStreamLegacy (driver_types.h)
+
+
+def _stream(device):
+    """The stream handle of a ``_dev`` call on ``device``: torch's current stream on a GPU, 0 on the CPU.  A NULL stream
+    would be the engine's own, unordered with the record assembly before the call.  torch's default stream has the
+    handle 0 and is CUDA's legacy default stream, which the C ABI takes as cudaStreamLegacy."""
+    import torch
+
+    if device.type != "cuda":
+        return 0
+    return torch.cuda.current_stream(device).cuda_stream or _CUDA_STREAM_LEGACY
+
+
+def _rank_share(cost, evaluate, device):
+    """Every walker's chi2 (a float64 tensor on ``device``) on every rank: the walkers are split by
+    ``parallel.balanced_assignment`` of ``cost``, ``evaluate(mine, idx)`` gives this rank's share (its walkers as a numpy
+    array and as a tensor on ``device``), and one ``parallel.gather_indexed_tensor`` collects them, joined even with an
+    empty share."""
+    import torch
+
+    from . import parallel
+
+    world, rank = parallel.world_rank()
+    sets = parallel.balanced_assignment(cost, world)
+    mine = sets[rank]
+    local = evaluate(mine, torch.as_tensor(mine, dtype=torch.long, device=device))
+    return parallel.gather_indexed_tensor(local, sets, len(cost))
 
 
 def _field_offset(path):
@@ -253,12 +291,8 @@ class DeviceLikelihood(BatchedLikelihood):
         extinction = None if av is None else (self._ext.data_ptr(), av.data_ptr())
         bands = [dict(b, n=b["t"].numel(), **{k: b[k].data_ptr() for k in ("t", "lnF_obs", "sigma_ln", "w")})
                  for b in self._bands]
-        stream = 0
-        if self.device.type == "cuda":
-            # A NULL stream would be the engine's own, unordered with the record assembly above.  torch's default
-            # stream has the handle 0 and is CUDA's legacy default stream, which the C ABI takes as cudaStreamLegacy.
-            stream = torch.cuda.current_stream(self.device).cuda_stream or _CUDA_STREAM_LEGACY
-        self.engine.chi2_dev(rec.data_ptr(), n, points, bands, chi2.data_ptr(), extinction=extinction, stream=stream)
+        self.engine.chi2_dev(rec.data_ptr(), n, points, bands, chi2.data_ptr(), extinction=extinction,
+                             stream=_stream(self.device))
         return chi2
 
     def chi2(self, samples: np.ndarray) -> np.ndarray:
@@ -268,16 +302,11 @@ class DeviceLikelihood(BatchedLikelihood):
         cols = torch.as_tensor(self.columns(samples), device=self.device)
         if not self.distributed:
             return self._chi2_dev(cols).cpu().numpy()
-        import torch.distributed as dist
-
         from . import parallel
 
-        world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
-        tt = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
+        tt = self._cost_times
         cost = parallel.cost_proxy(self.to_params(samples), float(np.min(tt)), float(np.max(tt)))
-        sets = parallel.balanced_assignment(cost, world)
-        mine = torch.as_tensor(sets[rank], dtype=torch.long, device=self.device)
-        return parallel.gather_indexed_tensor(self._chi2_dev(cols[mine]), sets, cols.shape[0]).cpu().numpy()
+        return _rank_share(cost, lambda _, idx: self._chi2_dev(cols[idx]), self.device).cpu().numpy()
 
 
 class LikelihoodStack:
@@ -293,20 +322,22 @@ class LikelihoodStack:
     Not supported (``NotImplementedError``): band-integrated data (stack such fits with ``BandLikelihoodStack``),
     ``distributed=True`` and ``DeviceLikelihood``."""
 
+    _band_data = False  # whether fits with band-integrated data (or without points) are accepted
+
     def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
         self.likelihoods = list(likelihoods)
         if not self.likelihoods:
-            raise ValueError("LikelihoodStack needs at least one likelihood")
+            raise ValueError(f"{type(self).__name__} needs at least one likelihood")
         for k, lk in enumerate(self.likelihoods):
             if isinstance(lk, DeviceLikelihood):
                 raise NotImplementedError(f"likelihood {k}: a DeviceLikelihood cannot be stacked (its data live in HBM)")
-            if lk.bands or not lk.t.size:
+            if not self._band_data and (lk.bands or not lk.t.size):
                 raise NotImplementedError(f"likelihood {k}: band-integrated data cannot be stacked (point data only)")
             if lk.distributed:
                 raise NotImplementedError(f"likelihood {k}: distributed=True cannot be stacked")
         self.engine = self.likelihoods[0].engine
-        self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) for lk in self.likelihoods]
-        self.fits_av = ["A_V" in lk.names for lk in self.likelihoods]
+        self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) if lk.t.size else None for lk in self.likelihoods]
+        self.fits_av = ["A_V" in lk.names and lk.t.size > 0 for lk in self.likelihoods]
 
     def _walkers(self, samples):
         """The valid walkers of every fit as one batch: (records, fit of each, A_V of each (0 where the fit has none),
@@ -340,10 +371,14 @@ class LikelihoodStack:
         P, ds, av, ok = self._walkers(samples)
         extinction = None
         if any(self.fits_av):
-            ext = [lk.ext_kernel if fit else np.zeros(lk.t.size) for lk, fit in zip(self.likelihoods, self.fits_av)]
+            ext = [None if not lk.t.size else lk.ext_kernel if fit else np.zeros(lk.t.size)
+                   for lk, fit in zip(self.likelihoods, self.fits_av)]
             extinction = (ext, av)
-        flat = self.engine.chi2_multi(P, self.datasets, ds, extinction=extinction) if P.size else np.zeros(0)
-        return self._split(flat, ok)
+        return self._split(self._engine_chi2(P, ds, extinction) if P.size else np.zeros(0), ok)
+
+    def _engine_chi2(self, P, dataset_of, extinction):
+        """chi2 of the stacked walkers in one engine call: ``chi2_multi`` here, ``chi2_multi_bands`` with bands."""
+        return self.engine.chi2_multi(P, self.datasets, dataset_of, extinction=extinction)
 
     def __call__(self, samples):
         if len(samples) != len(self.likelihoods):
@@ -362,31 +397,14 @@ class BandLikelihoodStack(LikelihoodStack):
     ``LikelihoodStack``'s.  A bands-only fit that names ``A_V`` ignores it, as ``BatchedLikelihood`` does without points.
     Not supported (``NotImplementedError``): ``distributed=True`` and ``DeviceLikelihood``."""
 
-    def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
-        self.likelihoods = list(likelihoods)
-        if not self.likelihoods:
-            raise ValueError("BandLikelihoodStack needs at least one likelihood")
-        for k, lk in enumerate(self.likelihoods):
-            if isinstance(lk, DeviceLikelihood):
-                raise NotImplementedError(f"likelihood {k}: a DeviceLikelihood cannot be stacked (its data live in HBM)")
-            if lk.distributed:
-                raise NotImplementedError(f"likelihood {k}: distributed=True cannot be stacked")
-        self.engine = self.likelihoods[0].engine
-        self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) if lk.t.size else None for lk in self.likelihoods]
-        self.bands = [lk.bands for lk in self.likelihoods]
-        self.fits_av = ["A_V" in lk.names and lk.t.size > 0 for lk in self.likelihoods]
+    _band_data = True
 
-    def chi2(self, samples):
-        """chi2 of every sample of every fit (a list of K arrays); +inf for parameter sets the constructors reject."""
-        P, ds, av, ok = self._walkers(samples)
-        extinction = None
-        if any(self.fits_av):
-            ext = [None if not lk.t.size else lk.ext_kernel if fit else np.zeros(lk.t.size)
-                   for lk, fit in zip(self.likelihoods, self.fits_av)]
-            extinction = (ext, av)
-        flat = (self.engine.chi2_multi_bands(P, self.datasets, self.bands, ds, extinction=extinction) if P.size
-                else np.zeros(0))
-        return self._split(flat, ok)
+    def __init__(self, likelihoods: Sequence[BatchedLikelihood]):
+        super().__init__(likelihoods)
+        self.bands = [lk.bands for lk in self.likelihoods]
+
+    def _engine_chi2(self, P, dataset_of, extinction):
+        return self.engine.chi2_multi_bands(P, self.datasets, self.bands, dataset_of, extinction=extinction)
 
 
 class DeviceLikelihoodStack(LikelihoodStack):
@@ -494,11 +512,8 @@ class DeviceLikelihoodStack(LikelihoodStack):
         points = None if self._pts is None else (*(a.data_ptr() for a in self._pts), self.n_points)
         av = X[:, -1].contiguous() if self._ext is not None else None
         extinction = None if av is None else (self._ext.data_ptr(), av.data_ptr())
-        stream = 0
-        if self.device.type == "cuda":  # as DeviceLikelihood._chi2_dev: ordered after the record assembly
-            stream = torch.cuda.current_stream(self.device).cuda_stream or _CUDA_STREAM_LEGACY
         self.engine.chi2_multi_bands_dev(rec.data_ptr(), n, dataset_of, self.sets, points, self._bands, chi2.data_ptr(),
-                                         extinction=extinction, stream=stream)
+                                         extinction=extinction, stream=_stream(self.device))
         return chi2
 
     def chi2(self, samples):
@@ -513,17 +528,12 @@ class DeviceLikelihoodStack(LikelihoodStack):
         if not self.distributed:
             flat = self._chi2_dev(X, fit_of, ds).cpu().numpy()
         else:
-            import torch.distributed as dist
-
             from . import parallel
 
-            world, rank = (dist.get_world_size(), dist.get_rank()) if dist.is_available() and dist.is_initialized() else (1, 0)
             cost = np.concatenate([parallel.cost_proxy(lk.to_params(s), *win) if s.shape[0] else np.zeros(0)
                                    for lk, s, win in zip(self.likelihoods, samples, self._window)])
-            sets = parallel.balanced_assignment(cost, world)
-            mine = sets[rank]
-            idx = torch.as_tensor(mine, dtype=torch.long, device=self.device)
-            flat = parallel.gather_indexed_tensor(self._chi2_dev(X[idx], fit_of[idx], ds[mine]), sets, n).cpu().numpy()
+            evaluate = lambda mine, idx: self._chi2_dev(X[idx], fit_of[idx], ds[mine])  # noqa: E731
+            flat = _rank_share(cost, evaluate, self.device).cpu().numpy()
         out, lo = [], 0
         for s in samples:
             out.append(flat[lo:lo + s.shape[0]])

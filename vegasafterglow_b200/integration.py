@@ -29,7 +29,7 @@ from typing import Callable, Sequence
 import numpy as np
 
 from . import abi
-from .fitting import band_obs
+from .fitting import _ensemble_chi2, band_obs
 
 _JET_CODE = {"tophat": abi.JET_TOPHAT, "uniform": abi.JET_TOPHAT, "gaussian": abi.JET_GAUSSIAN,
              "powerlaw": abi.JET_POWERLAW, "two_component": abi.JET_TWO_COMPONENT,
@@ -107,30 +107,13 @@ class GpuFitterEvaluator:
     def chi2(self, thetas: np.ndarray) -> np.ndarray:
         thetas = np.atleast_2d(np.asarray(thetas, dtype=np.float64))
         mp = [self.fitter._to_params(th) for th in thetas]
-        P = params_from_fitter(self.fitter, mp)
-        from .engine import Engine
-
-        ok = Engine.valid_mask(P)
-        per_walker = ()
+        A_V = None
         if self.ext_kernel is not None:
-            per_walker = (np.array([getattr(p, "A_V", 0.0) for p in mp], dtype=np.float64),)
-        out = np.full(len(mp), np.inf)
-        if ok.any():
-            if self.distributed:
-                from . import parallel
-
-                tt = self.points[0] if self.has_points else self.bands[0]["t"]
-                return parallel.partitioned_chi2(self.engine, P, tt, None, None, None, None, evaluate=self._run, valid=ok,
-                                                 per_walker=per_walker)
-            out[ok] = self._run(P[ok], *(a[ok] for a in per_walker))
-        return out
-
-    def _run(self, P, A_V=None):
-        if A_V is not None:
-            return self.engine.chi2(P, self.points, self.bands, extinction=(self.ext_kernel, A_V))
-        if not self.bands:
-            return self.engine.chi2_series(P, *self.points)
-        return self.engine.chi2(P, self.points, self.bands)
+            A_V = np.array([getattr(p, "A_V", 0.0) for p in mp], dtype=np.float64)
+        # the cost proxy of the distributed split spans the point times, or the first band's without points
+        window = (self.points[0] if self.has_points else self.bands[0]["t"]) if self.distributed else None
+        P = params_from_fitter(self.fitter, mp)
+        return _ensemble_chi2(self.engine, P, self.points, self.bands, self.ext_kernel, A_V, window)
 
     def log_likelihoods(self, thetas, log_likelihood_fn: Callable) -> np.ndarray:
         chi2 = self.chi2(thetas)

@@ -17,24 +17,13 @@ def partition(n: int, world: int, rank: int):
     return lo, min(lo + per, n)
 
 
-def gather_blocks(local: np.ndarray, n: int, device=None) -> np.ndarray:
-    """All-gather the per-rank float64 blocks of ``partition`` back into a length-``n`` vector."""
-    import torch
+def world_rank():
+    """(world size, rank) of the initialised ``torch.distributed`` process group; (1, 0) without one."""
     import torch.distributed as dist
 
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
-        return np.asarray(local, dtype=np.float64)
-    world = dist.get_world_size()
-    per = -(-n // world)
-    if device is None:
-        device = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu")
-    buf = torch.full((per,), float("inf"), dtype=torch.float64, device=device)
-    buf[: len(local)] = torch.as_tensor(np.asarray(local, dtype=np.float64), device=device)
-    out = torch.empty(per * world, dtype=torch.float64, device=device)
-    dist.all_gather_into_tensor(out, buf)
-    out = out.cpu().numpy()
-    pieces = [out[r * per: r * per + (partition(n, world, r)[1] - partition(n, world, r)[0])] for r in range(world)]
-    return np.concatenate(pieces)
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_world_size(), dist.get_rank()
+    return 1, 0
 
 
 def cost_proxy(params, t_min=1e2, t_max=1e7) -> np.ndarray:
@@ -79,27 +68,16 @@ def balanced_assignment(cost, world: int):
 
 
 def gather_indexed(local: np.ndarray, sets, n: int, device=None) -> np.ndarray:
-    """All-gather per-rank float64 vectors whose entries belong to the walkers ``sets[rank]`` into a length-``n`` vector."""
+    """All-gather per-rank float64 vectors whose entries belong to the walkers ``sets[rank]`` into a length-``n``
+    vector: ``gather_indexed_tensor`` on the collective's device (the current GPU under NCCL, else the CPU), as numpy."""
     import torch
     import torch.distributed as dist
 
-    world = len(sets)
-    if world == 1 or not (dist.is_available() and dist.is_initialized()):
-        out = np.full(n, np.inf)
-        out[sets[0]] = np.asarray(local, dtype=np.float64)
-        return out
-    per = max(len(s) for s in sets)
     if device is None:
-        device = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu")
-    buf = torch.full((max(per, 1),), float("inf"), dtype=torch.float64, device=device)
-    buf[: len(local)] = torch.as_tensor(np.asarray(local, dtype=np.float64), device=device)
-    got = torch.empty(max(per, 1) * world, dtype=torch.float64, device=device)
-    dist.all_gather_into_tensor(got, buf)
-    got = got.cpu().numpy()
-    out = np.full(n, np.inf)
-    for r, idx in enumerate(sets):
-        out[idx] = got[r * max(per, 1): r * max(per, 1) + len(idx)]
-    return out
+        nccl = dist.is_available() and dist.is_initialized() and dist.get_backend() == "nccl"
+        device = torch.device("cuda", torch.cuda.current_device()) if nccl else torch.device("cpu")
+    local = torch.as_tensor(np.asarray(local, dtype=np.float64), device=device)
+    return gather_indexed_tensor(local, sets, n).cpu().numpy()
 
 
 def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=True, valid=None,
@@ -114,13 +92,8 @@ def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=
       to exercise the partition / gather logic under gloo;
     * ``per_walker``: a tuple of length-n arrays (e.g. a fitted A_V), sliced with the rank's walkers like ``params``
       and passed to ``evaluate`` as extra arguments."""
-    import torch.distributed as dist
-
     n = len(params)
-    if dist.is_available() and dist.is_initialized():
-        world, rank = dist.get_world_size(), dist.get_rank()
-    else:
-        world, rank = 1, 0
+    world, rank = world_rank()
     keep = np.arange(n) if valid is None else np.nonzero(np.asarray(valid, dtype=bool))[0]
     if balance:
         sets = [keep[s] for s in balanced_assignment(cost_proxy(params[keep], float(np.min(t)), float(np.max(t))), world)]
@@ -135,8 +108,9 @@ def partitioned_chi2(engine, params, t, nu, lnF, sig, w, evaluate=None, balance=
 
 
 def gather_indexed_tensor(local, sets, n: int):
-    """``gather_indexed`` for a float64 tensor on the rank's device: the gather stays on that device (NCCL on GPUs, gloo
-    on the CPU) and the result is a length-``n`` tensor there, +inf where no rank wrote."""
+    """All-gather per-rank float64 tensors whose entries belong to the walkers ``sets[rank]``: the gather stays on the
+    rank's device (NCCL on GPUs, gloo on the CPU) and the result is a length-``n`` tensor there, +inf where no rank
+    wrote."""
     import torch
     import torch.distributed as dist
 
