@@ -208,8 +208,8 @@ int vag_chi2_ext(vag_context* ctx, const vag_params* params, size_t n_models, co
  * passes as the other entry points do.  Launches: those of vag_chi2_series / vag_flux_density_series on the same
  * total data, whatever n_sets (one CTA per data set inside the band search kernel).
  * Band-integrated data per data set: vag_flux_band_multi, vag_chi2_multi_bands below; on device buffers, planned on the
- * device: vag_chi2_multi_bands_dev (further below).  Not provided here: a device-buffer (_dev) variant of the two flux
- * calls, a public per-model grid (t x nu) request.
+ * device: vag_chi2_multi_bands_dev (further below).  A per-model grid (t x nu) request: vag_flux_density_grid_multi.
+ * Not provided here: a device-buffer (_dev) variant of the two flux calls.
  * The output mode (vag_set_output_mode) does not apply: every plane of `out` is written. */
 typedef struct vag_series_set {
     size_t offset, n; /* slice of the concatenated points */
@@ -272,6 +272,52 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
                          const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
                          const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
                          const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status);
+
+/* ---- a (t x nu) grid request per model, and posterior-predictive bands across models ------------------------------
+ * The times and frequencies of all grid sets are concatenated into t[n_t_total] and nu[n_nu_total]; set d is the times
+ * t[t0 .. t0 + n_t), ascending, finite and > 0, crossed with the frequencies nu[nu0 .. nu0 + n_nu) [Hz], finite and > 0.
+ * Model m is evaluated on set dataset_of[m] alone, as one evaluation of a single ragged grid request (the run of the band
+ * section above, with frequencies in Hz through the same unit conversion as vag_flux_density_grid's).  Its values are
+ * those of vag_flux_density_grid for that model on that set alone: bit for bit under the conditions stated for
+ * vag_flux_band_multi (no row split in either call -- from 2368 (model x shock) CTAs on 148 SMs -- and the same rows
+ * staged per pass; a model tiles its own n_nu as its own call does), otherwise to rounding.  An SSC model's tables span
+ * its own set's frequencies.  Batches over 32768 models run in passes.  The output mode does not apply.
+ * Checks, all before any work is enqueued (VAG_ERR_INVALID, the message names the set or the model; a failed call
+ * leaves the context usable and the outputs untouched): every set n_t > 0 and n_nu > 0, inside the arrays, its times
+ * ascending, finite and > 0, its frequencies finite and > 0; 0 <= dataset_of[m] < n_sets; parameter sets as
+ * vag_params_validate; n_t_total, n_nu_total, n_sets and n_models within a 32-bit int.  Sets no model uses are allowed.
+ * Not provided: device-buffer (_dev) forms of the two calls, bands of components other than total, weighted quantiles. */
+typedef struct vag_grid_set {
+    size_t t0, n_t;   /* slice of the concatenated times       */
+    size_t nu0, n_nu; /* slice of the concatenated frequencies */
+} vag_grid_set;
+
+/* PyModel::flux_density_grid (pybind/pymodel.cpp:498-514) of model m on its own set: model m's [VAG_NCOMP][n_nu][n_t]
+ * block starts at element VAG_NCOMP * off[m], off[m] = the sum of n_nu * n_t over the sets of models 0 .. m-1 (the
+ * layout of vag_flux_density_series_multi); every plane is written.  Launches: those of vag_flux_density_grid on one
+ * request, whatever n_sets. */
+int vag_flux_density_grid_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                const vag_grid_set* sets, size_t n_sets, const double* t, size_t n_t_total,
+                                const double* nu, size_t n_nu_total, double* out, int32_t* status);
+
+/* Posterior-predictive bands of many fits in one call: the run of vag_flux_density_grid_multi, then for every set d, every
+ * q[j] and every (nu, t) column, numpy.quantile(F_total[members of d], q[j], axis=0, method="linear") -- bit for bit (the
+ * sign of a zero aside) with numpy's rule on the same flux: h = (n - 1) q, lo = floor(h), hi = min(lo + 1, n - 1),
+ * g = h - lo, result a + (b - a) g, or b - (b - a) (1 - g) when g >= 0.5, with a, b the order statistics lo and hi.  The
+ * members of d are its models (dataset_of[m] == d) whose status has neither VAG_ST_ODE_FAIL500 (the reference throws)
+ * nor VAG_ST_CAPACITY (NaN output); the kernels read that from the run's status on the device.  A column with a NaN among
+ * its members gives NaN; a set without members gives NaN and n_used = 0.  The flux never leaves the device: the full
+ * ragged output sits in the context's output workspace, 8 * VAG_NCOMP * sum_m n_nu * n_t bytes.
+ * out: set d's [n_q][n_nu][n_t] block starts at n_q * the sum of n_nu * n_t over sets 0 .. d-1.  n_used[n_sets]: the
+ * members of every set.  status[n_models] may be NULL.  D2H traffic: out, n_used and status only.
+ * Checks: those of vag_flux_density_grid_multi, n_q >= 1 and every q[j] finite in [0, 1].
+ * Launches: those of vag_flux_density_grid_multi + 2 (the members of every set, a CTA per set; the selection, a CTA per
+ * set and 4 consecutive columns, a warp per column, exact MSB radix select over the order-preserving 64-bit image of the
+ * fluxes, in shared memory while the set's members fit 160 KB of staged keys, from global memory otherwise). */
+int vag_flux_quantiles_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                             const vag_grid_set* sets, size_t n_sets, const double* t, size_t n_t_total, const double* nu,
+                             size_t n_nu_total, const double* q, size_t n_q, double* out, int64_t* n_used,
+                             int32_t* status);
 
 /* ok[i] = 1 where vag_params_validate accepts params[i], else 0 (no error is raised for rejected sets). */
 int vag_params_validate_batch(const vag_params* params, size_t n, int32_t* ok);

@@ -61,6 +61,8 @@ def load():
     lib.vag_flux_band_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, ip]
     lib.vag_chi2_multi_bands.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, vp, sz, dp, ip]
     lib.vag_chi2_multi_bands_dev.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, vp, sz, dp, ip, vp]
+    lib.vag_flux_density_grid_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, sz, dp, sz, dp, ip]
+    lib.vag_flux_quantiles_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, sz, dp, sz, dp, sz, dp, vp, ip]
     lib.vag_debug_set_ode_limits.argtypes = [vp, C.c_int, C.c_int]
     lib.vag_last_total_alias.argtypes = [vp]
     lib.vag_set_series_mode.argtypes = [vp, C.c_int]
@@ -80,7 +82,7 @@ EXPORTS = [
     "vag_set_profiling", "vag_set_output_mode", "vag_last_stage_ms", "vag_last_launch_count", "vag_measure_fp64_peak", "vag_selftest_libm", "vag_chi2", "vag_params_validate_batch", "vag_debug_set_ode_limits", "vag_last_total_alias", "vag_last_work", "vag_set_series_mode", "vag_details_ic",
     "vag_set_grid_lanes", "vag_chi2_ext", "vag_params_validate_batch_dev", "vag_flux_band_dev", "vag_chi2_dev",
     "vag_flux_density_series_multi", "vag_chi2_multi", "vag_flux_band_multi", "vag_chi2_multi_bands",
-    "vag_chi2_multi_bands_dev",
+    "vag_chi2_multi_bands_dev", "vag_flux_density_grid_multi", "vag_flux_quantiles_multi",
 ]
 
 

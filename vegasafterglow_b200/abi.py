@@ -101,6 +101,13 @@ class MultiSet(C.Structure):
     _fields_ = [("offset", C.c_size_t), ("n", C.c_size_t), ("band0", C.c_size_t), ("n_bands", C.c_size_t)]
 
 
+class GridSet(C.Structure):
+    """``vag_grid_set`` (include/vag.h): one (t x nu) grid of a per-model grid request -- a slice of the concatenated
+    times and one of the concatenated frequencies."""
+
+    _fields_ = [("t0", C.c_size_t), ("n_t", C.c_size_t), ("nu0", C.c_size_t), ("n_nu", C.c_size_t)]
+
+
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
 

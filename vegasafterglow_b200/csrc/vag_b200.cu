@@ -25,6 +25,7 @@
 #include "../../include/vag.h"
 #include "vag_libm.cuh"
 #include "vag_pipeline.cuh"
+#include "vag_quantile.cuh"
 
 using namespace vag;
 
@@ -833,6 +834,88 @@ __global__ void k_gather_bands(const double* const* __restrict__ src, const Seri
     }
 }
 
+// ---- posterior-predictive bands (vag_flux_quantiles_multi) --------------------------------------------------------
+// The members of every set (CTA / set): of its candidates cand[c0[d] .. c0[d + 1]) -- the models whose dataset_of is d,
+// in model order -- those whose status has neither VAG_ST_ODE_FAIL500 (the reference throws) nor VAG_ST_CAPACITY (NaN
+// output), kept in order as the element offsets VAG_NCOMP * out_off[m] of their `total` planes in the ragged grid output;
+// n_used[d] = their number
+__global__ void __launch_bounds__(256) k_quant_members(const int* __restrict__ cand, const int* __restrict__ c0,
+                                                       const int32_t* __restrict__ status, const long long* __restrict__ out_off,
+                                                       long long* __restrict__ mem_off, long long* __restrict__ n_used) {
+    __shared__ int s_warp[8];
+    __shared__ int s_count;
+    const int d = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int lo = c0[d], hi = c0[d + 1];
+    if (threadIdx.x == 0) s_count = 0;
+    __syncthreads();
+    for (int base = lo; base < hi; base += blockDim.x) {
+        const int i = base + threadIdx.x;
+        const int m = i < hi ? cand[i] : -1;
+        const bool keep = m >= 0 && !(status[m] & (VAG_ST_ODE_FAIL500 | VAG_ST_CAPACITY));
+        const unsigned bal = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) s_warp[wid] = __popc(bal);
+        __syncthreads();
+        int pos = s_count + __popc(bal & ((1u << lane) - 1u));
+        for (int w = 0; w < wid; ++w) pos += s_warp[w];
+        if (keep) mem_off[lo + pos] = (long long)VAG_NCOMP * out_off[m];
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < 8; ++w) s_count += s_warp[w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) n_used[d] = s_count;
+}
+
+// numpy.quantile(method="linear") of every (set, column) over the set's members (vag_quantile.cuh), CTA / (set, tile of
+// QUANT_COLS consecutive columns of its [n_nu][n_t] grid), a warp / column.  tile0[d]: the first tile of set d, col0[d]:
+// its first column among the concatenated columns of all sets; set d's members' offsets start at mem_off[c0[d]].  The
+// members' rows of the tile are read coalesced; a set of at most rows_cap members is staged as keys in shared memory
+// ([QUANT_COLS][n]) and selected there, a larger one is selected from global memory (L2) in every pass.
+// out: set d's [n_q][n_nu][n_t] block at n_q * col0[d].
+constexpr int QUANT_COLS = 4;
+constexpr size_t QUANT_SMEM_BUDGET = 160 * 1024;  // dynamic shared memory k_quantiles may stage a tile in
+__global__ void __launch_bounds__(QUANT_COLS * 32) k_quantiles(const double* __restrict__ F, const long long* __restrict__ mem_off,
+                                                             const int* __restrict__ c0, const long long* __restrict__ n_used,
+                                                             const long long* __restrict__ tile0,
+                                                             const long long* __restrict__ col0, int n_sets,
+                                                             const double* __restrict__ q, int n_q, int rows_cap,
+                                                             double* __restrict__ out) {
+    extern __shared__ uint64_t s_keys[];
+    __shared__ unsigned s_hist[QUANT_COLS][QUANT_BINS];
+    const long long tile = blockIdx.x;
+    int d = 0;  // the last set whose first tile is <= tile (every set has one tile or more)
+    for (int hi = n_sets; hi - d > 1;) {
+        const int mid = (d + hi) / 2;
+        if (tile0[mid] <= tile)
+            d = mid;
+        else
+            hi = mid;
+    }
+    const long long cols = col0[d + 1] - col0[d], c_first = (tile - tile0[d]) * QUANT_COLS;
+    const int n = (int)n_used[d];
+    const long long* __restrict__ mo = mem_off + c0[d];
+    const int wid = threadIdx.x >> 5;
+    const bool staged = n <= rows_cap;
+    if (staged) {
+        for (int e = threadIdx.x; e < n * QUANT_COLS; e += blockDim.x) {
+            const int i = e / QUANT_COLS, k = e - i * QUANT_COLS;
+            if (c_first + k < cols) s_keys[(size_t)k * n + i] = quant_key(F[mo[i] + c_first + k]);
+        }
+        __syncthreads();
+    }
+    const long long c = c_first + wid;
+    if (c >= cols) return;
+    const QuantWarp grp{(int)(threadIdx.x & 31)};
+    double* o = out + n_q * col0[d] + c;
+    if (staged) {
+        const uint64_t* ks = s_keys + (size_t)wid * n;
+        quant_column(grp, [ks](int i) { return ks[i]; }, n, q, n_q, o, (size_t)cols, s_hist[wid]);
+    } else {
+        const double* f = F + c;
+        quant_column(grp, [f, mo](int i) { return quant_key(f[mo[i]]); }, n, q, n_q, o, (size_t)cols, s_hist[wid]);
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -1479,6 +1562,7 @@ int vag_create(int device, vag_context** out) {
             for (int kind = 0; kind < EATS_KINDS; ++kind)
                 CK(cudaFuncSetAttribute(eats_kernel(mode, kind, ragged), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         (int)EATS_SMEM_BUDGET));
+    CK(cudaFuncSetAttribute(k_quantiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANT_SMEM_BUDGET));
     {
         int blocks = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_ic_spectrum<false>, 128, 0) == cudaSuccess && blocks > 0)
@@ -2169,8 +2253,48 @@ static int check_models(const vag_params* params, size_t n_models) {
     return VAG_OK;
 }
 
-// The band pass: evaluation e evaluates record e of d_params on band band_of[e], all as one ragged grid request through
-// run_flux (passes of 32768 evaluations), then k_band_reduce_sets.  Times, frequency nodes (code units) and weights are
+// A ragged grid request: evaluation e (record e of the run) on set set_of[e] of `tab`, whose SeriesSet is its slice of
+// the concatenated times and of the concatenated frequencies.  put() adds the set table, the evaluations' sets and their
+// output offsets to the caller's one upload; bind() points the device table at that upload; run() evaluates them all as
+// one request through run_flux (passes of 32768 evaluations), evaluation e's [VAG_NCOMP][n_nu][n] block at element
+// VAG_NCOMP * off[e] of d_grid.  The band pass (quadrature nodes in code units) and vag_flux_density_grid_multi /
+// vag_flux_quantiles_multi (frequencies in Hz) run through it.
+struct GridSets {
+    std::vector<long long> off;  // [n_eval + 1] first (time x frequency) point of each evaluation's block
+    size_t n_sets = 0, max_n = 0, max_nu = 0, o_tab = 0, o_of = 0, o_off = 0;
+    SetsDev sd{};
+    void put(Pack& pk, const std::vector<SeriesSet>& tab, const int32_t* set_of, size_t n_eval) {
+        n_sets = tab.size();
+        off.assign(n_eval + 1, 0);
+        for (size_t e = 0; e < n_eval; ++e) {
+            const SeriesSet& S = tab[set_of[e]];
+            off[e + 1] = off[e] + (long long)S.n * S.n_nu;
+            max_n = std::max(max_n, (size_t)S.n);
+            max_nu = std::max(max_nu, (size_t)S.n_nu);
+        }
+        o_tab = pk.put(tab);
+        o_of = pk.put(set_of, n_eval);
+        o_off = pk.put(off);
+    }
+    const SetsDev& bind(void* base) {
+        sd = SetsDev{at<int>(base, o_of), at<SeriesSet>(base, o_tab), at<long long>(base, o_off)};
+        return sd;
+    }
+    size_t elems() const { return (size_t)off.back() * VAG_NCOMP; }
+    int run(vag_context* ctx, const vag_params* d_params, Caps caps, const double* d_t, size_t n_t, const double* d_nu,
+            size_t n_nu, bool nu_code_units, double* d_grid, int32_t* d_status, cudaStream_t s) const {
+        Request rq{false, d_t, d_nu, n_t, n_nu, nu_code_units};
+        rq.sets = &sd;
+        rq.h_off = off.data();
+        rq.n_sets = (int)n_sets;
+        rq.max_set = max_n;
+        rq.max_nu = max_nu;
+        return run_flux(ctx, d_params, off.size() - 1, caps, rq, d_grid, d_status, nullptr, s);
+    }
+};
+
+// The band pass: evaluation e evaluates record e of d_params on band band_of[e], all as one ragged grid request
+// (GridSets), then k_band_reduce_sets.  Times, frequency nodes (code units) and weights are
 // concatenated over the bands, and with `data` lnF_obs / sigma_ln / w at the times' offsets.  Its tables go to io_bands,
 // the grid and the band fluxes to io_out.  ctx->launches: run_flux's + 1.  With `device` (implies data) the bands' t /
 // lnF_obs / sigma_ln / w are device pointers: the host uploads a table of them with the other tables, and k_gather_bands
@@ -2207,25 +2331,18 @@ static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval
             w.insert(w.end(), B.w, B.w + B.n);
         }
     }
-    std::vector<long long> grid_off(n_eval + 1, 0);
     bp.h_red_off.assign(n_eval + 1, 0);
-    size_t max_n = 0, max_nu = 0;
-    for (size_t e = 0; e < n_eval; ++e) {
-        const SeriesSet& B = tab[band_of[e]];
-        grid_off[e + 1] = grid_off[e] + (long long)B.n * B.n_nu;
-        bp.h_red_off[e + 1] = bp.h_red_off[e] + B.n;
-        max_n = std::max(max_n, (size_t)B.n);
-        max_nu = std::max(max_nu, (size_t)B.n_nu);
-    }
+    for (size_t e = 0; e < n_eval; ++e) bp.h_red_off[e + 1] = bp.h_red_off[e] + tab[band_of[e]].n;
     Pack pk;
-    const size_t o_t = pk.put(t), o_nu = pk.put(nu), o_wgt = pk.put(wgt), o_tab = pk.put(tab), o_of = pk.put(band_of, n_eval),
-                 o_go = pk.put(grid_off), o_ro = pk.put(bp.h_red_off), o_lnF = pk.put(lnF), o_sig = pk.put(sig),
-                 o_w = pk.put(w), o_src = pk.put(src);
+    GridSets gs;
+    const size_t o_t = pk.put(t), o_nu = pk.put(nu), o_wgt = pk.put(wgt);
+    gs.put(pk, tab, band_of, n_eval);
+    const size_t o_ro = pk.put(bp.h_red_off), o_lnF = pk.put(lnF), o_sig = pk.put(sig), o_w = pk.put(w), o_src = pk.put(src);
     const size_t up = pk.h.size(), plane = device ? carve_sz<double>(n_t) / sizeof(double) : 0;
     CK(ctx->io_bands.ensure(up + 4 * sizeof(double) * plane));
     void* base = ctx->io_bands.p;
     CK(cudaMemcpyAsync(base, pk.h.data(), up, cudaMemcpyHostToDevice, s));
-    bp.sd = SetsDev{at<int>(base, o_of), at<SeriesSet>(base, o_tab), at<long long>(base, o_go)};
+    bp.sd = gs.bind(base);
     bp.red_off = at<long long>(base, o_ro);
     const double* d_t = at<double>(base, o_t);
     bp.lnF = data ? at<double>(base, o_lnF) : nullptr;
@@ -2239,17 +2356,11 @@ static int band_pass(vag_context* ctx, const vag_params* d_params, size_t n_eval
         bp.sig = planes + 2 * plane;
         bp.w = planes + 3 * plane;
     }
-    const size_t grid_elems = (size_t)grid_off[n_eval] * VAG_NCOMP, red_elems = (size_t)bp.h_red_off[n_eval] * VAG_NCOMP;
+    const size_t grid_elems = gs.elems(), red_elems = (size_t)bp.h_red_off[n_eval] * VAG_NCOMP;
     CK(ctx->io_out.ensure(sizeof(double) * (grid_elems + red_elems)));
     double* d_grid = static_cast<double*>(ctx->io_out.p);
     bp.red = d_grid + grid_elems;
-    Request rq{false, d_t, at<double>(base, o_nu), n_t, nu.size(), true};
-    rq.sets = &bp.sd;
-    rq.h_off = grid_off.data();
-    rq.n_sets = (int)n_bands;
-    rq.max_set = max_n;
-    rq.max_nu = max_nu;
-    if (int rc = run_flux(ctx, d_params, n_eval, caps, rq, d_grid, d_status, nullptr, s)) return rc;
+    if (int rc = gs.run(ctx, d_params, caps, d_t, n_t, at<double>(base, o_nu), nu.size(), true, d_grid, d_status, s)) return rc;
     k_band_reduce_sets<<<(unsigned)n_eval, 128, 0, s>>>(d_grid, at<double>(base, o_wgt), bp.red, bp.red_off, bp.sd);
     ctx->launches += device ? 2 : 1;  // (k_gather_bands ran before run_flux, which restarts the count)
     CK(cudaGetLastError());
@@ -2278,6 +2389,154 @@ int vag_flux_band_multi(vag_context* ctx, const vag_params* params, size_t n_mod
                            false, static_cast<int32_t*>(ctx->io_status.p), bp, s))
         return rc;
     CK(cudaMemcpyAsync(out, bp.red, sizeof(double) * VAG_NCOMP * bp.h_red_off[n_models], cudaMemcpyDeviceToHost, s));
+    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
+}
+
+// ---- per-model grid requests and their quantiles across models -----------------------------------------------------
+// The checks of vag_flux_density_grid_multi / vag_flux_quantiles_multi, all before any work is enqueued
+static int check_grid_multi(const vag_params* params, size_t n_models, const int32_t* dataset_of, const vag_grid_set* sets,
+                            size_t n_sets, const double* t, size_t n_t_total, const double* nu, size_t n_nu_total) {
+    if (!sets || n_sets == 0) return fail(VAG_ERR_INVALID, "no grid sets: sets is NULL or n_sets is 0");
+    if (!t || !nu) return fail(VAG_ERR_INVALID, "t or nu is NULL");
+    if (n_t_total > (size_t)INT_MAX || n_nu_total > (size_t)INT_MAX || n_sets > (size_t)INT_MAX ||
+        n_models > (size_t)INT_MAX)
+        return fail(VAG_ERR_INVALID, "n_t_total, n_nu_total, n_sets and n_models must fit in a 32-bit int");
+    if (n_models && !dataset_of) return fail(VAG_ERR_INVALID, "dataset_of is NULL");
+    for (size_t d = 0; d < n_sets; ++d) {
+        const std::string name = "set " + std::to_string(d) + ": ";
+        const vag_grid_set& S = sets[d];
+        if (S.n_t == 0) return fail(VAG_ERR_INVALID, name + "no times (n_t = 0)");
+        if (S.n_nu == 0) return fail(VAG_ERR_INVALID, name + "no frequencies (n_nu = 0)");
+        if (S.t0 > n_t_total || S.n_t > n_t_total - S.t0)
+            return fail(VAG_ERR_INVALID, name + "times [" + std::to_string(S.t0) + ", " + std::to_string(S.t0) + " + " +
+                                             std::to_string(S.n_t) + ") lie outside the " + std::to_string(n_t_total) + " times");
+        if (S.nu0 > n_nu_total || S.n_nu > n_nu_total - S.nu0)
+            return fail(VAG_ERR_INVALID, name + "frequencies [" + std::to_string(S.nu0) + ", " + std::to_string(S.nu0) + " + " +
+                                             std::to_string(S.n_nu) + ") lie outside the " + std::to_string(n_nu_total) +
+                                             " frequencies");
+        if (check_times(t + S.t0, S.n_t)) return fail(VAG_ERR_INVALID, name + g_err);
+        for (size_t i = S.nu0; i < S.nu0 + S.n_nu; ++i)
+            if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, name + "observation frequencies must be finite and > 0");
+    }
+    for (size_t m = 0; m < n_models; ++m)
+        if (dataset_of[m] < 0 || (size_t)dataset_of[m] >= n_sets)
+            return fail(VAG_ERR_INVALID, "model " + std::to_string(m) + ": dataset_of = " + std::to_string(dataset_of[m]) +
+                                             " is not a set index (n_sets = " + std::to_string(n_sets) + ")");
+    return check_models(params, n_models);
+}
+
+// The grid run of both calls on checked arguments, whose records prepare_params uploaded: pk holds the times, the
+// frequencies (Hz) and gs's tables, then whatever the caller packed behind them; one upload of it to io_sets with `room`
+// more bytes behind, then the run into io_out (status: io_status).  *base: the upload on the device.
+static int grid_multi_run(vag_context* ctx, Caps caps, const Pack& pk, size_t o_t, size_t n_t_total,
+                          size_t o_nu, size_t n_nu_total, GridSets& gs, size_t room, void** base, cudaStream_t s) {
+    CK(ctx->io_sets.ensure(pk.h.size() + room));
+    *base = ctx->io_sets.p;
+    CK(cudaMemcpyAsync(*base, pk.h.data(), pk.h.size(), cudaMemcpyHostToDevice, s));
+    gs.bind(*base);
+    CK(ctx->io_out.ensure(sizeof(double) * std::max<size_t>(gs.elems(), 1)));
+    return gs.run(ctx, static_cast<vag_params*>(ctx->io_params.p), caps, at<double>(*base, o_t), n_t_total,
+                  at<double>(*base, o_nu), n_nu_total, false, static_cast<double*>(ctx->io_out.p),
+                  static_cast<int32_t*>(ctx->io_status.p), s);
+}
+
+static std::vector<SeriesSet> grid_table(const vag_grid_set* sets, size_t n_sets) {
+    std::vector<SeriesSet> tab(n_sets);
+    for (size_t d = 0; d < n_sets; ++d)
+        tab[d] = SeriesSet{(int)sets[d].t0, (int)sets[d].n_t, (int)sets[d].n_nu, (int)sets[d].nu0};
+    return tab;
+}
+
+int vag_flux_density_grid_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                const vag_grid_set* sets, size_t n_sets, const double* t, size_t n_t_total,
+                                const double* nu, size_t n_nu_total, double* out, int32_t* status) {
+    if (!ctx || !out) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (int rc = check_grid_multi(params, n_models, dataset_of, sets, n_sets, t, n_t_total, nu, n_nu_total)) return rc;
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) return VAG_OK;
+    cudaStream_t s = ctx->stream;
+    Pack pk;
+    GridSets gs;
+    const size_t o_t = pk.put(t, n_t_total), o_nu = pk.put(nu, n_nu_total);
+    gs.put(pk, grid_table(sets, n_sets), dataset_of, n_models);
+    void* base = nullptr;
+    if (int rc = grid_multi_run(ctx, caps, pk, o_t, n_t_total, o_nu, n_nu_total, gs, 0, &base, s)) return rc;
+    CK(cudaMemcpyAsync(out, ctx->io_out.p, sizeof(double) * gs.elems(), cudaMemcpyDeviceToHost, s));
+    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
+}
+
+// The grid run of vag_flux_density_grid_multi, then k_quant_members and k_quantiles on its output in io_out: one upload
+// of the request, the run's tables, q and the quantile plan (the models of every set, in model order; every set's first
+// tile and first column), with room behind it for the members' offsets, n_used and the bands.
+int vag_flux_quantiles_multi(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                             const vag_grid_set* sets, size_t n_sets, const double* t, size_t n_t_total, const double* nu,
+                             size_t n_nu_total, const double* q, size_t n_q, double* out, int64_t* n_used,
+                             int32_t* status) {
+    if (!ctx || !out || !n_used) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (n_q == 0 || !q) return fail(VAG_ERR_INVALID, "no quantiles: q is NULL or n_q is 0");
+    if (n_q > (size_t)INT_MAX) return fail(VAG_ERR_INVALID, "n_q must fit in a 32-bit int");
+    for (size_t j = 0; j < n_q; ++j)
+        if (!(q[j] >= 0.0 && q[j] <= 1.0))
+            return fail(VAG_ERR_INVALID, "q[" + std::to_string(j) + "] must be finite and in [0, 1]");
+    if (int rc = check_grid_multi(params, n_models, dataset_of, sets, n_sets, t, n_t_total, nu, n_nu_total)) return rc;
+    std::vector<long long> tile0(n_sets + 1, 0), col0(n_sets + 1, 0);
+    for (size_t d = 0; d < n_sets; ++d) {
+        const long long cols = (long long)(sets[d].n_t * sets[d].n_nu);
+        col0[d + 1] = col0[d] + cols;
+        tile0[d + 1] = tile0[d] + (cols + QUANT_COLS - 1) / QUANT_COLS;
+    }
+    if (tile0[n_sets] > INT_MAX) return fail(VAG_ERR_INVALID, "too many (set, frequency, time) columns for one call");
+    const size_t n_out = n_q * (size_t)col0[n_sets];
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) {  // no set has members
+        std::fill(out, out + n_out, NAN);
+        std::fill(n_used, n_used + n_sets, 0);
+        return VAG_OK;
+    }
+    std::vector<int> c0(n_sets + 1, 0), cand(n_models);
+    for (size_t m = 0; m < n_models; ++m) ++c0[dataset_of[m] + 1];
+    int max_cand = 0;
+    for (size_t d = 0; d < n_sets; ++d) {
+        max_cand = std::max(max_cand, c0[d + 1]);
+        c0[d + 1] += c0[d];
+    }
+    {
+        std::vector<int> fill(c0.begin(), c0.end() - 1);
+        for (size_t m = 0; m < n_models; ++m) cand[fill[dataset_of[m]]++] = (int)m;
+    }
+    cudaStream_t s = ctx->stream;
+    Pack pk;
+    GridSets gs;
+    const size_t o_t = pk.put(t, n_t_total), o_nu = pk.put(nu, n_nu_total);
+    gs.put(pk, grid_table(sets, n_sets), dataset_of, n_models);
+    const size_t o_q = pk.put(q, n_q), o_cand = pk.put(cand), o_c0 = pk.put(c0), o_tile0 = pk.put(tile0),
+                 o_col0 = pk.put(col0), up = pk.h.size();
+    const size_t o_mem = up, o_used = o_mem + carve_sz<long long>(n_models), o_out = o_used + carve_sz<long long>(n_sets),
+                 end = o_out + carve_sz<double>(n_out);
+    void* base = nullptr;
+    if (int rc = grid_multi_run(ctx, caps, pk, o_t, n_t_total, o_nu, n_nu_total, gs, end - up, &base, s)) return rc;
+    const int launches = ctx->launches;
+    long long* d_used = at<long long>(base, o_used);
+    double* d_out = at<double>(base, o_out);
+    k_quant_members<<<(unsigned)n_sets, 256, 0, s>>>(at<int>(base, o_cand), at<int>(base, o_c0),
+                                                     static_cast<int32_t*>(ctx->io_status.p), gs.sd.out_off,
+                                                     at<long long>(base, o_mem), d_used);
+    // members staged in shared memory up to the budget; a larger set selects from global memory
+    const int rows_cap = (int)std::min<size_t>((size_t)max_cand, QUANT_SMEM_BUDGET / (QUANT_COLS * sizeof(uint64_t)));
+    k_quantiles<<<(unsigned)tile0[n_sets], QUANT_COLS * 32, (size_t)rows_cap * QUANT_COLS * sizeof(uint64_t), s>>>(
+        static_cast<double*>(ctx->io_out.p), at<long long>(base, o_mem), at<int>(base, o_c0), d_used,
+        at<long long>(base, o_tile0), at<long long>(base, o_col0), (int)n_sets, at<double>(base, o_q), (int)n_q, rows_cap,
+        d_out);
+    CK(cudaGetLastError());
+    ctx->launches = launches + 2;
+    CK(cudaMemcpyAsync(out, d_out, sizeof(double) * n_out, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(n_used, d_used, sizeof(int64_t) * n_sets, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;

@@ -298,6 +298,70 @@ class Engine:
                                                   st.ctypes.data))
         return (out, st) if return_status else out
 
+    # ---- a (t x nu) grid per model, and quantiles across models (vag_flux_density_grid_multi, vag_flux_quantiles_multi) --
+    @staticmethod
+    def _grid_sets(grids):
+        """``grids`` = [(t, nu), ...] -> (times and frequencies concatenated over the grids, ``abi.GridSet`` array,
+        int64[n_grids, 2] of (n_nu, n_t))."""
+        if not len(grids):
+            raise ValueError("no grids")
+        ts, nus = [], []
+        sets = (abi.GridSet * len(grids))()
+        shape = np.zeros((len(grids), 2), dtype=np.int64)
+        t0 = nu0 = 0
+        for d, g in enumerate(grids):
+            if len(g) != 2:
+                raise ValueError(f"grid {d} must be (t, nu)")
+            t, nu = _f64(g[0]).reshape(-1), _f64(g[1]).reshape(-1)
+            sets[d] = abi.GridSet(t0, t.size, nu0, nu.size)
+            shape[d] = nu.size, t.size
+            ts.append(t)
+            nus.append(nu)
+            t0, nu0 = t0 + t.size, nu0 + nu.size
+        return np.concatenate(ts), np.concatenate(nus), sets, shape
+
+    def flux_density_grid_multi(self, params, grids, dataset_of, return_status=False):
+        """``flux_density_grid`` of model m on its own grid ``grids[dataset_of[m]]`` = (t, nu), t ascending, all in one
+        batch.  Returns a list with one float64[5, n_nu, n_t] array per model; the arrays are views into one buffer in
+        model order (``vag_flux_density_grid_multi``)."""
+        p = self._params(params)
+        t, nu, sets, shape = self._grid_sets(grids)
+        ds = self._dataset_of(dataset_of, p.size)
+        in_range = p.size and ds.min() >= 0 and ds.max() < len(grids)
+        shp = shape[ds] if in_range else np.zeros((p.size, 2), dtype=np.int64)  # (else the call raises)
+        off = np.concatenate([[0], np.cumsum(shp[:, 0] * shp[:, 1])]).astype(np.int64)
+        buf = np.empty(abi.NCOMP * int(off[-1]))
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_flux_density_grid_multi(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p),
+                                                         len(sets), t.ctypes.data, t.size, nu.ctypes.data, nu.size,
+                                                         buf.ctypes.data, st.ctypes.data))
+        out = [buf[abi.NCOMP * off[m]:abi.NCOMP * off[m + 1]].reshape(abi.NCOMP, int(shp[m, 0]), int(shp[m, 1]))
+               for m in range(p.size)]
+        return (out, st) if return_status else out
+
+    def flux_quantiles_multi(self, params, grids, dataset_of, q, return_status=False):
+        """Posterior-predictive bands of many fits in one call: for every grid d, ``numpy.quantile`` of the ``total`` flux
+        of the models with ``dataset_of == d`` on ``grids[d]`` = (t, nu), at every ``q`` (method "linear"), computed on
+        the GPU where the flux is (``vag_flux_quantiles_multi``).  Models whose ODE failed (``abi.ST_ODE_FAIL500``) or
+        whose grid exceeded the capacity (``abi.ST_CAPACITY``) are left out.  Returns (a list with one
+        float64[n_q, n_nu, n_t] array per grid, int64 n_used[n_grids]: the models each grid's quantiles are over)."""
+        p = self._params(params)
+        t, nu, sets, shape = self._grid_sets(grids)
+        ds = self._dataset_of(dataset_of, p.size)
+        qs = _f64(q).reshape(-1)
+        cols = shape[:, 0] * shape[:, 1]
+        off = np.concatenate([[0], np.cumsum(cols)]).astype(np.int64)
+        buf = np.empty(qs.size * int(off[-1]))
+        n_used = np.zeros(len(grids), dtype=np.int64)
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_flux_quantiles_multi(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p),
+                                                      len(sets), t.ctypes.data, t.size, nu.ctypes.data, nu.size,
+                                                      qs.ctypes.data, qs.size, buf.ctypes.data, n_used.ctypes.data,
+                                                      st.ctypes.data))
+        bands = [buf[qs.size * off[d]:qs.size * off[d + 1]].reshape(qs.size, int(shape[d, 0]), int(shape[d, 1]))
+                 for d in range(len(grids))]
+        return (bands, n_used, st) if return_status else (bands, n_used)
+
     @staticmethod
     def valid_mask(params):
         """bool[n]: which parameter sets pass the constructor checks of the reference (vag_params_validate_batch)."""

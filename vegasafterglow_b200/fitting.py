@@ -188,6 +188,19 @@ class BatchedLikelihood:
         idx = self._in_bounds(samples)
         return self._log_prob(samples, idx, self.chi2(samples[idx]) if idx.size else np.zeros(0))
 
+    def flux_quantiles(self, samples: np.ndarray, t, nu, q=(0.16, 0.5, 0.84)):
+        """Posterior-predictive band of this fit: ``numpy.quantile`` over the posterior draws ``samples[n, ndim]`` of the
+        model's total flux density on the grid (t ascending, nu) at every ``q`` -> (float64[n_q, n_nu, n_t], the number of
+        draws used).  Draws the constructors reject are dropped, and so are draws whose ODE failed; bounds are not
+        applied (these are posterior draws), and ``A_V`` plays no part (it shifts the data, not the model).  One
+        ``Engine.flux_quantiles_multi`` call with one grid."""
+        from .engine import Engine
+
+        P = self.to_params(samples)
+        P = P[Engine.valid_mask(P)]
+        bands, n_used = self.engine.flux_quantiles_multi(P, [(t, nu)], np.zeros(P.size, dtype=np.int32), q)
+        return bands[0], int(n_used[0])
+
 
 _CUDA_STREAM_LEGACY = 0x1  # cudaStreamLegacy (driver_types.h)
 
@@ -379,6 +392,18 @@ class LikelihoodStack:
     def _engine_chi2(self, P, dataset_of, extinction):
         """chi2 of the stacked walkers in one engine call: ``chi2_multi`` here, ``chi2_multi_bands`` with bands."""
         return self.engine.chi2_multi(P, self.datasets, dataset_of, extinction=extinction)
+
+    def flux_quantiles(self, samples, grids, q=(0.16, 0.5, 0.84)):
+        """Posterior-predictive bands of the K fits in ONE ``Engine.flux_quantiles_multi`` call: fit k's draws
+        ``samples[k]`` (through its own ``to_params``) on its own grid ``grids[k]`` = (t ascending, nu).  Returns (a list
+        of K float64[n_q, n_nu, n_t] arrays, ``numpy.quantile`` of the total flux over the fit's draws at every ``q``;
+        int64[K] draws used per fit).  Draws the constructors reject (``Engine.valid_mask``) are dropped, and so are
+        draws whose ODE failed; bounds are not applied (these are posterior draws), and ``A_V`` plays no part (it shifts
+        the data, not the model).  Nothing is distributed: quantiles do not decompose over ranks."""
+        if len(samples) != len(self.likelihoods) or len(grids) != len(self.likelihoods):
+            raise ValueError(f"{len(samples)} sample arrays and {len(grids)} grids for {len(self.likelihoods)} likelihoods")
+        P, ds, _, _ = self._walkers(samples)
+        return self.engine.flux_quantiles_multi(P, grids, ds, q)
 
     def __call__(self, samples):
         if len(samples) != len(self.likelihoods):
