@@ -148,6 +148,19 @@ int vag_flux_density_grid(vag_context* ctx, const vag_params* params, size_t n_m
 int vag_flux_density_series(vag_context* ctx, const vag_params* params, size_t n_models, const double* t,
                             const double* nu, size_t n, double* out, int32_t* status);
 
+/* Replaces PyModel::flux_density_exposures (pybind/pymodel.cpp:412-496): point i is the average over its exposure
+ * expo_time[i] > 0 of num_points samples t[i] + j dt, dt = expo_time[i] / (num_points - 1), j = 0 .. num_points-1 (product
+ * and sum rounded separately).  t need not be sorted.  All n * num_points samples are sorted stably by time (ties: point
+ * index, then j) and run as ONE shared series request -- exactly vag_flux_density_series on them, with its series modes
+ * and output modes -- and a kernel averages on the device: a point's samples added to 0.0 in sorted order, divided by
+ * num_points.  Only out[n_models][VAG_NCOMP][n] crosses PCIe.  The result equals that series call followed by that host
+ * averaging bit for bit.  status as vag_flux_density_series.  Launches: those of vag_flux_density_series on the samples
+ * + 1.  Checks, all before any work is enqueued, in this order and with the messages of the reference's: num_points >= 2,
+ * every expo_time[i] finite and > 0, n > 0, t and nu finite and > 0; n * num_points within a 32-bit int. */
+int vag_flux_density_exposures(vag_context* ctx, const vag_params* params, size_t n_models, const double* t,
+                               const double* nu, const double* expo_time, size_t n, size_t num_points, double* out,
+                               int32_t* status);
+
 /* Replaces PyModel::flux (pybind/pymodel.cpp:391-410) = Observer::flux (src/core/observer.h:555-567):
  * flux integrated over [nu_min, nu_max] Hz with Boole weights on num_nu log-spaced frequencies
  * (src/core/quadrature.h:138-191).  out[n_models][VAG_NCOMP][n_t] in erg cm^-2 s^-1. */
@@ -272,6 +285,26 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
                          const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
                          const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
                          const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status);
+
+/* vag_chi2_multi_bands with exposure-averaged points.  expo_time[n_points_total] (point order, each finite and >= 0) and
+ * num_expo[n_sets] (>= 2 for every set with a point whose expo_time > 0; not read otherwise).  A point with e = expo_time
+ * > 0 of set d is the average of num_expo[d] samples over its exposure, by the rule of vag_flux_density_exposures; a point
+ * with e = 0 is one sample at its time (its value is that sample's flux exactly).  The series request of set d is all its
+ * samples, sorted stably by time (ties: point index, then j); that window also sets the set's grid.  The chi-squared rule
+ * is unchanged: w ((lnF_obs + A_V ext_k - ln max(F_avg, 1e-300)) / sigma_ln)^2, and so are the band terms, the status OR,
+ * VAG_ST_ODE_FAIL500 -> +inf, the passes of 32768 models and the series modes (applied to the sets of samples).  With
+ * every expo_time = 0 the result equals vag_chi2_multi_bands bit for bit.  The point pass runs the samples without the
+ * fused chi-squared, then one launch averages them (a CTA per point model) and one k_chi2 compares the averages with the
+ * points' data.  Launches, when the point models fit one pass of 32768: those of vag_chi2_multi_bands on the sets of
+ * samples + 1.  Checks, all before any work is enqueued (messages name the data set or the point; a failed call leaves
+ * the context usable): those of vag_chi2_multi_bands, then expo_time and num_expo, every sample time finite, and the
+ * samples of all sets within a 32-bit int.  Not provided: exposures on band data, a device-buffer (_dev) form. */
+int vag_chi2_multi_bands_exposures(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                   const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu,
+                                   const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k,
+                                   size_t n_points_total, const double* A_V, const double* expo_time,
+                                   const int32_t* num_expo, const vag_band_obs* bands, size_t n_bands_total, double* chi2,
+                                   int32_t* status);
 
 /* ---- a (t x nu) grid request per model, and posterior-predictive bands across models ------------------------------
  * The times and frequencies of all grid sets are concatenated into t[n_t_total] and nu[n_nu_total]; set d is the times

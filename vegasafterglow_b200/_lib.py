@@ -37,6 +37,7 @@ def load():
     lib.vag_params_default.argtypes = [vp]
     lib.vag_flux_density_grid.argtypes = [vp, vp, sz, dp, sz, dp, sz, dp, ip]
     lib.vag_flux_density_series.argtypes = [vp, vp, sz, dp, dp, sz, dp, ip]
+    lib.vag_flux_density_exposures.argtypes = [vp, vp, sz, dp, dp, dp, sz, sz, dp, ip]
     lib.vag_flux_band.argtypes = [vp, vp, sz, dp, sz, C.c_double, C.c_double, sz, dp, ip]
     lib.vag_chi2_series.argtypes = [vp, vp, sz, dp, dp, dp, dp, dp, sz, dp, ip]
     lib.vag_flux_density_grid_dev.argtypes = [vp, vp, sz, dp, sz, dp, sz, dp, ip, vp]
@@ -60,6 +61,8 @@ def load():
     lib.vag_chi2_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, dp, ip]
     lib.vag_flux_band_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, ip]
     lib.vag_chi2_multi_bands.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, vp, sz, dp, ip]
+    lib.vag_chi2_multi_bands_exposures.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, dp, ip, vp, sz,
+                                                   dp, ip]
     lib.vag_chi2_multi_bands_dev.argtypes = [vp, vp, sz, ip, vp, sz, dp, dp, dp, dp, dp, dp, sz, dp, vp, sz, dp, ip, vp]
     lib.vag_flux_density_grid_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, sz, dp, sz, dp, ip]
     lib.vag_flux_quantiles_multi.argtypes = [vp, vp, sz, ip, vp, sz, dp, sz, dp, sz, dp, sz, dp, vp, ip]
@@ -82,7 +85,8 @@ EXPORTS = [
     "vag_set_profiling", "vag_set_output_mode", "vag_last_stage_ms", "vag_last_launch_count", "vag_measure_fp64_peak", "vag_selftest_libm", "vag_chi2", "vag_params_validate_batch", "vag_debug_set_ode_limits", "vag_last_total_alias", "vag_last_work", "vag_set_series_mode", "vag_details_ic",
     "vag_set_grid_lanes", "vag_chi2_ext", "vag_params_validate_batch_dev", "vag_flux_band_dev", "vag_chi2_dev",
     "vag_flux_density_series_multi", "vag_chi2_multi", "vag_flux_band_multi", "vag_chi2_multi_bands",
-    "vag_chi2_multi_bands_dev", "vag_flux_density_grid_multi", "vag_flux_quantiles_multi",
+    "vag_chi2_multi_bands_dev", "vag_flux_density_grid_multi", "vag_flux_quantiles_multi", "vag_flux_density_exposures",
+    "vag_chi2_multi_bands_exposures",
 ]
 
 

@@ -26,6 +26,7 @@
 #include "vag_libm.cuh"
 #include "vag_pipeline.cuh"
 #include "vag_quantile.cuh"
+#include "vag_exposure.cuh"
 
 using namespace vag;
 
@@ -46,7 +47,8 @@ static_assert(sizeof(vag_params) == 320, "vag_params layout must match vegasafte
 struct SeriesSet {
     int off, n;  // slice of the concatenated points (grid request: of the concatenated times)
     int n_nu;    // series: distinct frequencies of the slice (k_series_bands_sets); grid: frequency nodes of the slice
-    int nu_off;  // grid: first node of the slice in the concatenated nodes
+    int nu_off;  // grid: first node of the slice in the concatenated nodes; the points of an exposure-averaged series
+                 // request (k_expo_average): the slice's first point in the sample plan
 };
 struct SetsDev {
     const int* set_of;         // [models of the pass] data set of each model
@@ -916,6 +918,34 @@ __global__ void __launch_bounds__(QUANT_COLS * 32) k_quantiles(const double* __r
     }
 }
 
+// ---- exposure averages (vag_flux_density_exposures, vag_chi2_multi_bands_exposures) -------------------------------
+// CTA / model, a thread / (component, point): out[c][i] = expo_mean of point i's samples in F (vag_exposure.cuh).  Shared
+// request: model m's samples are F[m][VAG_NCOMP][n_s], its points out[m][VAG_NCOMP][n], point i's samples at
+// pos[s0[i] .. s0[i + 1]).  RAGGED: model m's samples are its block of the ragged sample request (sx: the sets of samples),
+// its points its block of the ragged point output (sd: the sets of points, whose nu_off is the set's first point in s0).
+template <bool RAGGED>
+__global__ void __launch_bounds__(128) k_expo_average(const double* __restrict__ F, int n_s, int n, const int* __restrict__ s0,
+                                                      const int* __restrict__ pos, double* __restrict__ out, SetsDev sx,
+                                                      SetsDev sd) {
+    const int mi = blockIdx.x;
+    const double* f = F + (size_t)mi * VAG_NCOMP * n_s;
+    double* o = out + (size_t)mi * VAG_NCOMP * n;
+    if constexpr (RAGGED) {
+        const int d = sd.set_of[mi];
+        const SeriesSet S = sd.sets[d];
+        n_s = sx.sets[d].n;
+        n = S.n;
+        s0 += S.nu_off;
+        f = F + (size_t)(sx.out_off[mi] - sx.out_off[0]) * VAG_NCOMP;
+        o = out + (size_t)(sd.out_off[mi] - sd.out_off[0]) * VAG_NCOMP;
+    }
+    for (int q = threadIdx.x; q < VAG_NCOMP * n; q += blockDim.x) {
+        const int c = q / n, i = q - c * n;
+        const int a = s0[i];
+        o[q] = expo_mean(f + (size_t)c * n_s, pos + a, s0[i + 1] - a);
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -1771,12 +1801,13 @@ int vag_chi2_series_dev(vag_context* ctx, const vag_params* d_params, size_t n_m
 }
 
 // ---- host-buffer entry points --------------------------------------------------------------------
-// device -> host transfer of out[n_models][VAG_NCOMP][comp_sz] under the context's output mode
+// device -> host transfer of out[n_models][VAG_NCOMP][comp_sz] from src (NULL: io_out) under the context's output mode
 static int copy_out(vag_context* ctx, const vag_params* params, size_t n_models, size_t comp_sz, double* out,
-                    cudaStream_t s) {
+                    cudaStream_t s, const double* src_dev = nullptr) {
+    if (!src_dev) src_dev = static_cast<const double*>(ctx->io_out.p);
     const size_t row = sizeof(double) * comp_sz, pitch = row * VAG_NCOMP;
     if (ctx->out_mode == VAG_OUT_DENSE) {
-        CK(cudaMemcpyAsync(out, ctx->io_out.p, pitch * n_models, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(out, src_dev, pitch * n_models, cudaMemcpyDeviceToHost, s));
         return VAG_OK;
     }
     bool present[VAG_NCOMP] = {true, true, false, false, false};
@@ -1801,7 +1832,7 @@ static int copy_out(vag_context* ctx, const vag_params* params, size_t n_models,
             ctx->total_alias = which;
         }
     }
-    const char* src = static_cast<const char*>(ctx->io_out.p);
+    const char* src = reinterpret_cast<const char*>(src_dev);
     char* dst = reinterpret_cast<char*>(out);
     for (int c = 0; c < VAG_NCOMP;) {
         if (!present[c]) {
@@ -1844,6 +1875,53 @@ int vag_flux_density_grid(vag_context* ctx, const vag_params* params, size_t n_m
 int vag_flux_density_series(vag_context* ctx, const vag_params* params, size_t n_models, const double* t,
                             const double* nu, size_t n, double* out, int32_t* status) {
     return flux_host(ctx, params, n_models, true, t, n, nu, n, out, status);
+}
+
+// Model.flux_density_exposures (pybind/pymodel.cpp:412-496): the samples of every point (vag_exposure.cuh) as one
+// shared series request, then k_expo_average; only the averages cross PCIe.  Checks first, in the mirror's order.
+int vag_flux_density_exposures(vag_context* ctx, const vag_params* params, size_t n_models, const double* t,
+                               const double* nu, const double* expo_time, size_t n, size_t num_points, double* out,
+                               int32_t* status) {
+    if (!ctx || !out || (n && (!t || !nu || !expo_time))) return fail(VAG_ERR_INVALID, "NULL argument");
+    if (num_points < 2) return fail(VAG_ERR_INVALID, "num_points must be at least 2 to sample within each exposure time");
+    for (size_t i = 0; i < n; ++i)
+        if (!(std::isfinite(expo_time[i]) && expo_time[i] > 0))
+            return fail(VAG_ERR_INVALID, "expo_time[" + std::to_string(i) + "] must be finite and > 0, got " +
+                                             std::to_string(expo_time[i]));
+    if (n == 0) return fail(VAG_ERR_INVALID, "time array must be non-empty");
+    if (num_points > (size_t)INT_MAX / n) return fail(VAG_ERR_INVALID, "n * num_points samples must fit in a 32-bit int");
+    for (size_t i = 0; i < n; ++i)
+        if (!finite_pos(t[i])) return fail(VAG_ERR_INVALID, "observation times must be finite and > 0");
+    for (size_t i = 0; i < n; ++i)
+        if (!finite_pos(nu[i])) return fail(VAG_ERR_INVALID, "observation frequencies must be finite and > 0");
+    ExpoPlan P;
+    expo_plan_append(t, nu, expo_time, n, (int)num_points, P);
+    const size_t n_s = P.t.size();
+    if (int rc = check_times(P.t.data(), n_s)) return rc;  // a sample time that overflowed
+    Caps caps;
+    if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
+    if (n_models == 0) return VAG_OK;
+    cudaStream_t s = ctx->stream;
+    if (int rc = upload_request(ctx, P.t.data(), n_s, P.nu.data(), n_s)) return rc;
+    Pack pk;
+    const size_t o_s0 = pk.put(P.s0), o_pos = pk.put(P.pos);
+    CK(ctx->io_sets.ensure(pk.h.size()));
+    CK(cudaMemcpyAsync(ctx->io_sets.p, pk.h.data(), pk.h.size(), cudaMemcpyHostToDevice, s));
+    CK(ctx->io_out.ensure(sizeof(double) * n_models * VAG_NCOMP * (n_s + n)));
+    double* d_samples = static_cast<double*>(ctx->io_out.p);
+    double* d_avg = d_samples + n_models * VAG_NCOMP * n_s;
+    const Request rq{true, static_cast<double*>(ctx->io_t.p), static_cast<double*>(ctx->io_nu.p), n_s, n_s};
+    if (int rc = run_flux(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, caps, rq, d_samples,
+                          static_cast<int32_t*>(ctx->io_status.p), nullptr, s))
+        return rc;
+    k_expo_average<false><<<(unsigned)n_models, 128, 0, s>>>(d_samples, (int)n_s, (int)n, at<int>(ctx->io_sets.p, o_s0),
+                                                             at<int>(ctx->io_sets.p, o_pos), d_avg, SetsDev{}, SetsDev{});
+    ctx->launches++;
+    CK(cudaGetLastError());
+    if (int rc = copy_out(ctx, params, n_models, n, out, s, d_avg)) return rc;
+    if (status) CK(cudaMemcpyAsync(status, ctx->io_status.p, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return VAG_OK;
 }
 
 // Frequency grid (code units) and quadrature weights of PyModel::flux (pybind/pymodel.cpp:391-410): xt::logspace of the
@@ -2594,28 +2672,69 @@ static int check_multi_count(size_t n_models, const int32_t* dataset_of, const v
     return VAG_OK;
 }
 
+// The exposures of vag_chi2_multi_bands_exposures (checked): the samples of every set with points, in L.pt_sets' order
+// (vag_exposure.cuh, with the set's num_expo), whose nu_off becomes the set's first point in the plan; the point pass's
+// sets of samples and its models' blocks of samples.
+struct MultiExpo {
+    ExpoPlan plan;
+    std::vector<SeriesSet> sets;    // [sets with points] slices of the concatenated samples
+    std::vector<long long> off{0};  // [n_pt + 1] first sample of each point model's block
+    size_t max_set = 0;
+};
+static void multi_expo(const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* expo_time,
+                       const int32_t* num_expo, MultiLists& L, MultiExpo& X) {
+    for (size_t d = 0, q = 0; d < n_sets; ++d) {
+        const vag_multi_set& S = sets[d];
+        if (!S.n) continue;
+        const size_t first = X.plan.t.size();
+        L.pt_sets[q++].nu_off = (int)(X.plan.s0.size() - 1);
+        expo_plan_append(t + S.offset, nu + S.offset, expo_time + S.offset, S.n, num_expo[d], X.plan);
+        X.sets.push_back(SeriesSet{(int)first, (int)(X.plan.t.size() - first), 0, 0});
+        X.max_set = std::max(X.max_set, X.plan.t.size() - first);
+    }
+    for (size_t i = 0; i < L.n_pt; ++i) X.off.push_back(X.off.back() + X.sets[L.pt_set_of[i]].n);
+}
+
 // L's tables and the intermediate results on the device
 struct MultiDev {
     const int *pt_of, *e0;
     SetsDev pt_sd;              // the point pass: its models' data sets, the sets, the output offsets
     double* chi2_pts;           // [n_pt]
     int32_t *st_pts, *st_eval;  // [n_pt], [n_eval]
+    SetsDev pt_sx;              // with exposures: the point pass over the samples (pt_sd: its averages)
+    const int *s0, *pos;        // with exposures: the plan (MultiExpo)
 };
 
 // Steps 1, 2 (with 3) and 4 below on the records d_rec gathered for L (the point models', then the evaluations'): the point
 // pass on pts (pts.av: the A_V of each point model), the band pass (device: its data are device pointers), and
-// k_chi2_bands over all n_models.  *launches: the launches of the three.
+// k_chi2_bands over all n_models.  With exposures X, the point pass runs on the samples (pts.t / pts.nu), k_expo_average
+// averages them and k_chi2 compares the averages with the points' data.  *launches: the launches of the three.
 static int multi_passes(vag_context* ctx, const vag_params* d_rec, const MultiLists& L, Caps caps, const Chi2Points& pts,
                         const MultiDev& tb, const vag_band_obs* bands, size_t n_bands, const std::vector<BandGrid>& grids,
-                        bool device, size_t n_models, double* d_chi2, int32_t* d_status, cudaStream_t s, int* launches) {
+                        bool device, size_t n_models, double* d_chi2, int32_t* d_status, cudaStream_t s, int* launches,
+                        const MultiExpo* X = nullptr) {
     *launches = 0;
-    if (L.n_pt) {
+    if (L.n_pt && !X) {
         CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (size_t)L.pt_off[L.n_pt]));
         if (int rc = run_flux(ctx, d_rec, L.n_pt, caps, points_request(pts, &tb.pt_sd, L.pt_off.data(), L.pt_sets.size(),
                                                                        L.max_set),
                               static_cast<double*>(ctx->io_out.p), tb.st_pts, tb.chi2_pts, s))
             return rc;
         *launches += ctx->launches;
+    } else if (L.n_pt) {
+        const size_t n_samples = (size_t)X->off[L.n_pt];
+        CK(ctx->io_out.ensure(sizeof(double) * VAG_NCOMP * (n_samples + (size_t)L.pt_off[L.n_pt])));
+        double* d_samples = static_cast<double*>(ctx->io_out.p);
+        double* d_avg = d_samples + VAG_NCOMP * n_samples;
+        const Chi2Points flux{pts.t, pts.nu, nullptr, nullptr, nullptr, nullptr, nullptr, X->plan.t.size()};
+        if (int rc = run_flux(ctx, d_rec, L.n_pt, caps, points_request(flux, &tb.pt_sx, X->off.data(), X->sets.size(),
+                                                                       X->max_set),
+                              d_samples, tb.st_pts, nullptr, s))
+            return rc;
+        k_expo_average<true><<<(unsigned)L.n_pt, 128, 0, s>>>(d_samples, 0, 0, tb.s0, tb.pos, d_avg, tb.pt_sx, tb.pt_sd);
+        k_chi2<true><<<(unsigned)((L.n_pt * 32 + 127) / 128), 128, 0, s>>>(d_avg, L.n_pt, 0, pts.lnF, pts.sig, pts.w, pts.av,
+                                                                           pts.ext, tb.chi2_pts, tb.st_pts, 0, tb.pt_sd);
+        *launches += ctx->launches + 2;
     }
     BandPass bp{};
     if (L.n_eval) {
@@ -2636,17 +2755,27 @@ static int multi_passes(vag_context* ctx, const vag_params* d_rec, const MultiLi
 // the device: one upload of the lists and the point pass's tables -- and, from host memory (`host`), of the points pts and
 // A_V[n_models] -- then room for the gathered records, the point models' A_V and the results.  k_gather_params_av gathers
 // the records of both lists and the A_V, and multi_passes runs steps 1 to 4.  chi2 / status [n_models]: device outputs,
-// or NULL to place them in io_sets.  *launches: k_gather_params_av's and multi_passes'.
+// or NULL to place them in io_sets.  With exposures X (host only) the uploaded t / nu are X's samples, with X's tables.
+// *launches: k_gather_params_av's and multi_passes'.
 static int multi_chi2(vag_context* ctx, const vag_params* d_params, size_t n_models, const MultiLists& L, Caps caps,
                       Chi2Points pts, const double* A_V, bool host, const vag_band_obs* bands, size_t n_bands,
-                      const std::vector<BandGrid>& grids, double*& chi2, int32_t*& status, cudaStream_t s, int* launches) {
+                      const std::vector<BandGrid>& grids, double*& chi2, int32_t*& status, cudaStream_t s, int* launches,
+                      const MultiExpo* X = nullptr) {
     const size_t n_pt = L.n_pt, n_eval = L.n_eval, n_up = host && n_pt ? pts.n : 0, n_av = A_V ? n_pt : 0;
+    const size_t n_tnu = X ? (n_up ? X->plan.t.size() : 0) : n_up;
     Pack pk;
     const size_t o_gather = pk.put(L.gather), o_pt_of = pk.put(L.pt_of), o_e0 = pk.put(L.e0), o_sets = pk.put(L.pt_sets),
-                 o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off), o_t = pk.put(pts.t, n_up),
-                 o_nu = pk.put(pts.nu, n_up), o_lnF = pk.put(pts.lnF, n_up), o_sig = pk.put(pts.sig, n_up),
-                 o_w = pk.put(pts.w, n_up), o_ext = pk.put(pts.ext, pts.ext ? n_up : 0),
-                 o_A_V = pk.put(A_V, host && A_V ? n_models : 0);
+                 o_set_of = pk.put(L.pt_set_of), o_off = pk.put(L.pt_off),
+                 o_t = pk.put(X ? X->plan.t.data() : pts.t, n_tnu), o_nu = pk.put(X ? X->plan.nu.data() : pts.nu, n_tnu),
+                 o_lnF = pk.put(pts.lnF, n_up), o_sig = pk.put(pts.sig, n_up), o_w = pk.put(pts.w, n_up),
+                 o_ext = pk.put(pts.ext, pts.ext ? n_up : 0), o_A_V = pk.put(A_V, host && A_V ? n_models : 0);
+    size_t o_sx = 0, o_offx = 0, o_s0 = 0, o_pos = 0;
+    if (X) {
+        o_sx = pk.put(X->sets);
+        o_offx = pk.put(X->off);
+        o_s0 = pk.put(X->plan.s0);
+        o_pos = pk.put(X->plan.pos);
+    }
     const size_t up = pk.h.size(), o_rec = up, o_av = o_rec + carve_sz<vag_params>(n_pt + n_eval),
                  o_chi2_pts = o_av + carve_sz<double>(n_av), o_st_pts = o_chi2_pts + carve_sz<double>(n_pt),
                  o_st_eval = o_st_pts + carve_sz<int>(n_pt), o_chi2 = o_st_eval + carve_sz<int>(n_eval),
@@ -2664,22 +2793,62 @@ static int multi_chi2(vag_context* ctx, const vag_params* d_params, size_t n_mod
     vag_params* d_rec = at<vag_params>(base, o_rec);
     k_gather_params_av<<<(unsigned)((n_pt + n_eval + 127) / 128), 128, 0, s>>>(
         d_params, at<int>(base, o_gather), n_pt + n_eval, d_rec, host && A_V ? at<double>(base, o_A_V) : A_V, n_av, at<double>(base, o_av));
-    const MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
-                      SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
-                      at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval)};
-    if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands, grids, !host, n_models, chi2, status, s, launches))
+    MultiDev tb{at<int>(base, o_pt_of), at<int>(base, o_e0),
+                SetsDev{at<int>(base, o_set_of), at<SeriesSet>(base, o_sets), at<long long>(base, o_off)},
+                at<double>(base, o_chi2_pts), at<int32_t>(base, o_st_pts), at<int32_t>(base, o_st_eval), SetsDev{},
+                nullptr, nullptr};
+    if (X) {
+        tb.pt_sx = SetsDev{tb.pt_sd.set_of, at<SeriesSet>(base, o_sx), at<long long>(base, o_offx)};
+        tb.s0 = at<int>(base, o_s0);
+        tb.pos = at<int>(base, o_pos);
+    }
+    if (int rc = multi_passes(ctx, d_rec, L, caps, pts, tb, bands, n_bands, grids, !host, n_models, chi2, status, s, launches,
+                              X))
         return rc;
     *launches += 1;  // k_gather_params_av
     return VAG_OK;
 }
 
+// The exposure checks of vag_chi2_multi_bands_exposures, after those of vag_chi2_multi_bands: every expo_time finite and
+// >= 0, num_expo >= 2 for every set with points of which one has an exposure, every sample time finite, the samples
+// within a 32-bit int
+static int check_multi_expo(const vag_multi_set* sets, size_t n_sets, const double* t, size_t n_points_total,
+                            const double* expo_time, const int32_t* num_expo) {
+    if (n_points_total && !expo_time) return fail(VAG_ERR_INVALID, "expo_time is NULL");
+    if (!num_expo) return fail(VAG_ERR_INVALID, "num_expo is NULL");
+    for (size_t i = 0; i < n_points_total; ++i)
+        if (!(std::isfinite(expo_time[i]) && expo_time[i] >= 0))
+            return fail(VAG_ERR_INVALID, "point " + std::to_string(i) + ": expo_time = " + std::to_string(expo_time[i]) +
+                                             " must be finite and >= 0");
+    size_t total = 0;
+    for (size_t d = 0; d < n_sets; ++d) {
+        const vag_multi_set& S = sets[d];
+        const std::string name = "data set " + std::to_string(d) + ": ";
+        size_t n_exp = 0;
+        for (size_t i = S.offset; i < S.offset + S.n; ++i) n_exp += expo_time[i] > 0;
+        if (n_exp && num_expo[d] < 2)
+            return fail(VAG_ERR_INVALID, name + "num_expo = " + std::to_string(num_expo[d]) +
+                                             " must be at least 2 (the set has exposures)");
+        for (size_t i = S.offset; i < S.offset + S.n; ++i) {  // the last sample, the latest of the point's
+            if (!(expo_time[i] > 0)) continue;
+            volatile double step = (double)(num_expo[d] - 1) * (expo_time[i] / (double)(num_expo[d] - 1));
+            if (!std::isfinite(t[i] + step))
+                return fail(VAG_ERR_INVALID, name + "point " + std::to_string(i) + ": its last sample time is not finite");
+        }
+        total += S.n + n_exp * (size_t)(n_exp ? num_expo[d] - 1 : 0);
+        if (total > (size_t)INT_MAX) return fail(VAG_ERR_INVALID, "the samples of all data sets must fit in a 32-bit int");
+    }
+    return VAG_OK;
+}
+
 // 1. the ragged point pass over the models whose set has points (vag_chi2_multi's, on those models and the sets with
-// points), 2. the band pass over every (model, band) evaluation, model-major, 3. its reduction, 4. k_chi2_bands, through
-// multi_chi2 on the records uploaded by prepare_params
-int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
-                         const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
-                         const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
-                         const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status) {
+// points; with exposures on their samples, then averaged), 2. the band pass over every (model, band) evaluation,
+// model-major, 3. its reduction, 4. k_chi2_bands, through multi_chi2 on the records uploaded by prepare_params
+static int multi_bands_host(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                            const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                            const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
+                            const double* A_V, bool exposures, const double* expo_time, const int32_t* num_expo,
+                            const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status) {
     if (!ctx || !chi2) return fail(VAG_ERR_INVALID, "NULL argument");
     if (n_bands_total && !bands) return fail(VAG_ERR_INVALID, "bands is NULL");
     if (int rc = check_points(n_points_total, t && nu && lnF_obs && sigma_ln && w, ext_k, A_V, false)) return rc;
@@ -2688,8 +2857,12 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
     if (int rc = check_bands(bands, n_bands_total, true, grids)) return rc;
     if (int rc = check_models(params, n_models)) return rc;
     if (int rc = check_multi_count(n_models, dataset_of, sets)) return rc;
+    if (exposures)
+        if (int rc = check_multi_expo(sets, n_sets, t, n_points_total, expo_time, num_expo)) return rc;
     MultiLists L;
     multi_lists(n_models, dataset_of, sets, n_sets, nullptr, L);
+    MultiExpo X;
+    if (exposures) multi_expo(sets, n_sets, t, nu, expo_time, num_expo, L, X);
     Caps caps;
     if (int rc = prepare_params(ctx, params, n_models, &caps)) return rc;
     if (n_models == 0) return VAG_OK;
@@ -2699,13 +2872,31 @@ int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_mo
     int launches = 0;
     if (int rc = multi_chi2(ctx, static_cast<vag_params*>(ctx->io_params.p), n_models, L, caps,
                             Chi2Points{t, nu, lnF_obs, sigma_ln, w, ext_k, nullptr, n_points_total}, A_V, true, bands,
-                            n_bands_total, grids, d_chi2, d_status, s, &launches))
+                            n_bands_total, grids, d_chi2, d_status, s, &launches, exposures ? &X : nullptr))
         return rc;
     ctx->launches = launches;
     CK(cudaMemcpyAsync(chi2, d_chi2, sizeof(double) * n_models, cudaMemcpyDeviceToHost, s));
     if (status) CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * n_models, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return VAG_OK;
+}
+
+int vag_chi2_multi_bands(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                         const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu, const double* lnF_obs,
+                         const double* sigma_ln, const double* w, const double* ext_k, size_t n_points_total,
+                         const double* A_V, const vag_band_obs* bands, size_t n_bands_total, double* chi2, int32_t* status) {
+    return multi_bands_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, lnF_obs, sigma_ln, w, ext_k,
+                            n_points_total, A_V, false, nullptr, nullptr, bands, n_bands_total, chi2, status);
+}
+
+int vag_chi2_multi_bands_exposures(vag_context* ctx, const vag_params* params, size_t n_models, const int32_t* dataset_of,
+                                   const vag_multi_set* sets, size_t n_sets, const double* t, const double* nu,
+                                   const double* lnF_obs, const double* sigma_ln, const double* w, const double* ext_k,
+                                   size_t n_points_total, const double* A_V, const double* expo_time,
+                                   const int32_t* num_expo, const vag_band_obs* bands, size_t n_bands_total, double* chi2,
+                                   int32_t* status) {
+    return multi_bands_host(ctx, params, n_models, dataset_of, sets, n_sets, t, nu, lnF_obs, sigma_ln, w, ext_k,
+                            n_points_total, A_V, true, expo_time, num_expo, bands, n_bands_total, chi2, status);
 }
 
 // ---- device-buffer entry points that plan on the device --------------------------------------------------------

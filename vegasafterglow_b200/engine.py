@@ -74,27 +74,18 @@ class Engine:
         return (out, st) if return_status else out
 
     def flux_density_exposures(self, params, t, nu, expo_time, num_points=10, return_status=False):
-        """Batched ``Model.flux_density_exposures`` (pybind/pymodel.cpp:412-496): each point is the
-        average of ``num_points`` samples spread over its exposure window (host-side sampling and
-        averaging exactly as the reference does; the series itself runs on the GPU)."""
+        """Batched ``Model.flux_density_exposures`` (pybind/pymodel.cpp:412-496) -> float64[n_models, 5, n]: each point
+        is the average of ``num_points`` samples spread over its exposure window, sampled, evaluated and averaged on the
+        GPU (``vag_flux_density_exposures``); t need not be sorted."""
+        p = self._params(params)
         t, nu, expo_time = (_f64(a).reshape(-1) for a in (t, nu, expo_time))
         if not (t.size == nu.size == expo_time.size):
             raise ValueError("time, frequency, and exposure time arrays must have the same size")
-        if num_points < 2:
-            raise ValueError("num_points must be at least 2 to sample within each exposure time")
-        if not np.all(np.isfinite(expo_time) & (expo_time > 0)):
-            bad = int(np.nonzero(~(np.isfinite(expo_time) & (expo_time > 0)))[0][0])
-            raise ValueError(f"expo_time[{bad}] must be finite and > 0, got {expo_time[bad]}")
-        k = np.arange(num_points, dtype=np.float64)
-        ts = (t[:, None] + k[None, :] * (expo_time / (num_points - 1))[:, None]).reshape(-1)
-        nus = np.repeat(nu, num_points)
-        idx = np.repeat(np.arange(t.size), num_points)
-        order = np.argsort(ts, kind="stable")
-        res = self.flux_density_series(params, ts[order], nus[order], return_status=True)
-        f, st = res
-        out = np.zeros((f.shape[0], abi.NCOMP, t.size))
-        np.add.at(out, (slice(None), slice(None), idx[order]), f)
-        out /= float(num_points)
+        out = (np.zeros if getattr(self, "_present_only", False) else np.empty)((p.size, abi.NCOMP, t.size))
+        st = np.zeros(p.size, dtype=np.int32)
+        _lib.check(self._lib.vag_flux_density_exposures(self._h, p.ctypes.data, p.size, t.ctypes.data, nu.ctypes.data,
+                                                        expo_time.ctypes.data, t.size, max(int(num_points), 0),
+                                                        out.ctypes.data, st.ctypes.data))
         return (out, st) if return_status else out
 
     def chi2_series(self, params, t, nu, lnF_obs, sigma_ln, w, return_status=False):
@@ -258,12 +249,15 @@ class Engine:
         out = [buf[abi.NCOMP * off[m]:abi.NCOMP * off[m + 1]].reshape(abi.NCOMP, int(n_m[m])) for m in range(p.size)]
         return (out, st) if return_status else out
 
-    def chi2_multi_bands(self, params, datasets, bands, dataset_of, extinction=None, return_status=False):
+    def chi2_multi_bands(self, params, datasets, bands, dataset_of, extinction=None, return_status=False, exposures=None):
         """``chi2`` of model m on its own data set, all in one batch -> chi2[n_models].  Data set d is its point data
         ``datasets[d]`` = (t, nu, lnF_obs, sigma_ln, w), t ascending, or None when it has none, and its band-integrated data
         ``bands[d]``, a list of ``fitting.band_obs`` dicts (may be empty when it has points).  ``extinction`` = (ext_k, A_V):
         ext_k a list with one array per data set (None for a set without points), A_V[n_models]; model m's points are then
-        compared as lnF_obs + A_V[m] * ext_k, its band terms unchanged (``vag_chi2_multi_bands``)."""
+        compared as lnF_obs + A_V[m] * ext_k, its band terms unchanged (``vag_chi2_multi_bands``).  ``exposures``: one
+        entry per data set, None or (expo_time, num_points) -- expo_time per point (>= 0, in the order of its points); a
+        point with expo_time > 0 is compared with the model averaged over num_points samples of its exposure, as
+        ``flux_density_exposures`` computes it (``vag_chi2_multi_bands_exposures``).  None everywhere: the call without."""
         p = self._params(params)
         if len(bands) != len(datasets):
             raise ValueError(f"{len(bands)} band lists for {len(datasets)} data sets")
@@ -288,15 +282,45 @@ class Engine:
             b0 += len(bands[d])
         ds = self._dataset_of(dataset_of, p.size)
         ext, av = self._extinction(extinction, n_pts, p.size)
+        expo = self._exposures(exposures, n_pts)
         out = np.empty(p.size)
         st = np.zeros(p.size, dtype=np.int32)
         pts = [a.ctypes.data if t.size else None for a in (t, nu, lnF, sig, w)]
-        _lib.check(self._lib.vag_chi2_multi_bands(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p),
-                                                  len(datasets), *pts, None if ext is None else ext.ctypes.data, t.size,
-                                                  None if av is None else av.ctypes.data,
-                                                  C.cast(arr, C.c_void_p) if flat else None, len(flat), out.ctypes.data,
-                                                  st.ctypes.data))
+        fn, expo_args = self._lib.vag_chi2_multi_bands, ()
+        if expo is not None:
+            fn, expo_args = self._lib.vag_chi2_multi_bands_exposures, (expo[0].ctypes.data if t.size else None,
+                                                                       expo[1].ctypes.data)
+        _lib.check(fn(self._h, p.ctypes.data, p.size, ds.ctypes.data, C.cast(sets, C.c_void_p), len(datasets), *pts,
+                      None if ext is None else ext.ctypes.data, t.size, None if av is None else av.ctypes.data, *expo_args,
+                      C.cast(arr, C.c_void_p) if flat else None, len(flat), out.ctypes.data, st.ctypes.data))
         return (out, st) if return_status else out
+
+    @staticmethod
+    def _exposures(exposures, sizes):
+        """``exposures`` of a batch of several data sets (one entry per set: None or (expo_time, num_points)) -> (expo_time
+        concatenated over the sets, 0 for a set without, int32 num_points[n_sets], 0 for a set without), or None when no
+        set has an entry."""
+        if exposures is None:
+            return None
+        if len(exposures) != len(sizes):
+            raise ValueError(f"exposures has {len(exposures)} entries for {len(sizes)} data sets")
+        if all(e is None for e in exposures):
+            return None
+        cols, num = [], np.zeros(len(sizes), dtype=np.int32)
+        for d, (e, n) in enumerate(zip(exposures, sizes)):
+            if e is None:
+                cols.append(np.zeros(int(n)))
+                continue
+            if len(e) != 2:
+                raise ValueError(f"data set {d}: exposures must be (expo_time, num_points) or None")
+            et, k = _f64(e[0]).reshape(-1), int(e[1])
+            if et.size != n:
+                raise ValueError(f"data set {d}: expo_time has {et.size} values for {n} points")
+            if not -2**31 <= k < 2**31:
+                raise ValueError(f"data set {d}: num_points = {k} must fit in a 32-bit int")
+            cols.append(et)
+            num[d] = k
+        return np.concatenate(cols), num
 
     # ---- a (t x nu) grid per model, and quantiles across models (vag_flux_density_grid_multi, vag_flux_quantiles_multi) --
     @staticmethod

@@ -59,9 +59,14 @@ def band_obs(t, flux, err, nu_min, nu_max, num_points=5, weights=None):
             "nu_min": float(nu_min), "nu_max": float(nu_max), "num_nu": int(num_points)}
 
 
-def _chi2_batch(engine, P, points, bands, ext_kernel=None, A_V=None):
+def _chi2_batch(engine, P, points, bands, ext_kernel=None, A_V=None, exposure=None):
     """chi2 of the records ``P`` in one engine call: ``chi2_series`` for points alone, ``chi2`` with bands, and
-    ``chi2(extinction=(ext_kernel, A_V))`` with a per-walker A_V.  The stored arrays are passed as they are."""
+    ``chi2(extinction=(ext_kernel, A_V))`` with a per-walker A_V.  With ``exposure`` = (expo_time, num_points), one
+    single-set ``chi2_multi_bands(exposures=...)``.  The stored arrays are passed as they are."""
+    if exposure is not None:
+        ext = None if A_V is None else ([ext_kernel], A_V)
+        return engine.chi2_multi_bands(P, [points], [bands], np.zeros(P.size, dtype=np.int32), extinction=ext,
+                                       exposures=[exposure])
     if A_V is not None:
         return engine.chi2(P, points, bands, extinction=(ext_kernel, A_V))
     if not bands:
@@ -69,7 +74,7 @@ def _chi2_batch(engine, P, points, bands, ext_kernel=None, A_V=None):
     return engine.chi2(P, points, bands)
 
 
-def _ensemble_chi2(engine, P, points, bands, ext_kernel=None, A_V=None, window=None):
+def _ensemble_chi2(engine, P, points, bands, ext_kernel=None, A_V=None, window=None, exposure=None):
     """chi2 of every record of ``P``; +inf for a record the model constructor rejects (the reference maps that exception
     to logL = -inf, samplers.py:63-70).  ``A_V`` (per walker) shifts the point data and is dropped without points.
     ``window``: None evaluates every walker here; else the ensemble is split over the ranks by the cost proxy over the
@@ -79,7 +84,10 @@ def _ensemble_chi2(engine, P, points, bands, ext_kernel=None, A_V=None, window=N
 
     ok = Engine.valid_mask(P)
     per_walker = (A_V,) if A_V is not None and points is not None else ()
-    evaluate = lambda Q, *av: _chi2_batch(engine, Q, points, bands, ext_kernel, *av)  # noqa: E731
+
+    def evaluate(Q, *av):
+        return _chi2_batch(engine, Q, points, bands, ext_kernel, av[0] if av else None, exposure)
+
     if window is not None:
         from . import parallel
 
@@ -101,12 +109,16 @@ class BatchedLikelihood:
     A name ``"A_V"`` fits host-galaxy extinction: ``ext_kernel`` (per point, in the caller's order) is the
     extinction law at each point, and a sample's point data are compared as ln F_obs + A_V * ext_kernel
     (``Engine.chi2(extinction=...)``).  Band data are not shifted.
+
+    ``expo_time`` (per point, in the caller's order, each >= 0) compares each point with an exposure with the model
+    averaged over ``expo_points`` samples of its exposure, the rule of ``Model.flux_density_exposures``; a point with 0
+    is compared with the model at its time (``Engine.chi2_multi_bands(exposures=...)``).  Band data have no exposures.
     """
 
     def __init__(self, engine, template, names: Sequence[str], log_scale: Sequence[bool], t, nu, flux, err,
                  weights=None, lower=None, upper=None, log_prior: Optional[Callable] = None,
                  log_likelihood_fn: Callable = lambda chi2: -0.5 * chi2, distributed: bool = False, bands=(),
-                 ext_kernel=None):
+                 ext_kernel=None, expo_time=None, expo_points=10):
         self.engine = engine
         self.template = np.ascontiguousarray(template, dtype=abi.PARAMS_DTYPE).reshape(-1)[:1].copy()
         self.names = list(names)
@@ -126,12 +138,25 @@ class BatchedLikelihood:
             if ext.size != self.t.size:
                 raise ValueError(f"ext_kernel has {ext.size} values for {self.t.size} points")
             self.ext_kernel = ext[time_order(t)]
+        self.expo_time, self.expo_points = None, int(expo_points)
+        if expo_time is not None:
+            e = np.asarray(expo_time, dtype=np.float64).reshape(-1)
+            if e.size != self.t.size or not self.t.size:
+                raise ValueError(f"expo_time has {e.size} values for {self.t.size} points")
+            if not np.all(np.isfinite(e) & (e >= 0)):
+                raise ValueError("expo_time must be finite and >= 0")
+            if np.any(e > 0) and self.expo_points < 2:
+                raise ValueError("expo_points must be at least 2 to sample within each exposure time")
+            self.expo_time = e[time_order(t)]
         # band-integrated data sets (Fitter.add_flux -> BandObs; fitter.py:525-531 evaluates Model.flux on each)
         self.bands = [band_obs(**b) for b in bands]
         if not self.t.size and not self.bands:
             raise ValueError("no data")
         # the times of the distributed split's cost proxy: the points', or every band's without points
         self._cost_times = self.t if self.t.size else np.concatenate([b["t"] for b in self.bands])
+        if self.expo_time is not None:  # and the last sample of each exposure (vag_exposure.cuh)
+            k = max(self.expo_points - 1, 1)
+            self._cost_times = np.concatenate([self.t, self.t + k * (self.expo_time / k)])
         self.lower = None if lower is None else np.asarray(lower, dtype=np.float64)
         self.upper = None if upper is None else np.asarray(upper, dtype=np.float64)
         self.log_prior = log_prior
@@ -161,7 +186,11 @@ class BatchedLikelihood:
         pts = (self.t, self.nu, self.lnF, self.sig, self.w) if self.t.size else None
         A_V = self._column(samples, self.names.index("A_V")) if "A_V" in self.names else None
         return _ensemble_chi2(self.engine, self.to_params(samples), pts, self.bands, self.ext_kernel, A_V,
-                              self._cost_times if self.distributed else None)
+                              self._cost_times if self.distributed else None, self._exposure())
+
+    def _exposure(self):
+        """(expo_time, expo_points) in time order, or None"""
+        return None if self.expo_time is None else (self.expo_time, self.expo_points)
 
     def _in_bounds(self, samples: np.ndarray) -> np.ndarray:
         """Indices of the samples inside [lower, upper]."""
@@ -257,6 +286,8 @@ class DeviceLikelihood(BatchedLikelihood):
         import torch
 
         super().__init__(engine, *args, **kwargs)
+        if self.expo_time is not None:
+            raise NotImplementedError("DeviceLikelihood: expo_time is not supported (use BatchedLikelihood)")
         self.device = torch.device("cuda", engine.device) if device is None else torch.device(device)
 
         def dev(a):
@@ -331,7 +362,9 @@ class LikelihoodStack:
     Each likelihood keeps its own template, names, point data, bounds, prior, ``log_likelihood_fn`` and optional fitted
     ``A_V``; fit k's walkers are evaluated on fit k's data set.  Bounds, rejected parameter sets and non-finite chi2 give
     -inf as in ``BatchedLikelihood.__call__``.  When only some fits sample ``A_V``, the others run with ext_k = 0 and
-    A_V = 0, and lnF_obs + 0 * 0 is lnF_obs exactly.  The engine is the first likelihood's.
+    A_V = 0, and lnF_obs + 0 * 0 is lnF_obs exactly.  Fits with ``expo_time`` keep their own exposures and
+    ``expo_points``, and the others get zero exposures: the stack then makes one ``chi2_multi_bands(exposures=...)`` call
+    instead.  The engine is the first likelihood's.
     Not supported (``NotImplementedError``): band-integrated data (stack such fits with ``BandLikelihoodStack``),
     ``distributed=True`` and ``DeviceLikelihood``."""
 
@@ -351,6 +384,9 @@ class LikelihoodStack:
         self.engine = self.likelihoods[0].engine
         self.datasets = [(lk.t, lk.nu, lk.lnF, lk.sig, lk.w) if lk.t.size else None for lk in self.likelihoods]
         self.fits_av = ["A_V" in lk.names and lk.t.size > 0 for lk in self.likelihoods]
+        self.exposures = [lk._exposure() for lk in self.likelihoods]
+        if all(e is None for e in self.exposures):
+            self.exposures = None
 
     def _walkers(self, samples):
         """The valid walkers of every fit as one batch: (records, fit of each, A_V of each (0 where the fit has none),
@@ -390,8 +426,12 @@ class LikelihoodStack:
         return self._split(self._engine_chi2(P, ds, extinction) if P.size else np.zeros(0), ok)
 
     def _engine_chi2(self, P, dataset_of, extinction):
-        """chi2 of the stacked walkers in one engine call: ``chi2_multi`` here, ``chi2_multi_bands`` with bands."""
-        return self.engine.chi2_multi(P, self.datasets, dataset_of, extinction=extinction)
+        """chi2 of the stacked walkers in one engine call: ``chi2_multi`` here, ``chi2_multi_bands`` with bands or
+        exposures."""
+        if self.exposures is None:
+            return self.engine.chi2_multi(P, self.datasets, dataset_of, extinction=extinction)
+        return self.engine.chi2_multi_bands(P, self.datasets, [[] for _ in self.datasets], dataset_of, extinction=extinction,
+                                            exposures=self.exposures)
 
     def flux_quantiles(self, samples, grids, q=(0.16, 0.5, 0.84)):
         """Posterior-predictive bands of the K fits in ONE ``Engine.flux_quantiles_multi`` call: fit k's draws
@@ -429,7 +469,8 @@ class BandLikelihoodStack(LikelihoodStack):
         self.bands = [lk.bands for lk in self.likelihoods]
 
     def _engine_chi2(self, P, dataset_of, extinction):
-        return self.engine.chi2_multi_bands(P, self.datasets, self.bands, dataset_of, extinction=extinction)
+        expo = {} if self.exposures is None else {"exposures": self.exposures}
+        return self.engine.chi2_multi_bands(P, self.datasets, self.bands, dataset_of, extinction=extinction, **expo)
 
 
 class DeviceLikelihoodStack(LikelihoodStack):

@@ -242,8 +242,8 @@ class Model {
         return pack(out, {(py::ssize_t)n_t});
     }
 
-    // PyModel::flux_density_exposures (pybind/pymodel.cpp:412-496): host-side sampling of each
-    // exposure window, one series evaluation on the GPU, host-side averaging.
+    // PyModel::flux_density_exposures (pybind/pymodel.cpp:412-496): sampling, evaluation and averaging on the GPU
+    // (vag_flux_density_exposures checks the rest with the reference's messages)
     FluxDict flux_density_exposures(py::array_t<double, py::array::c_style | py::array::forcecast> t,
                                     py::array_t<double, py::array::c_style | py::array::forcecast> nu,
                                     py::array_t<double, py::array::c_style | py::array::forcecast> expo_time,
@@ -251,39 +251,13 @@ class Model {
         const size_t n = t.size();
         require(n == (size_t)nu.size() && n == (size_t)expo_time.size(),
                 "time, frequency, and exposure time arrays must have the same size");
-        require(num_points >= 2, "num_points must be at least 2 to sample within each exposure time");
-        for (size_t i = 0; i < n; ++i)
-            require(std::isfinite(expo_time.data()[i]) && expo_time.data()[i] > 0,
-                    "expo_time[" + std::to_string(i) + "] must be finite and > 0, got " + std::to_string(expo_time.data()[i]));
-        const size_t total = n * num_points;
-        std::vector<double> ts(total), nus(total);
-        std::vector<size_t> idx(total), order(total);
-        for (size_t i = 0, j = 0; i < n; ++i) {
-            const double dt = expo_time.data()[i] / static_cast<double>(num_points - 1);
-            for (size_t k = 0; k < num_points; ++k, ++j) {
-                ts[j] = t.data()[i] + k * dt;
-                nus[j] = nu.data()[i];
-                idx[j] = i;
-                order[j] = j;
-            }
-        }
-        std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return ts[a] < ts[b]; });
-        std::vector<double> ts_s(total), nus_s(total);
-        for (size_t j = 0; j < total; ++j) {
-            ts_s[j] = ts[order[j]];
-            nus_s[j] = nus[order[j]];
-        }
-        std::vector<double> raw(VAG_NCOMP * total);
+        std::vector<double> out(VAG_NCOMP * n);
         {
             py::gil_scoped_release rel;
             auto ctx = context(device_);
             std::lock_guard<std::mutex> lk(ctx->mu);
-            check(vag_flux_density_series(ctx->h, &p_, 1, ts_s.data(), nus_s.data(), total, raw.data(), nullptr));
-        }
-        std::vector<double> out(VAG_NCOMP * n, 0.0);
-        for (int c = 0; c < VAG_NCOMP; ++c) {
-            for (size_t j = 0; j < total; ++j) out[c * n + idx[order[j]]] += raw[c * total + j];
-            for (size_t i = 0; i < n; ++i) out[c * n + i] /= static_cast<double>(num_points);
+            check(vag_flux_density_exposures(ctx->h, &p_, 1, t.data(), nu.data(), expo_time.data(), n, num_points,
+                                             out.data(), nullptr));
         }
         return pack(out, {(py::ssize_t)n});
     }
